@@ -2,7 +2,7 @@
 """Headline benchmark: ESRGAN/RRDBNet generator inference throughput (HR-output Mpixel/s) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|cfg2_default|cfg1|cfg3|...]
-                    [--mode infer|train]
+                    [--mode infer|train] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): Hydra generator (nf=64, nb=11, gc=16, in_channels=4), batch 64 of 256x256 HR tiles
 (LR 64x64) per GPU, synthetic inputs, random-init weights.  One "step" = one generator forward over the batch.
@@ -20,7 +20,10 @@ Workload (BASELINE.json configs[1]): Hydra generator (nf=64, nb=11, gc=16, in_ch
   gpu_eager_baseline (N = 1): the reference graph in stock PyTorch eager + cuDNN (bf16 autocast, channels_last,
            cudnn.benchmark) on the same GPU - "the kernel to beat" of BASELINE.md section 4
 N > 1 (torchrun): independent tile batches per rank, no data-path collective -> "weak" scaling.
---impl reference: times the reference's CPU implementation (oracle port; /root/reference does not exist on the GPU box).
+--impl reference: times the reference's CPU implementation (the oracle port, oracle/generator.py).
+--dump-outputs DIR: after the timed steps, the arrays the last timed step computed (inference: the generator output "sr";
+           train: "sr", "loss" and the flat parameter gradients "grads") go to DIR/<name>.npy as float32, rank 0 only.  Inputs
+           and weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -200,6 +203,26 @@ def recorded_dram_traffic():
     return None, "no ncu DRAM pass recorded for this build"
 
 
+DUMP_BYTES = 60_000_000      # below 64 MB however the MB is counted
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: writes every tensor of `arrays` (name -> tensor) as <path>/<name>.npy in float32.  If they would take more
+    than DUMP_BYTES together, each is cut to the same fraction of its elements: a seeded sample of the flattened tensor that
+    depends only on the sizes, so runs with the same arguments store the same elements."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    total = 4 * sum(t.numel() for t in arrays.values())
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if total > DUMP_BYTES:
+            keep = a.numel() * DUMP_BYTES // total
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, name + ".npy"), a.numpy())
+
+
 
 def run_ours(args):
     import torch
@@ -257,6 +280,8 @@ def run_ours(args):
             barrier()
             ms_total = e0.elapsed_time(e1)
         launches = kernel_launch_count() - l0
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"sr": out})
         ms_step = max_over_ranks(ms_total / args.steps)
         # ---------------- end-to-end timing (host pinned -> device -> host) through the public pipeline API:
         # every step copies its x/elev/mask from pinned host memory and its result back; copies of neighbouring steps
@@ -330,7 +355,7 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
-def train_measure(workload, steps, warmup, dev, world, rank, overlap=True, e2e=True):
+def train_measure(workload, steps, warmup, dev, world, rank, overlap=True, e2e=True, dump=None):
     """Generator training step (SURVEY.md section 8d cfg3, generator part): forward on a training plan, L1 pixel loss
     (core/task.py:141), backward (dgrad + wgrad kernels), gradient all-reduce when N > 1 - by default the bf16 exchange
     overlapped with the segmented backward (climsr_b200.parallel.attach_ddp) -, fused AdamW step (conf/optimizers/adamw.yaml:
@@ -358,14 +383,17 @@ def train_measure(workload, steps, warmup, dev, world, rank, overlap=True, e2e=T
     xd, ed, md, hd = (t.to(dev) for t in (x, elev, mask, hr))
     loss_host = torch.empty((), dtype=torch.float32).pin_memory()
     mode = {"sync": world > 1}
+    last_sr = [None]
 
     def step():
         opt.zero_grad(set_to_none=True)
-        lv = losses.l1_loss(net(xd, ed, md), hd)
+        sr = net(xd, ed, md)
+        lv = losses.l1_loss(sr, hd)
         lv.backward()
         if mode["sync"] and sync is None:
             bucketer.allreduce()
         opt.step()
+        last_sr[0] = sr
         return lv
 
     def barrier():
@@ -402,6 +430,8 @@ def train_measure(workload, steps, warmup, dev, world, rank, overlap=True, e2e=T
     # (a host-side hiccup - the step is launch-bound at this size), which says nothing about the path
     ms_again, lv = timed(steps)
     ms_step = min(ms_step, ms_again)
+    if dump and rank == 0:
+        dump_outputs(dump, {"sr": last_sr[0], "loss": lv, "grads": torch.cat([p.grad.reshape(-1) for p in net.parameters()])})
     last_loss = float(lv.detach())
     out = {"ms_per_step": ms_step, "mpixel_per_s": world * tiles * H * W / (ms_step * 1e-3) / 1e6, "loss_first": first_loss,
            "loss_last": last_loss, "gpu_launches": int(launches), "clocks": clk.summary(),
@@ -472,7 +502,7 @@ def run_train(args):
     dev = torch.device("cuda", local)
     in_ch, nb, gc, tiles, h, w = WORKLOADS[args.workload]
     H, W = 4 * h, 4 * w
-    m = train_measure(args.workload, args.steps, args.warmup, dev, world, rank, overlap=not args.no_overlap)
+    m = train_measure(args.workload, args.steps, args.warmup, dev, world, rank, overlap=not args.no_overlap, dump=args.dump_outputs)
     peaks = load_peaks()
     line = {
         "metric": "generator_train_hr_mpixel_per_s", "value": m["mpixel_per_s"], "unit": "Mpixel/s",
@@ -604,10 +634,17 @@ def gpu_eager_measure(workload, dev, steps=5):
                     "autocast(bf16), channels_last, cudnn.benchmark=True", "workload": workload}
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"expected a count >= 1, got {s}")
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=positive_int, default=20, help="timed steps of the headline measurement")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="cfg2", choices=sorted(WORKLOADS))
@@ -617,7 +654,11 @@ def main():
                     help="train: bucketed all-reduce AFTER backward (GradientBucketer) instead of the default exchange overlapped with the "
                          "segmented backward (attach_ddp)")
     ap.add_argument("--no-extras", action="store_true", help="inference line only: skip the train / halo_tiled / gpu_eager_baseline measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the arrays the last timed step computed to DIR/<name>.npy (float32, "
+                                                          "at most 64 MB in all)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl != "reference" and os.environ.get("CSR_OPTS"):
         # tuning hook: CSR_OPTS="18=0,19=0" applies csr_set_option(key, value) pairs before anything is built
         sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "climate-super-resolution_b200"))
