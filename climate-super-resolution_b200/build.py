@@ -2,8 +2,7 @@
 
 Every translation unit is compiled to an object file in parallel (build/ is git-ignored), then linked into
 climsr_b200/libclimsr_b200.so.  ``python build.py --force`` rebuilds everything, ``-v`` adds ptxas resource usage,
-``CSR_BUILD_TRACE=1`` compiles the per-role clock stamps of tools/trace_conv.py in, ``CSR_EXPERIMENTS=1`` the measured-and-
-rejected kernel variants (CTA pairs, unstaged stores, dense-block regrouping; see DESIGN.md section 3.1).
+``CSR_BUILD_TRACE=1`` compiles the per-role clock stamps of tools/trace_conv.py in.
 """
 from __future__ import annotations
 
@@ -26,8 +25,6 @@ def _defines():
     d = []
     if os.environ.get("CSR_BUILD_TRACE") == "1":
         d.append("-DCSR_ENABLE_TRACE")          # per-role clock stamps (tools/trace_conv.py)
-    if os.environ.get("CSR_EXPERIMENTS") == "1":
-        d.append("-DCSR_EXPERIMENTS")
     return d
 
 

@@ -37,41 +37,23 @@ static int g_opt_force_generic = 0;
 static int g_opt_one_mma = 0;
 static int g_opt_graphs = 1;
 static int g_opt_graph_max_px = 1 << 21;   // forward: replay a CUDA graph up to this many HR pixels per call (larger batches are GPU-bound)
-static int g_opt_issue_order = 1;       // MMA warps take strict turns tile by tile: 0 never, 1 in CTA-pair launches, 2 in every launch
 static int g_opt_wgrad_atomic = 1;      // weight-gradient partial sums through red.global.add.v4.f32 instead of per-CTA slices + reduce kernel
 static int g_opt_eight_acc = 1;         // eight accumulator buffers for two-tile windows when TMEM has room (KW*npad <= 64)
 static int g_opt_tall = 1;              // two M tiles per window for thin layers
 static int g_opt_narrow_box = 1;        // 16- / 32-channel window boxes for layers over <= 16 / 32 input channels
-static int g_opt_regroup = 0;           // dense blocks regrouped by source in the forward (see fwd_exec_table): -3 % alone, but the plain
-                                        // layout gains more from two-tile windows (5.76 vs 5.85 ms), so it is off by default
 static int g_opt_trace_cta = 0;         // debug: CTA recorded by csr_debug_set_trace
 static int g_opt_reserve_sms = 0;       // plans created afterwards size their persistent grids to (SM count - this): the SMs left free run the
                                         // gradient all-reduce (NCCL, capped to as many CTAs) concurrently with the backward kernels
-static int g_opt_l2_prefetch = 0;       // conv layers that stream from HBM: prefetch windows this many tile iterations ahead into L2 (cp.async.bulk.prefetch.tensor).
-                                        // Measured: no effect at depth 2/4/8 (HRconv 317-323 us either way) - the HR tail is not bound by HBM latency
-static int g_dbg_dense = 0;             // DenseParams::dbg (timing experiments)
 static int g_opt_dense_min = 2;         // ... only when a block has at least this many windows per SM: with <= 1 window per CTA nothing pipelines
                                         // across layers and the counters only cost (cfg1 / one Europe raster / cfg3: 7-10 % slower, r02 A/B)
 static int g_opt_tap_pack = 1;          // conv_last's tap sum fused with the SRCNN input im2col (tap_pack_kernel)
-static int g_opt_hyb = 1;               // hybrid tap fold (conv_tc.cu HYB_T): bit 0 early-release layers (HRconv 338 -> 294 us); experiments build only:
-                                        // bit 1 conv5 / trunk_conv, bit 2 four accumulators there (measured slower: those are not epilogue-bound)
+static int g_opt_hyb = 1;               // hybrid tap fold (conv_tc.cu HYB_T) on the early-release layers (HRconv 338 -> 294 us)
 static int g_opt_merge_phases = 1;      // sub-pixel phase pairs of nearest-x2 + conv as one launch (gridDim.y)
 static int g_opt_fuse_tail = 3;         // inference, second MMA over the staged tile: bit 0 srcnn.conv2 inside srcnn.conv1's epilogue, bit 1 conv_last's
                                         // nine tap planes inside HRconv's epilogue (+ tap_sum_kernel)
-[[maybe_unused]] static int g_opt_dense9 = 0;            // dense blocks with all nine taps folded into N = 144 (rdb9_tc.cu) instead of N = 48 (rdb_tc.cu)
 static int g_opt_dense = 1;             // conv1..conv4 of every gc = 16 dense block as ONE persistent launch with tile-level dependencies (rdb_tc.cu)
-static int g_opt_early = 1;             // early-release epilogue (conv_tc.cu, EARLY_T): 1 = wide residual-free layers; 2 = also the residual layers (RDB conv5 with one
-                                        // staging buffer and a third window slot, trunk_conv): measured slower in situ (42.0 / 55.5 vs 39.6 / 51.7 us per conv5)
-static int g_opt_pair = 0;              // CTA-pair (cta_group::2) launches for 3x3 layers with >= 96 KB of weights.  Measured (cfg2): MMAs run at the
-                                        // 108 clk/MMA pair rate instead of ~140, but two SMs in lock-step on two accumulators expose the epilogue:
-                                        // 6.11 vs 5.90 ms per step, so it stays off by default
-static int g_opt_no_single_group = 3;   // epilogue groups of two-accumulator layers: 1 = always two groups of 8 warps (one tile each); 0 = one group of
-                                        // 16 warps when that deepens the window ring (RDB conv5: measured slower, the single group paces the tile);
-                                        // 2 = one group everywhere; 3 (default) = one group for layers with < 96 KB of weights and no residual /
-                                        // gate operand (HRconv, upconv, conv_first, srcnn.conv1: epilogue-bound, 16 warps on one tile shorten its
-                                        // latency chain: -2 % per inference step; the gated input-gradient convs of the backward lose with it)
+static int g_opt_early = 1;             // early-release epilogue (conv_tc.cu, EARLY_T) for the wide residual-free layers
 static int g_dbg_wgrad[5] = {0, 0, 0, 0, 0};   // a_lbo, a_sbo, b_lbo, b_sbo, flags overrides of the MN-major descriptors
-static int g_opt_no_direct32 = 1;   // measured: no gain over staging on cfg2 (tools/ab_bench.py), kept as an option
 
 static int fail(int code, const char* fmt, ...) {
   va_list ap;
@@ -163,12 +145,8 @@ struct LayerSpec {
   float wscale = 1.f;      // constant folded into the packed weights
   int src = -1;            // backward tables: index of the forward layer whose weight tensor is packed
   struct Block { int src, ci_lo, n, src_ci_off, src_cin; float wscale; };
-  // backward tables (transposed): executed input-channel blocks gathered from several forward layers;
-  // forward execution table: executed OUTPUT-channel blocks [ci_lo, ci_lo+n) = filters of layer `src` over its input
-  // channels [src_ci_off, src_ci_off + cin)
+  // backward tables (transposed): executed input-channel blocks gathered from several forward layers
   std::vector<Block> blocks;
-  int block_bias = 0;      // forward blocks: 1 = the bias segments come from the source layers, 0 = zero bias
-  int act_upto = 0;        // forward blocks: > 0 = the layer's LeakyReLU applies to output channels < act_upto only
   int ekw() const { return fold ? 1 : kw; }
   int ecin() const { return fold ? cin * kw : cin; }
 };
@@ -205,42 +183,18 @@ static std::vector<LayerSpec> layer_table(const CsrNetDesc& d) {
   return v;
 }
 
-// Forward EXECUTION table.  Same length and order as the state_dict table, but each dense block (esrgan.py:32-38) is
-// regrouped by source: since x_k = lrelu(W_k * [x, x1..x_{k-1}]) and the first 64 input channels of every conv_k are the
-// block input x, ONE launch computes conv1 and the x-parts of conv2..conv4 side by side (64 -> 4*gc channels, UMMA
-// N = 3*64 instead of 3*16 for the same A-tile reads) and writes [x1 | p2 | p3 | p4] into the concat slots of x1..x4;
-// conv_k (k = 2..4) then only runs over x1..x_{k-1} ((k-1)*gc input channels) and adds p_k - read from the very slot it
-// overwrites - before its LeakyReLU.  66 narrow MMAs per tile become 12 wide + 18 narrow ones and conv2..4 read one
-// 64-channel box instead of two.  p_k passes through bf16 once (the concat buffer's type).
-static int fwd_index_rdb(int i, int r, int k);
+// Forward EXECUTION table: the state_dict table plus a view of conv_last's weights.
 static std::vector<LayerSpec> fwd_exec_table(const CsrNetDesc& d, const std::vector<LayerSpec>& f) {
   std::vector<LayerSpec> v = f;
   for (size_t i = 0; i < v.size(); ++i) v[i].src = (int)i;
-  {
-    // conv_last (64 -> 1, 3x3) seen as a 1x1 layer with nine "output channels" = its nine taps: tap[t](y, x) = sum_c W[0][c][t] * in(y, x)[c].
-    // Inference runs it as a second MMA inside HRconv's epilogue (conv_tc.cu FUSE_T = 2) and sums the shifted taps afterwards
-    // (tap_sum_kernel), so HRconv's 64-channel HR map never reaches memory.  W[0][c][ky][kx] flattened is [c][t]: the transposed read
-    // of a (cout = 9, cin = 64, 1 x 1) layer.  Always the LAST entry, so state_dict indices keep their meaning.
-    LayerSpec T{"conv_last.taps", 9, d.nf, 1, 1};
-    T.transposed = 1;
-    T.src = (int)f.size() - 4;                             // conv_last
-    v.push_back(T);
-  }
-  if (!g_opt_regroup) return v;
-  for (int i = 0; i < d.nb; ++i)
-    for (int r = 0; r < 3; ++r) {
-      LayerSpec& X = v[fwd_index_rdb(i, r, 1)];
-      X.name += "+x_parts";
-      X.cout = 4 * d.gc; X.cin = d.nf; X.block_bias = 1; X.act_upto = d.gc;
-      for (int k = 1; k <= 4; ++k)
-        X.blocks.push_back({fwd_index_rdb(i, r, k), (k - 1) * d.gc, d.gc, 0, d.nf + (k - 1) * d.gc, 1.f});
-      for (int k = 2; k <= 4; ++k) {
-        LayerSpec& Lk = v[fwd_index_rdb(i, r, k)];
-        Lk.name += ".dense_part";
-        Lk.cin = (k - 1) * d.gc;
-        Lk.blocks.push_back({fwd_index_rdb(i, r, k), 0, d.gc, d.nf, d.nf + (k - 1) * d.gc, 1.f});
-      }
-    }
+  // conv_last (64 -> 1, 3x3) seen as a 1x1 layer with nine "output channels" = its nine taps: tap[t](y, x) = sum_c W[0][c][t] * in(y, x)[c].
+  // Inference runs it as a second MMA inside HRconv's epilogue (conv_tc.cu FUSE_T = 2) and sums the shifted taps afterwards
+  // (tap_sum_kernel), so HRconv's 64-channel HR map never reaches memory.  W[0][c][ky][kx] flattened is [c][t]: the transposed read
+  // of a (cout = 9, cin = 64, 1 x 1) layer.  Always the LAST entry, so state_dict indices keep their meaning.
+  LayerSpec T{"conv_last.taps", 9, d.nf, 1, 1};
+  T.transposed = 1;
+  T.src = (int)f.size() - 4;                               // conv_last
+  v.push_back(T);
   return v;
 }
 
@@ -364,8 +318,6 @@ struct ConvIO {
   void* out = nullptr; int out_C = 0, out_coff = 0; int out_kind = kOutBf16;
   int act = CSR_ACT_NONE;
   const void* r1 = nullptr; int r1_C = 0, r1_coff = 0; float s1 = 1.f;
-  int r1_pre = 0;          // r1 is added before the activation
-  int act_upto = 0;        // > 0: LeakyReLU on output channels < act_upto only (of the whole layer, before the cout split)
   const void* r2 = nullptr; int r2_C = 0, r2_coff = 0; float s2 = 1.f;
   const void* gate = nullptr; int gate_C = 0, gate_coff = 0, gate_from = 0; float gate_neg = 0.2f;
 };
@@ -393,26 +345,12 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
   p.n_groups = p.n_acc;
   Tiling tl;
   int rc = CSR_OK;
-  // CTA pair (tcgen05 cta_group::2) for 3x3 layers with >= 96 KB of weights (RDB conv5 and the matching input-gradient
-  // convs): each CTA keeps half of the weights, so the window ring gets 5 slots instead of 2.  Needs an even tile count
-  // (the two CTAs of a pair always work on adjacent tiles) and one of the specialised epilogues.
-  const int res_bits = (io.r1 ? 1 : 0) | (io.r2 ? 2 : 0) | (io.gate ? 4 : 0);
-  if (g_opt_pair && !pp.stream && tma_out && p.KW == 3 && p.PW == 1 && (p.KW * p.npad) % 16 == 0 && p.w_bytes >= 96 * 1024 && io.act == CSR_ACT_NONE &&
-      (res_bits == 1 || res_bits == 3 || res_bits == 4 || res_bits == 5) && !g_opt_force_generic) {
-    Tiling tp;
-    const int pair_groups = g_opt_pair == 2 ? 1 : p.n_groups;   // 2: one 16-warp epilogue group per CTA (shorter accumulator hand-back)
-    if (choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes / 2, p.n_kblocks, p.stage_row_bytes, pair_groups, &tp) == CSR_OK &&
-        (((long long)ceil_div(W, tp.TW) * ceil_div(H, tp.TH) * N) & 1) == 0) {
-      tl = tp;
-      p.pair = 1;
-      p.n_groups = pair_groups;
-    }
-  }
+  const bool has_res = io.r1 || io.r2 || io.gate;
   // Layers over <= 32 input channels (the dense-block parts over x1 / x1,x2) only move those channels: 32- or 64-byte
   // window rows with the matching TMA / UMMA swizzle instead of a whole 64-channel box.  These launches are bound by
   // the bytes the SM can take in per clock, not by MMAs.
   p.box_c = 64;
-  if (g_opt_narrow_box && p.n_kblocks == 1 && !p.pair) p.box_c = p.cin <= 16 ? 16 : p.cin <= 32 ? 32 : 64;
+  if (g_opt_narrow_box && p.n_kblocks == 1) p.box_c = p.cin <= 16 ? 16 : p.cin <= 32 ? 32 : 64;
   // Thin layers (<= 32 output channels: four accumulator buffers) are bound by the per-tile work of the producer and
   // MMA-issuer warps (~110 / ~250 scalar instructions at ~5 clk each), not by MMAs or bytes: give them windows of two M
   // tiles, which halves that work per tile and shrinks the halo from 6/4 to 10/8 rows.
@@ -422,8 +360,8 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
     p.wkb_bytes = pp.kh * 4 * pp.kw * pp.npad * 32;
     rc = choose_tiling(H, W, pp.kh, pp.kw, 0, p.n_kblocks, p.stage_row_bytes, p.n_groups, &tl, 128, 1, p.wkb_bytes);
     if (!rc && tl.n_slots < 2) rc = fail(CSR_ERR_UNSUPPORTED, "streamed-weight conv: window ring too shallow");
-  } else if (!p.pair) rc = choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, p.n_groups, &tl, p.box_c * 2);
-  if (!rc && g_opt_tall && !p.pair && p.n_acc == 4 && p.n_groups == 4) {
+  } else rc = choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, p.n_groups, &tl, p.box_c * 2);
+  if (!rc && g_opt_tall && p.n_acc == 4 && p.n_groups == 4) {
     Tiling t2;   // taken unless the second M tile would mostly hang below the image
     if (choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, p.n_groups, &t2, p.box_c * 2, 2) == CSR_OK &&
         t2.eff >= 0.85 * tl.eff && t2.n_slots >= 2) {
@@ -435,52 +373,24 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
     }
   }
   if (rc) return rc;
-  if (!p.pair && tma_out && p.n_groups == 2 && (g_opt_no_single_group == 2 || (g_opt_no_single_group == 3 && p.w_bytes < 96 * 1024 && res_bits == 0))) {
-    // experiment: all 16 epilogue warps on one tile at a time (two chunks per warp) for every two-accumulator layer
+  if (tma_out && p.n_groups == 2 && p.w_bytes < 96 * 1024 && !has_res) {
+    // One epilogue group of 16 warps on one tile at a time (two chunks per warp) for the two-accumulator layers with < 96 KB of
+    // weights and no residual / gate operand (HRconv, upconv, conv_first, srcnn.conv1): they are epilogue-bound, and 16 warps on
+    // one tile shorten its latency chain (-2 % per inference step).  RDB conv5 and the gated input-gradient convs of the backward
+    // lose with it: there the single group paces the tile.
     Tiling t1;
     if (choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, 1, &t1, p.box_c * 2) == CSR_OK) {
       tl = t1;
       p.n_groups = 1;
     }
   }
-  if (!p.pair && tma_out && p.n_groups == 2 && tl.n_slots < 3 && !g_opt_no_single_group) {
-    // Weights leave little shared memory (RDB conv5: 144 KB): one epilogue group (16 warps, still two accumulator
-    // buffers) needs one staging buffer instead of two, which buys a third window slot - the MMAs of such a layer take
-    // far longer than its epilogue, and with two slots every tile waited ~2400 clk for its TMA load.
-    Tiling t1;
-    if (choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, 1, &t1, p.box_c * 2) == CSR_OK && t1.n_slots > tl.n_slots) {
-      tl = t1;
-      p.n_groups = 1;
-    }
-  }
-  if (!p.pair && tma_out && tl.n_slots < 2 * p.n_kblocks && pp.n_store % 16 == 0 && io.out_C % 16 == 0 && (io.out_coff + pp.co_lo) % 16 == 0 &&
-      !g_opt_no_direct32) {
-    // The resident weights leave too little shared memory for staging AND a window ring that prefetches across tiles
-    // (RDB conv5: 144 KB of weights): store whole 32-byte sectors straight from registers instead.
-    Tiling t2;
-    if (choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, 0, 0, &t2, p.box_c * 2) == CSR_OK && t2.n_slots >= 2 * p.n_kblocks) {
-      tl = t2;
-      p.store_mode = kStoreDirect32;
-      p.stage_row_bytes = 0;
-    }
-  }
-  // final activation code of this part (act_upto splits a LeakyReLU over the output-channel parts)
   p.act = io.act;
-  if (io.act_upto > 0 && io.act == CSR_ACT_LRELU02) {
-    const int upto = io.act_upto - pp.co_lo;               // in this part's channels
-    if (upto <= 0) p.act = CSR_ACT_NONE;
-    else if (upto < pp.n_store) { p.act = 3; p.act_upto = upto; }
-  }
   p.n_stage = p.n_groups;
   // Early-release epilogue (conv_tc.cu, EARLY_T): wide residual-free layers that run with one 16-warp group.  Two staging
   // buffers; KW <= 2 layers also get four accumulator buffers (4 x KW x 64 <= 512 TMEM columns).
-  const bool early_plain = res_bits == 0 && p.n_groups == 1 &&
-      ((p.KW == 3 && p.PW == 1 && (p.act == 0 || p.act == 1 || p.act == 3)) || (p.KW == 2 && p.PW <= 1 && p.act == 1) ||
-       (p.KW == 1 && p.PW == 0 && p.act == 2));
-  // ... and the residual layers (RDB conv5, trunk_conv): with the accumulator handed back early one 16-warp group no longer
-  // paces the tile, and a single staging buffer buys RDB conv5 (144 KB of weights) a third window slot
-  const bool early_res = g_opt_early >= 2 && (res_bits == 1 || res_bits == 3) && !io.r1_pre && p.KW == 3 && p.PW == 1 && p.act == 0 && p.n_groups <= 2;
-  if (g_opt_early && !p.pair && !p.tall_shift && tma_out && p.npad == 64 && pp.n_store == 64 && !g_opt_force_generic && (early_plain || early_res)) {
+  const bool early_plain = !has_res && p.n_groups == 1 &&
+      ((p.KW == 3 && p.PW == 1 && (p.act == 0 || p.act == 1)) || (p.KW == 2 && p.PW <= 1 && p.act == 1) || (p.KW == 1 && p.PW == 0 && p.act == 2));
+  if (g_opt_early && early_plain && !p.tall_shift && tma_out && p.npad == 64 && pp.n_store == 64 && !g_opt_force_generic) {
     Tiling te2, te1;
     const bool ok2 = choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, 2, &te2, p.box_c * 2) == CSR_OK;
     const bool ok1 = choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, 1, &te1, p.box_c * 2) == CSR_OK;
@@ -490,7 +400,7 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
     else if (ok1 && (!ok2 || te1.n_slots > te2.n_slots)) stages = 1;
     else if (ok2) stages = 2;
     const Tiling& te = stages == 1 ? te1 : te2;
-    if (stages && te.n_slots >= std::min(2, p.n_kblocks + 1) && (early_plain || te.n_slots > tl.n_slots || te.n_slots >= want)) {
+    if (stages && te.n_slots >= std::min(2, p.n_kblocks + 1)) {
       tl = te;
       p.early = 1;
       p.n_groups = 1;
@@ -498,24 +408,12 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
       if (4 * p.KW * p.npad <= 512 && !g_opt_two_acc) p.n_acc = 4;
     }
   }
-  // Hybrid tap fold (conv_tc.cu HYB_T) for the 64-channel 3x3 / 2x2 layers, which are epilogue-bound: the last horizontal tap is its own
-  // MMA on an A operand shifted by one pixel and accumulates into the previous tap's columns - a third (half) fewer accumulator
-  // columns to read and one shuffle-sum fewer, at 22 % more MMA time.  Bit 0: early-release layers, bit 1: RDB conv5 / trunk_conv,
-  // bit 2: four accumulators for the latter.
-  {
-    const bool hyb_early = (g_opt_hyb & 1) && p.early && ((p.KW == 3 && p.PW == 1) || (p.KW == 2 && p.PW <= 1));
-#ifdef CSR_EXPERIMENTS
-    const bool hyb_res = (g_opt_hyb & 2) && !p.early && p.KW == 3 && p.PW == 1 && p.act == 0 && (res_bits == 1 || res_bits == 3) && !io.r1_pre &&
-                         p.n_groups == 2;
-#else
-    const bool hyb_res = false;
-#endif
-    if ((hyb_early || hyb_res) && !p.pair && !p.tall_shift && p.store_mode == kStoreStaged && p.npad == 64 && pp.n_store == 64 && p.box_c == 64 &&
-        !p.stream_w && !g_opt_force_generic) {
-      p.hyb = 1;
-      const int acc_cols = (p.KW - 1) * p.npad;
-      if (4 * acc_cols <= 512 && !g_opt_two_acc && (p.early || (g_opt_hyb & 4))) p.n_acc = 4;
-    }
+  // Hybrid tap fold (conv_tc.cu HYB_T) for the early-release 64-channel 3x3 / 2x2 layers, which are epilogue-bound: the last horizontal
+  // tap is its own MMA on an A operand shifted by one pixel and accumulates into the previous tap's columns - a third (half) fewer
+  // accumulator columns to read and one shuffle-sum fewer, at 22 % more MMA time.
+  if (g_opt_hyb && p.early && ((p.KW == 3 && p.PW == 1) || (p.KW == 2 && p.PW <= 1)) && p.box_c == 64 && !p.stream_w) {
+    p.hyb = 1;
+    if (4 * (p.KW - 1) * p.npad <= 512 && !g_opt_two_acc) p.n_acc = 4;
   }
   p.SW = tl.SW; p.TH = tl.TH; p.TW = tl.TW;
   p.sw_shift = 0;
@@ -532,7 +430,6 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
   p.win_slot_bytes = (int)align_up(tl.win_bytes, 1024);
   p.stage_bytes = tl.stage_bytes;
   p.n_mma = g_opt_one_mma ? 1 : 2;
-  p.issue_order = (p.n_mma == 2) && (g_opt_issue_order == 2 || (g_opt_issue_order == 1 && p.pair));
   int cols = 32;
   while (cols < p.n_acc * (p.hyb ? p.KW - 1 : p.KW) * p.npad) cols *= 2;
   if (cols > 512 || p.KW * p.npad > 256) return fail(CSR_ERR_UNSUPPORTED, "KW*npad = %d exceeds the UMMA N / TMEM budget", p.KW * p.npad);
@@ -540,9 +437,7 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
   p.trace = g_trace;
   p.trace_cta = g_opt_trace_cta;
   p.use_pdl = g_opt_pdl;
-  p.l2_prefetch = ((size_t)N * H * W * io.in_C * 2 > (size_t)48 << 20) ? g_opt_l2_prefetch : 0;   // only layers that stream from HBM
   p.force_generic = g_opt_force_generic;
-  p.r1_pre = io.r1 ? io.r1_pre : 0;
   p.s1 = io.s1; p.s2 = io.s2;
   p.r1 = io.r1; p.r1_C = io.r1_C; p.r1_coff = io.r1_coff + pp.co_lo;
   p.r2 = io.r2; p.r2_C = io.r2_C; p.r2_coff = io.r2_coff + pp.co_lo;
@@ -889,7 +784,7 @@ static int build_dense(const std::vector<PackLayer>& packs, int li, int N, int H
   DenseParams& p = dl->p;
   memset(&p, 0, sizeof(p));
   if (gc != 16 || C % 8) return fail(CSR_ERR_UNSUPPORTED, "dense-block kernel: gc must be 16");
-  p.N = N; p.H = H; p.W = W; p.n_layers = 4; p.C = C; p.buf = buf; p.flags = flags; p.use_pdl = g_opt_pdl; p.dbg = g_dbg_dense;
+  p.N = N; p.H = H; p.W = W; p.n_layers = 4; p.C = C; p.buf = buf; p.flags = flags; p.use_pdl = g_opt_pdl;
   // forward: x_{k+1} = lrelu(conv_{k+1}(...)).  backward (gate given): layer k = the gated gradient of x_{4-k}, gate = x_{4-k} of the
   // forward concat buffer (channels nf + (3-k) gc ...), no activation
   p.act = gate ? 0 : 1; p.gate = gate; p.gate_C = gate_C; p.gate_neg = 0.2f;
@@ -907,24 +802,6 @@ static int build_dense(const std::vector<PackLayer>& packs, int li, int N, int H
     wmax = std::max(wmax, pl.parts[0].w_bytes);
   }
   p.wbuf_bytes = (int)align_up(wmax, 1024);
-#ifdef CSR_EXPERIMENTS
-  if (g_opt_dense9) {
-    // all nine taps folded into N = 144 (rdb9_tc.cu): windows of 16 x 16 input pixels, 14 x 14 outputs
-    p.fold9 = 1;
-    p.SW = 16; p.sw_shift = 4; p.TH = 8; p.TW = 14;
-    p.tiles_x = ceil_div(W, 14); p.tiles_y = ceil_div(H, 14);
-    p.tiles_per_img = p.tiles_x * p.tiles_y;
-    p.num_tiles = p.tiles_per_img * N;
-    if ((long long)p.tiles_per_img * N >= (1 << 24) || p.tiles_per_img >= (1 << 16)) return fail(CSR_ERR_UNSUPPORTED, "dense-block kernel: too many windows");
-    p.magic_img = ((1ull << 40) / (unsigned)p.tiles_per_img) + 1;
-    p.magic_row = ((1ull << 40) / (unsigned)p.tiles_x) + 1;
-    p.win_bytes = 16 * 16 * 128; p.slot_bytes = p.win_bytes;
-    p.n_slots = 8;
-    while (p.n_slots > 2 && dense9_smem_bytes(p) > (size_t)kSmemLimit) --p.n_slots;
-    if (dense9_smem_bytes(p) > (size_t)kSmemLimit || p.n_slots < 3) return fail(CSR_ERR_UNSUPPORTED, "dense-block kernel (N=144): window ring too shallow");
-    return encode_act_map(&dl->tmap, buf, N, H, W, C, 16, 16, 64);
-  }
-#endif
   Tiling tl;
   int rc = choose_tiling(H, W, 3, 3, 2 * p.wbuf_bytes, 2, 32, 4, &tl, 128, 2);
   if (rc) return rc;
@@ -1039,7 +916,7 @@ static int plan_build(CsrPlan* P, void* ws) {
       const int j = 3 * i + r;
       void* src = cat(j);
       void* dst = P->train ? cat(j + 1) : (r < 2 ? cat(j + 1) : cat(3 * i));
-      if (g_opt_dense && !g_opt_regroup && gc == 16 && !g_opt_force_generic) {
+      if (g_opt_dense && gc == 16 && !g_opt_force_generic) {
         // conv1..conv4 as ONE persistent launch with tile-level dependencies between the layers (rdb_tc.cu)
         DenseLaunch dl;
         const size_t per_block = (size_t)kDenseMaxLayers * N * ceil_div(h, 8) * ceil_div(w, 14);
@@ -1057,16 +934,7 @@ static int plan_build(CsrPlan* P, void* ws) {
       }
       for (int k = 1; k <= 4; ++k) {
         // x_k = lrelu(conv_k(cat(x, x1..x_{k-1})))  written into its concat slice  (esrgan.py:33-36)
-        ConvIO io = io_of(src, C, src, C, nf + (k - 1) * gc, CSR_ACT_LRELU02);
-        if (g_opt_regroup) {
-          if (k == 1) {
-            io.act_upto = gc;                                // [x1 | p2 | p3 | p4] -> channels [nf, nf + 4 gc)
-          } else {
-            io.cin_off = nf;                                 // reads x1..x_{k-1} only ...
-            io.r1 = src; io.r1_C = C; io.r1_coff = nf + (k - 1) * gc; io.r1_pre = 1;   // ... and adds p_k from its own slot
-          }
-        }
-        rc = add(h, w, io);
+        rc = add(h, w, io_of(src, C, src, C, nf + (k - 1) * gc, CSR_ACT_LRELU02));
         if (rc) return rc;
       }
     conv5:
@@ -1534,12 +1402,8 @@ int csr_device_check(void) {
 }
 
 int csr_set_option(int32_t key, int32_t value) {
-  // the table with defaults and meanings is in INTEGRATION.md section 6
-#ifndef CSR_EXPERIMENTS
-  // measured-and-rejected kernel variants are not part of the default build (conv_tc.cu launch_conv_tc)
-  if ((key == 13 && value != 0) || (key == 16 && value != 0) || (key == 8 && value == 0) || (key == 32 && value != 0) || (key == 35 && (value & ~1)))
-    return fail(CSR_ERR_UNSUPPORTED, "option %d=%d selects an experimental kernel variant: rebuild with CSR_EXPERIMENTS=1 python build.py --force", key, value);
-#endif
+  // the table with defaults and meanings is in INTEGRATION.md section 6.  Keys 8, 9, 13, 14, 16, 28, 29 and 32 are retired (they
+  // selected removed kernel variants): do not reuse them, callers of older versions may still set them
   switch (key) {
     case 1: g_opt_pdl = value ? 1 : 0; return CSR_OK;              // programmatic dependent launch on/off
     case 2: g_opt_force_sw = value; return CSR_OK;                 // debug: force the window pitch
@@ -1548,14 +1412,9 @@ int csr_set_option(int32_t key, int32_t value) {
     case 5: g_opt_two_acc = value ? 1 : 0; return CSR_OK;          // debug: never more than two accumulator buffers
     case 6: g_opt_force_generic = value ? 1 : 0; return CSR_OK;    // debug: runtime-switched kernels only
     case 7: g_opt_one_mma = value ? 1 : 0; return CSR_OK;          // debug: a single MMA issuer warp
-    case 8: g_opt_no_direct32 = value ? 1 : 0; return CSR_OK;      // 0: allow unstaged 32-byte stores when staging starves the window ring
-    case 9: g_opt_no_single_group = value; return CSR_OK;          // epilogue groups of two-accumulator layers (see g_opt_no_single_group)
     case 11: g_opt_graphs = value ? 1 : 0; return CSR_OK;          // CUDA-graph replay of plan forward / backward_flat
     case 12: g_opt_graph_max_px = value; return CSR_OK;
-    case 13: g_opt_pair = value; return CSR_OK;                    // CTA-pair launches (default off; 2 = with one epilogue group per CTA: 5.53 vs 5.38 vs 5.15 ms without pairs)
-    case 14: g_opt_issue_order = value; return CSR_OK;
     case 15: g_opt_trace_cta = value; return CSR_OK;
-    case 16: g_opt_regroup = value ? 1 : 0; return CSR_OK;         // takes effect for weights packed / plans created afterwards
     case 17: g_opt_narrow_box = value ? 1 : 0; return CSR_OK;
     case 18: g_opt_tall = value ? 1 : 0; return CSR_OK;
     case 19: g_opt_eight_acc = value ? 1 : 0; return CSR_OK;
@@ -1563,28 +1422,23 @@ int csr_set_option(int32_t key, int32_t value) {
     case 25: g_opt_wgrad_atomic = value ? 1 : 0; return CSR_OK;    // plans created afterwards
     case 27: g_opt_dense = value ? 1 : 0; return CSR_OK;           // plans created afterwards
     case 36: g_opt_tap_pack = value ? 1 : 0; return CSR_OK;
-    case 35: g_opt_hyb = value; return CSR_OK;                    // plans created afterwards
+    case 35:                                                       // plans created afterwards
+      if (value != 0 && value != 1) return fail(CSR_ERR_BAD_ARG, "option 35: 0 or 1");
+      g_opt_hyb = value; return CSR_OK;
     case 34: g_opt_merge_phases = value ? 1 : 0; return CSR_OK;    // plans created afterwards
     case 33: g_opt_fuse_tail = value & 3; return CSR_OK;       // plans created afterwards
-    case 32: g_opt_dense9 = value ? 1 : 0; return CSR_OK;          // plans created afterwards
     case 31: if (value < 0 || value > 64) return fail(CSR_ERR_BAD_ARG, "option 31: windows per SM in [0, 64]"); g_opt_dense_min = value; return CSR_OK;
-    case 28: g_dbg_dense = value; return CSR_OK;
-    case 29: g_opt_l2_prefetch = value; return CSR_OK;
     case 30: g_opt_reserve_sms = value < 0 ? 0 : value; return CSR_OK;
-    case 26: g_opt_early = value; return CSR_OK;           // early-release epilogue of the wide residual-free layers
+    case 26:                                                       // early-release epilogue of the wide residual-free layers
+      if (value != 0 && value != 1) return fail(CSR_ERR_BAD_ARG, "option 26: 0 or 1");
+      g_opt_early = value; return CSR_OK;
     default: return fail(CSR_ERR_BAD_ARG, "unknown option key %d", key);
   }
 }
 
 int64_t csr_kernel_launch_count(void) { return g_launches.load(); }
 
-int csr_has_experiments(void) {
-#ifdef CSR_EXPERIMENTS
-  return 1;
-#else
-  return 0;
-#endif
-}
+int csr_has_experiments(void) { return 0; }   // kept for ABI version 2: the experimental kernel variants are gone
 
 int csr_debug_set_trace(void* device_buffer) {
 #ifdef CSR_ENABLE_TRACE
@@ -1669,17 +1523,9 @@ int csr_pack_weights(const CsrNetDesc* net, const float* const* w, const float* 
   for (size_t i = 0; i < layers.size(); ++i) {
     const LayerSpec& L = layers[i];
     if (i < n_real && (!w[i] || !b[i])) return fail(CSR_ERR_BAD_ARG, "null weight/bias pointer for layer %zu", i);
-    for (const PackPart& pp : packs[i].parts) {
-      float* bdst = reinterpret_cast<float*>(base + pp.b_off);
-      if (L.blocks.empty()) {
-        jobs.push_back({i < n_real ? w[i] : w[L.src], i < n_real ? b[i] : nullptr, base + pp.w_off, bdst, L.cout, L.cin, L.kh, L.kw, L.fold, pp.phase,
-                        L.transposed, L.wscale, pp.co_lo, pp.npad, packs[i].cin_pad, 0, 0, 0, 0});
-      } else {
-        for (const LayerSpec::Block& B : L.blocks)         // output-channel blocks gathered from several state_dict layers
-          jobs.push_back({w[B.src], L.block_bias ? b[B.src] : nullptr, base + pp.w_off, bdst, L.cout, L.cin, L.kh, L.kw, 0, pp.phase, 0,
-                          B.wscale, pp.co_lo, pp.npad, packs[i].cin_pad, B.ci_lo, B.n, B.src_ci_off, B.src_cin});
-      }
-    }
+    for (const PackPart& pp : packs[i].parts)
+      jobs.push_back({i < n_real ? w[i] : w[L.src], i < n_real ? b[i] : nullptr, base + pp.w_off, reinterpret_cast<float*>(base + pp.b_off), L.cout,
+                      L.cin, L.kh, L.kw, L.fold, pp.phase, L.transposed, L.wscale, pp.co_lo, pp.npad, packs[i].cin_pad, 0, 0, 0, 0});
   }
   return run_pack_jobs(jobs, packed, s);
 }

@@ -132,13 +132,9 @@ __device__ __forceinline__ uint4 ldg16(const void* base, size_t pix, int C, int 
 
 // Compile-time specialisation of the epilogue (it is instruction-issue bound, so every runtime switch costs):
 //   KW_T  horizontal taps (0 = runtime p.KW, taps gathered one at a time);  PW_T left padding when KW_T > 0
-//   ACT_T activation (-1 = runtime p.act; 3 = LeakyReLU on channels below p.act_upto only);  RES_T bit0 r1, bit1 r2,
-//         bit2 gate, bit3 r1 is added BEFORE the activation (-1 = runtime pointers / p.r1_pre)
-//   ST_T  1 = staged bf16 stores only, 2 = direct 32-byte bf16 stores only, 3 = fp32 planar single-channel output only
-//         (conv_last, srcnn.conv3: just channel 0 is computed), -1 = runtime p.store_mode
-//   PAIR_T 1 = CTA pair (cluster of 2, tcgen05 cta_group::2): the two CTAs take adjacent tiles, the leader issues one
-//          M = 256 MMA for both, and each CTA keeps only HALF of the layer's weights resident (B rows [0,N/2) / [N/2,N)),
-//          which is what buys RDB conv5 (144 KB of weights) a window ring deep enough to prefetch across tiles.
+//   ACT_T activation (-1 = runtime p.act);  RES_T bit0 r1, bit1 r2, bit2 gate (-1 = runtime pointers)
+//   ST_T  1 = staged bf16 stores only, 3 = fp32 planar single-channel output only (conv_last, srcnn.conv3: just channel 0
+//         is computed), -1 = runtime p.store_mode
 //   TALL_T 1 = two M tiles per window (ConvParams::tall_shift), compile-time so that the common kernels carry none of it
 //   HYB_T 1 = (3x3, early-release epilogue) only TWO of the three horizontal taps are folded into N: per (dy, k-step) one N = 2*npad MMA
 //            (taps dx = 0, 1) plus one N = npad MMA for tap dx = 2 whose A operand starts one pixel later and which accumulates into the
@@ -155,23 +151,23 @@ __device__ __forceinline__ uint4 ldg16(const void* base, size_t pix, int C, int 
 //          ~2450 clk per 128 x 64 tile against ~1400 clk of MMAs, because an accumulator stayed busy for the whole
 //          ~1000-clk arithmetic phase and only two of them fit TMEM; tools/tmem_probe.cu shows the TMEM read port itself
 //          delivers a 128 x 192 fp32 tile to 16 warps in ~260 clk.)
-template <int KW_T, int PW_T, int ACT_T, int RES_T, int ST_T, int PAIR_T = 0, int TALL_T = 0, int EARLY_T = 0, int FUSE_T = 0, int HYB_T = 0>
+template <int KW_T, int PW_T, int ACT_T, int RES_T, int ST_T, int TALL_T = 0, int EARLY_T = 0, int FUSE_T = 0, int HYB_T = 0>
 __global__ void __launch_bounds__(kConvThreads, 1)
 conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
+  static_assert(!HYB_T || EARLY_T, "hybrid tap fold: early-release epilogue only");
   extern __shared__ uint8_t smem_raw[];
   // 1024-byte alignment: the 128B-swizzle pattern repeats every 8 rows x 128 B.
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t slots_addr = smem_base;
   const uint32_t stage_addr = slots_addr + static_cast<uint32_t>(p.n_slots) * p.slot_bytes;   // one staging buffer per epilogue group
   const uint32_t w_addr = stage_addr + static_cast<uint32_t>(p.n_stage) * p.stage_bytes;
-  const uint32_t crank = PAIR_T ? cluster_ctarank() : 0u;   // rank in the CTA pair; rank 0 (leader) issues the MMAs
-  const int w_local = p.stream_w ? 0 : (PAIR_T ? (p.w_bytes >> 1) : p.w_bytes);  // resident weight bytes of this CTA
+  const int w_local = p.stream_w ? 0 : p.w_bytes;       // resident weight bytes
   // fused 1x1 successor (FUSE_T): its packed weights and bias sit right behind the layer's own weights
   const uint32_t w2_addr = w_addr + ((w_local + 127) & ~127);
   const uint32_t b2_addr = w2_addr + (FUSE_T ? static_cast<uint32_t>(p.w2_bytes) : 0u);
   const uint32_t bias_addr = b2_addr + (FUSE_T ? 128u : 0u);
   const uint32_t bar_addr = bias_addr + 256;            // up to 64 fp32 biases
-  // barriers: [0] weights, [1..S] a_full, [1+S..2S] a_empty, then acc_full[8], acc_empty[8], token[2]
+  // barriers: [0] weights, [1..S] a_full, [1+S..2S] a_empty, then acc_full[8], acc_empty[8], d2
   const int S = p.n_slots;
   const int NA = p.n_acc;                               // accumulator buffers in TMEM (2, 4 or 8)
   const int NG = p.n_groups;                            // epilogue warp groups (1, 2 or 4; NG <= NA): tiles in flight in the epilogue
@@ -181,12 +177,8 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
   auto bar_a_empty = [&](int s) { return bar_addr + 8u * (1 + S + s); };
   auto bar_acc_full = [&](int b) { return bar_addr + 8u * (1 + 2 * S + b); };
   auto bar_acc_empty = [&](int b) { return bar_addr + 8u * (9 + 2 * S + b); };
-  auto bar_token = [&](int w) { return bar_addr + 8u * (17 + 2 * S + w); };  // "MMA warp w has issued its tile" (issue_order)
-  const uint32_t bar_d2 = bar_addr + 8u * (19 + 2 * S);              // FUSE_T: the second MMA of a tile has completed
-  const uint32_t tmem_slot_addr = bar_addr + 8u * (20 + 2 * S);      // [0] TMEM base, [1..2] issuer progress words
-  // CTA pair: the barriers the LEADER waits on (weights, a_full, acc_empty) live in the leader's shared memory; the peer
-  // reaches them through the cluster window at the same offsets.
-  const uint32_t lead_off = PAIR_T ? (map_to_cta(bar_addr, 0) - bar_addr) : 0u;
+  const uint32_t bar_d2 = bar_addr + 8u * (17 + 2 * S);              // FUSE_T: the second MMA of a tile has completed
+  const uint32_t tmem_slot_addr = bar_addr + 8u * (18 + 2 * S);      // [0] TMEM base, [1..2] issuer progress words
   uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
   float* bias_s = reinterpret_cast<float*>(smem_gen + (bias_addr - smem_base));
   volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(smem_gen + (tmem_slot_addr - smem_base));
@@ -206,49 +198,33 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
   if (threadIdx.x == 0) {
     progress[0] = 0;
     progress[1] = 0;
-    mbar_init(bar_token(0), 1);
-    mbar_init(bar_token(1), 1);
     mbar_init(bar_d2, 1);
     tma_prefetch_desc(&tmap);
-    mbar_init(bar_w, (PAIR_T && crank == 0) ? 2 : 1);     // pair leader: + the peer's "my half has landed" arrival
+    mbar_init(bar_w, 1);
     for (int s = 0; s < S; ++s) {
       mbar_init(bar_a_full(s), 1);
       mbar_init(bar_a_empty(s), 1);
     }
     for (int b = 0; b < NA; ++b) {
       mbar_init(bar_acc_full(b), 1);
-      mbar_init(bar_acc_empty(b), PAIR_T ? 2 * wpg : wpg);   // pair: the epilogue warps of both CTAs release the leader's buffer
+      mbar_init(bar_acc_empty(b), wpg);
     }
     fence_mbar_init();
     fence_proxy_async_smem();
   }
-  if constexpr (PAIR_T) cluster_sync_all();               // both CTAs' barriers exist before anything arrives on them remotely
   if (threadIdx.x == 0 && !p.stream_w) {
     // layer weights (constant data, not produced by the previous kernel): resident for the whole CTA
     const uint8_t* wsrc = reinterpret_cast<const uint8_t*>(p.wpk) + static_cast<size_t>(blockIdx.y) * p.part_w_bytes;
-    if constexpr (PAIR_T) {
-      // every (k-block, dy, k-step) block of N rows x 16 K: this CTA keeps rows [crank*N/2, +N/2)
-      const int full = (KW_T ? KW_T : p.KW) * p.npad * 32, half = full >> 1;
-      mbar_arrive_expect_tx(bar_w, w_local);
-      for (int off = 0, loc = 0; off < p.w_bytes; off += full, loc += half)
-        bulk_load(w_addr + loc, wsrc + off + crank * half, half, bar_w);
-    } else {
-      mbar_arrive_expect_tx(bar_w, p.w_bytes + (FUSE_T ? p.w2_bytes : 0));
-      for (int off = 0; off < p.w_bytes; off += 32768) {
-        const int nbytes = min(32768, p.w_bytes - off);
-        bulk_load(w_addr + off, wsrc + off, nbytes, bar_w);
-      }
-      if constexpr (FUSE_T) bulk_load(w2_addr, p.w2, p.w2_bytes, bar_w);
+    mbar_arrive_expect_tx(bar_w, p.w_bytes + (FUSE_T ? p.w2_bytes : 0));
+    for (int off = 0; off < p.w_bytes; off += 32768) {
+      const int nbytes = min(32768, p.w_bytes - off);
+      bulk_load(w_addr + off, wsrc + off, nbytes, bar_w);
     }
+    if constexpr (FUSE_T) bulk_load(w2_addr, p.w2, p.w2_bytes, bar_w);
   }
   if (warp == 1) {
-    if constexpr (PAIR_T) {
-      tmem_alloc_pair(tmem_slot_addr, p.tmem_cols);
-      tmem_relinquish_pair();
-    } else {
-      tmem_alloc(tmem_slot_addr, p.tmem_cols);
-      tmem_relinquish();
-    }
+    tmem_alloc(tmem_slot_addr, p.tmem_cols);
+    tmem_relinquish();
   }
   for (int i = threadIdx.x; i < p.npad; i += blockDim.x) bias_s[i] = p.bias[blockIdx.y * p.part_b_floats + i];
   if constexpr (FUSE_T) {
@@ -274,14 +250,6 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
     uint32_t phase = 0;
     for (int t = blockIdx.x; t < p.num_tiles; t += gridDim.x, ++pit) {
       const Tile tl = decode_tile<TALL_T>(p, t);
-      if (p.l2_prefetch > 0) {
-        const int tp = t + p.l2_prefetch * static_cast<int>(gridDim.x);
-        if (tp < p.num_tiles && elect_one()) {
-          const Tile tq = decode_tile<TALL_T>(p, tp);
-          for (int kb = 0; kb < p.n_kblocks; ++kb) tma_prefetch_l2_4d(&tmap, p.cin_off + kb * 64, tq.x0 - p.PW, tq.y0 - ph_eff, tq.n);
-        }
-        __syncwarp();
-      }
       for (int kb = 0; kb < p.n_kblocks; ++kb) {
         if (kb == 0 && lane == 0) CSR_TRACE(0, pit, 0);
         mbar_wait_spin(bar_a_empty(slot), phase ^ 1);
@@ -296,14 +264,10 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
                                   static_cast<size_t>(kb) * p.wkb_bytes;
             const uint32_t wdst = slots_addr + slot * p.slot_bytes + p.win_slot_bytes;
             for (int off = 0; off < wbytes; off += 32768) bulk_load(wdst + off, wsrc + off, min(32768, wbytes - off), bar_a_full(slot));
-          } else
-          // pair: both CTAs' windows are counted on the leader's barrier, which the MMA issuer waits on
-          if (crank == 0) mbar_arrive_expect_tx(bar_a_full(slot), PAIR_T ? 2 * p.win_bytes : p.win_bytes);
-          if constexpr (PAIR_T)
-            tma_load_4d_pair(slots_addr + slot * p.slot_bytes, &tmap, bar_a_full(slot) + lead_off, p.cin_off + kb * 64, tl.x0 - p.PW,
-                             tl.y0 - ph_eff, tl.n);
-          else
-            tma_load_4d(slots_addr + slot * p.slot_bytes, &tmap, bar_a_full(slot), p.cin_off + kb * 64, tl.x0 - p.PW, tl.y0 - ph_eff, tl.n);
+          } else {
+            mbar_arrive_expect_tx(bar_a_full(slot), p.win_bytes);
+          }
+          tma_load_4d(slots_addr + slot * p.slot_bytes, &tmap, bar_a_full(slot), p.cin_off + kb * 64, tl.x0 - p.PW, tl.y0 - ph_eff, tl.n);
         }
         __syncwarp();
         if (++slot == S) { slot = 0; phase ^= 1; }
@@ -311,13 +275,6 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
     }
   } else if (warp <= kMmaWarps) {
     if (warp > p.n_mma) goto done;                       // single-issuer launches: warp 2 idles
-    if (PAIR_T && crank != 0) {                          // CTA pair: only the leader issues; the peer reports its weight half
-      if (warp == 1) {
-        mbar_wait_spin(bar_w, 0);
-        if (lane == 0) mbar_arrive_cluster(bar_w + lead_off);
-      }
-      goto done;
-    }
     // ===================== MMA issuers (warps 1 and 2 take alternate tiles) =====================
     // tcgen05.mma issue proceeds at execution pace (the issuing thread stalls while the tensor pipe is busy), so with a
     // single issuer the ~600 clk of mbarrier round trips between tiles leave the pipe idle.  With two issuers one warp's
@@ -327,8 +284,8 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
     // from the other issuer's progress word otherwise.  All 32 lanes run the warp-uniform control flow; one elected lane issues.  Per
     // MMA only the 14-bit start-address fields of the two descriptors change.
     const int mw = warp - 1;
-    const uint32_t idesc = make_idesc_bf16(PAIR_T ? 2 * kTileM : kTileM, nmma);
-    const uint32_t b_step16 = static_cast<uint32_t>(nmma * (PAIR_T ? 16 : 32)) >> 4;   // one (dy,kstep) weight block in 16-byte units
+    const uint32_t idesc = make_idesc_bf16(kTileM, nmma);
+    const uint32_t b_step16 = static_cast<uint32_t>(nmma * 32) >> 4;         // one (dy,kstep) weight block in 16-byte units
     const uint32_t kb_w16 = static_cast<uint32_t>(p.KH * 4) * b_step16;       // one full k-block of weights
     // A window: one pixel = one row of box_c channels (128 / 64 / 32 bytes, swizzled with the matching TMA mode)
     const uint32_t row_bytes = static_cast<uint32_t>(p.box_c) * 2u;
@@ -370,15 +327,6 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
         mbar_wait_spin(bar_a_full(slot), phase);
         if (p.n_mma > 1) progress[mw] = static_cast<uint32_t>(entry) + 1u;
         tc_fence_after();
-        if (p.issue_order && kb == 0 && it > 0) {
-          // The tensor pipe executes MMAs in issue order.  With a deep window ring both issuers would interleave their
-          // tiles MMA by MMA, finish both accumulators at the same moment and then leave the pipe idle while both
-          // epilogues run; taking turns (tile it starts once tile it-1 is fully issued) keeps one accumulator draining
-          // while the other fills.
-          // (an mbarrier, not a shared-memory spin: a spinning warp steals issue slots from the epilogue warps on its
-          // scheduler.)  Strict alternation keeps the waiter at most one phase behind, so the parity is unambiguous.
-          mbar_wait_spin(bar_token(1 - mw), static_cast<uint32_t>((it - 1) / p.n_mma) & 1u);
-        }
         if (kb == 0 && lane == 0) CSR_TRACE(1, it, 2);
         const int ks_here = min(4, ksteps_total - kb * 4);
         uint32_t a16 = ((slots_addr + slot * p.slot_bytes) >> 4) | a_lbo;
@@ -405,8 +353,7 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
             } else
             for (int dy = 0; dy < p.KH; ++dy, a16 += row16) {
               for (int ks = 0; ks < ks_here; ++ks, b16 += b_step16) {
-                if constexpr (PAIR_T) umma_bf16_split_pair(d_tmem, a16 + ks * 2, a_hi, b16, b_hi, idesc, acc);
-                else umma_bf16_split(d_tmem, a16 + ks * 2, a_hi, b16, b_hi, idesc, acc);
+                umma_bf16_split(d_tmem, a16 + ks * 2, a_hi, b16, b_hi, idesc, acc);
                 acc = 1;
               }
             }
@@ -425,20 +372,12 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
             }
           }
           if (last_kb) CSR_TRACE(1, it, 4);
-          if constexpr (PAIR_T) {
-            umma_commit_pair(bar_a_empty(slot));                           // both CTAs' window slots
-            if (last_kb) umma_commit_pair(bar_acc_full(buf));
-          } else {
-            umma_commit(bar_a_empty(slot));                                // window slot reusable once these MMAs have read it
-            if (last_kb) umma_commit(bar_acc_full(buf + tall - 1));        // accumulator complete -> epilogue
-          }
+          umma_commit(bar_a_empty(slot));                                  // window slot reusable once these MMAs have read it
+          if (last_kb) umma_commit(bar_acc_full(buf + tall - 1));          // accumulator complete -> epilogue
           if (kb == p.n_kblocks - 1) CSR_TRACE(1, it, 5);
         }
         __syncwarp();
-        if (kb == p.n_kblocks - 1 && lane == 0) {
-          if (p.issue_order) mbar_arrive(bar_token(mw));
-          CSR_TRACE(1, it, 3);
-        }
+        if (kb == p.n_kblocks - 1 && lane == 0) CSR_TRACE(1, it, 3);
         ring_advance(1);
       }
       if (p.n_mma > 1) {                                                   // skip the other issuer's tile
@@ -475,7 +414,6 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
     const bool has_r1 = RES_T >= 0 ? (RES_T & 1) != 0 : p.r1 != nullptr;
     const bool has_r2 = RES_T >= 0 ? (RES_T & 2) != 0 : p.r2 != nullptr;
     const bool has_gate = RES_T >= 0 ? (RES_T & 4) != 0 : p.gate != nullptr;
-    const bool r1_pre = RES_T >= 0 ? (RES_T & 8) != 0 : p.r1_pre != 0;    // r1 is a partial pre-activation sum (dense-block regrouping)
     const bool tma_store = ST_T >= 0 ? ST_T == 1 : (p.store_mode == kStoreStaged);
     const bool need_pix = !tma_store || has_r1 || has_r2 || has_gate;    // warp-uniform
     const uint32_t swz = (p.stage_row_bytes == 128) ? static_cast<uint32_t>(srow & 7) : 0u;   // SWIZZLE_128B staging rows
@@ -506,8 +444,7 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
     uint32_t acc_phase = 0;
     if constexpr (EARLY_T) {
       // One group of 16 warps, 64 output channels: warp (quadrant q, sub s) owns channels [16 s, 16 s + 16) of rows [32 q, 32 q + 32).
-      static_assert(KW_T >= 1 && KW_T <= 3 && (RES_T == 0 || RES_T == 1 || RES_T == 3) && ST_T == 1 && PAIR_T == 0 && TALL_T == 0,
-                    "early-release epilogue: wide layers without gate / pre-activation addend");
+      static_assert(KW_T >= 1 && KW_T <= 3 && RES_T == 0 && ST_T == 1 && TALL_T == 0, "early-release epilogue: wide residual-free layers");
       const int ch_lo = sub * 16;
       uint32_t sb = 0;                                    // staging buffer of this tile
       const bool two_stage = p.n_stage == 2;
@@ -558,19 +495,6 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
         if (t >= p.num_tiles) break;
         if (tracer) CSR_TRACE(2, it, 3);
         const Tile tl = decode_tile<0>(p, t);
-        // residual operands do not depend on the accumulator: fetch them before waiting for the MMAs
-        uint4 q1[2], q2[2];
-        if constexpr (RES_T != 0) {
-          const int y = tl.y0 + ty, x = tl.x0 - PW_T + tx;
-          const bool valid = col_ok && (y < p.H) && (x < p.W);
-          const size_t pix = (static_cast<size_t>(tl.n) * p.H + y) * p.W + x;
-#pragma unroll
-          for (int jj = 0; jj < 2; ++jj) {
-            const int ch0 = ch_lo + jj * 8;
-            q1[jj] = valid ? ldg16(p.r1, pix, p.r1_C, p.r1_coff + ch0) : make_uint4(0, 0, 0, 0);
-            if constexpr (RES_T == 3) q2[jj] = valid ? ldg16(p.r2, pix, p.r2_C, p.r2_coff + ch0) : make_uint4(0, 0, 0, 0);
-          }
-        }
         if (!two_stage && it > 0) named_bar_sync(1, gthreads);   // one staging buffer: every copy-out of the previous tile has been issued
         const uint32_t t_addr = t_lane + buf * nacc + ch_lo;
         mbar_wait(bar_acc_full(buf), acc_phase);           // the one bounded wait (see mbar_wait_spin)
@@ -599,13 +523,7 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
           }
 #pragma unroll
           for (int dx = 0; dx < KW_E; ++dx) gather_add8(v, raw[jj][dx], dx - PW_T, lane);
-          if (act == 3) {
-            if (ch0 < p.act_upto) apply_act8(v, 1);
-          } else {
-            apply_act8(v, act);
-          }
-          if constexpr (RES_T != 0) fma_residual8(v, q1[jj], p.s1);
-          if constexpr (RES_T == 3) fma_residual8(v, q2[jj], p.s2);
+          apply_act8(v, act);
           if (col_ok && ch0 < p.n_store)
             st_shared_v4(srow_addr + sb * p.stage_bytes + ((static_cast<uint32_t>(ch0 >> 3) ^ swz) << 4), pack_bf16x2(v[0], v[1]),
                          pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
@@ -717,7 +635,6 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
       mbar_wait(bar_acc_full(buf), acc_phase);             // the one bounded wait (see mbar_wait_spin)
       tc_fence_after();
       if (tracer) CSR_TRACE(2, it, 1);
-      uint4 held = make_uint4(0, 0, 0, 0);                // first half of a 32-byte direct store
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         const int c = 2 * (sub + (j >> 1) * cstep) + (j & 1);   // adjacent chunk pairs: 16 channels = one 32-byte sector
@@ -736,18 +653,6 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
             tmem_ld8(t_addr + ch0, r0);
             tmem_ld_wait();
             gather_add8(v, r0, 0, lane);
-          } else if constexpr (KW_T == 2 && HYB_T) {      // hybrid fold: both taps in one column group
-            uint32_t r0[8];
-            tmem_ld8(t_addr + ch0, r0);
-            tmem_ld_wait();
-            gather_add8(v, r0, d0, lane);
-          } else if constexpr (KW_T == 3 && HYB_T) {      // hybrid fold: tap 2 accumulated into tap 1's columns
-            uint32_t r0[8], r1[8];
-            tmem_ld8(t_addr + ch0, r0);
-            tmem_ld8(t_addr + p.npad + ch0, r1);
-            tmem_ld_wait();
-            gather_add8(v, r0, d0, lane);
-            gather_add8(v, r1, d1, lane);
           } else if constexpr (KW_T == 2) {
             uint32_t r0[8], r1[8];
             tmem_ld8(t_addr + ch0, r0);
@@ -772,14 +677,9 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
               gather_add8(v, r, dx - PW, lane);
             }
           }
-          if (r1_pre) fma_residual8(v, q1[j], 1.f);
-          if (act == 3) {
-            if (ch0 < p.act_upto) apply_act8(v, 1);
-          } else {
-            apply_act8(v, act, p.act_slope);
-          }
+          apply_act8(v, act, p.act_slope);
           if (need_pix) {
-            if (has_r1 && !r1_pre) fma_residual8(v, q1[j], p.s1);
+            if (has_r1) fma_residual8(v, q1[j], p.s1);
             if (has_gate) gate8(v, q2[j], p.gate_neg);
             else if (has_r2) fma_residual8(v, q2[j], p.s2);
           }
@@ -789,15 +689,8 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
                            pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
           } else if (valid) {
             const size_t opix = (static_cast<size_t>(tl.n) * p.out_H + (y * p.out_sy + oy_eff)) * p.out_W + (x * p.out_sx + p.out_ox);
-            const int smode = ST_T == 2 ? static_cast<int>(kStoreDirect32) : ST_T == 3 ? static_cast<int>(kStoreF32Planar) : p.store_mode;
-            if (smode == kStoreDirect32) {
-              // whole 32-byte sectors per lane (16 channels): no partial-sector writes reach L2
-              uint4 o;
-              o.x = pack_bf16x2(v[0], v[1]); o.y = pack_bf16x2(v[2], v[3]); o.z = pack_bf16x2(v[4], v[5]); o.w = pack_bf16x2(v[6], v[7]);
-              if ((j & 1) == 0) held = o;
-              else if (ch0 < p.n_store)
-                st_global_v8(reinterpret_cast<__nv_bfloat16*>(p.out) + opix * p.out_C + p.out_coff + static_cast<int>(blockIdx.y) * p.part_c + ch0 - 8, held, o);
-            } else if (smode == kStoreF32Planar) {
+            const int smode = ST_T == 3 ? static_cast<int>(kStoreF32Planar) : p.store_mode;
+            if (smode == kStoreF32Planar) {
               if (c == 0) reinterpret_cast<float*>(p.out)[opix] = v[0];
             } else {
 #pragma unroll
@@ -817,10 +710,7 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
       // all TMEM reads of this warp are complete (wait::ld above): hand the accumulator buffer back to the MMA warp
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if constexpr (PAIR_T) mbar_arrive_cluster(bar_acc_empty(buf) + lead_off);
-        else mbar_arrive(bar_acc_empty(buf));
-      }
+      if (lane == 0) mbar_arrive(bar_acc_empty(buf));
       if (tma_store) {
         named_bar_sync(1 + g, gthreads);                  // the staged tile is complete
         if (tracer) CSR_TRACE(2, it, 7);
@@ -849,28 +739,26 @@ done:
   tc_fence_before();
   __syncthreads();
   timeline_end(p.timeline, p.launch_id);
-  if constexpr (PAIR_T) cluster_sync_all();              // the leader's MMAs read the peer's shared memory and TMEM until here
   if (warp == 1) {
     __syncwarp();
     tc_fence_after();
-    if constexpr (PAIR_T) tmem_dealloc_pair(tmem_base, p.tmem_cols);
-    else tmem_dealloc(tmem_base, p.tmem_cols);
+    tmem_dealloc(tmem_base, p.tmem_cols);
   }
 }
 
 size_t conv_smem_bytes(const ConvParams& p) {
   return 1024 /*alignment slack*/ + static_cast<size_t>(p.n_slots) * p.slot_bytes + static_cast<size_t>(p.n_stage) * p.stage_bytes +
-         (((p.stream_w ? 0 : p.pair ? p.w_bytes / 2 : p.w_bytes) + 127) & ~127) + (p.fuse2 ? p.w2_bytes + 128 : 0) + 256 /*bias*/ +
-         8 * (20 + 2 * p.n_slots) + 32;
+         (((p.stream_w ? 0 : p.w_bytes) + 127) & ~127) + (p.fuse2 ? p.w2_bytes + 128 : 0) + 256 /*bias*/ +
+         8 * (18 + 2 * p.n_slots) + 32;
 }
 
-template <int KW_T, int PW_T, int ACT_T, int RES_T, int ST_T, int PAIR_T = 0, int TALL_T = 0, int EARLY_T = 0, int FUSE_T = 0, int HYB_T = 0>
+template <int KW_T, int PW_T, int ACT_T, int RES_T, int ST_T, int TALL_T = 0, int EARLY_T = 0, int FUSE_T = 0, int HYB_T = 0>
 static int launch_t(const ConvParams& p, const CUtensorMap& tmap, int num_sms, cudaStream_t stream) {
   const size_t smem = conv_smem_bytes(p);
   if (smem > static_cast<size_t>(kSmemLimit)) return static_cast<int>(cudaErrorInvalidValue);
   // the attribute is per device (and per template instantiation): one process may drive several GPUs
   static bool configured[64] = {};
-  auto kern = conv_tc_kernel<KW_T, PW_T, ACT_T, RES_T, ST_T, PAIR_T, TALL_T, EARLY_T, FUSE_T, HYB_T>;
+  auto kern = conv_tc_kernel<KW_T, PW_T, ACT_T, RES_T, ST_T, TALL_T, EARLY_T, FUSE_T, HYB_T>;
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return static_cast<int>(cudaErrorInvalidDevice);
   if (!configured[dev]) {
@@ -883,131 +771,85 @@ static int launch_t(const ConvParams& p, const CUtensorMap& tmap, int num_sms, c
   const int parts = p.parts > 1 ? p.parts : 1;
   const int per_part = num_sms / parts > 0 ? num_sms / parts : 1;
   cfg.gridDim = dim3(p.num_tiles < per_part ? p.num_tiles : per_part, parts);
-  if (PAIR_T) cfg.gridDim.x &= ~1u;                       // whole pairs (the host only selects pair mode for an even tile count)
   cfg.blockDim = dim3(kConvThreads);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
+  cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = p.use_pdl ? 1 : 0;
-  attr[1].id = cudaLaunchAttributeClusterDimension;
-  attr[1].val.clusterDim.x = 2;
-  attr[1].val.clusterDim.y = 1;
-  attr[1].val.clusterDim.z = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = PAIR_T ? 2 : 1;
+  cfg.numAttrs = 1;
   return static_cast<int>(cudaLaunchKernelEx(&cfg, kern, p, tmap));
 }
 
 int launch_conv_tc(const ConvParams& p, const CUtensorMap& tmap, int num_sms, cudaStream_t stream) {
-  const int res = (p.r1 ? 1 : 0) | (p.r2 ? 2 : 0) | (p.gate ? 4 : 0) | ((p.r1 && p.r1_pre) ? 8 : 0);
+  const int res = (p.r1 ? 1 : 0) | (p.r2 ? 2 : 0) | (p.gate ? 4 : 0);
   if ((res & 6) == 6) return static_cast<int>(cudaErrorInvalidValue);   // r2 and gate share an operand slot
-  // Measured-and-rejected variants (CTA pairs, unstaged 32-byte stores, dense blocks regrouped by source as per-layer launches)
-  // are only instantiated in a -DCSR_EXPERIMENTS build (CSR_EXPERIMENTS=1 python build.py): the default library carries the
-  // kernels that run.  DESIGN.md section 3.1 has their numbers.
-  if (p.pair) {
-#ifdef CSR_EXPERIMENTS
-    // CTA-pair variants: 3x3 layers whose resident weights would otherwise starve the window ring
-    if (p.store_mode != kStoreStaged || p.KW != 3 || p.PW != 1 || p.act != 0 || (p.num_tiles & 1) || p.force_generic)
-      return static_cast<int>(cudaErrorInvalidValue);
-    switch (res) {
-      case 1: return launch_t<3, 1, 0, 1, 1, 1>(p, tmap, num_sms, stream);
-      case 3: return launch_t<3, 1, 0, 3, 1, 1>(p, tmap, num_sms, stream);
-      case 4: return launch_t<3, 1, 0, 4, 1, 1>(p, tmap, num_sms, stream);
-      case 5: return launch_t<3, 1, 0, 5, 1, 1>(p, tmap, num_sms, stream);
-      default: return static_cast<int>(cudaErrorInvalidValue);
-    }
-#else
-    return static_cast<int>(cudaErrorNotSupported);
-#endif
-  }
   if (p.tall_shift) {
     // two-M-tile windows: the thin layers only (four accumulator buffers)
     if ((p.n_acc != 4 && p.n_acc != 8) || p.n_groups != 4) return static_cast<int>(cudaErrorInvalidValue);
     if (p.store_mode == kStoreStaged && !p.force_generic && p.KW == 3 && p.PW == 1 && p.act == 1 && res == 0)
-      return launch_t<3, 1, 1, 0, 1, 0, 1>(p, tmap, num_sms, stream);      // RDB conv1-4 (not regrouped)
-#ifdef CSR_EXPERIMENTS
-    if (p.store_mode == kStoreStaged && !p.force_generic && p.KW == 3 && p.PW == 1 && p.act == 1 && res == 9)
-      return launch_t<3, 1, 1, 9, 1, 0, 1>(p, tmap, num_sms, stream);      // RDB conv2-4 over x1..x_{k-1}
-#endif
+      return launch_t<3, 1, 1, 0, 1, 1>(p, tmap, num_sms, stream);         // RDB conv1-4
     if (p.store_mode == kStoreStaged && !p.force_generic && p.KW == 1 && p.PW == 0 && p.act == 2 && res == 0)
-      return launch_t<1, 0, 2, 0, 1, 0, 1>(p, tmap, num_sms, stream);      // srcnn.conv2
+      return launch_t<1, 0, 2, 0, 1, 1>(p, tmap, num_sms, stream);         // srcnn.conv2
     if (p.store_mode == kStoreStaged && !p.force_generic && p.KW == 3 && p.PW == 1 && p.act == 0 && res == 4)
-      return launch_t<3, 1, 0, 4, 1, 0, 1>(p, tmap, num_sms, stream);      // dense-block input gradients of x1..x4 (gated)
+      return launch_t<3, 1, 0, 4, 1, 1>(p, tmap, num_sms, stream);         // dense-block input gradients of x1..x4 (gated)
     if (p.store_mode == kStoreStaged && !p.force_generic && p.KW == 3 && p.PW == 1 && p.act == 0 && res == 5)
-      return launch_t<3, 1, 0, 5, 1, 0, 1>(p, tmap, num_sms, stream);
+      return launch_t<3, 1, 0, 5, 1, 1>(p, tmap, num_sms, stream);
     if (p.store_mode == kStoreStaged && !p.force_generic && p.KW == 1 && p.PW == 0 && p.act == 0 && res == 4)
-      return launch_t<1, 0, 0, 4, 1, 0, 1>(p, tmap, num_sms, stream);      // srcnn.conv3 input gradient over the gradient im2col
+      return launch_t<1, 0, 0, 4, 1, 1>(p, tmap, num_sms, stream);         // srcnn.conv3 input gradient over the gradient im2col
     if (p.store_mode == kStoreF32Planar && !p.force_generic && p.KW == 3 && p.PW == 1 && p.act == 0 && res == 0)
-      return launch_t<3, 1, 0, 0, 3, 0, 1>(p, tmap, num_sms, stream);      // conv_last
+      return launch_t<3, 1, 0, 0, 3, 1>(p, tmap, num_sms, stream);         // conv_last
     if (p.store_mode == kStoreF32Planar && !p.force_generic && p.KW == 5 && p.PW == 2 && p.act == 0 && res == 0)
-      return launch_t<5, 2, 0, 0, 3, 0, 1>(p, tmap, num_sms, stream);      // srcnn.conv3
+      return launch_t<5, 2, 0, 0, 3, 1>(p, tmap, num_sms, stream);         // srcnn.conv3
     switch (p.KW) {
-      case 1: return launch_t<1, 0, -1, -1, -1, 0, 1>(p, tmap, num_sms, stream);
-      case 3: if (p.PW == 1) return launch_t<3, 1, -1, -1, -1, 0, 1>(p, tmap, num_sms, stream);
-      default: return launch_t<0, 0, -1, -1, -1, 0, 1>(p, tmap, num_sms, stream);
+      case 1: return launch_t<1, 0, -1, -1, -1, 1>(p, tmap, num_sms, stream);
+      case 3: if (p.PW == 1) return launch_t<3, 1, -1, -1, -1, 1>(p, tmap, num_sms, stream);
+      default: return launch_t<0, 0, -1, -1, -1, 1>(p, tmap, num_sms, stream);
     }
   }
   if (p.early) {
     // wide residual-free layers with the early-release epilogue (one 16-warp group, two staging buffers)
-    if (p.store_mode != kStoreStaged || p.n_groups != 1 || p.n_stage < 1 || p.n_stage > 2 || p.npad != 64 || p.force_generic)
+    if (p.store_mode != kStoreStaged || p.n_groups != 1 || p.n_stage < 1 || p.n_stage > 2 || p.npad != 64 || res != 0 || p.force_generic)
       return static_cast<int>(cudaErrorInvalidValue);
     if (p.fuse2 == 2) {
       // HRconv (3x3, LeakyReLU) + the nine tap planes of conv_last (3x3, 64 -> 1) in one launch
-      if (p.KW != 3 || p.PW != 1 || p.act != 1 || res != 0 || p.stage_row_bytes != 128 || p.w2_bytes != 2048 || p.n2 != 9 || p.out2_plane <= 0 ||
+      if (p.KW != 3 || p.PW != 1 || p.act != 1 || p.stage_row_bytes != 128 || p.w2_bytes != 2048 || p.n2 != 9 || p.out2_plane <= 0 ||
           p.tmem_cols < p.n_acc * (p.hyb ? p.KW - 1 : p.KW) * p.npad + 16 || p.parts > 1)
         return static_cast<int>(cudaErrorInvalidValue);
-      if (p.hyb) return launch_t<3, 1, 1, 0, 1, 0, 0, 1, 2, 1>(p, tmap, num_sms, stream);
-      return launch_t<3, 1, 1, 0, 1, 0, 0, 1, 2>(p, tmap, num_sms, stream);
+      if (p.hyb) return launch_t<3, 1, 1, 0, 1, 0, 1, 2, 1>(p, tmap, num_sms, stream);
+      return launch_t<3, 1, 1, 0, 1, 0, 1, 2>(p, tmap, num_sms, stream);
     }
     if (p.fuse2) {
       // srcnn.conv1 (x-im2col folded, ReLU) + srcnn.conv2 (1x1, ReLU) in one launch
-      if (p.KW != 1 || p.PW != 0 || p.act != 2 || res != 0 || p.stage_row_bytes != 128 || p.w2_bytes != 4096 || p.n2 < 8 || p.n2 > 32 || (p.n2 & 7) ||
+      if (p.KW != 1 || p.PW != 0 || p.act != 2 || p.stage_row_bytes != 128 || p.w2_bytes != 4096 || p.n2 < 8 || p.n2 > 32 || (p.n2 & 7) ||
           p.tmem_cols < p.n_acc * p.KW * p.npad + 32 || p.parts > 1)
         return static_cast<int>(cudaErrorInvalidValue);
-      return launch_t<1, 0, 2, 0, 1, 0, 0, 1, 1>(p, tmap, num_sms, stream);
+      return launch_t<1, 0, 2, 0, 1, 0, 1, 1>(p, tmap, num_sms, stream);
     }
-#define CSR_EARLY(KW_, PW_, ACT_, RES_) \
-    if (p.KW == KW_ && p.PW == PW_ && p.act == ACT_ && res == RES_) {                                                                   \
-      if constexpr (KW_ >= 2) { if (p.hyb) return launch_t<KW_, PW_, ACT_, RES_, 1, 0, 0, 1, 0, 1>(p, tmap, num_sms, stream); }            \
-      return launch_t<KW_, PW_, ACT_, RES_, 1, 0, 0, 1>(p, tmap, num_sms, stream);                                                      \
+#define CSR_EARLY(KW_, PW_, ACT_)                                                                                    \
+    if (p.KW == KW_ && p.PW == PW_ && p.act == ACT_) {                                                                 \
+      if constexpr (KW_ >= 2) { if (p.hyb) return launch_t<KW_, PW_, ACT_, 0, 1, 0, 1, 0, 1>(p, tmap, num_sms, stream); } \
+      return launch_t<KW_, PW_, ACT_, 0, 1, 0, 1>(p, tmap, num_sms, stream);                                           \
     }
-    CSR_EARLY(3, 1, 1, 0)   // HRconv
-    CSR_EARLY(3, 1, 0, 0)   // conv_first
-#ifdef CSR_EXPERIMENTS
-    CSR_EARLY(3, 1, 3, 0)   // dense block regrouped by source: conv1 + the x-parts of conv2-4
-#endif
-    CSR_EARLY(2, 0, 1, 0)   // upconv sub-pixel phases
-    CSR_EARLY(2, 1, 1, 0)
-    CSR_EARLY(1, 0, 2, 0)   // srcnn.conv1 (x-im2col folded)
-    CSR_EARLY(3, 1, 0, 1)   // RDB conv5 (*0.2 + x), trunk_conv (+ fea): one staging buffer when the weights leave no room for two
-    CSR_EARLY(3, 1, 0, 3)   // RDB3 conv5 (*0.2 + x, *0.2 + x_rrdb)
+    CSR_EARLY(3, 1, 1)   // HRconv
+    CSR_EARLY(3, 1, 0)   // conv_first
+    CSR_EARLY(2, 0, 1)   // upconv sub-pixel phases
+    CSR_EARLY(2, 1, 1)
+    CSR_EARLY(1, 0, 2)   // srcnn.conv1 (x-im2col folded)
 #undef CSR_EARLY
     return static_cast<int>(cudaErrorInvalidValue);
   }
 #define CSR_CASE(KW_, PW_, ACT_, RES_, ST_)                                                                  \
-  if (p.store_mode == (ST_ == 1 ? kStoreStaged : ST_ == 3 ? kStoreF32Planar : kStoreDirect32) && !p.force_generic && p.KW == KW_ && \
+  if (p.store_mode == (ST_ == 1 ? kStoreStaged : kStoreF32Planar) && !p.force_generic && p.KW == KW_ &&   \
       p.PW == PW_ && p.act == ACT_ && res == RES_)                                                           \
     return launch_t<KW_, PW_, ACT_, RES_, ST_>(p, tmap, num_sms, stream);
   // the layer shapes of the generator forward (esrgan.py / srcnn.py) ...
   CSR_CASE(3, 1, 1, 0, 1)   // RDB conv1-4, HRconv: lrelu
   CSR_CASE(3, 1, 0, 0, 1)   // conv_first
   CSR_CASE(3, 1, 4, 0, 1)   // discriminator convs: LeakyReLU(act_slope)
-  if (p.hyb && p.store_mode == kStoreStaged && !p.force_generic && p.KW == 3 && p.PW == 1 && p.act == 0) {   // hybrid tap fold (HYB_T)
-#ifdef CSR_EXPERIMENTS
-    if (res == 1) return launch_t<3, 1, 0, 1, 1, 0, 0, 0, 0, 1>(p, tmap, num_sms, stream);
-    if (res == 3) return launch_t<3, 1, 0, 3, 1, 0, 0, 0, 0, 1>(p, tmap, num_sms, stream);
-#endif
-    return static_cast<int>(cudaErrorInvalidValue);
-  }
   CSR_CASE(3, 1, 0, 1, 1)   // RDB conv5 (*0.2 + x), trunk_conv (+ fea)
   CSR_CASE(3, 1, 0, 3, 1)   // RDB3 conv5 (*0.2 + x, *0.2 + x_rrdb)
-#ifdef CSR_EXPERIMENTS
-  CSR_CASE(3, 1, 0, 1, 2)   // ... the same with unstaged stores (weights leave no room for staging + a deep window ring)
-  CSR_CASE(3, 1, 0, 3, 2)
-  CSR_CASE(3, 1, 3, 0, 1)   // dense block regrouped by source: conv1 and the x-parts of conv2-4 in one launch (lrelu on conv1's channels)
-  CSR_CASE(3, 1, 1, 9, 1)   // ... conv2-4 over x1..x_{k-1} only, the x-part added before the lrelu
-#endif
   CSR_CASE(2, 0, 1, 0, 1)   // upconv sub-pixel phases
   CSR_CASE(2, 1, 1, 0, 1)
   CSR_CASE(1, 0, 2, 0, 1)   // srcnn.conv1 (x-im2col folded), srcnn.conv2: relu

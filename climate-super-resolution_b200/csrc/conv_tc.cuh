@@ -18,9 +18,7 @@ enum StoreMode {
   kStoreStaged = 0,     // bf16 NHWC through a swizzled shared-memory staging tile, copied out as whole pixel rows
   kStoreDirect = 1,     // bf16 NHWC, per-element global stores (ragged channel counts)
   kStoreF32Planar = 2,  // fp32 (N,1,H,W), channel 0 only
-  kStoreF32Nhwc = 3,    // fp32 NHWC (n_store channels per pixel, pitch out_C): gradient / debug outputs
-  kStoreDirect32 = 4    // bf16 NHWC, one 32-byte store per lane and 16-channel chunk pair straight from registers
-                        // (no staging; n_store, out_C and out_coff multiples of 16)
+  kStoreF32Nhwc = 3     // fp32 NHWC (n_store channels per pixel, pitch out_C): gradient / debug outputs
 };
 
 struct ConvParams {
@@ -50,18 +48,15 @@ struct ConvParams {
   int early;       // 1 = early-release epilogue (conv_tc.cu, EARLY_T): wide residual-free layers, one 16-warp group
   int tmem_cols;   // power of two >= max(32, n_acc*KW*npad)
   int force_generic;  // debug: skip the compile-time specialised kernels
-  int issue_order; // 1 = the two MMA warps take strict turns tile by tile (only meaningful with n_mma == 2)
   int trace_cta;   // debug: the CTA whose role timestamps go to `trace`
   int box_c;       // channels per window pixel in shared memory: 64 (128-byte rows), or 32 / 16 for single-k-block layers with cin <= 32 / 16
   int tall_shift;  // 1: a window holds TWO vertically adjacent M tiles (2*TH + KH - 1 rows, one TMA load, one MMA-issuer iteration,
                    //    two accumulator buffers): halves the per-tile control cost of thin layers; needs n_acc == 4.  tiles_* / num_tiles
                    //    then count windows.  0: one M tile per window
-  int pair;        // 1 = CTA-pair launch (cluster of 2, M = 256 MMAs, half of the weights resident per CTA); needs an even tile count
   int stream_w;    // 1: the layer's weights do NOT stay resident (layers with >= 256 input channels: > 150 KB per 64 output channels): every
                    //    window slot also receives the packed weights of its 64-channel k-block (wkb_bytes, at offset win_slot_bytes)
   int wkb_bytes;   // packed weights of one full k-block: KH * 4 * KW * npad * 32
   int win_slot_bytes;
-  int l2_prefetch; // > 0: the producer prefetches the window of the tile `l2_prefetch` iterations ahead into L2 (layers that stream from HBM)
   int use_pdl;     // launch with programmatic stream serialization (prologue overlaps the previous kernel's tail)
   // Output-channel parts of ONE layer as one launch (gridDim.y = parts): every part has this launch's geometry and reads the same input;
   // part k takes its weights at wpk + k*part_w_bytes, its bias at bias + k*part_b_floats and writes output channels out_coff + k*part_c.
@@ -77,13 +72,11 @@ struct ConvParams {
   void* out2; int out2_C, out2_coff;
   // fuse2 == 2: the successor is a 3x3 -> 1 conv seen as nine 1x1 'tap' channels (n2 = 9): fp32 tap planes out2[tap * out2_plane + pixel]
   long long out2_plane;
-  // epilogue:  v = act(acc + bias [+ r1 if r1_pre]);  if r1 (not r1_pre): v = v*s1 + r1;  if r2: v = v*s2 + r2;  if gate: v *= (gate > 0 ? 1 : gate_neg)
+  // epilogue:  v = act(acc + bias);  if r1: v = v*s1 + r1;  if r2: v = v*s2 + r2;  if gate: v *= (gate > 0 ? 1 : gate_neg)
   const float* bias;   // [npad] fp32 (zero padded)
   const void* wpk;     // packed bf16 weights (global), layout [kblock][dy][kstep in kblock][KW*npad/8][2][8][8]
-  int act;             // 0 none, 1 leaky-relu 0.2, 2 relu, 3 leaky-relu 0.2 on output channels < act_upto only, 4 leaky-relu(act_slope)
-  int act_upto;
+  int act;             // 0 none, 1 leaky-relu 0.2, 2 relu, 4 leaky-relu(act_slope)
   float act_slope;     // act == 4: LeakyReLU negative slope
-  int r1_pre;          // 1: r1 is added BEFORE the activation (v = act(acc + bias + r1)) instead of after it
   float s1, s2;
   const void* r1; int r1_C, r1_coff;
   const void* r2; int r2_C, r2_coff;

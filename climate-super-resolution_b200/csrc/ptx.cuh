@@ -86,12 +86,6 @@ __device__ __forceinline__ void tma_load_4d(uint32_t dst, const void* tmap, uint
       ::"r"(dst), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
       : "memory");
 }
-// L2 prefetch of a tensor box (no shared-memory destination): decouples HBM latency from the depth of the window ring
-__device__ __forceinline__ void tma_prefetch_l2_4d(const void* tmap, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.prefetch.tensor.4d.L2.global.tile [%0, {%1, %2, %3, %4}];"
-               ::"l"(reinterpret_cast<uint64_t>(tmap)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-               : "memory");
-}
 __device__ __forceinline__ void bulk_load(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                ::"r"(dst), "l"(reinterpret_cast<uint64_t>(src)), "r"(bytes), "r"(bar)
@@ -116,11 +110,6 @@ __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
 // fire-and-forget vector fp32 add into global memory (sm_90+): one L2 atomic per 16 bytes
 __device__ __forceinline__ void red_add_v4_f32(float* ptr, float a, float b, float c, float d) {
   asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(ptr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
-}
-__device__ __forceinline__ void st_global_v8(void* ptr, const uint4& a, const uint4& b) {
-  asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(ptr), "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w), "r"(b.x),
-               "r"(b.y), "r"(b.z), "r"(b.w)
-               : "memory");
 }
 __device__ __forceinline__ uint4 ld_shared_v4(uint32_t addr) {
   uint4 v;
@@ -181,60 +170,6 @@ __device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t adesc, uint6
 // All previously issued MMAs of this thread arrive on `bar` when they complete (implies fence::before_thread_sync).
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// ---- CTA pair (cluster of two CTAs on one TPC, tcgen05 cta_group::2) ----
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire;" ::: "memory");
-}
-// shared::cluster address of `addr` (a shared::cta address of this CTA) inside CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t map_to_cta(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_bar) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_bar) : "memory");
-}
-// TMA window load of a CTA pair: lands in THIS CTA's shared memory, completes bytes on `cluster_bar`, a shared::cluster
-// address that may belong to the peer CTA (the leader's barrier) - that is what .cta_group::2 permits.
-__device__ __forceinline__ void tma_load_4d_pair(uint32_t dst, const void* tmap, uint32_t cluster_bar, int c0, int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(cluster_bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t smem_dst, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void tmem_relinquish_pair() {
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-// M = 256 MMA issued by the leader CTA: A rows [0,128) / [128,256) and B rows [0,N/2) / [N/2,N) are read from the same
-// shared-memory offsets of CTA 0 / CTA 1; each CTA's TMEM receives its own 128 accumulator rows, all N columns.
-__device__ __forceinline__ void umma_bf16_split_pair(uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi,
-                                                     uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-      "mov.b64 da, {%1, %2};\n\t"
-      "mov.b64 db, {%3, %4};\n\t"
-      "setp.ne.b32 p, %6, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %5, p;\n\t}"
-      ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// commit arriving on the barrier at the same shared-memory offset in both CTAs of the pair
-__device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"(static_cast<uint16_t>(3)) : "memory");
 }
 // 32 lanes x 16 consecutive fp32 columns -> 16 registers per thread (lane i of the warp reads TMEM lane base+i).
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {

@@ -165,7 +165,7 @@ dense_block_kernel(const DenseParams p, const __grid_constant__ CUtensorMap tmap
       const unsigned* fl = p.flags + static_cast<size_t>(l > 0 ? l - 1 : 0) * p.num_tiles;
       for (int t = blockIdx.x; t < p.num_tiles; t += G) {
         const Win w = decode_win(p, t);
-        if (l > 0 && !(p.dbg & 2)) {
+        if (l > 0) {
           // the windows of layer l-1 this window reads (1-pixel halo): itself and its <= 8 neighbours inside the image
           if (lane < 9) {
             const int dy = lane / 3 - 1, dx = lane - (lane / 3) * 3 - 1;
@@ -183,7 +183,7 @@ dense_block_kernel(const DenseParams p, const __grid_constant__ CUtensorMap tmap
           // other CTAs' generic-proxy stores (acquired above) -> this warp's async-proxy reads.  Once per window, not per TMA
           // issue: the fence also waits for the warp's loads in flight (62 -> 53 us per dense block); without any proxy fence the
           // block takes 50 us, a writer-side fence.proxy.async.global in the epilogue 52 us (profiles/r02_dense_block_notes.txt)
-          if (!(p.dbg & 4)) fence_proxy_async_all();
+          fence_proxy_async_all();
         }
         for (int kb = 0; kb < p.L[l].n_kblocks; ++kb) {
           mbar_wait_spin(bar_a_empty(slot), phase ^ 1);
@@ -390,7 +390,7 @@ dense_block_kernel(const DenseParams p, const __grid_constant__ CUtensorMap tmap
       }
       named_bar_sync(1 + g, 128);                           // every store of the tile has been issued (and the staging buffer is free)
       if (wj == 0 && lane == 0) {
-        if (!(p.dbg & 1)) __threadfence();                  // cumulative: the group's stores, ordered before this by the barrier
+        __threadfence();                                    // cumulative: the group's stores, ordered before this by the barrier
         red_release_gpu_add(p.flags + static_cast<size_t>(l) * p.num_tiles + t, 1u);
       }
       // next M tile of this group: m + 4 -> q + 2
@@ -415,11 +415,6 @@ size_t dense_smem_bytes(const DenseParams& p) {
 }
 
 int launch_dense_block(const DenseParams& p, const CUtensorMap& tmap, int num_sms, cudaStream_t stream) {
-#ifdef CSR_EXPERIMENTS
-  if (p.fold9) return launch_dense9_block(p, tmap, num_sms, stream);
-#else
-  if (p.fold9) return static_cast<int>(cudaErrorInvalidValue);
-#endif
   const size_t smem = dense_smem_bytes(p);
   if (smem > static_cast<size_t>(kSmemLimit) || p.n_layers < 1 || p.n_layers > kDenseMaxLayers || p.n_slots < 2)
     return static_cast<int>(cudaErrorInvalidValue);

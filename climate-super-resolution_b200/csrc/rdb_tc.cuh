@@ -42,17 +42,11 @@ struct DenseParams {
   float gate_neg;
   unsigned long long* timeline;   // debug: see ConvParams::timeline
   int launch_id;
-  int fold9;                      // 1: dense9_block_kernel (rdb9_tc.cu): all nine taps folded into N = 144, windows of 16 x 16 input pixels
-                                  //    (SW = 16, TH = 8 rows per M tile, 14 x 14 outputs per window; tiles_y counts 14-row windows)
-  int dbg;                        // timing experiments only (wrong results): bit 0 = no fence before the counter update, bit 1 = no dependency waits, bit 2 = no proxy fence
   DenseLayerParams L[kDenseMaxLayers];
 };
 
 size_t dense_smem_bytes(const DenseParams& p);
 // tmap: 4-D (C, W, H, N) bf16 map of the concat buffer, box (64, SW, 2*TH+2, 1), SWIZZLE_128B, zero fill.  Returns cudaError_t.
 int launch_dense_block(const DenseParams& p, const CUtensorMap& tmap, int num_sms, cudaStream_t stream);
-// fold9 form: tmap box (64, 16, 16, 1)
-size_t dense9_smem_bytes(const DenseParams& p);
-int launch_dense9_block(const DenseParams& p, const CUtensorMap& tmap, int num_sms, cudaStream_t stream);
 
 }  // namespace csr

@@ -100,7 +100,7 @@ int         csr_set_option(int32_t key, int32_t value);
 int64_t     csr_kernel_launch_count(void);           /* kernels launched by this library so far   */
 /* debug: device buffer of 3*64*8 int64 receiving per-role clock64 timestamps of CTA 0 for convs built afterwards
  * (NULL switches tracing off).  Layout [role: producer, mma, epilogue][tile 0..63][event 0..7].                   */
-int         csr_has_experiments(void);   /* 1: built with -DCSR_EXPERIMENTS (measured-and-rejected kernel variants selectable via csr_set_option) */
+int         csr_has_experiments(void);   /* always 0: the measured-and-rejected kernel variants were removed; kept so that ABI version 2 stays intact */
 int         csr_debug_set_trace(void* device_buffer);
 /* debug: in-situ timeline of the launches of csr_plan_forward (direct launches, no graph replay).  device_u64: 2 * capacity
  * uint64 in device memory, even entries preset to ~0, odd entries to 0; launch i then leaves [2i] = earliest CTA start after

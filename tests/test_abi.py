@@ -58,6 +58,17 @@ def test_argument_validation_without_gpu():
     assert lib.csr_plan_create(C.byref(good), 1, 8, 8, None, 0, None) == -1
 
 
+def test_retired_option_keys_are_rejected():
+    """Keys of the removed kernel variants are unknown keys; 26 and 35 take only 0 / 1."""
+    from climsr_b200._lib import lib
+    for key in (8, 9, 13, 14, 16, 28, 29, 32):
+        assert lib.csr_set_option(key, 0) == -1 and lib.csr_set_option(key, 1) == -1, key
+    for key in (26, 35):
+        assert lib.csr_set_option(key, 2) == -1 and lib.csr_set_option(key, -1) == -1, key
+        assert lib.csr_set_option(key, 1) == 0, key                    # the default
+    assert lib.csr_has_experiments() == 0
+
+
 def test_no_cpu_fallback():
     import torch
     from climsr_b200 import CsrError

@@ -126,40 +126,6 @@ def test_conv_epilogue_variants():
     assert torch.equal(a, c)
 
 
-def _need_experiments():
-    from climsr_b200._lib import lib
-    if not lib.csr_has_experiments():
-        pytest.skip("measured-and-rejected kernel variant: only in a CSR_EXPERIMENTS=1 build")
-
-
-def test_conv_cta_pair_matches_single_cta():
-    """CTA-pair launches (tcgen05 cta_group::2, option 13; off by default) of the RDB conv5 shape - 128 -> 64 channels with
-    the x5*0.2 + x residuals of esrgan.py:38,54 - must reproduce the single-CTA kernel bit for bit: same MMAs, same
-    accumulation order, only the operand halves come from two CTAs."""
-    from climsr_b200 import ops
-    from climsr_b200._lib import lib
-    _need_experiments()
-    g = torch.Generator().manual_seed(21)
-    n, h, w = 4, 16, 60                          # 4 x 4 x 2 = 32 tiles: an even count, which pair mode needs
-    x = torch.rand((n, 128, h, w), generator=g) * 2 - 1
-    wt = (torch.rand((64, 128, 3, 3), generator=g) * 2 - 1) / 34
-    b = torch.rand((64,), generator=g) - 0.5
-    r2 = torch.rand((n, 64, h, w), generator=g) * 2 - 1
-    xin = _nhwc(x, 128)
-    outs = []
-    for pair in (0, 1):
-        lib.csr_set_option(13, pair)
-        try:
-            o1 = ops.conv2d_nhwc(xin, wt.cuda(), b.cuda(), res1=xin, scale1=0.2)
-            o2 = ops.conv2d_nhwc(xin, wt.cuda(), b.cuda(), res1=xin, scale1=0.2, res2=_nhwc(r2, 64), scale2=0.2)
-        finally:
-            lib.csr_set_option(13, 0)
-        outs.append((o1, o2))
-    assert torch.equal(outs[0][0], outs[1][0]) and torch.equal(outs[0][1], outs[1][1])
-    want = _ref_conv(x, wt, b, "none") * 0.2 + _bf(x[:, :64])
-    assert float((outs[1][0].float().cpu().permute(0, 3, 1, 2) - want).abs().max()) <= 2.0 ** -7 * max(1.0, float(want.abs().max()))
-
-
 @pytest.mark.parametrize("n,h,w,cin,cout,k,in_c,in_coff", [
     (2, 5, 33, 64, 16, 3, 128, 0),      # second M tile of the window mostly below the image
     (1, 12, 61, 112, 16, 3, 128, 0),    # one and a half windows, two k-blocks
@@ -715,66 +681,6 @@ def test_fused_hr_tail_matches_separate_launches(n, in_ch, h, w):
     assert torch.equal(outs[3], outs[2])
     scale = max(1.0, float(outs[0].abs().max()))
     assert float((outs[3] - outs[0]).abs().max()) <= 2e-3 * scale, float((outs[3] - outs[0]).abs().max())
-
-
-@pytest.mark.parametrize("n,in_ch,h,w,nb", [(4, 4, 64, 64, 3), (1, 3, 113, 113, 2), (3, 4, 20, 36, 2), (1, 1, 9, 7, 1), (16, 4, 32, 32, 2), (150, 4, 16, 16, 1),
-                                            (2, 4, 28, 14, 1), (1, 4, 29, 15, 1)])
-def test_dense_block_nine_tap_fold_matches_per_layer_launches(n, in_ch, h, w, nb):
-    """(Experiments build only - measured slower, see rdb9_tc.cu.)  Option 32: conv1..conv4 of every dense block with ALL NINE taps folded into the UMMA N dimension (rdb9_tc.cu: N = 144, 16 x 16
-    windows, the row-shifted accumulator rows summed in the epilogue) against four per-layer launches.  Same products, another fp32
-    summation order -> equal up to bf16 rounding flips of single activations: a small fraction of the output scale.  Shapes as in the
-    bit-identity test plus rasters that end exactly on / one past a 14-pixel window edge."""
-    _need_experiments()
-    from climsr_b200._lib import lib
-    from climsr_b200.models import ESRGANGenerator
-    from oracle import synth
-    sd = synth.make_state_dict(in_ch, 1, 64, nb, 16, seed=6, gain=1.4)
-    x, elev, mask = synth.make_inputs(n, in_ch, h, w, seed=7)
-    outs = []
-    try:
-        lib.csr_set_option(31, 0)
-        for fold9, dense in ((1, 1), (0, 0), (1, 1)):
-            lib.csr_set_option(32, fold9)
-            lib.csr_set_option(27, dense)
-            net = ESRGANGenerator(in_ch, 1, 64, nb, 16)
-            net.load_state_dict(sd)
-            net = net.cuda().eval()
-            with torch.no_grad():
-                a = net(x.cuda(), elev.cuda(), mask.cuda())
-                b = net(x.cuda(), elev.cuda(), mask.cuda())          # second call: CUDA-graph replay where the plan uses one
-            assert torch.equal(a, b)
-            outs.append(a.cpu())
-            del net
-    finally:
-        lib.csr_set_option(27, 1)
-        lib.csr_set_option(31, 2)
-        lib.csr_set_option(32, 0)
-    assert torch.equal(outs[0], outs[2])                              # run-to-run deterministic
-    scale = float(outs[1].abs().max())
-    assert float((outs[0] - outs[1]).abs().max()) <= 4e-3 * max(scale, 1.0), (float((outs[0] - outs[1]).abs().max()), scale)
-
-
-def test_dense_block_regrouping_matches_plain_forward(golden_dir):
-    """Option 16: dense blocks regrouped by source (conv1 + x-parts of conv2-4 in one wide launch, partial sums through the
-    bf16 concat slots) against the plain layer-by-layer forward and the reference golden output."""
-    from climsr_b200._lib import lib
-    from oracle import synth
-    _need_experiments()
-    z = np.load(os.path.join(golden_dir, "gen_hydra_seeded.npz"))
-    in_ch, nb, gc, n, h, w = (int(v) for v in z["meta"])
-    sd = synth.make_state_dict(in_ch, 1, 64, nb, gc, seed=0, gain=float(z["gains"][1]))     # the "trained-like" weight scale
-    x, elev, mask = synth.make_inputs(n, in_ch, h, w, seed=1)
-    outs = []
-    try:
-        for regroup in (0, 1):
-            lib.csr_set_option(16, regroup)
-            outs.append(_run_generator(sd, x, elev, mask, in_ch, nb, gc))
-    finally:
-        lib.csr_set_option(16, 0)
-    want = torch.from_numpy(z["sr_trained"])
-    assert float((outs[0] - want).abs().max()) <= 1e-2 and float((outs[1] - want).abs().max()) <= 1e-2
-    assert float((outs[0] - outs[1]).abs().max()) <= 1e-2
-    assert not torch.equal(outs[0], outs[1])      # the option really changes the execution (one more bf16 rounding of p_k)
 
 
 @pytest.mark.parametrize("tag", ["small", "hydra"])

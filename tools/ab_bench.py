@@ -12,28 +12,19 @@ from climsr_b200.models import ESRGANGenerator  # noqa: E402
 VARIANTS = {
     "default": {},
     "one_mma": {7: 1},
-    "direct32": {8: 0},
     "two_acc": {5: 1},
     "slots4": {3: 4},
     "slots3": {3: 3},
     "no_pdl": {1: 0},
-    "single_group_conv5": {9: 0},
-    "single_group_all": {9: 2},
-    "two_groups": {9: 1},
-    "pair": {13: 1},
-    "pair_single_group": {13: 2},
-    "regroup": {16: 1},
     "no_eight_acc": {19: 0},
     "no_narrow_box": {17: 0},
     "no_tall": {18: 0},
-    "pair_unordered": {13: 1, 14: 0},
-    "order_all": {14: 2},
 }
 
 
 def run(name, opts, n=64, h=64, w=64, steps=20):
-    for k in (1, 3, 5, 7, 8, 9, 13, 14, 16, 17, 18, 19):
-        lib.csr_set_option(k, {1: 1, 3: 8, 8: 1, 9: 3, 14: 1, 17: 1, 18: 1, 19: 1}.get(k, 0))
+    for k in (1, 3, 5, 7, 17, 18, 19):
+        lib.csr_set_option(k, {1: 1, 3: 8, 17: 1, 18: 1, 19: 1}.get(k, 0))
     for k, v in opts.items():
         lib.csr_set_option(k, v)
     torch.manual_seed(0)

@@ -56,16 +56,8 @@ def run(name, n, h, w, cin, cout, k, in_c, act="lrelu", out_coff=0, res=False, i
 if __name__ == "__main__":
     if os.environ.get("CSR_SLOTS"):
         lib.csr_set_option(3, int(os.environ["CSR_SLOTS"]))
-    if os.environ.get("CSR_DIRECT32"):
-        lib.csr_set_option(8, 0)
     if os.environ.get("CSR_CONV5"):
-        x = None
-        for pair, cta in ((0, 0), (1, 0), (1, 1)):
-            lib.csr_set_option(13, pair)
-            lib.csr_set_option(15, cta)
-            run(f"rdb.conv5+res pair={pair} cta={cta}", 64, 64, 64, 128, 64, 3, 128, act="none", res=True)
-        lib.csr_set_option(13, 0)
-        lib.csr_set_option(15, 0)
+        run("rdb.conv5+res", 64, 64, 64, 128, 64, 3, 128, act="none", res=True)
         sys.exit(0)
     if os.environ.get("CSR_DENSE"):
         run("dense x-pass 64->64", 64, 64, 64, 64, 64, 3, 128, out_coff=64)
