@@ -299,10 +299,6 @@ struct ConvLaunch {
   CUtensorMap tmap;
   size_t w_off = 0, b_off = 0;  // offsets into the packed blob (resolved at forward time)
   size_t w2_off = 0, b2_off = 0;  // fused 1x1 successor (ConvParams::fuse2)
-  int tapsum = 0;               // 1: not a conv - conv_last finished from the tap planes HRconv's fused epilogue wrote (tap_sum_kernel)
-  const float* taps = nullptr; long tap_plane = 0; int tap_H = 0, tap_W = 0;
-  bool final_out = false;       // fp32-planar output that IS the caller's `out` tensor
-  int dense = -1;               // >= 0: this entry stands for a whole dense-block launch (CsrPlan::dense[dense]), not a conv
 };
 
 // conv1..conv4 of one dense block as one launch (rdb_tc.cu)
@@ -514,16 +510,9 @@ static int build_wgrad(int sms, int N, int H, int W, int KW, int PW, int dy_off,
   return CSR_OK;
 }
 
-// Weight (and bias) gradient of one conv layer, accumulated into dw / db (fp32 OIHW / (cout)):
-//   dw += scale * sum_p g[p][co] x[p + tap][ci]   over executed taps; see wgrad_scatter_kernel for fold / phase.
-// x: (N,H,W,x_C) bf16 (the layer's INPUT, low resolution for an up2 layer); g: gradient w.r.t. the layer's pre-activation
-// output.  For phase >= 0, g is the (2H, 2W) buffer and the phase's pixels are read through a strided view.
-struct WgradLayer {
-  int cout, cin, kh, kw, fold, up2;
-};
 constexpr int kMaxParts = 160;   // >= SM count: per-CTA partial-sum slices
-static size_t wgrad_scratch_floats(const WgradLayer& L) {
-  const int ekh = L.up2 ? 2 : L.kh, ekw = L.up2 ? 2 : (L.fold ? 1 : L.kw);
+static size_t wgrad_scratch_floats(const LayerSpec& L) {
+  const int ekh = L.up2 ? 2 : L.kh, ekw = L.up2 ? 2 : L.ekw();
   const int ld_n = (L.cout + 15) / 16 * 16;
   return (size_t)ekh * kMaxParts * ekw * 128 * ld_n;
 }
@@ -546,75 +535,22 @@ static int encode_phase_map(CUtensorMap* m, const void* base, int N, int H, int 
   return CSR_OK;
 }
 
-static int run_wgrad_layer(const WgradLayer& L, int N, int H, int W, const void* x, int x_C, int x_coff, const void* g, int g_C, int g_coff,
-                           float scale, float* dw, float* db, float* scratch, int sms, cudaStream_t s, long long* launches) {
-  const int ld_n = (L.cout + 15) / 16 * 16;
-  if (ld_n > 128) return fail(CSR_ERR_UNSUPPORTED, "wgrad: cout %d > 128", L.cout);
-  const int ecin = L.fold ? L.cin * L.kw : L.cin;
-  const int ekh = L.up2 ? 2 : L.kh, ekw = L.up2 ? 2 : (L.fold ? 1 : L.kw);
-  if (sms > kMaxParts) return fail(CSR_ERR_UNSUPPORTED, "wgrad: %d SMs > %d", sms, kMaxParts);
-  const long part_stride = (long)ekh * ekw * 128 * ld_n;
-  const int per = wgrad_taps_per_launch(ekw, ld_n);
-  for (int phase = L.up2 ? 0 : -1; phase < (L.up2 ? 4 : 0); ++phase) {
-    const int ph = L.up2 ? 1 - (phase >> 1) : L.kh / 2;
-    const int pw = L.up2 ? 1 - (phase & 1) : (L.fold ? 0 : L.kw / 2);
-    for (int ci0 = 0; ci0 < ecin; ci0 += 128) {
-      int n_parts = 0;
-      if (g_opt_wgrad_atomic) {
-        CSR_CUDA(cudaMemsetAsync(scratch, 0, (size_t)part_stride * sizeof(float), s));
-        ++*launches;
-      }
-      for (int dy = 0; dy < ekh; dy += per) {
-        WgradLaunch wl;
-        // output-gradient columns [64, 128) come through a second 64-channel box of the same buffer
-        int rc = build_wgrad(sms, N, H, W, ekw, pw, dy - ph, std::min(per, ekh - dy), x, x_C, x_coff + ci0, g, g_C, g_coff, ld_n > 64 ? g : nullptr,
-                             ld_n > 64 ? g_C : 0, ld_n > 64 ? g_coff + 64 : 0, ld_n,
-                             scratch + (size_t)dy * ekw * 128 * ld_n, part_stride, ld_n, &wl);
-        n_parts = wl.p.n_parts;
-        if (rc) return rc;
-        wl.p.atomic = g_opt_wgrad_atomic;
-        if (phase >= 0) {
-          rc = encode_phase_map(&wl.tg0, g, N, H, W, g_C, phase, wl.p.SW, wl.p.TH);
-          if (rc) return rc;
-          wl.tg1 = wl.tg0;
-        }
-        int e = launch_wgrad_tc(wl.p, wl.tx0, wl.tx1, wl.tg0, wl.tg1, sms, s);
-        if (e) return fail(CSR_ERR_CUDA, "wgrad launch failed: %s", cudaGetErrorString((cudaError_t)e));
-        ++*launches;
-      }
-      if (!g_opt_wgrad_atomic) {
-        CSR_CUDA(launch_wgrad_reduce(scratch, part_stride, n_parts, part_stride, s));
-        ++*launches;
-      }
-      CSR_CUDA(launch_wgrad_scatter(scratch, ld_n, dw, L.cout, L.cin, L.kh, L.kw, L.fold, phase, ci0, std::min(128, ecin - ci0), 0, scale, 0, s));
-      ++*launches;
-    }
-  }
-  if (db) {
-    const long npix = (long)N * H * W * (L.up2 ? 4 : 1);
-    float* dbs[1] = {db};
-    CSR_CUDA(launch_bias_grad(g, npix, g_C, g_coff, L.cout, scale, dbs, 1, s));
-    ++*launches;
-  }
-  return CSR_OK;
-}
-
 // Job mode (wgrad_tc.cuh): layers with many channels and few pixels (the discriminator: 64..512 channels on 130^2..6^2 grids).
 // ONE GEMM launch per layer - CTAs own (128-input-channel chunk, output-channel chunk, vertical-tap group) blocks of the weight
 // gradient and loop over pixel tiles - instead of one launch (whose 128-pixel K slices each end in ~200 KB of atomics) per block.
-static bool wgrad_jobs_applicable(const WgradLayer& L, int N, int H, int W, int sms) {
+static bool wgrad_jobs_applicable(const LayerSpec& L, int N, int H, int W, int sms) {
   if (L.up2 || L.fold || L.kh != L.kw || L.kw > 3) return false;
   const long tiles = (long)N * ceil_div(H, 4) * ceil_div(W, 30);
   return L.cout > 128 || (L.cin > 128 && tiles < 4L * sms);
 }
-static size_t wgrad_jobs_scratch_floats(const WgradLayer& L) {
+static size_t wgrad_jobs_scratch_floats(const LayerSpec& L) {
   const int n_cols = L.cout >= 128 ? 128 : (L.cout + 15) / 16 * 16;
   const int per = wgrad_taps_per_launch(L.kw, n_cols);
   const long jobs = (long)ceil_div(L.cin, 128) * ceil_div(L.cout, n_cols) * ceil_div(L.kh, per);
   return (size_t)jobs * per * L.kw * 128 * n_cols;
 }
-static int run_wgrad_layer_jobs(const WgradLayer& L, int N, int H, int W, const void* x, int x_C, int x_coff, const void* g, int g_C, int g_coff,
-                                float scale, float* dw, float* db, float* scratch, int sms, cudaStream_t s, long long* launches) {
+static int run_wgrad_layer_jobs(const LayerSpec& L, int N, int H, int W, const void* x, int x_C, int x_coff, const void* g, int g_C, int g_coff,
+                                float scale, float* dw, float* db, float* scratch, int sms, cudaStream_t s) {
   const int n_cols = L.cout >= 128 ? 128 : (L.cout + 15) / 16 * 16;
   if (L.cout > 128 && L.cout % 128) return fail(CSR_ERR_UNSUPPORTED, "wgrad: cout %d > 128 must be a multiple of 128", L.cout);
   const int per = wgrad_taps_per_launch(L.kw, n_cols);
@@ -634,19 +570,195 @@ static int run_wgrad_layer_jobs(const WgradLayer& L, int N, int H, int W, const 
   int e = launch_wgrad_tc(p, wl.tx0, wl.tx1, wl.tg0, wl.tg1, sms, s);
   if (e) return fail(CSR_ERR_CUDA, "wgrad (job mode) launch failed: %s", cudaGetErrorString((cudaError_t)e));
   CSR_CUDA(launch_wgrad_scatter_jobs(scratch, dw, L.cout, L.cin, L.kh, L.kw, n_cols, p.jobs_co, p.jobs_dy, per, p.job_stride, scale, s));
-  *launches += 3;
+  g_launches += 3;
   if (db) {
     const long npix = (long)N * H * W;
     if (L.cout > 128 && L.cout % 128 == 0) {
       CSR_CUDA(launch_bias_grad_wide(g, npix, g_C, g_coff, L.cout / 128, scale, db, s));
-      ++*launches;
+      ++g_launches;
     } else {
       for (int co = 0; co < L.cout; co += 128) {
         float* dbs[1] = {db + co};
         CSR_CUDA(launch_bias_grad(g, npix, g_C, g_coff + co, std::min(128, L.cout - co), scale, dbs, 1, s));
-        ++*launches;
+        ++g_launches;
       }
     }
+  }
+  return CSR_OK;
+}
+
+// ------------------------------------------------------------------------------------------- launch lists
+// One launch of a launch list: a plan's forward or backward (CsrPlan::fwd / bwd) or one layer's weight gradient.  Operands that
+// change from call to call are null here and supplied by run_ops from its Bindings; every other pointer is fixed when the op is built.
+struct Op {
+  enum Kind { kNchw, kConv, kDense, kTapSum, kTapPack, kPackSrcnn, kGcol, kScale, kWgrad, kReduce, kScatter, kBias, kBiasPlanar, kMemset } kind;
+  ConvLaunch conv;               // kConv; p.out == nullptr: the caller's `out`
+  DenseLaunch dense;             // kDense: conv1..conv4 of a dense block, or (backward) its four gated input-gradient convs (rdb_tc.cu)
+  WgradLaunch wg;                // kWgrad
+  // kScatter / kBias*: which layer's gradient (index into Bindings::dw / db), and how
+  int layer = -1, fold = 0, phase = -1, ci0 = 0, ci_n = 0, col0 = 0, ld_n = 0, n_parts = 0, nseg = 1;
+  int taps_t = 0;                         // kScatter: columns are taps of a single-output-channel layer (dw[ci][tap])
+  int cout = 0, cin = 0, kh = 0, kw = 0;  // kScatter: the forward layer's shape; kGcol: taps
+  int seg_layers[4] = {-1, -1, -1, -1};   // kBias with nseg > 1: one layer per channel segment
+  int N = 0, H = 0, W = 0;                // kNchw: the input grid (C channels); kTapSum / kTapPack / kPackSrcnn / kGcol: the HR grid
+  float scale = 1.f;
+  const void* src = nullptr; void* dst = nullptr;   // src == nullptr: x (kNchw), dL/dout (kGcol, kBiasPlanar)
+  long count = 0; int C = 0, coff = 0;
+  size_t b_off = 0;                       // kTapSum / kTapPack: conv_last's bias inside the packed blob
+};
+
+// What run_ops binds at run time.
+struct Bindings {
+  const void* packed = nullptr;           // packed weights (kConv, kDense, kTapSum, kTapPack)
+  const float* x = nullptr; const float* elev = nullptr; const float* mask = nullptr; float* out = nullptr;
+  const float* grad_out = nullptr;        // dL/dout, fp32 planar
+  float* const* dw = nullptr; float* const* db = nullptr;   // per layer
+  unsigned long long* timeline = nullptr; int timeline_cap = 0;   // csr_debug_set_timeline: launch id = op index
+};
+
+static int run_ops(const std::vector<Op>& ops, size_t lo, size_t hi, const Bindings& b, int sms, cudaStream_t s) {
+  const uint8_t* pk = reinterpret_cast<const uint8_t*>(b.packed);
+  hi = std::min(hi, ops.size());
+  for (size_t i = lo; i < hi; ++i) {
+    const Op& op = ops[i];
+    unsigned long long* tl = (long long)i < b.timeline_cap ? b.timeline : nullptr;
+    switch (op.kind) {
+      case Op::kNchw:
+        CSR_CUDA(launch_nchw_to_nhwc(b.x, op.dst, op.N, op.C, op.H, op.W, 64, 16, s));
+        break;
+      case Op::kConv: {
+        ConvParams p = op.conv.p;
+        p.wpk = pk + op.conv.w_off;
+        p.bias = reinterpret_cast<const float*>(pk + op.conv.b_off);
+        if (p.fuse2) { p.w2 = pk + op.conv.w2_off; p.b2 = p.fuse2 == 1 ? reinterpret_cast<const float*>(pk + op.conv.b2_off) : nullptr; }
+        if (!p.out) p.out = b.out;
+        if (tl) { p.timeline = tl; p.launch_id = (int)i; }
+        int e = launch_conv_tc(p, op.conv.tmap, sms, s);
+        if (e) return fail(CSR_ERR_CUDA, "conv launch %zu failed: %s", i, cudaGetErrorString((cudaError_t)e));
+        break;
+      }
+      case Op::kDense: {
+        DenseParams p = op.dense.p;
+        for (int k = 0; k < p.n_layers; ++k) {
+          p.L[k].wpk = pk + op.dense.w_off[k];
+          p.L[k].bias = reinterpret_cast<const float*>(pk + op.dense.b_off[k]);
+        }
+        if (tl) { p.timeline = tl; p.launch_id = (int)i; }
+        int e = launch_dense_block(p, op.dense.tmap, sms, s);
+        if (e) return fail(CSR_ERR_CUDA, "dense-block launch %zu failed: %s", i, cudaGetErrorString((cudaError_t)e));
+        break;
+      }
+      case Op::kTapSum:
+        CSR_CUDA(launch_tap_sum(reinterpret_cast<const float*>(op.src), op.count, reinterpret_cast<const float*>(pk + op.b_off),
+                                reinterpret_cast<float*>(op.dst), op.H, op.W, op.count, s));
+        break;
+      case Op::kTapPack:
+        CSR_CUDA(launch_tap_pack(reinterpret_cast<const float*>(op.src), op.count, reinterpret_cast<const float*>(pk + op.b_off), b.elev, b.mask,
+                                 op.dst, op.N, op.H, op.W, s));
+        break;
+      case Op::kPackSrcnn:
+        CSR_CUDA(launch_pack_srcnn_in(reinterpret_cast<const float*>(op.src), b.elev, b.mask, op.dst, op.W, op.count, op.C, s));
+        break;
+      case Op::kGcol:
+        CSR_CUDA(launch_gcol_pack(op.src ? op.src : b.grad_out, op.C, op.dst, op.coff, op.H, op.W, op.count, op.kh, op.kw, s));
+        break;
+      case Op::kScale:
+        CSR_CUDA(launch_scale_copy64(op.src, op.C, op.dst, op.coff, op.count, op.scale, s));
+        break;
+      case Op::kWgrad: {
+        int e = launch_wgrad_tc(op.wg.p, op.wg.tx0, op.wg.tx1, op.wg.tg0, op.wg.tg1, sms, s);
+        if (e) return fail(CSR_ERR_CUDA, "wgrad launch %zu failed: %s", i, cudaGetErrorString((cudaError_t)e));
+        break;
+      }
+      case Op::kReduce:
+        CSR_CUDA(launch_wgrad_reduce(reinterpret_cast<float*>(op.dst), op.count, op.n_parts, op.count, s));
+        break;
+      case Op::kScatter:
+        if (!b.dw[op.layer]) return fail(CSR_ERR_BAD_ARG, "null weight-gradient pointer for layer %d", op.layer);
+        CSR_CUDA(launch_wgrad_scatter(reinterpret_cast<const float*>(op.src), op.ld_n, b.dw[op.layer], op.cout, op.cin, op.kh, op.kw, op.fold, op.phase,
+                                      op.ci0, op.ci_n, op.col0, op.scale, op.taps_t, s));
+        break;
+      case Op::kBias: {
+        float* dbs[4] = {nullptr, nullptr, nullptr, nullptr};
+        for (int q = 0; q < op.nseg; ++q) {
+          dbs[q] = b.db[op.nseg > 1 ? op.seg_layers[q] : op.layer];
+          if (!dbs[q]) return fail(CSR_ERR_BAD_ARG, "null bias-gradient pointer for layer %d", op.layer);
+        }
+        CSR_CUDA(launch_bias_grad(op.src, op.count, op.C, op.coff, op.cout, op.scale, dbs, op.nseg, s));
+        break;
+      }
+      case Op::kBiasPlanar:
+        CSR_CUDA(launch_bias_grad_planar(op.src ? reinterpret_cast<const float*>(op.src) : b.grad_out, op.count, op.scale, b.db[op.layer], s));
+        break;
+      case Op::kMemset:
+        CSR_CUDA(cudaMemsetAsync(op.dst, 0, op.count, s));
+        break;
+    }
+    ++g_launches;
+  }
+  return CSR_OK;
+}
+
+static Op memset_op(void* dst, size_t bytes) {
+  Op op;
+  op.kind = Op::kMemset; op.dst = dst; op.count = (long)bytes;
+  return op;
+}
+
+// One weight-gradient accumulation group: the GEMM launches `wg` sum into dacc[0, floats).  Option 25 on: dacc is zeroed and the
+// GEMMs add into it with red.global.add.v4.f32; off: every CTA writes its own partial slice and a reduce kernel sums the slices.
+static void push_acc_group(std::vector<Op>& ops, std::vector<WgradLaunch>& wg, float* dacc, long floats) {
+  if (g_opt_wgrad_atomic) ops.push_back(memset_op(dacc, (size_t)floats * sizeof(float)));
+  for (WgradLaunch& wl : wg) {
+    Op op; op.kind = Op::kWgrad; op.wg = wl; op.wg.p.atomic = g_opt_wgrad_atomic;
+    ops.push_back(op);
+  }
+  if (!g_opt_wgrad_atomic) {
+    Op rd; rd.kind = Op::kReduce; rd.dst = dacc; rd.n_parts = wg.back().p.n_parts; rd.count = floats;
+    ops.push_back(rd);
+  }
+}
+
+// Weight (and, with `bias`, bias) gradient of one conv layer, accumulated into Bindings::dw / db [layer] (fp32 OIHW / (cout)):
+//   dw += scale * sum_p g[p][co] x[p + tap][ci]   over executed taps; see wgrad_scatter_kernel for fold / phase.
+// x: (N,H,W,x_C) bf16 (the layer's INPUT, low resolution for an up2 layer); g: gradient w.r.t. the layer's pre-activation
+// output.  For an up2 layer, g is the (2H, 2W) buffer and each phase's pixels are read through a strided view.
+static int emit_wgrad(std::vector<Op>& ops, const LayerSpec& L, int layer, int N, int H, int W, const void* x, int x_C, int x_coff, const void* g,
+                      int g_C, int g_coff, float scale, bool bias, float* dacc, int sms) {
+  const int ld_n = (L.cout + 15) / 16 * 16;
+  if (ld_n > 128) return fail(CSR_ERR_UNSUPPORTED, "wgrad: cout %d > 128 needs job mode (a 3x3 or 1x1 layer)", L.cout);
+  if (sms > kMaxParts) return fail(CSR_ERR_UNSUPPORTED, "wgrad: %d SMs > %d", sms, kMaxParts);
+  const int ecin = L.ecin(), ekh = L.up2 ? 2 : L.kh, ekw = L.up2 ? 2 : L.ekw();
+  const long part_stride = (long)ekh * ekw * 128 * ld_n;
+  const int per = wgrad_taps_per_launch(ekw, ld_n);
+  const void* gB = ld_n > 64 ? g : nullptr;   // output-gradient columns [64, 128) come through a second 64-channel box of the same buffer
+  for (int phase = L.up2 ? 0 : -1; phase < (L.up2 ? 4 : 0); ++phase) {
+    const int ph = L.up2 ? 1 - (phase >> 1) : L.kh / 2;
+    const int pw = L.up2 ? 1 - (phase & 1) : L.ekw() / 2;
+    for (int ci0 = 0; ci0 < ecin; ci0 += 128) {
+      std::vector<WgradLaunch> wg;
+      for (int dy = 0; dy < ekh; dy += per) {
+        WgradLaunch wl;
+        int rc = build_wgrad(sms, N, H, W, ekw, pw, dy - ph, std::min(per, ekh - dy), x, x_C, x_coff + ci0, g, g_C, g_coff, gB, gB ? g_C : 0,
+                             gB ? g_coff + 64 : 0, ld_n, dacc + (size_t)dy * ekw * 128 * ld_n, part_stride, ld_n, &wl);
+        if (rc) return rc;
+        if (phase >= 0) {
+          rc = encode_phase_map(&wl.tg0, g, N, H, W, g_C, phase, wl.p.SW, wl.p.TH);
+          if (rc) return rc;
+          wl.tg1 = wl.tg0;
+        }
+        wg.push_back(wl);
+      }
+      push_acc_group(ops, wg, dacc, part_stride);
+      Op sc; sc.kind = Op::kScatter; sc.src = dacc; sc.layer = layer; sc.fold = L.fold; sc.phase = phase; sc.ci0 = ci0; sc.ci_n = std::min(128, ecin - ci0);
+      sc.ld_n = ld_n; sc.scale = scale; sc.cout = L.cout; sc.cin = L.cin; sc.kh = L.kh; sc.kw = L.kw;
+      ops.push_back(sc);
+    }
+  }
+  if (bias) {
+    Op bo; bo.kind = Op::kBias; bo.layer = layer; bo.src = g; bo.count = (long)N * H * W * (L.up2 ? 4 : 1); bo.C = g_C; bo.coff = g_coff;
+    bo.cout = L.cout; bo.scale = scale;
+    ops.push_back(bo);
   }
   return CSR_OK;
 }
@@ -654,42 +766,22 @@ static int run_wgrad_layer_jobs(const WgradLayer& L, int N, int H, int W, const 
 // ------------------------------------------------------------------------------------------- plan
 }  // namespace csr
 
-// Backward op list entry (training plans).
-struct BwdOp {
-  enum Kind { kConv, kWgrad, kReduce, kScatter, kBias, kBiasPlanar, kScale, kMemset, kGcol, kDense } kind;
-  csr::DenseLaunch dense;        // kDense: the four gated input-gradient convs of a dense block as one dataflow launch (rdb_tc.cu)
-  csr::ConvLaunch conv;          // kConv (dgrad); w_off/b_off index the BACKWARD packed blob
-  csr::WgradLaunch wg;           // kWgrad
-  // kScatter / kBias*: which forward layer's gradient, and how
-  int layer = -1, fold = 0, phase = -1, ci0 = 0, ci_n = 0, col0 = 0, ld_n = 0, n_parts = 0, nseg = 1;
-  long dy_stride = 0;
-  int taps_t = 0;                         // kScatter: columns are taps of a single-output-channel layer (dw[ci][tap])
-  int kh = 0, kw = 0;                     // kGcol: taps; src planar fp32 (C == 0) or bf16 NHWC pitch C; dst pitch coff
-  int seg_layers[4] = {-1, -1, -1, -1};   // kBias with nseg > 1: one forward layer per channel segment
-  float scale = 1.f;
-  const void* src = nullptr; void* dst = nullptr;   // kScale (bf16 NHWC 64 ch: dst = scale*src), kBias (g buffer), kMemset
-  long count = 0; int C = 0, coff = 0, cout = 0;
-};
-
 struct CsrPlan {
   CsrNetDesc net;
   int N, h, w;
   int sms;
   int train = 0;
-  std::vector<csr::ConvLaunch> convs;   // forward, in execution order
-  std::vector<csr::DenseLaunch> dense;  // dense-block launches referenced by convs[i].dense
+  std::vector<csr::Op> fwd, bwd;        // forward (op 0: the input conversion) and, in training plans, backward launch lists
   std::vector<size_t> dbg_cat;          // csr_plan_buffer: byte offsets of the concat buffers / HR-tail activations inside the workspace
   size_t dbg_tail[5] = {0, 0, 0, 0, 0};  // m1, hrA, hrB, hrD, hrE
   int ccat = 0;
-  unsigned int* flags = nullptr;        // completion counters of the dense-block launches (zeroed at the start of every forward)
+  unsigned int* flags = nullptr;        // completion counters of the dense-block launches
   size_t flags_bytes = 0;
-  int idx_srcnn1;                       // the SRCNN x-im2col pack kernel runs right before this conv
+  bool fwd_dense = false;               // the forward has dense-block launches: it zeroes `flags` after the input conversion
   int srcnn_pitch = 64;                 // channel pitch of the SRCNN input im2col (27 -> 32 channels) and of srcnn.conv2's output (32 channels):
                                         // 32 in inference plans - the TMA loads promote to whole 128/256-byte L2 lines, so a 64-channel
                                         // pitch doubled the HBM reads of srcnn.conv1 and srcnn.conv3 -, 64 in training plans (the
                                         // weight-gradient GEMMs read 64-channel boxes)
-  void* xin; void* sin; float* tlast;
-  size_t packed_bytes;
   // CUDA-graph replay (launch-bound batches: a forward is ~180 launches, a training step ~800): the launch sequence is
   // captured once per packed-weight blob with plan-owned staging buffers for every pointer that changes between calls
   struct GraphCache { cudaGraphExec_t exec = nullptr; const void* packed = nullptr; bool failed = false; long launches = 0; int calls = 0; };
@@ -702,15 +794,21 @@ struct CsrPlan {
   float* sgout = nullptr; float* sgrad = nullptr;                                                // staged dL/dout, flat gradients
   std::vector<size_t> grad_off;          // per layer: float offset of dW, db inside the flat gradient buffer (2 entries each)
   size_t grad_floats = 0;
-  // training
-  std::vector<BwdOp> bwd;
-  std::vector<csr::LayerSpec> fwd_layers;
-  void* gout_nhwc = nullptr;            // (N,H,W,16) bf16: dL/dout in channel 0
-  float* dacc = nullptr;                // fp32 scratch of the weight-gradient GEMMs
-  size_t packed_bwd_bytes = 0;
 };
 
 namespace csr {
+
+// Float offsets of every layer's dW and db inside the flat gradient buffer (2 entries per layer); *total: its size in floats.
+static std::vector<size_t> grad_offsets(const std::vector<LayerSpec>& layers, size_t* total) {
+  std::vector<size_t> off;
+  size_t o = 0;
+  for (const LayerSpec& Ls : layers) {
+    off.push_back(o); o += align_up((size_t)Ls.cout * Ls.cin * Ls.kh * Ls.kw, 4);
+    off.push_back(o); o += align_up((size_t)Ls.cout, 4);
+  }
+  *total = o;
+  return off;
+}
 
 struct WsLayout {
   size_t xin, fea0, t0, m1, hrA, hrB, hrC, hrD, hrE, tlast, total;
@@ -748,7 +846,7 @@ static WsLayout ws_layout(const CsrNetDesc& d, int N, int h, int w, int train) {
   if (train) {
     L.sgout = take(hr * 4);
     size_t gf = 0;
-    for (const LayerSpec& Ls : layer_table(d)) gf += align_up((size_t)Ls.cout * Ls.cin * Ls.kh * Ls.kw, 4) + align_up((size_t)Ls.cout, 4);
+    grad_offsets(layer_table(d), &gf);
     L.sgrad = take(gf * 4);
     L.hrD = take(hr * 64 * 2); // srcnn.conv1 output (inference: reuses hrA)
     L.hrE = take(hr * 64 * 2); // srcnn.conv2 output (inference: reuses hrB)
@@ -769,6 +867,24 @@ static WsLayout ws_layout(const CsrNetDesc& d, int N, int h, int w, int train) {
   }
   L.total = off;
   return L;
+}
+
+// The buffers of a WsLayout inside one workspace (the training-only ones point at its start in inference plans).
+struct WsPtrs {
+  void *xin, *fea0, *t0, *m1, *hrA, *hrB, *hrC, *hrD, *hrE, *gO, *gcolB, *gT, *gP, *gQ, *gm1, *gt0, *gcat[3];
+  std::vector<void*> cat;
+  float *tlast, *dacc;
+};
+static WsPtrs ws_carve(const WsLayout& L, void* ws) {
+  uint8_t* b = reinterpret_cast<uint8_t*>(ws);
+  WsPtrs p;
+  p.xin = b + L.xin; p.fea0 = b + L.fea0; p.t0 = b + L.t0; p.m1 = b + L.m1; p.hrA = b + L.hrA; p.hrB = b + L.hrB; p.hrC = b + L.hrC;
+  p.hrD = b + L.hrD; p.hrE = b + L.hrE; p.gO = b + L.gO; p.gcolB = b + L.gcolB; p.gT = b + L.gT; p.gP = b + L.gP; p.gQ = b + L.gQ;
+  p.gm1 = b + L.gm1; p.gt0 = b + L.gt0;
+  for (int i = 0; i < 3; ++i) p.gcat[i] = b + L.gcat[i];
+  for (size_t o : L.cat) p.cat.push_back(b + o);
+  p.tlast = reinterpret_cast<float*>(b + L.tlast); p.dacc = reinterpret_cast<float*>(b + L.dacc);
+  return p;
 }
 
 static ConvIO io_of(const void* in, int in_C, void* out, int out_C, int out_coff, int act) {
@@ -820,53 +936,50 @@ static int build_dense(const std::vector<PackLayer>& packs, int li, int N, int H
   return encode_act_map(&dl->tmap, buf, N, H, W, C, p.SW, 2 * p.TH + 2, 64);
 }
 
-static int plan_build(CsrPlan* P, void* ws) {
+static bool dense_enabled(const CsrNetDesc& d) { return g_opt_dense && d.gc == 16 && !g_opt_force_generic; }
+
+// The four convs of dense block j (concat buffer `buf`, pack layers li..li+3) as ONE persistent launch with tile-level
+// dependencies between the layers: conv1..conv4 of the forward, or with `gate` the backward's four gated input-gradient convs.
+// False: run them as one launch per layer (option 27 off, no tile shape fits, or fewer than option 31's windows per SM).
+static bool try_dense(const CsrPlan* P, const std::vector<PackLayer>& packs, int li, int j, void* buf, const void* gate, Op* op) {
+  const CsrNetDesc& d = P->net;
+  if (!dense_enabled(d)) return false;
+  const size_t per_block = (size_t)kDenseMaxLayers * P->N * ceil_div(P->h, 8) * ceil_div(P->w, 14);   // ws_layout's flags
+  op->kind = Op::kDense;
+  return build_dense(packs, li, P->N, P->h, P->w, buf, P->ccat, d.nf, d.gc, P->flags + (size_t)j * per_block, &op->dense, gate, gate ? P->ccat : 0) ==
+             CSR_OK &&
+         (size_t)op->dense.p.num_tiles * kDenseMaxLayers <= per_block && op->dense.p.num_tiles >= g_opt_dense_min * P->sms;
+}
+
+// The forward launch list, in launch order.
+static int plan_build(CsrPlan* P, const WsPtrs& ws, const std::vector<LayerSpec>& layers) {
   const CsrNetDesc& d = P->net;
   const int N = P->N, h = P->h, w = P->w;
-  const WsLayout L = ws_layout(d, N, h, w, P->train);
-  uint8_t* base = reinterpret_cast<uint8_t*>(ws);
-  void* xin = base + L.xin; void* fea0 = base + L.fea0;
-  auto cat = [&](int j) -> void* { return base + L.cat[P->train ? j : j % 3]; };
-  void* t0 = base + L.t0; void* m1 = base + L.m1; void* hrA = base + L.hrA; void* hrB = base + L.hrB; void* hrC = base + L.hrC;
-  void* hrD = base + L.hrD; void* hrE = base + L.hrE;
-  P->xin = xin; P->sin = hrC; P->tlast = reinterpret_cast<float*>(base + L.tlast);
-  P->sx = reinterpret_cast<float*>(base + L.sx); P->selev = reinterpret_cast<float*>(base + L.selev);
-  P->smask = reinterpret_cast<float*>(base + L.smask); P->sout = reinterpret_cast<float*>(base + L.sout);
-  P->flags = reinterpret_cast<unsigned int*>(base + L.flags); P->flags_bytes = L.flags_bytes;
-  P->dbg_cat = L.cat; P->ccat = L.ccat;
-  P->dbg_tail[0] = L.m1; P->dbg_tail[1] = L.hrA; P->dbg_tail[2] = L.hrB; P->dbg_tail[3] = L.hrD; P->dbg_tail[4] = L.hrE;
-  const std::vector<LayerSpec> layers = layer_table(d);
-  P->fwd_layers = layers;
-  {
-    size_t off = 0;
-    for (const LayerSpec& Ls : layers) {
-      P->grad_off.push_back(off); off += align_up((size_t)Ls.cout * Ls.cin * Ls.kh * Ls.kw, 4);
-      P->grad_off.push_back(off); off += align_up((size_t)Ls.cout, 4);
-    }
-    P->grad_floats = off;
-  }
-  if (P->train) { P->sgout = reinterpret_cast<float*>(base + L.sgout); P->sgrad = reinterpret_cast<float*>(base + L.sgrad); }
+  auto cat = [&](int j) -> void* { return ws.cat[P->train ? j : j % 3]; };
   size_t total = 0;
-  const std::vector<LayerSpec> exec = fwd_exec_table(d, layers);
-  const std::vector<PackLayer> packs = pack_layout(exec, &total);
-  P->packed_bytes = total;
-  const int C = L.ccat, nf = d.nf, gc = d.gc;
+  const std::vector<PackLayer> packs = pack_layout(fwd_exec_table(d, layers), &total);
+  const int C = P->ccat, nf = d.nf, gc = d.gc;
+  std::vector<Op>& ops = P->fwd;
+  {
+    Op op; op.kind = Op::kNchw; op.dst = ws.xin; op.N = N; op.C = d.in_channels; op.H = h; op.W = w;
+    ops.push_back(op);
+  }
   int li = 0;
   auto add = [&](int H, int W, const ConvIO& io, bool advance = true) -> int {
     const PackLayer& pl = packs[li];
-    const size_t first = P->convs.size();
+    const size_t first = ops.size();
     for (const PackPart& pp : pl.parts) {
-      ConvLaunch cl;
-      int rc = build_conv(pl, pp, N, H, W, io, &cl);
+      Op op; op.kind = Op::kConv;
+      int rc = build_conv(pl, pp, N, H, W, io, &op.conv);
       if (rc) return rc;
-      P->convs.push_back(cl);
+      ops.push_back(op);
     }
     // nearest-x2 + conv = four sub-pixel phases (a, b) in phase order 2a + b: the two phases with the same b share the kernel
     // specialisation (PW = 1 - b) and go out as ONE launch with a on gridDim.y (weights / bias at a constant stride, PH = 1 - a,
     // output rows 2y + a): two launches instead of four, each over twice the tiles
     if (g_opt_merge_phases && pl.parts.size() == 4 && pl.parts[0].phase == 0 && pl.parts[3].phase == 3 && !io.r1 && !io.r2 && !io.gate) {
-      ConvLaunch a0 = P->convs[first], a1 = P->convs[first + 1];
-      const ConvLaunch& c2 = P->convs[first + 2]; const ConvLaunch& c3 = P->convs[first + 3];
+      ConvLaunch& a0 = ops[first].conv; ConvLaunch& a1 = ops[first + 1].conv;
+      const ConvLaunch& c2 = ops[first + 2].conv; const ConvLaunch& c3 = ops[first + 3].conv;
       auto pair_ok = [](const ConvLaunch& u, const ConvLaunch& v) {
         return u.p.PW == v.p.PW && u.p.KW == v.p.KW && u.p.KH == v.p.KH && u.p.num_tiles == v.p.num_tiles && u.p.SW == v.p.SW && u.p.TH == v.p.TH &&
                u.p.n_slots == v.p.n_slots && u.p.w_bytes == v.p.w_bytes && u.p.early == v.p.early && u.p.n_acc == v.p.n_acc &&
@@ -883,9 +996,7 @@ static int plan_build(CsrPlan* P, void* ws) {
         };
         merge2(a0, c2);
         merge2(a1, c3);
-        P->convs.resize(first);
-        P->convs.push_back(a0);
-        P->convs.push_back(a1);
+        ops.resize(first + 2);
       }
     }
     if (advance) ++li;
@@ -894,18 +1005,19 @@ static int plan_build(CsrPlan* P, void* ws) {
   int rc;
   // conv_first (esrgan.py:90) has two consumers: the first RRDB (reads x from its concat buffer) and the trunk skip-add
   // 33 layers later.  The layer is tiny (K = 16), so it is simply run into both places.
-  rc = add(h, w, io_of(xin, 64, cat(0), C, 0, CSR_ACT_NONE), false);
+  const size_t c0 = ops.size();
+  rc = add(h, w, io_of(ws.xin, 64, cat(0), C, 0, CSR_ACT_NONE), false);
   if (rc) return rc;
-  if (g_opt_merge_phases && P->convs.size() == 1 && P->convs[0].p.early && P->convs[0].p.store_mode == kStoreStaged && P->convs[0].p.KW == 3 &&
-      P->convs[0].p.act == 0 && !P->convs[0].p.r1) {
+  ConvParams& f = ops[c0].conv.p;
+  if (g_opt_merge_phases && ops.size() == c0 + 1 && f.early && f.store_mode == kStoreStaged && f.KW == 3 && f.act == 0 && !f.r1) {
     // ... with the early-release epilogue the staged tile is simply stored twice (conv_tc.cu, out_dup)
-    P->convs[0].p.out_dup = fea0; P->convs[0].p.dup_C = 64; P->convs[0].p.dup_coff = 0;
+    f.out_dup = ws.fea0; f.dup_C = 64; f.dup_coff = 0;
     ++li;
   } else {
-    P->convs.clear();
-    rc = add(h, w, io_of(xin, 64, fea0, 64, 0, CSR_ACT_NONE), false);
+    ops.resize(c0);
+    rc = add(h, w, io_of(ws.xin, 64, ws.fea0, 64, 0, CSR_ACT_NONE), false);
     if (rc) return rc;
-    rc = add(h, w, io_of(xin, 64, cat(0), C, 0, CSR_ACT_NONE));
+    rc = add(h, w, io_of(ws.xin, 64, cat(0), C, 0, CSR_ACT_NONE));
     if (rc) return rc;
   }
   for (int i = 0; i < d.nb; ++i) {
@@ -916,28 +1028,18 @@ static int plan_build(CsrPlan* P, void* ws) {
       const int j = 3 * i + r;
       void* src = cat(j);
       void* dst = P->train ? cat(j + 1) : (r < 2 ? cat(j + 1) : cat(3 * i));
-      if (g_opt_dense && gc == 16 && !g_opt_force_generic) {
-        // conv1..conv4 as ONE persistent launch with tile-level dependencies between the layers (rdb_tc.cu)
-        DenseLaunch dl;
-        const size_t per_block = (size_t)kDenseMaxLayers * N * ceil_div(h, 8) * ceil_div(w, 14);
-        unsigned int* fl = P->flags + (size_t)j * per_block;
-        if (build_dense(packs, li, N, h, w, src, C, nf, gc, fl, &dl) == CSR_OK && (size_t)dl.p.num_tiles * kDenseMaxLayers <= per_block &&
-            dl.p.num_tiles >= g_opt_dense_min * P->sms) {
-          ConvLaunch stub;
-          memset(&stub.p, 0, sizeof(stub.p));
-          stub.dense = (int)P->dense.size();
-          P->dense.push_back(dl);
-          P->convs.push_back(stub);
-          li += 4;
-          goto conv5;
+      Op dop;
+      if (try_dense(P, packs, li, j, src, nullptr, &dop)) {
+        ops.push_back(dop);
+        P->fwd_dense = true;
+        li += 4;
+      } else {
+        for (int k = 1; k <= 4; ++k) {
+          // x_k = lrelu(conv_k(cat(x, x1..x_{k-1})))  written into its concat slice  (esrgan.py:33-36)
+          rc = add(h, w, io_of(src, C, src, C, nf + (k - 1) * gc, CSR_ACT_LRELU02));
+          if (rc) return rc;
         }
       }
-      for (int k = 1; k <= 4; ++k) {
-        // x_k = lrelu(conv_k(cat(x, x1..x_{k-1})))  written into its concat slice  (esrgan.py:33-36)
-        rc = add(h, w, io_of(src, C, src, C, nf + (k - 1) * gc, CSR_ACT_LRELU02));
-        if (rc) return rc;
-      }
-    conv5:
       // x5*0.2 + x  (esrgan.py:37-38); RDB3 additionally applies the RRDB residual out*0.2 + x_rrdb (esrgan.py:54)
       ConvIO io = io_of(src, C, dst, C, 0, CSR_ACT_NONE);
       io.r1 = src; io.r1_C = C; io.s1 = 0.2f;
@@ -949,30 +1051,33 @@ static int plan_build(CsrPlan* P, void* ws) {
   void* trunk_out = P->train ? cat(3 * d.nb) : cat(0);
   // trunk_conv + skip (esrgan.py:91-92)
   {
-    ConvIO io = io_of(trunk_out, C, t0, 64, 0, CSR_ACT_NONE);
-    io.r1 = fea0; io.r1_C = 64; io.s1 = 1.f;
+    ConvIO io = io_of(trunk_out, C, ws.t0, 64, 0, CSR_ACT_NONE);
+    io.r1 = ws.fea0; io.r1_C = 64; io.s1 = 1.f;
     rc = add(h, w, io);
     if (rc) return rc;
   }
   // lrelu(upconv1(nearest x2)) and lrelu(upconv2(nearest x2)) (esrgan.py:94,97): four sub-pixel phases each
-  rc = add(h, w, io_of(t0, 64, m1, 64, 0, CSR_ACT_LRELU02));
+  rc = add(h, w, io_of(ws.t0, 64, ws.m1, 64, 0, CSR_ACT_LRELU02));
   if (rc) return rc;
-  rc = add(2 * h, 2 * w, io_of(m1, 64, hrA, 64, 0, CSR_ACT_LRELU02));
+  rc = add(2 * h, 2 * w, io_of(ws.m1, 64, ws.hrA, 64, 0, CSR_ACT_LRELU02));
   if (rc) return rc;
   const int H = 4 * h, W = 4 * w;
-  rc = add(H, W, io_of(hrA, 64, hrB, 64, 0, CSR_ACT_LRELU02));  // HRconv (esrgan.py:99)
+  rc = add(H, W, io_of(ws.hrA, 64, ws.hrB, 64, 0, CSR_ACT_LRELU02));  // HRconv (esrgan.py:99)
   if (rc) return rc;
   // conv_last -> fp32 planar temp; then [out, elev, mask] is packed (with srcnn.conv1's horizontal window) into hrC
+  P->srcnn_pitch = P->train ? 64 : 32;
+  const int sp = P->srcnn_pitch;
+  bool tap_pack = false;
   {
     // Inference: HRconv's 64-channel output never reaches memory - its fused epilogue writes the nine tap planes of conv_last (second
     // MMA over the staged tile, conv_tc.cu FUSE_T = 2) into hrB and tap_sum_kernel adds the shifted taps + bias into tlast.
-    ConvLaunch& hc = P->convs.back();
+    ConvLaunch& hc = ops.back().conv;
     const PackLayer& pt = packs.back();                          // "conv_last.taps" (fwd_exec_table)
     bool fused = false;
     if ((g_opt_fuse_tail & 2) && !P->train && hc.p.early && hc.p.KW == 3 && hc.p.PW == 1 && hc.p.npad == 64 && hc.p.stage_row_bytes == 128 &&
         pt.parts.size() == 1 && pt.parts[0].npad == 16 && pt.parts[0].w_bytes == 2048 && pt.cin_pad == 64) {
       ConvParams q = hc.p;
-      q.fuse2 = 2; q.w2_bytes = pt.parts[0].w_bytes; q.n2 = 9; q.out2 = hrB; q.out2_plane = (long long)N * H * W;
+      q.fuse2 = 2; q.w2_bytes = pt.parts[0].w_bytes; q.n2 = 9; q.out2 = ws.hrB; q.out2_plane = (long long)N * H * W;
       if (q.hyb) q.n_acc = 2;                                  // hybrid fold: 2 x 128 + 16 columns (four accumulators would fill TMEM)
       int cols = 32;
       while (cols < q.n_acc * (q.hyb ? 2 : q.KW) * q.npad + 16) cols *= 2;
@@ -980,37 +1085,39 @@ static int plan_build(CsrPlan* P, void* ws) {
       if (cols <= 512 && conv_smem_bytes(q) <= (size_t)kSmemLimit && (size_t)9 * N * H * W * sizeof(float) <= (size_t)N * H * W * 64 * 2) {
         hc.p = q;
         hc.w2_off = pt.parts[0].w_off;
-        ConvLaunch ts;
-        memset(&ts.p, 0, sizeof(ts.p));
-        ts.tapsum = 1; ts.taps = reinterpret_cast<const float*>(hrB); ts.tap_plane = (long)N * H * W; ts.tap_H = H; ts.tap_W = W;
-        ts.b_off = packs[li].parts[0].b_off;                      // conv_last's own bias
-        P->convs.push_back(ts);
+        // option 36: the tap sum and the SRCNN input im2col in one pass (tap_pack_kernel)
+        tap_pack = g_opt_tap_pack != 0;
+        Op ts; ts.kind = tap_pack ? Op::kTapPack : Op::kTapSum;
+        ts.src = ws.hrB; ts.dst = tap_pack ? ws.hrC : (void*)ws.tlast; ts.count = (long)N * H * W; ts.N = N; ts.H = H; ts.W = W;
+        ts.b_off = packs[li].parts[0].b_off;                     // conv_last's own bias
+        ops.push_back(ts);
         ++li;                                                    // conv_last has no conv launch
         fused = true;
       }
     }
     if (!fused) {
-      ConvIO io = io_of(hrB, 64, P->tlast, 1, 0, CSR_ACT_NONE);
+      ConvIO io = io_of(ws.hrB, 64, ws.tlast, 1, 0, CSR_ACT_NONE);
       io.out_kind = kOutF32Planar;
       rc = add(H, W, io);
       if (rc) return rc;
     }
   }
-  P->idx_srcnn1 = (int)P->convs.size();
-  P->srcnn_pitch = P->train ? 64 : 32;
-  const int sp = P->srcnn_pitch;
-  rc = add(H, W, io_of(hrC, sp, hrD, 64, 0, CSR_ACT_RELU));     // srcnn.conv1 (9x1 folded)
+  if (!tap_pack) {
+    Op op; op.kind = Op::kPackSrcnn; op.src = ws.tlast; op.dst = ws.hrC; op.W = W; op.count = (long)N * H * W; op.C = sp;
+    ops.push_back(op);
+  }
+  rc = add(H, W, io_of(ws.hrC, sp, ws.hrD, 64, 0, CSR_ACT_RELU));     // srcnn.conv1 (9x1 folded)
   if (rc) return rc;
   {
     // Inference: srcnn.conv2 (1x1, 64 -> 32, ReLU) runs inside srcnn.conv1's epilogue as a second MMA over the staged tile; the
     // 64-channel HR map is never written (conv_tc.cu FUSE_T).  Training plans keep both layers (the backward needs the intermediate).
-    ConvLaunch& c1 = P->convs.back();
+    ConvLaunch& c1 = ops.back().conv;
     const PackLayer& p2 = packs[li];
     bool fused = false;
     if ((g_opt_fuse_tail & 1) && !P->train && c1.p.early && c1.p.KW == 1 && c1.p.PW == 0 && c1.p.npad == 64 && c1.p.stage_row_bytes == 128 &&
         p2.parts.size() == 1 && p2.parts[0].npad == 32 && p2.parts[0].w_bytes == 4096 && p2.cin_pad == 64 && sp % 8 == 0) {
       ConvParams q = c1.p;
-      q.fuse2 = 1; q.w2_bytes = p2.parts[0].w_bytes; q.n2 = 32; q.out2 = hrE; q.out2_C = sp; q.out2_coff = 0;
+      q.fuse2 = 1; q.w2_bytes = p2.parts[0].w_bytes; q.n2 = 32; q.out2 = ws.hrE; q.out2_C = sp; q.out2_coff = 0;
       int cols = 32;
       while (cols < q.n_acc * q.KW * q.npad + 32) cols *= 2;
       q.tmem_cols = cols;
@@ -1022,18 +1129,13 @@ static int plan_build(CsrPlan* P, void* ws) {
       }
     }
     if (!fused) {
-      rc = add(H, W, io_of(hrD, 64, hrE, sp, 0, CSR_ACT_RELU));   // srcnn.conv2 1x1
+      rc = add(H, W, io_of(ws.hrD, 64, ws.hrE, sp, 0, CSR_ACT_RELU));   // srcnn.conv2 1x1
       if (rc) return rc;
     }
   }
-  {
-    ConvIO io = io_of(hrE, sp, nullptr, 1, 0, CSR_ACT_NONE);    // srcnn.conv3 5x5 -> the caller's output tensor
-    io.out_kind = kOutF32Planar;
-    rc = add(H, W, io);
-    if (rc) return rc;
-    P->convs.back().final_out = true;
-  }
-  return rc;
+  ConvIO io = io_of(ws.hrE, sp, nullptr, 1, 0, CSR_ACT_NONE);    // srcnn.conv3 5x5 -> the caller's output tensor (bound by run_ops)
+  io.out_kind = kOutF32Planar;
+  return add(H, W, io);
 }
 
 // ------------------------------------------------------------------------------------------- backward plan
@@ -1088,54 +1190,25 @@ static std::vector<LayerSpec> bwd_layer_table(const CsrNetDesc& d, const std::ve
   return v;
 }
 
-// Weight-gradient accumulation through L2 vector atomics (option 25, default on): each group [wgrad launches..., reduce]
-// becomes [memset of part 0, wgrad launches (atomic)...] - the reduce kernel and the per-CTA partial slices disappear.
-static void wgrad_ops_to_atomic(std::vector<BwdOp>& ops, float* dacc) {
-  if (!g_opt_wgrad_atomic) return;
-  std::vector<BwdOp> out;
-  out.reserve(ops.size());
-  for (size_t i = 0; i < ops.size(); ++i) {
-    if (ops[i].kind != BwdOp::kReduce) { out.push_back(ops[i]); continue; }
-    size_t first = out.size();
-    while (first > 0 && out[first - 1].kind == BwdOp::kWgrad) --first;
-    for (size_t j = first; j < out.size(); ++j) out[j].wg.p.atomic = 1;
-    BwdOp ms; ms.kind = BwdOp::kMemset; ms.dst = dacc; ms.count = ops[i].count * (long)sizeof(float);
-    out.insert(out.begin() + first, ms);
-  }
-  ops.swap(out);
-}
-
-static int bwd_build(CsrPlan* P, void* ws) {
+static int bwd_build(CsrPlan* P, const WsPtrs& ws, const std::vector<LayerSpec>& F) {
   const CsrNetDesc& d = P->net;
   const int N = P->N, h = P->h, w = P->w, H = 4 * h, W = 4 * w;
-  const WsLayout L = ws_layout(d, N, h, w, 1);
-  uint8_t* base = reinterpret_cast<uint8_t*>(ws);
-  auto cat = [&](int j) -> void* { return base + L.cat[j]; };
-  void* xin = base + L.xin;
-  void* t0 = base + L.t0; void* m1 = base + L.m1; void* hrA = base + L.hrA; void* hrB = base + L.hrB; void* hrC = base + L.hrC;
-  void* hrD = base + L.hrD; void* hrE = base + L.hrE;
-  void* gO = base + L.gO; void* gcolB = base + L.gcolB; void* gT = base + L.gT; void* gP = base + L.gP; void* gQ = base + L.gQ; void* gm1 = base + L.gm1;
-  void* gt0 = base + L.gt0;
-  void* gcat[3] = {base + L.gcat[0], base + L.gcat[1], base + L.gcat[2]};
-  float* dacc = reinterpret_cast<float*>(base + L.dacc);
-  P->gout_nhwc = gO; P->dacc = dacc;
-  const std::vector<LayerSpec>& F = P->fwd_layers;
+  float* dacc = ws.dacc;
   const std::vector<LayerSpec> B = bwd_layer_table(d, F);
   size_t total = 0;
   const std::vector<PackLayer> packs = pack_layout(B, &total);
-  P->packed_bwd_bytes = total;
-  const int C = L.ccat, nf = d.nf, gc = d.gc;
+  const int C = P->ccat, nf = d.nf, gc = d.gc;
   const int base_tail = 1 + d.nb * 15;
   int bi = 0;                                             // next backward layer
-  std::vector<BwdOp>& ops = P->bwd;
+  std::vector<Op>& ops = P->bwd;
 
-  auto dgrad = [&](int Hh, int Ww, const ConvIO& io, const void* phase_src = nullptr, int src_H = 0, int src_W = 0) -> int {
+  // the parts of backward layer bi
+  auto dgrad = [&](int Hh, int Ww, const ConvIO& io, const void* phase_src = nullptr) -> int {
     const PackLayer& pl = packs[bi];
     const bool up2 = B[bi].up2 != 0;
-    int launch = 0;
     for (const PackPart& pp : pl.parts) {
-      BwdOp op;
-      op.kind = BwdOp::kConv;
+      Op op;
+      op.kind = Op::kConv;
       ConvIO io2 = io;
       if (up2) {
         // phases accumulate into the same low-resolution gradient: first writes, later ones add, the last one gates
@@ -1152,53 +1225,12 @@ static int bwd_build(CsrPlan* P, void* ws) {
         if (rc) return rc;
       }
       ops.push_back(op);
-      ++launch;
     }
     ++bi;
     return CSR_OK;
   };
-  auto wgrad_plain = [&](int layer, int Hh, int Ww, const void* x, int x_C, int x_coff, const void* g, int g_C, int g_coff, float scale,
-                         bool planar_bias = false, const float* gplanar = nullptr) -> int {
-    const LayerSpec& Ls = F[layer];
-    const int ld_n = (Ls.cout + 15) / 16 * 16;
-    const int ecin = Ls.fold ? Ls.cin * Ls.kw : Ls.cin;
-    const int ekh = Ls.up2 ? 2 : Ls.kh, ekw = Ls.up2 ? 2 : (Ls.fold ? 1 : Ls.kw);
-    for (int phase = Ls.up2 ? 0 : -1; phase < (Ls.up2 ? 4 : 0); ++phase) {
-      const int ph = Ls.up2 ? 1 - (phase >> 1) : Ls.kh / 2;
-      const int pw = Ls.up2 ? 1 - (phase & 1) : (Ls.fold ? 0 : Ls.kw / 2);
-      const long part_stride = (long)ekh * ekw * 128 * ld_n;
-      const int per = wgrad_taps_per_launch(ekw, ld_n);
-      for (int ci0 = 0; ci0 < ecin; ci0 += 128) {
-        int n_parts = 0;
-        for (int dy = 0; dy < ekh; dy += per) {
-          BwdOp op; op.kind = BwdOp::kWgrad;
-          int rc = build_wgrad(P->sms, N, Hh, Ww, ekw, pw, dy - ph, std::min(per, ekh - dy), x, x_C, x_coff + ci0, g, g_C, g_coff, nullptr, 0, 0,
-                               ld_n, dacc + (size_t)dy * ekw * 128 * ld_n, part_stride, ld_n, &op.wg);
-          if (rc) return rc;
-          n_parts = op.wg.p.n_parts;
-          if (phase >= 0) {
-            rc = encode_phase_map(&op.wg.tg0, g, N, Hh, Ww, g_C, phase, op.wg.p.SW, op.wg.p.TH);
-            if (rc) return rc;
-            op.wg.tg1 = op.wg.tg0;
-          }
-          ops.push_back(op);
-        }
-        BwdOp rd; rd.kind = BwdOp::kReduce; rd.n_parts = n_parts; rd.dy_stride = part_stride; rd.count = part_stride;
-        ops.push_back(rd);
-        BwdOp sc; sc.kind = BwdOp::kScatter; sc.layer = layer; sc.fold = Ls.fold; sc.phase = phase; sc.ci0 = ci0;
-        sc.ci_n = std::min(128, ecin - ci0); sc.col0 = 0; sc.ld_n = ld_n; sc.scale = scale;
-        ops.push_back(sc);
-      }
-    }
-    BwdOp bo;
-    if (planar_bias) {
-      bo.kind = BwdOp::kBiasPlanar; bo.layer = layer; bo.src = gplanar; bo.count = (long)N * H * W; bo.scale = scale;
-    } else {
-      bo.kind = BwdOp::kBias; bo.layer = layer; bo.src = g; bo.count = (long)N * Hh * Ww * (Ls.up2 ? 4 : 1); bo.C = g_C; bo.coff = g_coff;
-      bo.cout = Ls.cout; bo.scale = scale;
-    }
-    ops.push_back(bo);
-    return CSR_OK;
+  auto wgrad_plain = [&](int layer, int Hh, int Ww, const void* x, int x_C, int x_coff, const void* g, int g_C, int g_coff, float scale) -> int {
+    return emit_wgrad(ops, F[layer], layer, N, Hh, Ww, x, x_C, x_coff, g, g_C, g_coff, scale, true, dacc, P->sms);
   };
   // weight gradient of a single-output-channel layer as ONE 1x1 GEMM: x (cin channels) against the im2col of its output
   // gradient (taps as columns); the scatter writes dw[ci][tap]
@@ -1208,14 +1240,12 @@ static int bwd_build(CsrPlan* P, void* ws) {
     const int ld_n = (ntaps + 15) / 16 * 16;
     const long part_stride = (long)128 * ld_n;
     for (int ci0 = 0; ci0 < Ls.cin; ci0 += 128) {
-      BwdOp op; op.kind = BwdOp::kWgrad;
-      int rc = build_wgrad(P->sms, N, Hh, Ww, 1, 0, 0, 1, x, x_C, ci0, gcol, gcol_C, 0, nullptr, 0, 0, ld_n, dacc, part_stride, ld_n, &op.wg);
+      std::vector<WgradLaunch> wg(1);
+      int rc = build_wgrad(P->sms, N, Hh, Ww, 1, 0, 0, 1, x, x_C, ci0, gcol, gcol_C, 0, nullptr, 0, 0, ld_n, dacc, part_stride, ld_n, &wg[0]);
       if (rc) return rc;
-      ops.push_back(op);
-      BwdOp rd; rd.kind = BwdOp::kReduce; rd.n_parts = op.wg.p.n_parts; rd.dy_stride = part_stride; rd.count = part_stride;
-      ops.push_back(rd);
-      BwdOp sc; sc.kind = BwdOp::kScatter; sc.layer = layer; sc.ci0 = ci0; sc.ci_n = std::min(128, Ls.cin - ci0); sc.col0 = 0; sc.ld_n = ld_n;
-      sc.scale = 1.f; sc.taps_t = ntaps;
+      push_acc_group(ops, wg, dacc, part_stride);
+      Op sc; sc.kind = Op::kScatter; sc.src = dacc; sc.layer = layer; sc.ci0 = ci0; sc.ci_n = std::min(128, Ls.cin - ci0); sc.ld_n = ld_n;
+      sc.taps_t = ntaps; sc.cout = ntaps; sc.cin = Ls.cin; sc.kh = sc.kw = 1;
       ops.push_back(sc);
     }
     return CSR_OK;
@@ -1226,53 +1256,55 @@ static int bwd_build(CsrPlan* P, void* ws) {
   };
 
   int rc;
-  if (g_opt_dense && gc == 16 && !g_opt_force_generic) {
-    // completion counters of the dense-block launches of the backward (the forward zeroed and used the same region)
-    BwdOp ms; ms.kind = BwdOp::kMemset; ms.dst = P->flags; ms.count = (long)P->flags_bytes;
-    ops.push_back(ms);
-  }
+  // completion counters of the dense-block launches of the backward (the forward zeroed and used the same region)
+  if (dense_enabled(d)) ops.push_back(memset_op(P->flags, P->flags_bytes));
   // ---- SRCNN tail (srcnn.py:13-18) -------------------------------------------------------------------------------
   // srcnn.conv3 (32 -> 1, 5x5): im2col of dL/dout (25 taps as channels) makes both of its gradients 1x1 GEMMs
-  { BwdOp op; op.kind = BwdOp::kGcol; op.src = nullptr; op.C = 0; op.dst = gO; op.coff = 32; op.kh = 5; op.kw = 5; ops.push_back(op); }
-  rc = wgrad_cols(base_tail + 7, H, W, hrE, 64, gO, 32);
+  auto gcol = [&](const void* src, int src_C, void* dst, int dst_C, int k) {
+    Op op; op.kind = Op::kGcol; op.src = src; op.C = src_C; op.dst = dst; op.coff = dst_C; op.kh = op.kw = k;
+    op.H = H; op.W = W; op.count = (long)N * H * W;
+    ops.push_back(op);
+  };
+  gcol(nullptr, 0, ws.gO, 32, 5);
+  rc = wgrad_cols(base_tail + 7, H, W, ws.hrE, 64, ws.gO, 32);
   if (rc) return rc;
-  { BwdOp bo; bo.kind = BwdOp::kBiasPlanar; bo.layer = base_tail + 7; bo.src = nullptr; bo.count = (long)N * H * W; bo.scale = 1.f; ops.push_back(bo); }
-  rc = dgrad(H, W, gated(io_of(gO, 32, gP, 64, 0, CSR_ACT_NONE), hrE, 64, 0, 0, 0.f));  // -> d/d relu(conv2) * relu'
+  { Op bo; bo.kind = Op::kBiasPlanar; bo.layer = base_tail + 7; bo.count = (long)N * H * W; ops.push_back(bo); }
+  rc = dgrad(H, W, gated(io_of(ws.gO, 32, ws.gP, 64, 0, CSR_ACT_NONE), ws.hrE, 64, 0, 0, 0.f));  // -> d/d relu(conv2) * relu'
   if (rc) return rc;
-  rc = wgrad_plain(base_tail + 6, H, W, hrD, 64, 0, gP, 64, 0, 1.f);                  // srcnn.conv2
+  rc = wgrad_plain(base_tail + 6, H, W, ws.hrD, 64, 0, ws.gP, 64, 0, 1.f);                  // srcnn.conv2
   if (rc) return rc;
-  rc = dgrad(H, W, gated(io_of(gP, 64, gQ, 64, 0, CSR_ACT_NONE), hrD, 64, 0, 0, 0.f));
+  rc = dgrad(H, W, gated(io_of(ws.gP, 64, ws.gQ, 64, 0, CSR_ACT_NONE), ws.hrD, 64, 0, 0, 0.f));
   if (rc) return rc;
-  rc = wgrad_plain(base_tail + 5, H, W, hrC, 64, 0, gQ, 64, 0, 1.f);                  // srcnn.conv1 (folded 9x1 over 27 ch)
+  rc = wgrad_plain(base_tail + 5, H, W, ws.hrC, 64, 0, ws.gQ, 64, 0, 1.f);                  // srcnn.conv1 (folded 9x1 over 27 ch)
   if (rc) return rc;
-  rc = dgrad(H, W, io_of(gQ, 64, gT, 16, 0, CSR_ACT_NONE));                           // d/d[out, elev, mask]; channel 0 is used
+  rc = dgrad(H, W, io_of(ws.gQ, 64, ws.gT, 16, 0, CSR_ACT_NONE));                           // d/d[out, elev, mask]; channel 0 is used
   if (rc) return rc;
   // ---- conv_last, HRconv (esrgan.py:99) ----------------------------------------------------------------------------
-  { BwdOp op; op.kind = BwdOp::kGcol; op.src = gT; op.C = 16; op.dst = gcolB; op.coff = 16; op.kh = 3; op.kw = 3; ops.push_back(op); }
-  rc = wgrad_cols(base_tail + 4, H, W, hrB, 64, gcolB, 16);
+  gcol(ws.gT, 16, ws.gcolB, 16, 3);
+  rc = wgrad_cols(base_tail + 4, H, W, ws.hrB, 64, ws.gcolB, 16);
   if (rc) return rc;
-  { BwdOp bo; bo.kind = BwdOp::kBias; bo.layer = base_tail + 4; bo.src = gT; bo.count = (long)N * H * W; bo.C = 16; bo.coff = 0; bo.cout = 1;
-    bo.scale = 1.f; ops.push_back(bo); }
-  rc = dgrad(H, W, gated(io_of(gcolB, 16, gP, 64, 0, CSR_ACT_NONE), hrB, 64, 0, 0, 0.2f));
+  { Op bo; bo.kind = Op::kBias; bo.layer = base_tail + 4; bo.src = ws.gT; bo.count = (long)N * H * W; bo.C = 16; bo.coff = 0; bo.cout = 1;
+    ops.push_back(bo); }
+  rc = dgrad(H, W, gated(io_of(ws.gcolB, 16, ws.gP, 64, 0, CSR_ACT_NONE), ws.hrB, 64, 0, 0, 0.2f));
   if (rc) return rc;
-  rc = wgrad_plain(base_tail + 3, H, W, hrA, 64, 0, gP, 64, 0, 1.f);
+  rc = wgrad_plain(base_tail + 3, H, W, ws.hrA, 64, 0, ws.gP, 64, 0, 1.f);
   if (rc) return rc;
-  rc = dgrad(H, W, gated(io_of(gP, 64, gQ, 64, 0, CSR_ACT_NONE), hrA, 64, 0, 0, 0.2f));
+  rc = dgrad(H, W, gated(io_of(ws.gP, 64, ws.gQ, 64, 0, CSR_ACT_NONE), ws.hrA, 64, 0, 0, 0.2f));
   if (rc) return rc;
   // ---- upconv2 / upconv1 (esrgan.py:94,97): nearest-x2 + conv, transposed phase by phase ---------------------------
-  rc = wgrad_plain(base_tail + 2, 2 * h, 2 * w, m1, 64, 0, gQ, 64, 0, 1.f);
+  rc = wgrad_plain(base_tail + 2, 2 * h, 2 * w, ws.m1, 64, 0, ws.gQ, 64, 0, 1.f);
   if (rc) return rc;
-  rc = dgrad(2 * h, 2 * w, gated(io_of(gQ, 64, gm1, 64, 0, CSR_ACT_NONE), m1, 64, 0, 0, 0.2f), gQ);
+  rc = dgrad(2 * h, 2 * w, gated(io_of(ws.gQ, 64, ws.gm1, 64, 0, CSR_ACT_NONE), ws.m1, 64, 0, 0, 0.2f), ws.gQ);
   if (rc) return rc;
-  rc = wgrad_plain(base_tail + 1, h, w, t0, 64, 0, gm1, 64, 0, 1.f);
+  rc = wgrad_plain(base_tail + 1, h, w, ws.t0, 64, 0, ws.gm1, 64, 0, 1.f);
   if (rc) return rc;
-  rc = dgrad(h, w, io_of(gm1, 64, gt0, 64, 0, CSR_ACT_NONE), gm1);
+  rc = dgrad(h, w, io_of(ws.gm1, 64, ws.gt0, 64, 0, CSR_ACT_NONE), ws.gm1);
   if (rc) return rc;
   // ---- trunk_conv + skip (esrgan.py:91-92): gt0 is also the skip-path gradient of conv_first's output --------------
-  rc = wgrad_plain(base_tail + 0, h, w, cat(3 * d.nb), C, 0, gt0, 64, 0, 1.f);
+  rc = wgrad_plain(base_tail + 0, h, w, ws.cat[3 * d.nb], C, 0, ws.gt0, 64, 0, 1.f);
   if (rc) return rc;
   int Pb = 0;                                             // gcat buffer whose channels [0,64) hold dL/d(RRDB output)
-  rc = dgrad(h, w, io_of(gt0, 64, gcat[Pb], C, 0, CSR_ACT_NONE));
+  rc = dgrad(h, w, io_of(ws.gt0, 64, ws.gcat[Pb], C, 0, CSR_ACT_NONE));
   if (rc) return rc;
   // ---- RRDB trunk, reversed (esrgan.py:32-38, 50-54) ----------------------------------------------------------------
   // Per dense block one gradient concat buffer Gb = [g_y (64) | g4 | g3 | g2 | g1] (bwd_layer_table): four narrow convs
@@ -1281,105 +1313,77 @@ static int bwd_build(CsrPlan* P, void* ws) {
   for (int i = d.nb - 1; i >= 0; --i) {
     const int Qb = (Pb + 1) % 3, Rb = (Pb + 2) % 3;
     // out = RDB3_out*0.2 + x_rrdb: the gradient entering RDB3 is 0.2*G  ->  Gb(RDB3)[0:64]
-    { BwdOp op; op.kind = BwdOp::kScale; op.src = gcat[Pb]; op.C = C; op.dst = gcat[Qb]; op.coff = C; op.count = (long)N * h * w; op.scale = 0.2f;
+    { Op op; op.kind = Op::kScale; op.src = ws.gcat[Pb]; op.C = C; op.dst = ws.gcat[Qb]; op.coff = C; op.count = (long)N * h * w; op.scale = 0.2f;
       ops.push_back(op); }
     const int gbuf[3] = {Qb, Rb, Qb};                     // Gb of RDB3, RDB2, RDB1
     const int xout[3] = {Rb, Qb, Rb};                     // where each block's input gradient goes: the next Gb[0:64]
     for (int r = 2; r >= 0; --r) {
       const int j = 3 * i + r;
-      void* Gb = gcat[gbuf[2 - r]];
-      void* Xo = gcat[xout[2 - r]];
-      bool dense_done = false;
-      if (g_opt_dense && gc == 16 && !g_opt_force_generic) {
-        // the four gated convs as ONE persistent launch with tile-level dependencies, like the forward's conv1..conv4
-        BwdOp op; op.kind = BwdOp::kDense;
-        const size_t per_block = (size_t)kDenseMaxLayers * N * ceil_div(h, 8) * ceil_div(w, 14);
-        unsigned int* fl = P->flags + (size_t)j * per_block;
-        if (build_dense(packs, bi, N, h, w, Gb, C, nf, gc, fl, &op.dense, cat(j), C) == CSR_OK && (size_t)op.dense.p.num_tiles * kDenseMaxLayers <= per_block &&
-            op.dense.p.num_tiles >= g_opt_dense_min * P->sms) {
-          ops.push_back(op);
-          bi += 4;
-          dense_done = true;
-        }
-      }
-      for (int sidx = 4; sidx >= 1 && !dense_done; --sidx) {
-        // g_s = lrelu'(x_s) * conv_T([g_y | g4 .. g_{s+1}])  ->  Gb slice of x_s
-        ConvIO io = io_of(Gb, C, Gb, C, nf + (4 - sidx) * gc, CSR_ACT_NONE);
-        io = gated(io, cat(j), C, nf + (sidx - 1) * gc, 0, 0.2f);
-        const PackLayer& pl = packs[bi];
-        for (const PackPart& pp : pl.parts) {
-          BwdOp op; op.kind = BwdOp::kConv;
-          rc = build_conv(pl, pp, N, h, w, io, &op.conv);
+      void* Gb = ws.gcat[gbuf[2 - r]];
+      void* Xo = ws.gcat[xout[2 - r]];
+      Op dop;
+      if (try_dense(P, packs, bi, j, Gb, ws.cat[j], &dop)) {
+        ops.push_back(dop);
+        bi += 4;
+      } else {
+        for (int sidx = 4; sidx >= 1; --sidx) {
+          // g_s = lrelu'(x_s) * conv_T([g_y | g4 .. g_{s+1}])  ->  Gb slice of x_s
+          rc = dgrad(h, w, gated(io_of(Gb, C, Gb, C, nf + (4 - sidx) * gc, CSR_ACT_NONE), ws.cat[j], C, nf + (sidx - 1) * gc, 0, 0.2f));
           if (rc) return rc;
-          ops.push_back(op);
         }
-        ++bi;
       }
       // weight gradients of the whole dense block as ONE GEMM per vertical tap (gc = 16): x = the block's forward concat
       // buffer (128 ch), g columns [0,64) = [g4 g3 g2 g1], columns [64,128) = g_y (conv5, scale 0.2).  Issued before the
       // input-gradient conv below, whose output may overwrite a buffer another block's GEMM has just read.
-      {
-        if (C > 128 || 4 * gc > 64) {
-          // gc = 32: concat pitch 192 -> per-layer weight gradients
-          for (int k = 1; k <= 4; ++k) {
-            rc = wgrad_plain(fwd_index_rdb(i, r, k), h, w, cat(j), C, 0, Gb, C, nf + (4 - k) * gc, 1.f);
-            if (rc) return rc;
-          }
-          rc = wgrad_plain(fwd_index_rdb(i, r, 5), h, w, cat(j), C, 0, Gb, C, 0, 0.2f);
+      if (C > 128 || 4 * gc > 64) {
+        // gc = 32: concat pitch 192 -> per-layer weight gradients
+        for (int k = 1; k <= 4; ++k) {
+          rc = wgrad_plain(fwd_index_rdb(i, r, k), h, w, ws.cat[j], C, 0, Gb, C, nf + (4 - k) * gc, 1.f);
           if (rc) return rc;
-        } else {
-          const long part_stride = (long)9 * 128 * 128;
-          int n_parts = 0;
-          for (int dy = 0; dy < 3; ++dy) {
-            BwdOp op; op.kind = BwdOp::kWgrad;
-            rc = build_wgrad(P->sms, N, h, w, 3, 1, dy - 1, 1, cat(j), C, 0, Gb, C, nf, Gb, C, 0, 128, dacc + (size_t)dy * 3 * 128 * 128, part_stride,
-                             128, &op.wg);
-            if (rc) return rc;
-            n_parts = op.wg.p.n_parts;
-            ops.push_back(op);
-          }
-          { BwdOp rd; rd.kind = BwdOp::kReduce; rd.n_parts = n_parts; rd.dy_stride = part_stride; rd.count = part_stride; ops.push_back(rd); }
-          for (int k = 1; k <= 5; ++k) {
-            const int layer = fwd_index_rdb(i, r, k);
-            BwdOp sc; sc.kind = BwdOp::kScatter; sc.layer = layer; sc.ci0 = 0; sc.ci_n = (k < 5) ? nf + (k - 1) * gc : nf + 4 * gc;
-            sc.col0 = (k < 5) ? (4 - k) * gc : 64; sc.ld_n = 128; sc.scale = (k < 5) ? 1.f : 0.2f;
-            ops.push_back(sc);
-          }
-          // bias gradients: the four narrow convs in one pass over the gradient-concat slices, conv5 from g_y
-          BwdOp bo; bo.kind = BwdOp::kBias; bo.count = (long)N * h * w; bo.cout = 4 * gc; bo.nseg = 4;
-          for (int q = 0; q < 4; ++q) bo.seg_layers[q] = fwd_index_rdb(i, r, 4 - q);      // slice order g4, g3, g2, g1
-          bo.layer = bo.seg_layers[0]; bo.src = Gb; bo.C = C; bo.coff = nf; bo.scale = 1.f;
-          ops.push_back(bo);
-          BwdOp b5; b5.kind = BwdOp::kBias; b5.layer = fwd_index_rdb(i, r, 5); b5.count = (long)N * h * w; b5.cout = nf;
-          b5.src = Gb; b5.C = C; b5.coff = 0; b5.scale = 0.2f;
-          ops.push_back(b5);
         }
+        rc = wgrad_plain(fwd_index_rdb(i, r, 5), h, w, ws.cat[j], C, 0, Gb, C, 0, 0.2f);
+        if (rc) return rc;
+      } else {
+        const long part_stride = (long)9 * 128 * 128;
+        std::vector<WgradLaunch> wg(3);
+        for (int dy = 0; dy < 3; ++dy) {
+          rc = build_wgrad(P->sms, N, h, w, 3, 1, dy - 1, 1, ws.cat[j], C, 0, Gb, C, nf, Gb, C, 0, 128, dacc + (size_t)dy * 3 * 128 * 128, part_stride,
+                           128, &wg[dy]);
+          if (rc) return rc;
+        }
+        push_acc_group(ops, wg, dacc, part_stride);
+        for (int k = 1; k <= 5; ++k) {
+          const LayerSpec& Ls = F[fwd_index_rdb(i, r, k)];
+          Op sc; sc.kind = Op::kScatter; sc.src = dacc; sc.layer = fwd_index_rdb(i, r, k); sc.ci0 = 0; sc.ci_n = Ls.cin;
+          sc.col0 = (k < 5) ? (4 - k) * gc : 64; sc.ld_n = 128; sc.scale = (k < 5) ? 1.f : 0.2f;
+          sc.cout = Ls.cout; sc.cin = Ls.cin; sc.kh = Ls.kh; sc.kw = Ls.kw;
+          ops.push_back(sc);
+        }
+        // bias gradients: the four narrow convs in one pass over the gradient-concat slices, conv5 from g_y
+        Op bo; bo.kind = Op::kBias; bo.count = (long)N * h * w; bo.cout = 4 * gc; bo.nseg = 4;
+        for (int q = 0; q < 4; ++q) bo.seg_layers[q] = fwd_index_rdb(i, r, 4 - q);      // slice order g4, g3, g2, g1
+        bo.layer = bo.seg_layers[0]; bo.src = Gb; bo.C = C; bo.coff = nf;
+        ops.push_back(bo);
+        Op b5; b5.kind = Op::kBias; b5.layer = fwd_index_rdb(i, r, 5); b5.count = (long)N * h * w; b5.cout = nf;
+        b5.src = Gb; b5.C = C; b5.coff = 0; b5.scale = 0.2f;
+        ops.push_back(b5);
       }
       // gradient of the block input: conv_T([g_y | g4 | g3 | g2 | g1]) + g_y (identity path of x5*0.2 + x)
       // (+ G for RDB1: identity path of the RRDB, out*0.2 + x_rrdb)
-      {
-        ConvIO io = io_of(Gb, C, Xo, C, 0, CSR_ACT_NONE);
-        io.r1 = Gb; io.r1_C = C; io.r1_coff = 0; io.s1 = 1.f;
-        if (r == 0) { io.r2 = gcat[Pb]; io.r2_C = C; io.r2_coff = 0; io.s2 = 1.f; }
-        const PackLayer& pl = packs[bi];
-        for (const PackPart& pp : pl.parts) {
-          BwdOp op; op.kind = BwdOp::kConv;
-          rc = build_conv(pl, pp, N, h, w, io, &op.conv);
-          if (rc) return rc;
-          ops.push_back(op);
-        }
-        ++bi;
-      }
+      ConvIO io = io_of(Gb, C, Xo, C, 0, CSR_ACT_NONE);
+      io.r1 = Gb; io.r1_C = C; io.r1_coff = 0; io.s1 = 1.f;
+      if (r == 0) { io.r2 = ws.gcat[Pb]; io.r2_C = C; io.r2_coff = 0; io.s2 = 1.f; }
+      rc = dgrad(h, w, io);
+      if (rc) return rc;
     }
     Pb = Rb;                                               // RDB1 wrote dL/d(RRDB input) (incl. + G) into R[0:64]
   }
   // ---- conv_first (esrgan.py:90): total gradient of its output = trunk path (gcat[Pb][0:64]) + skip path (gt0) ----
-  rc = wgrad_plain(0, h, w, xin, 64, 0, gcat[Pb], C, 0, 1.f);
+  rc = wgrad_plain(0, h, w, ws.xin, 64, 0, ws.gcat[Pb], C, 0, 1.f);
   if (rc) return rc;
-  rc = wgrad_plain(0, h, w, xin, 64, 0, gt0, 64, 0, 1.f);
+  rc = wgrad_plain(0, h, w, ws.xin, 64, 0, ws.gt0, 64, 0, 1.f);
   if (rc) return rc;
   if (bi != (int)B.size()) return fail(CSR_ERR_BAD_ARG, "internal: backward table mismatch (%d of %zu)", bi, B.size());
-  wgrad_ops_to_atomic(ops, dacc);
   return CSR_OK;
 }
 
@@ -1554,14 +1558,23 @@ static int plan_create_impl(const CsrNetDesc* net, int32_t n, int32_t h, int32_t
   if (rc) return rc;
   CsrPlan* P = new CsrPlan();
   P->net = *net; P->N = n; P->h = h; P->w = w; P->sms = std::max(1, di.sms - (train ? g_opt_reserve_sms : 0)); P->train = train;
-  rc = plan_build(P, workspace);
+  const std::vector<LayerSpec> layers = layer_table(*net);
+  P->grad_off = grad_offsets(layers, &P->grad_floats);
+  uint8_t* base = reinterpret_cast<uint8_t*>(workspace);
+  P->sx = reinterpret_cast<float*>(base + L.sx); P->selev = reinterpret_cast<float*>(base + L.selev);
+  P->smask = reinterpret_cast<float*>(base + L.smask); P->sout = reinterpret_cast<float*>(base + L.sout);
+  if (train) { P->sgout = reinterpret_cast<float*>(base + L.sgout); P->sgrad = reinterpret_cast<float*>(base + L.sgrad); }
+  P->flags = reinterpret_cast<unsigned int*>(base + L.flags); P->flags_bytes = L.flags_bytes;
+  P->dbg_cat = L.cat; P->ccat = L.ccat;
+  P->dbg_tail[0] = L.m1; P->dbg_tail[1] = L.hrA; P->dbg_tail[2] = L.hrB; P->dbg_tail[3] = L.hrD; P->dbg_tail[4] = L.hrE;
+  const WsPtrs ws = ws_carve(L, workspace);
+  rc = plan_build(P, ws, layers);
   if (!rc && train) {
-    rc = bwd_build(P, workspace);
+    rc = bwd_build(P, ws, layers);
     if (!rc) {
       // the narrow gradient maps are read 16 channels wide but written 1-3 channels wide: start them from zero
-      uint8_t* base = reinterpret_cast<uint8_t*>(workspace);
       const size_t hr16 = (size_t)n * h * w * 16 * 16 * 2;
-      cudaError_t e = cudaMemset(base + L.gT, 0, hr16);
+      cudaError_t e = cudaMemset(ws.gT, 0, hr16);
       if (e != cudaSuccess) rc = fail(CSR_ERR_CUDA, "cudaMemset: %s", cudaGetErrorString(e));
     }
   }
@@ -1677,13 +1690,22 @@ static int run_graphed(CsrPlan::GraphCache& gc, const void* packed, cudaStream_t
 
 extern "C" {
 
-static int backward_launches(CsrPlan* P, const void* packed_bwd, const float* grad_out, float* const* dw, float* const* db, cudaStream_t s,
-                             size_t op_lo = 0, size_t op_hi = (size_t)-1);
-
 int csr_plan_backward(CsrPlan* P, const void* packed_bwd, const float* grad_out, float* const* dw, float* const* db, void* stream) {
   if (!P || !packed_bwd || !grad_out || !dw || !db) return fail(CSR_ERR_BAD_ARG, "null pointer");
   if (!P->train) return fail(CSR_ERR_BAD_ARG, "csr_plan_backward needs a plan made by csr_train_plan_create");
-  return backward_launches(P, packed_bwd, grad_out, dw, db, reinterpret_cast<cudaStream_t>(stream));
+  Bindings b;
+  b.packed = packed_bwd; b.grad_out = grad_out; b.dw = dw; b.db = db;
+  return run_ops(P->bwd, 0, P->bwd.size(), b, P->sms, reinterpret_cast<cudaStream_t>(stream));
+}
+
+// Bindings of the flat-gradient backward: dL/dout and the gradients live in the plan's staging buffers.
+static Bindings flat_bindings(const CsrPlan* P, const void* packed_bwd, std::vector<float*>& dw, std::vector<float*>& db) {
+  const size_t nl = P->grad_off.size() / 2;
+  dw.resize(nl); db.resize(nl);
+  for (size_t i = 0; i < nl; ++i) { dw[i] = P->sgrad + P->grad_off[2 * i]; db[i] = P->sgrad + P->grad_off[2 * i + 1]; }
+  Bindings b;
+  b.packed = packed_bwd; b.grad_out = P->sgout; b.dw = dw.data(); b.db = db.data();
+  return b;
 }
 
 size_t csr_plan_grad_floats(const CsrPlan* P) { return P ? P->grad_floats : 0; }
@@ -1705,12 +1727,12 @@ int csr_plan_backward_segments(CsrPlan* P, int32_t nseg) {
   if (!P || !P->train) return fail(CSR_ERR_BAD_ARG, "needs a plan made by csr_train_plan_create");
   if (nseg < 1) return fail(CSR_ERR_BAD_ARG, "nseg must be positive");
   // last op that writes each layer's gradient
-  const size_t nl = P->fwd_layers.size();
+  const size_t nl = P->grad_off.size() / 2;
   std::vector<size_t> last(nl, 0);
   for (size_t oi = 0; oi < P->bwd.size(); ++oi) {
-    const BwdOp& op = P->bwd[oi];
-    if (op.kind == BwdOp::kScatter || op.kind == BwdOp::kBiasPlanar) last[op.layer] = oi;
-    if (op.kind == BwdOp::kBias)
+    const Op& op = P->bwd[oi];
+    if (op.kind == Op::kScatter || op.kind == Op::kBiasPlanar) last[op.layer] = oi;
+    if (op.kind == Op::kBias)
       for (int q = 0; q < op.nseg; ++q) last[op.nseg > 1 ? op.seg_layers[q] : op.layer] = oi;
   }
   // done_after[oi] = lowest float offset such that every layer at or above it is complete once ops [0, oi] have run
@@ -1753,15 +1775,14 @@ int csr_plan_backward_flat_seg(CsrPlan* P, const void* packed_bwd, const float* 
   if (!P || !packed_bwd || !grad_out || !flat_grads || !lo || !hi) return fail(CSR_ERR_BAD_ARG, "null pointer");
   if (!P->train || seg < 0 || (size_t)seg >= P->seg_lo.size()) return fail(CSR_ERR_BAD_ARG, "bad segment (call csr_plan_backward_segments first)");
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  const size_t nl = P->fwd_layers.size();
   if (seg == 0)
     CSR_CUDA(cudaMemcpyAsync(P->sgout, grad_out, (size_t)P->N * 16 * P->h * P->w * sizeof(float), cudaMemcpyDeviceToDevice, s));
-  std::vector<float*> dw(nl), db(nl);
-  for (size_t i = 0; i < nl; ++i) { dw[i] = P->sgrad + P->grad_off[2 * i]; db[i] = P->sgrad + P->grad_off[2 * i + 1]; }
+  std::vector<float*> dw, db;
+  const Bindings b = flat_bindings(P, packed_bwd, dw, db);
   const size_t o0 = P->seg_op[seg], o1 = P->seg_op[seg + 1];
   int rc = run_graphed(P->g_seg[seg], packed_bwd, s, [&](cudaStream_t st) -> int {
     if (seg == 0) CSR_CUDA(cudaMemsetAsync(P->sgrad, 0, P->grad_floats * sizeof(float), st));
-    return backward_launches(P, packed_bwd, P->sgout, dw.data(), db.data(), st, o0, o1);
+    return run_ops(P->bwd, o0, o1, b, P->sms, st);
   });
   if (rc) return rc;
   *lo = P->seg_lo[seg]; *hi = P->seg_hi[seg];
@@ -1773,84 +1794,17 @@ int csr_plan_backward_flat(CsrPlan* P, const void* packed_bwd, const float* grad
   if (!P || !packed_bwd || !grad_out || !flat_grads) return fail(CSR_ERR_BAD_ARG, "null pointer");
   if (!P->train) return fail(CSR_ERR_BAD_ARG, "csr_plan_backward_flat needs a plan made by csr_train_plan_create");
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  const size_t nl = P->fwd_layers.size();
   const size_t hr_bytes = (size_t)P->N * 16 * P->h * P->w * sizeof(float);
   // the replayed graph works on plan-owned buffers: stage dL/dout in, copy the flat gradients out
   CSR_CUDA(cudaMemcpyAsync(P->sgout, grad_out, hr_bytes, cudaMemcpyDeviceToDevice, s));
-  std::vector<float*> dw(nl), db(nl);
-  for (size_t i = 0; i < nl; ++i) { dw[i] = P->sgrad + P->grad_off[2 * i]; db[i] = P->sgrad + P->grad_off[2 * i + 1]; }
+  std::vector<float*> dw, db;
+  const Bindings b = flat_bindings(P, packed_bwd, dw, db);
   int rc = run_graphed(P->g_bwd, packed_bwd, s, [&](cudaStream_t st) -> int {
     CSR_CUDA(cudaMemsetAsync(P->sgrad, 0, P->grad_floats * sizeof(float), st));
-    return backward_launches(P, packed_bwd, P->sgout, dw.data(), db.data(), st);
+    return run_ops(P->bwd, 0, P->bwd.size(), b, P->sms, st);
   });
   if (rc) return rc;
   CSR_CUDA(cudaMemcpyAsync(flat_grads, P->sgrad, P->grad_floats * sizeof(float), cudaMemcpyDeviceToDevice, s));
-  return CSR_OK;
-}
-
-static int backward_launches(CsrPlan* P, const void* packed_bwd, const float* grad_out, float* const* dw, float* const* db, cudaStream_t s,
-                             size_t op_lo, size_t op_hi) {
-  const uint8_t* pk = reinterpret_cast<const uint8_t*>(packed_bwd);
-  const int H = 4 * P->h, W = 4 * P->w;
-  op_hi = std::min(op_hi, P->bwd.size());
-  for (size_t oi = op_lo; oi < op_hi; ++oi) {
-    BwdOp& op = P->bwd[oi];
-    switch (op.kind) {
-      case BwdOp::kGcol:
-        CSR_CUDA(launch_gcol_pack(op.src ? op.src : grad_out, op.C, op.dst, op.coff, H, W, (long)P->N * H * W, op.kh, op.kw, s));
-        break;
-      case BwdOp::kConv: {
-        op.conv.p.wpk = pk + op.conv.w_off;
-        op.conv.p.bias = reinterpret_cast<const float*>(pk + op.conv.b_off);
-        int e = launch_conv_tc(op.conv.p, op.conv.tmap, P->sms, s);
-        if (e) return fail(CSR_ERR_CUDA, "dgrad launch failed: %s", cudaGetErrorString((cudaError_t)e));
-        break;
-      }
-      case BwdOp::kDense: {
-        for (int k = 0; k < op.dense.p.n_layers; ++k) {
-          op.dense.p.L[k].wpk = pk + op.dense.w_off[k];
-          op.dense.p.L[k].bias = reinterpret_cast<const float*>(pk + op.dense.b_off[k]);
-        }
-        int e = launch_dense_block(op.dense.p, op.dense.tmap, P->sms, s);
-        if (e) return fail(CSR_ERR_CUDA, "dense-block dgrad launch failed: %s", cudaGetErrorString((cudaError_t)e));
-        break;
-      }
-      case BwdOp::kWgrad: {
-        int e = launch_wgrad_tc(op.wg.p, op.wg.tx0, op.wg.tx1, op.wg.tg0, op.wg.tg1, P->sms, s);
-        if (e) return fail(CSR_ERR_CUDA, "wgrad launch failed: %s", cudaGetErrorString((cudaError_t)e));
-        break;
-      }
-      case BwdOp::kReduce:
-        CSR_CUDA(launch_wgrad_reduce(P->dacc, op.dy_stride, op.n_parts, op.count, s));
-        break;
-      case BwdOp::kScatter: {
-        const LayerSpec& L = P->fwd_layers[op.layer];
-        if (!dw[op.layer]) return fail(CSR_ERR_BAD_ARG, "null weight-gradient pointer for layer %d", op.layer);
-        CSR_CUDA(launch_wgrad_scatter(P->dacc, op.ld_n, dw[op.layer], op.taps_t ? op.taps_t : L.cout, L.cin, op.taps_t ? 1 : L.kh, op.taps_t ? 1 : L.kw, op.fold, op.phase, op.ci0, op.ci_n, op.col0,
-                                      op.scale, op.taps_t, s));
-        break;
-      }
-      case BwdOp::kBias: {
-        float* dbs[4] = {nullptr, nullptr, nullptr, nullptr};
-        for (int q = 0; q < op.nseg; ++q) {
-          dbs[q] = db[op.nseg > 1 ? op.seg_layers[q] : op.layer];
-          if (!dbs[q]) return fail(CSR_ERR_BAD_ARG, "null bias-gradient pointer for layer %d", op.layer);
-        }
-        CSR_CUDA(launch_bias_grad(op.src, op.count, op.C, op.coff, op.cout, op.scale, dbs, op.nseg, s));
-        break;
-      }
-      case BwdOp::kBiasPlanar:
-        CSR_CUDA(launch_bias_grad_planar(op.src ? reinterpret_cast<const float*>(op.src) : grad_out, op.count, op.scale, db[op.layer], s));
-        break;
-      case BwdOp::kScale:
-        CSR_CUDA(launch_scale_copy64(op.src, op.C, op.dst, op.coff, op.count, op.scale, s));
-        break;
-      case BwdOp::kMemset:
-        CSR_CUDA(cudaMemsetAsync(op.dst, 0, op.count, s));
-        break;
-    }
-    ++g_launches;
-  }
   return CSR_OK;
 }
 
@@ -1875,7 +1829,7 @@ int csr_plan_buffer(const CsrPlan* P, int32_t kind, int32_t index, size_t* offse
 
 int csr_plan_num_backward_ops(const CsrPlan* plan) { return plan ? (int)plan->bwd.size() : 0; }
 
-int csr_plan_num_launches(const CsrPlan* plan) { return plan ? (int)plan->convs.size() + 2 : 0; }
+int csr_plan_num_launches(const CsrPlan* plan) { return plan ? (int)plan->fwd.size() : 0; }
 
 void csr_plan_destroy(CsrPlan* plan) {
   if (!plan) return;
@@ -1885,68 +1839,30 @@ void csr_plan_destroy(CsrPlan* plan) {
   delete plan;
 }
 
-static int forward_launches(CsrPlan* P, const void* packed, const float* x, const float* elev, const float* mask, float* out, cudaStream_t s);
-
 int csr_plan_forward(CsrPlan* P, const void* packed, const float* x, const float* elev, const float* mask, float* out, void* stream) {
   if (!P || !packed || !x || !elev || !mask || !out) return fail(CSR_ERR_BAD_ARG, "null pointer");
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  Bindings b;
+  b.packed = packed; b.timeline = g_timeline; b.timeline_cap = g_timeline_cap;
+  auto body = [&](cudaStream_t st) -> int {
+    int rc = run_ops(P->fwd, 0, 1, b, P->sms, st);           // op 0: the input conversion
+    if (rc) return rc;
+    if (P->fwd_dense) CSR_CUDA(cudaMemsetAsync(P->flags, 0, P->flags_bytes, st));
+    return run_ops(P->fwd, 1, P->fwd.size(), b, P->sms, st);
+  };
   // Graph replay pays three staging copies; it wins when the forward is launch-bound (small rasters / batches).
   const size_t hr_px = (size_t)P->N * 16 * P->h * P->w;
-  if (!g_opt_graphs || P->g_fwd.failed || hr_px > (size_t)g_opt_graph_max_px) return forward_launches(P, packed, x, elev, mask, out, s);
+  if (!g_opt_graphs || P->g_fwd.failed || hr_px > (size_t)g_opt_graph_max_px) {
+    b.x = x; b.elev = elev; b.mask = mask; b.out = out;
+    return body(s);
+  }
   CSR_CUDA(cudaMemcpyAsync(P->sx, x, (size_t)P->N * P->net.in_channels * P->h * P->w * sizeof(float), cudaMemcpyDeviceToDevice, s));
   CSR_CUDA(cudaMemcpyAsync(P->selev, elev, hr_px * sizeof(float), cudaMemcpyDeviceToDevice, s));
   CSR_CUDA(cudaMemcpyAsync(P->smask, mask, hr_px * sizeof(float), cudaMemcpyDeviceToDevice, s));
-  int rc = run_graphed(P->g_fwd, packed, s, [&](cudaStream_t st) -> int { return forward_launches(P, packed, P->sx, P->selev, P->smask, P->sout, st); });
+  b.x = P->sx; b.elev = P->selev; b.mask = P->smask; b.out = P->sout;
+  int rc = run_graphed(P->g_fwd, packed, s, body);
   if (rc) return rc;
   CSR_CUDA(cudaMemcpyAsync(out, P->sout, hr_px * sizeof(float), cudaMemcpyDeviceToDevice, s));
-  return CSR_OK;
-}
-
-static int forward_launches(CsrPlan* P, const void* packed, const float* x, const float* elev, const float* mask, float* out, cudaStream_t s) {
-  const uint8_t* pk = reinterpret_cast<const uint8_t*>(packed);
-  CSR_CUDA(launch_nchw_to_nhwc(x, P->xin, P->N, P->net.in_channels, P->h, P->w, 64, 16, s));
-  ++g_launches;
-  if (!P->dense.empty()) CSR_CUDA(cudaMemsetAsync(P->flags, 0, P->flags_bytes, s));   // completion counters of the dense-block launches
-  const ConvLaunch* tap_pack = nullptr;
-  for (size_t i = 0; i < P->convs.size(); ++i) {
-    if ((int)i == P->idx_srcnn1) {
-      if (tap_pack) {
-        // conv_last's tap sum and the SRCNN input im2col in one pass
-        CSR_CUDA(launch_tap_pack(tap_pack->taps, tap_pack->tap_plane, reinterpret_cast<const float*>(pk + tap_pack->b_off), elev, mask, P->sin, P->N,
-                                 tap_pack->tap_H, tap_pack->tap_W, s));
-      } else {
-        CSR_CUDA(launch_pack_srcnn_in(P->tlast, elev, mask, P->sin, 4 * P->w, (long)P->N * P->h * P->w * 16, P->srcnn_pitch, s));
-      }
-      ++g_launches;
-    }
-    ConvLaunch& cl = P->convs[i];
-    if (cl.dense >= 0) {
-      DenseLaunch& dl = P->dense[cl.dense];
-      for (int k = 0; k < dl.p.n_layers; ++k) {
-        dl.p.L[k].wpk = pk + dl.w_off[k];
-        dl.p.L[k].bias = reinterpret_cast<const float*>(pk + dl.b_off[k]);
-      }
-      dl.p.timeline = ((int)i < g_timeline_cap) ? g_timeline : nullptr; dl.p.launch_id = (int)i;
-      int e = launch_dense_block(dl.p, dl.tmap, P->sms, s);
-      if (e) return fail(CSR_ERR_CUDA, "dense-block launch %zu failed: %s", i, cudaGetErrorString((cudaError_t)e));
-      ++g_launches;
-      continue;
-    }
-    if (cl.tapsum && P->srcnn_pitch == 32 && g_opt_tap_pack) { tap_pack = &cl; continue; }   // finished by tap_pack_kernel right before srcnn.conv1
-    if (cl.tapsum) {
-      CSR_CUDA(launch_tap_sum(cl.taps, cl.tap_plane, reinterpret_cast<const float*>(pk + cl.b_off), P->tlast, cl.tap_H, cl.tap_W, cl.tap_plane, s));
-      ++g_launches;
-      continue;
-    }
-    cl.p.wpk = pk + cl.w_off;
-    cl.p.bias = reinterpret_cast<const float*>(pk + cl.b_off);
-    if (cl.p.fuse2) { cl.p.w2 = pk + cl.w2_off; cl.p.b2 = cl.p.fuse2 == 1 ? reinterpret_cast<const float*>(pk + cl.b2_off) : nullptr; }
-    if (cl.final_out) cl.p.out = out;
-    cl.p.timeline = ((int)i < g_timeline_cap) ? g_timeline : nullptr; cl.p.launch_id = (int)i;
-    int e = launch_conv_tc(cl.p, cl.tmap, P->sms, s);
-    if (e) return fail(CSR_ERR_CUDA, "conv launch %zu failed: %s", i, cudaGetErrorString((cudaError_t)e));
-    ++g_launches;
-  }
   return CSR_OK;
 }
 
@@ -2066,7 +1982,7 @@ int csr_conv2d_nhwc(const CsrConvDesc* d, const void* in, const float* weight, c
 // ---- single-layer weight gradient (building block; used by the parity tests) ---------------------------
 size_t csr_conv2d_wgrad_scratch_bytes(const CsrWgradDesc* d) {
   if (!d || d->cout < 1 || d->cin < 1) return 0;
-  WgradLayer L = {d->cout, d->cin, d->kh, d->kw, 0, d->in_up2 ? 1 : 0};
+  const LayerSpec L = {"wgrad", d->cout, d->cin, d->kh, d->kw, 0, d->in_up2 ? 1 : 0};
   const size_t jobs = (!L.up2 && L.kh == L.kw && L.kw <= 3) ? wgrad_jobs_scratch_floats(L) : 0;
   if (d->cout > 128) return jobs * sizeof(float);
   return std::max(jobs, wgrad_scratch_floats(L)) * sizeof(float);
@@ -2078,23 +1994,21 @@ int csr_conv2d_wgrad(const CsrWgradDesc* d, const void* x, const void* g, float*
   if (d->n < 1 || d->h < 1 || d->w < 1 || d->cin < 1 || d->cout < 1 || d->cout > 1024) return fail(CSR_ERR_BAD_ARG, "bad wgrad shape");
   if (!(d->kh & 1) || !(d->kw & 1) || d->kh > 9 || d->kw > 9) return fail(CSR_ERR_UNSUPPORTED, "kernel %dx%d", d->kh, d->kw);
   if (d->in_up2 && (d->kh != 3 || d->kw != 3)) return fail(CSR_ERR_UNSUPPORTED, "nearest-x2 input needs a 3x3 kernel");
-  WgradLayer L = {d->cout, d->cin, d->kh, d->kw, 0, d->in_up2 ? 1 : 0};
+  const LayerSpec L = {"wgrad", d->cout, d->cin, d->kh, d->kw, 0, d->in_up2 ? 1 : 0};
   if (scratch_bytes < csr_conv2d_wgrad_scratch_bytes(d)) return fail(CSR_ERR_WORKSPACE, "wgrad scratch too small");
   DeviceInfo di;
   int rc = device_info(&di);
   if (rc) return rc;
-  long long launches = 0;
-  if (wgrad_jobs_applicable(L, d->n, d->h, d->w, di.sms)) {
-    rc = run_wgrad_layer_jobs(L, d->n, d->h, d->w, x, d->x_c, d->x_coff, g, d->g_c, d->g_coff, d->scale, dw, db, reinterpret_cast<float*>(scratch),
-                              di.sms, reinterpret_cast<cudaStream_t>(stream), &launches);
-    g_launches += launches;
-    return rc;
-  }
-  if (d->cout > 128) return fail(CSR_ERR_UNSUPPORTED, "wgrad: cout %d > 128 needs a 3x3 (or 1x1) stride-1 layer", d->cout);
-  rc = run_wgrad_layer(L, d->n, d->h, d->w, x, d->x_c, d->x_coff, g, d->g_c, d->g_coff, d->scale, dw, db, reinterpret_cast<float*>(scratch),
-                       di.sms, reinterpret_cast<cudaStream_t>(stream), &launches);
-  g_launches += launches;
-  return rc;
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  float* dacc = reinterpret_cast<float*>(scratch);
+  if (wgrad_jobs_applicable(L, d->n, d->h, d->w, di.sms))
+    return run_wgrad_layer_jobs(L, d->n, d->h, d->w, x, d->x_c, d->x_coff, g, d->g_c, d->g_coff, d->scale, dw, db, dacc, di.sms, s);
+  std::vector<Op> ops;
+  rc = emit_wgrad(ops, L, 0, d->n, d->h, d->w, x, d->x_c, d->x_coff, g, d->g_c, d->g_coff, d->scale, db != nullptr, dacc, di.sms);
+  if (rc) return rc;
+  Bindings b;
+  b.dw = &dw; b.db = &db;
+  return run_ops(ops, 0, ops.size(), b, di.sms, s);
 }
 
 // ---- layout helpers -----------------------------------------------------------------------------------

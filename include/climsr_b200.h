@@ -125,6 +125,7 @@ int     csr_plan_create(const CsrNetDesc* net, int32_t n, int32_t h, int32_t w,
                         void* workspace, size_t workspace_bytes, CsrPlan** plan);
 int     csr_plan_forward(CsrPlan* plan, const void* packed, const float* x, const float* elev,
                          const float* mask, float* out, void* stream);
+/* launches of one forward: what a forward without graph replay adds to csr_kernel_launch_count */
 int     csr_plan_num_launches(const CsrPlan* plan);
 void    csr_plan_destroy(CsrPlan* plan);
 /* one-shot convenience: plan_create + plan_forward + plan_destroy                               */

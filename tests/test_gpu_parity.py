@@ -683,6 +683,32 @@ def test_fused_hr_tail_matches_separate_launches(n, in_ch, h, w):
     assert float((outs[3] - outs[0]).abs().max()) <= 2e-3 * scale, float((outs[3] - outs[0]).abs().max())
 
 
+@pytest.mark.parametrize("key,value", [(None, None), (33, 0), (36, 0)])
+def test_plan_num_launches_matches_a_forward(key, value):
+    """csr_plan_num_launches is exactly what one forward without graph replay adds to the launch counter, for the default HR tail
+    (tap sum inside the SRCNN input pack), the separate tap sum (option 36 = 0) and the unfused tail (option 33 = 0); cfg4 shapes."""
+    from climsr_b200 import kernel_launch_count
+    from climsr_b200._lib import lib
+    from climsr_b200.models import ESRGANGenerator
+    from oracle import synth
+    x, elev, mask = (t.cuda() for t in synth.make_inputs(1, 3, 113, 113, seed=41))
+    lib.csr_set_option(11, 0)
+    if key is not None:
+        lib.csr_set_option(key, value)
+    try:
+        net = ESRGANGenerator(3, 1, 64, 11, 16).cuda().eval()
+        with torch.no_grad():
+            net(x, elev, mask)                       # packs the weights and creates the plan
+            before = kernel_launch_count()
+            net(x, elev, mask)
+            launched = kernel_launch_count() - before
+        assert launched == lib.csr_plan_num_launches(net._plan(1, 113, 113, x.device))
+    finally:
+        lib.csr_set_option(11, 1)
+        if key is not None:
+            lib.csr_set_option(key, {33: 3, 36: 1}[key])
+
+
 @pytest.mark.parametrize("tag", ["small", "hydra"])
 def test_rcan_matches_reference_golden(golden_dir, tag):
     """SURVEY 8f row 4: climsr_b200.models.rcan.RCAN (conv kernel + channel-attention / PixelShuffle kernels) against the outputs

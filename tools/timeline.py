@@ -1,5 +1,6 @@
 """In-situ timeline of one generator forward (PDL overlap intact): per launch the time from the previous launch's last CTA end
-to this launch's first CTA start (gap), and its own span.  python tools/timeline.py [workload] ; CSR_OPTS as in bench.py."""
+to this launch's first CTA start (gap), and its own span; launch i is op i of the plan's forward (op 0, the input conversion, has no
+stamps).  python tools/timeline.py [workload] ; CSR_OPTS as in bench.py."""
 import os
 import sys
 
