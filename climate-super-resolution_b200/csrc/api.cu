@@ -1636,9 +1636,14 @@ int csr_pack_weights_bwd(const CsrNetDesc* net, const float* const* w, void* pac
 // Run `body` (a launch sequence on stream s) through a cached CUDA graph: captured at the second call for a given packed
 // blob (the first call runs directly, so one-time attribute / symbol setup never happens inside a capture) and replayed
 // afterwards.  Any capture / instantiate failure falls back to direct launches for the lifetime of the plan.
+// When the caller is itself capturing s (torch.cuda.graph around a forward or backward), the launches go straight into the
+// caller's capture: no private stream or nested capture is started there, and the call does not advance the cache.
 template <typename Body>
 static int run_graphed(CsrPlan::GraphCache& gc, const void* packed, cudaStream_t s, Body body) {
   if (!g_opt_graphs || gc.failed) return body(s);
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(s, &cap) != cudaSuccess) { cudaGetLastError(); return body(s); }
+  if (cap != cudaStreamCaptureStatusNone) return body(s);
   if (gc.exec && gc.packed == packed) {
     CSR_CUDA(cudaGraphLaunch(gc.exec, s));
     g_launches += gc.launches;
@@ -1693,6 +1698,14 @@ extern "C" {
 int csr_plan_backward(CsrPlan* P, const void* packed_bwd, const float* grad_out, float* const* dw, float* const* db, void* stream) {
   if (!P || !packed_bwd || !grad_out || !dw || !db) return fail(CSR_ERR_BAD_ARG, "null pointer");
   if (!P->train) return fail(CSR_ERR_BAD_ARG, "csr_plan_backward needs a plan made by csr_train_plan_create");
+  // every gradient pointer is checked before the first launch: a refused call leaves dw / db untouched
+  for (const Op& op : P->bwd) {
+    if (op.kind == Op::kScatter && !dw[op.layer]) return fail(CSR_ERR_BAD_ARG, "null weight-gradient pointer for layer %d", op.layer);
+    if (op.kind == Op::kBiasPlanar && !db[op.layer]) return fail(CSR_ERR_BAD_ARG, "null bias-gradient pointer for layer %d", op.layer);
+    if (op.kind == Op::kBias)
+      for (int q = 0; q < op.nseg; ++q)
+        if (!db[op.nseg > 1 ? op.seg_layers[q] : op.layer]) return fail(CSR_ERR_BAD_ARG, "null bias-gradient pointer for layer %d", op.layer);
+  }
   Bindings b;
   b.packed = packed_bwd; b.grad_out = grad_out; b.dw = dw; b.db = db;
   return run_ops(P->bwd, 0, P->bwd.size(), b, P->sms, reinterpret_cast<cudaStream_t>(stream));

@@ -138,7 +138,10 @@ int     csr_generator_forward(const CsrNetDesc* net, const void* packed, const f
  * A training plan keeps every dense block's concat buffer and the HR-tail activations (the saved state autograd would
  * keep).  csr_plan_forward works on it unchanged; csr_plan_backward then ACCUMULATES (+=) d loss / d weight and
  * d loss / d bias of every conv layer into dw[i] / db[i] (HOST arrays of csr_num_layers() DEVICE pointers, fp32, the
- * parameters' OIHW / (cout) shapes) given grad_out = d loss / d out, fp32 (N,1,4h,4w).
+ * parameters' OIHW / (cout) shapes) given grad_out = d loss / d out, fp32 (N,1,4h,4w).  A null dw[i] / db[i] returns
+ * CSR_ERR_BAD_ARG before anything is launched.
+ * csr_plan_forward and csr_plan_backward_flat may be called on a stream the caller is capturing (after one call outside
+ * the capture): their launches then go into the caller's graph and the plan's own graph cache is left as it was.
  * <- autograd backward of ESRGANGenerator.forward (esrgan.py:89-102), invoked by Lightning's loss.backward().       */
 size_t  csr_train_workspace_bytes(const CsrNetDesc* net, int32_t n, int32_t h, int32_t w);
 int     csr_train_plan_create(const CsrNetDesc* net, int32_t n, int32_t h, int32_t w,
