@@ -107,7 +107,10 @@ def _load():
         "csr_linear_forward": (C.c_int, [vp, vp, vp, vp, i32, i32, i32, vp]),
         "csr_linear_backward": (C.c_int, [vp, vp, vp, vp, vp, vp, i32, i32, i32, vp]),
         "csr_channel_attention": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]),
+        "csr_channel_attention_backward_scratch_bytes": (sz, [i32, i32]),
+        "csr_channel_attention_backward": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, i32, i32, i32, i32, i32, vp]),
         "csr_pixel_shuffle2": (C.c_int, [vp, vp, i32, i32, i32, i32, vp]),
+        "csr_pixel_unshuffle2": (C.c_int, [vp, vp, i32, i32, i32, i32, vp]),
         "csr_grad_pack_bf16": (C.c_int, [vp, vp, sz, f32, vp]),
         "csr_grad_unpack_bf16": (C.c_int, [vp, vp, sz, f32, vp]),
         "csr_lr_input_from_hr": (C.c_int, [vp, vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp]),
@@ -128,7 +131,8 @@ EXPORTS = ("csr_abi_version", "csr_last_error", "csr_device_check", "csr_set_opt
            "csr_conv2d_nhwc", "csr_conv2d_pack", "csr_conv2d_wgrad_scratch_bytes", "csr_conv2d_wgrad", "csr_nchw_f32_to_nhwc_bf16", "csr_nhwc_bf16_to_nchw_f32", "csr_pixel_loss_scratch_bytes", "csr_l1_loss", "csr_mse_loss",
            "csr_metrics_scratch_bytes", "csr_masked_metrics", "csr_minmax_normalize", "csr_minmax_denormalize_mask", "csr_disc_gather", "csr_disc_collect", "csr_disc_bn_scratch_bytes", "csr_disc_bn_forward",
            "csr_disc_bn_backward", "csr_disc_flatten", "csr_disc_unflatten", "csr_linear_forward", "csr_linear_backward",
-           "csr_channel_attention", "csr_pixel_shuffle2", "csr_grad_pack_bf16", "csr_grad_unpack_bf16", "csr_lr_input_from_hr")
+           "csr_channel_attention", "csr_channel_attention_backward_scratch_bytes", "csr_channel_attention_backward", "csr_pixel_shuffle2",
+           "csr_pixel_unshuffle2", "csr_grad_pack_bf16", "csr_grad_unpack_bf16", "csr_lr_input_from_hr")
 
 
 def check(rc: int, what: str = "") -> None:

@@ -1,5 +1,5 @@
-"""Drop-in ``RCAN`` generator (the reference's default ``generator_type``, climsr/core/config.py:64) on the sm_100a kernels -
-inference path (SURVEY.md section 8f row 4).
+"""Drop-in ``RCAN`` generator (the reference's default ``generator_type``, climsr/core/config.py:64) on the sm_100a kernels,
+inference and training (SURVEY.md section 8f row 4).
 
 Mirrors climsr/models/rcan.py:137-217: same constructor signature (``conv`` is accepted and must be the default), same
 sub-module / parameter names (``head``, ``body.{g}.body.{b}.body.{0,2}`` + ``.body.3.conv_du.{0,2}``, ``tail.0.{0,2}``,
@@ -10,13 +10,21 @@ same ``forward(x, elev, mask) -> (N, 1, 4h, 4w)``.
 Every 3x3 convolution runs on the tcgen05 conv kernel (csr_conv2d_nhwc) with bias / ReLU / the ResidualGroup and body
 skip-adds fused in the epilogue; CALayer (global average pool -> 1x1 -> ReLU -> 1x1 -> sigmoid -> scale) together with the
 RCAB skip is csr_channel_attention, PixelShuffle(2) is csr_pixel_shuffle2, the SRCNN tail runs on the same conv kernel.
-Packed weights are cached per weight version.  Training (autograd) is not implemented for this model: forward under
-``torch.enable_grad()`` with parameters that require gradients raises.  There is no CPU fallback.
+Packed weights are cached per weight version.
+
+Training: in ``train()`` mode with gradients enabled the forward runs the same launch sequence through ``_RCANFunction``,
+which keeps the activations the backward needs on its autograd node (freed with the graph).  ``loss.backward()`` runs the
+input-gradient convs on the same conv kernel (transposed packs, ReLU' as the epilogue gate, the skip gradients as epilogue
+residuals), csr_channel_attention_backward for CALayer, csr_pixel_unshuffle2 for PixelShuffle, and csr_conv2d_wgrad for every
+conv, and hands back ordinary fp32 ``.grad`` tensors (views of one zeroed buffer in ``parameters()`` order).  Gradients
+w.r.t. x, elev and mask are not produced.  In ``eval()`` mode a forward under ``torch.enable_grad()`` with parameters that
+require gradients raises, as it always has.  There is no CPU fallback.
 """
 from __future__ import annotations
 
 import logging
 import math
+from typing import Optional
 
 import torch
 import torch.nn as nn
@@ -111,19 +119,23 @@ class RCAN(nn.Module):
                 raise KeyError(f'missing keys in state_dict: "{missing}"')
 
     # ------------------------------------------------------------------ packed-weight cache (see Discriminator._packed)
-    def _packed(self, conv: nn.Conv2d):
+    def _packed(self, conv: nn.Conv2d, transposed: bool = False, force: bool = False):
+        """(scratch, prepacked): the layer's pack scratch and whether it already holds the current weights.  force: the caller packs
+        in its conv call (training: optimizers such as fused AdamW update weights without bumping the version counters), and the
+        entry is left without a key so that the next inference forward repacks too."""
         from .esrgan import _WEIGHT_EPOCH
         cache = self.__dict__.setdefault("_pack_cache", {})
         w, b = conv.weight, conv.bias
         key = (w.data_ptr(), w._version, b.data_ptr(), b._version, _WEIGHT_EPOCH[0], w.device)
-        ent = cache.get(id(conv))
-        if ent is not None and ent[1] == key:
+        ent = cache.get((id(conv), transposed))
+        if not force and ent is not None and ent[1] == key:
             return ent[0], True
         kh, kw = conv.kernel_size
-        nbytes = ops.conv2d_scratch_bytes(conv.out_channels, conv.in_channels, kh, kw)
+        nbytes = ops.conv2d_scratch_bytes(conv.in_channels, conv.out_channels, kh, kw, True) if transposed else \
+            ops.conv2d_scratch_bytes(conv.out_channels, conv.in_channels, kh, kw)
         scratch = ent[0] if ent is not None and ent[0].numel() >= nbytes and ent[0].device == w.device else \
             torch.empty(max(nbytes, 16), dtype=torch.uint8, device=w.device)
-        cache[id(conv)] = (scratch, key)
+        cache[(id(conv), transposed)] = (scratch, None if force else key)
         return scratch, False
 
     def __getstate__(self):
@@ -140,10 +152,16 @@ class RCAN(nn.Module):
                 new.__dict__[k] = copy.deepcopy(v, memo)
         return new
 
-    def _conv(self, inp: Tensor, conv: nn.Conv2d, act: str = "none", res1=None, out_mode: str = "nhwc") -> Tensor:
-        scratch, pre = self._packed(conv)
+    def _conv(self, inp: Tensor, conv: nn.Conv2d, act: str = "none", res1=None, out_mode: str = "nhwc", train: bool = False) -> Tensor:
+        scratch, pre = self._packed(conv, force=train)
         return ops.conv2d_nhwc(inp, conv.weight.detach().contiguous().float(), conv.bias.detach().contiguous().float(), act=act, res1=res1,
                                out_mode=out_mode, scratch=scratch, prepacked=pre)
+
+    def _conv_t(self, g: Tensor, conv: nn.Conv2d, res1=None, res2=None, gate=None) -> Tensor:
+        """Input gradient of ``conv`` (+ res1 + res2, then * ReLU'(gate)), packed transposed on every call."""
+        scratch, _ = self._packed(conv, transposed=True, force=True)
+        return ops.conv2d_nhwc(g, conv.weight.detach().contiguous().float(), None, transposed=True, res1=res1, res2=res2, gate=gate,
+                               gate_neg=0.0, scratch=scratch)
 
     # ------------------------------------------------------------------ forward (rcan.py:175-186)
     def forward(self, x: Tensor, elev: Tensor, mask: Tensor) -> Tensor:
@@ -158,39 +176,158 @@ class RCAN(nn.Module):
         if not x.is_cuda:
             raise CsrError("climsr_b200 RCAN runs on CUDA (sm_100a) only; there is no CPU fallback")
         if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters())):
-            raise CsrError("climsr_b200 RCAN is inference-only (its backward is not implemented on the sm_100a path): call it under "
-                           "torch.no_grad() or freeze its parameters")
+            if not self.training:
+                raise CsrError("climsr_b200 RCAN trains in train() mode only (eval() mode runs the inference path): call .train() "
+                               "before the training forward, or run inference under torch.no_grad() / with frozen parameters")
+            return _RCANFunction.apply(self, x, elev, mask, *self.parameters())
+        return self._run(x, elev, mask)
+
+    def _run(self, x: Tensor, elev: Tensor, mask: Tensor, saved: Optional[dict] = None) -> Tensor:
+        """The forward launch sequence.  saved (training): filled with the activations the backward reads, every RCAB with its own
+        pooled sums; the weights are packed in every conv call."""
+        n, _, h, w = x.shape
         dev = x.device
+        train = saved is not None
         f32 = lambda t: t.detach().contiguous().float()  # noqa: E731
         with torch.cuda.device(dev):
             a = ops.nchw_to_nhwc_bf16(x.detach(), 64)
-            head = self._conv(a, self.head[0])                                   # x = self.head(x)
+            head = self._conv(a, self.head[0], train=train)                      # x = self.head(x)
             cur = head
-            pooled = torch.empty((n, 64), dtype=torch.float32, device=dev)
+            pooled = None if train else torch.empty((n, 64), dtype=torch.float32, device=dev)
+            blocks, groups = [], []
             for grp in list(self.body)[:-1]:                                     # ResidualGroup (rcan.py:104-134)
                 g_in = cur
                 for blk in list(grp.body)[:-1]:                                  # RCAB (rcan.py:71-101)
-                    t = self._conv(cur, blk.body[0], act="relu")
-                    r = self._conv(t, blk.body[2])
+                    t = self._conv(cur, blk.body[0], act="relu", train=train)
+                    r = self._conv(t, blk.body[2], train=train)
                     ca = blk.body[3].conv_du
                     out = torch.empty_like(r)
+                    if train:
+                        pooled = torch.empty((n, 64), dtype=torch.float32, device=dev)
+                        blocks.append((cur, t, r, pooled))
                     check(lib.csr_channel_attention(r.data_ptr(), cur.data_ptr(), f32(ca[0].weight).data_ptr(), f32(ca[0].bias).data_ptr(),
                                                     f32(ca[2].weight).data_ptr(), f32(ca[2].bias).data_ptr(), out.data_ptr(), pooled.data_ptr(),
                                                     n, h, w, 64, ca[0].out_channels, current_stream_ptr()), "csr_channel_attention")
                     cur = out
-                cur = self._conv(cur, grp.body[-1], res1=g_in)                   # res = body(x); res += x
-            res = self._conv(cur, self.body[-1], res1=head)                      # res = self.body(x); res += x
+                groups.append(cur)
+                cur = self._conv(cur, grp.body[-1], res1=g_in, train=train)      # res = body(x); res += x
+            body_in = cur
+            res = self._conv(cur, self.body[-1], res1=head, train=train)         # res = self.body(x); res += x
             up = self.tail[0]
             t, hh, ww = res, h, w
+            up_in = []
             for i in range(0, len(up), 2):                                       # Upsampler: conv 64 -> 256, PixelShuffle(2)
-                y4 = self._conv(t, up[i])
+                up_in.append(t)
+                y4 = self._conv(t, up[i], train=train)
                 t = torch.empty((n, 2 * hh, 2 * ww, 64), dtype=torch.bfloat16, device=dev)
                 check(lib.csr_pixel_shuffle2(y4.data_ptr(), t.data_ptr(), n, hh, ww, 64, current_stream_ptr()), "csr_pixel_shuffle2")
                 hh, ww = 2 * hh, 2 * ww
-            y = self._conv(t, self.tail[1], out_mode="f32_planar")               # (N,1,H,W) fp32
+            y = self._conv(t, self.tail[1], out_mode="f32_planar", train=train)  # (N,1,H,W) fp32
             # x = self.srcnn(torch.cat([x, elev, mask], 1))   (srcnn.py:13-18)
             cat = torch.cat([y, elev.detach().to(dev).float(), mask.detach().to(dev).float()], 1).contiguous()
             s_in = ops.nchw_to_nhwc_bf16(cat, 64)
-            s1 = self._conv(s_in, self.srcnn.conv1, act="relu")
-            s2 = self._conv(s1, self.srcnn.conv2, act="relu")
-            return self._conv(s2, self.srcnn.conv3, out_mode="f32_planar")
+            s1 = self._conv(s_in, self.srcnn.conv1, act="relu", train=train)
+            s2 = self._conv(s1, self.srcnn.conv2, act="relu", train=train)
+            if train:
+                saved.update(n=n, h=h, w=w, a=a, head=head, blocks=blocks, groups=groups, body_in=body_in, up_in=up_in, tail_in=t,
+                             s_in=s_in, s1=s1, s2=s2)
+            return self._conv(s2, self.srcnn.conv3, out_mode="f32_planar", train=train)
+
+    # ------------------------------------------------------------------ backward (autograd of rcan.py:175-186)
+    def _backward(self, sv: dict, grad_out: Tensor) -> list:
+        """Gradients of every parameter, in ``parameters()`` order, as views of one zeroed fp32 buffer."""
+        dev = grad_out.device
+        n, h, w = sv["n"], sv["h"], sv["w"]
+        params = list(self.parameters())
+        flat = torch.zeros(sum(p.numel() for p in params), dtype=torch.float32, device=dev)
+        views, off = {}, 0
+        for p in params:
+            views[p] = flat[off:off + p.numel()].view(p.shape)
+            off += p.numel()
+        f32 = lambda t: t.detach().contiguous().float()  # noqa: E731
+
+        def wgrad(x, g, conv):
+            ops.conv2d_wgrad(x, g, tuple(conv.weight.shape), dw=views[conv.weight], db=views[conv.bias])
+
+        with torch.cuda.device(dev):
+            g = ops.nchw_to_nhwc_bf16(grad_out.detach().contiguous().float(), 64)
+            # SRCNN tail: conv3 <- relu(conv2) <- relu(conv1) <- cat([y, elev, mask])
+            sr = self.srcnn
+            wgrad(sv["s2"], g, sr.conv3)
+            g = self._conv_t(g, sr.conv3, gate=sv["s2"])
+            wgrad(sv["s1"], g, sr.conv2)
+            g = self._conv_t(g, sr.conv2, gate=sv["s1"])
+            wgrad(sv["s_in"], g, sr.conv1)
+            g = self._conv_t(g, sr.conv1)                                # channel 0: dL/dy (1, 2: elev / mask, unused)
+            # Upsampler: tail.1 <- PixelShuffle <- tail.0.2 <- PixelShuffle <- tail.0.0
+            wgrad(sv["tail_in"], g, self.tail[1])
+            g = self._conv_t(g, self.tail[1])
+            up = self.tail[0]
+            for i, t in zip(range(len(up) - 2, -1, -2), reversed(sv["up_in"])):
+                hh, ww = t.shape[1], t.shape[2]
+                g4 = torch.empty((n, hh, ww, 256), dtype=torch.bfloat16, device=dev)
+                check(lib.csr_pixel_unshuffle2(g.data_ptr(), g4.data_ptr(), n, hh, ww, 64, current_stream_ptr()), "csr_pixel_unshuffle2")
+                wgrad(t, g4, up[i])
+                g = self._conv_t(g4, up[i])
+            # body: res = body(head) + head; each group: out = conv(RCABs(g_in)) + g_in; each RCAB: out = CA(res) + cur
+            d_res = g
+            wgrad(sv["body_in"], d_res, self.body[-1])
+            g = self._conv_t(d_res, self.body[-1])
+            blocks = iter(reversed(sv["blocks"]))
+            scratch = torch.empty(max(lib.csr_channel_attention_backward_scratch_bytes(n, 64), 16), dtype=torch.uint8, device=dev)
+            for grp, grp_last_in in zip(reversed(list(self.body)[:-1]), reversed(sv["groups"])):
+                d_out = g                                                  # gradient at the group output = at its input (skip)
+                wgrad(grp_last_in, d_out, grp.body[-1])
+                rcabs = list(grp.body)[:-1]
+                if not rcabs:
+                    g = self._conv_t(d_out, grp.body[-1], res1=d_out)
+                    continue
+                g = self._conv_t(d_out, grp.body[-1])
+                for k in range(len(rcabs) - 1, -1, -1):
+                    blk = rcabs[k]
+                    cur, t, r, pooled = next(blocks)
+                    ca = blk.body[3].conv_du
+                    dr = torch.empty_like(r)
+                    check(lib.csr_channel_attention_backward(g.data_ptr(), r.data_ptr(), pooled.data_ptr(), f32(ca[0].weight).data_ptr(),
+                                                             f32(ca[0].bias).data_ptr(), f32(ca[2].weight).data_ptr(), f32(ca[2].bias).data_ptr(),
+                                                             dr.data_ptr(), views[ca[0].weight].data_ptr(), views[ca[0].bias].data_ptr(),
+                                                             views[ca[2].weight].data_ptr(), views[ca[2].bias].data_ptr(), scratch.data_ptr(),
+                                                             scratch.numel(), n, h, w, 64, ca[0].out_channels, current_stream_ptr()),
+                          "csr_channel_attention_backward")
+                    wgrad(t, dr, blk.body[2])
+                    dt = self._conv_t(dr, blk.body[2], gate=t)
+                    wgrad(cur, dt, blk.body[0])
+                    # RCAB skip (+ the group skip at the group's first block)
+                    g = self._conv_t(dt, blk.body[0], res1=g, res2=d_out if k == 0 else None)
+            # dL/dhead = g + d_res (body skip): the weight gradient is linear in it - two accumulating calls instead of an add pass
+            wgrad(sv["a"], g, self.head[0])
+            wgrad(sv["a"], d_res, self.head[0])
+        return [views[p] for p in params]
+
+
+class _RCANFunction(torch.autograd.Function):
+    """Training forward / backward of RCAN on the sm_100a kernels.  The saved activations live on this node (``ctx.saved``) and
+    are released by its backward or with the graph."""
+
+    @staticmethod
+    def forward(ctx, module, x, elev, mask, *params):
+        saved = {}
+        out = module._run(x, elev, mask, saved)
+        ctx.module, ctx.saved = module, saved
+        ctx.set_materialize_grads(False)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        n_in = 4 + len(list(ctx.module.parameters()))
+        if grad_out is None:
+            return (None,) * n_in
+        if ctx.needs_input_grad[1]:
+            raise CsrError("climsr_b200: the generator does not produce a gradient for its input x (it is data in the reference's "
+                           "training loop, climsr/task/pl_generator_pre_training.py:18-33); detach x or clear requires_grad")
+        if ctx.saved is None:
+            raise CsrError("RCAN's saved activations were released by its first backward; a second backward through the same forward "
+                           "(retain_graph=True) is not supported - run the forward again")
+        grads = ctx.module._backward(ctx.saved, grad_out)
+        ctx.saved = None
+        return (None, None, None, None) + tuple(grads)

@@ -350,7 +350,10 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
   // Thin layers (<= 32 output channels: four accumulator buffers) are bound by the per-tile work of the producer and
   // MMA-issuer warps (~110 / ~250 scalar instructions at ~5 clk each), not by MMAs or bytes: give them windows of two M
   // tiles, which halves that work per tile and shrinks the halo from 6/4 to 10/8 rows.
-  if (pp.stream) {
+  // A layer of ONE k-block (<= 64 input channels, e.g. the 9x9 input gradient of srcnn.conv1) streams its whole weights as that
+  // k-block: two slots never fit, so it keeps the weights resident next to a shallower window ring instead.
+  const bool stream_w = pp.stream && p.n_kblocks > 1;
+  if (stream_w) {
     p.stream_w = 1;
     p.n_groups = 1;                                        // one staging buffer: two (window + weight k-block) slots of ~96 KB must fit
     p.wkb_bytes = pp.kh * 4 * pp.kw * pp.npad * 32;
@@ -2016,12 +2019,24 @@ int csr_conv2d_wgrad(const CsrWgradDesc* d, const void* x, const void* g, float*
   float* dacc = reinterpret_cast<float*>(scratch);
   if (wgrad_jobs_applicable(L, d->n, d->h, d->w, di.sms))
     return run_wgrad_layer_jobs(L, d->n, d->h, d->w, x, d->x_c, d->x_coff, g, d->g_c, d->g_coff, d->scale, dw, db, dacc, di.sms, s);
-  std::vector<Op> ops;
-  rc = emit_wgrad(ops, L, 0, d->n, d->h, d->w, x, d->x_c, d->x_coff, g, d->g_c, d->g_coff, d->scale, db != nullptr, dacc, di.sms);
-  if (rc) return rc;
-  Bindings b;
-  b.dw = &dw; b.db = &db;
-  return run_ops(ops, 0, ops.size(), b, di.sms, s);
+  // Output channels in chunks whose KW x chunk accumulator columns fit the 512 TMEM columns (one chunk for every layer up to 5x5 / 64
+  // channels; the 9x9 srcnn.conv1 with 64 output channels takes two).
+  const int ekw = L.up2 ? 2 : L.kw;
+  const int chunk = std::max(16, std::min((L.cout + 15) / 16 * 16, 512 / ekw / 16 * 16));
+  for (int co0 = 0; co0 < L.cout; co0 += chunk) {
+    LayerSpec Lc = L;
+    Lc.cout = std::min(chunk, L.cout - co0);
+    std::vector<Op> ops;
+    rc = emit_wgrad(ops, Lc, 0, d->n, d->h, d->w, x, d->x_c, d->x_coff, g, d->g_c, d->g_coff + co0, d->scale, db != nullptr, dacc, di.sms);
+    if (rc) return rc;
+    float* dwc = dw + (size_t)co0 * L.cin * L.kh * L.kw;
+    float* dbc = db ? db + co0 : nullptr;
+    Bindings b;
+    b.dw = &dwc; b.db = &dbc;
+    rc = run_ops(ops, 0, ops.size(), b, di.sms, s);
+    if (rc) return rc;
+  }
+  return CSR_OK;
 }
 
 // ---- layout helpers -----------------------------------------------------------------------------------
@@ -2203,7 +2218,7 @@ int csr_linear_backward(const float* x, const float* w, const float* gy, float* 
   return CSR_OK;
 }
 
-// ---- RCAN generator: glue between the convolutions (rcan.cu) ---------------------------------------------------------
+// ---- RCAN generator: glue between the convolutions (rcan.cu), forward and backward ---------------------------------------------------------
 int csr_channel_attention(const void* res, const void* x, const float* w1, const float* b1, const float* w2, const float* b2, void* out,
                           float* pooled_scratch, int32_t n, int32_t h, int32_t w, int32_t c, int32_t c_reduced, void* stream) {
   if (!res || !x || !w1 || !b1 || !w2 || !b2 || !out || !pooled_scratch) return fail(CSR_ERR_BAD_ARG, "null pointer");
@@ -2218,6 +2233,26 @@ int csr_channel_attention(const void* res, const void* x, const float* w1, const
 int csr_pixel_shuffle2(const void* src, void* dst, int32_t n, int32_t h, int32_t w, int32_t c, void* stream) {
   if (!src || !dst || n < 1 || h < 1 || w < 1 || c < 8 || c % 8) return fail(CSR_ERR_BAD_ARG, "csr_pixel_shuffle2: bad arguments");
   CSR_CUDA(launch_pixel_shuffle2(src, dst, n, h, w, c, reinterpret_cast<cudaStream_t>(stream)));
+  ++g_launches;
+  return CSR_OK;
+}
+size_t csr_channel_attention_backward_scratch_bytes(int32_t n, int32_t c) { return n > 0 && c > 0 ? (size_t)n * c * sizeof(float) : 0; }
+int csr_channel_attention_backward(const void* dout, const void* res, const float* pooled, const float* w1, const float* b1, const float* w2,
+                                   const float* b2, void* dres, float* dw1, float* db1, float* dw2, float* db2, void* scratch,
+                                   size_t scratch_bytes, int32_t n, int32_t h, int32_t w, int32_t c, int32_t c_reduced, void* stream) {
+  if (!dout || !res || !pooled || !w1 || !b1 || !w2 || !b2 || !dres || !dw1 || !db1 || !dw2 || !db2 || !scratch)
+    return fail(CSR_ERR_BAD_ARG, "null pointer");
+  if (n < 1 || n > 65535 || h < 1 || w < 1 || c < 8 || c % 8 || c > 512 || c_reduced < 1 || c_reduced > c)
+    return fail(CSR_ERR_BAD_ARG, "csr_channel_attention_backward: bad shape n=%d h=%d w=%d c=%d c_reduced=%d", n, h, w, c, c_reduced);
+  if (scratch_bytes < csr_channel_attention_backward_scratch_bytes(n, c)) return fail(CSR_ERR_WORKSPACE, "channel-attention backward scratch too small");
+  CSR_CUDA(launch_ca_backward(dout, res, pooled, w1, b1, w2, b2, dres, dw1, db1, dw2, db2, reinterpret_cast<float*>(scratch), n, (long)h * w, c,
+                              c_reduced, reinterpret_cast<cudaStream_t>(stream)));
+  g_launches += 2;
+  return CSR_OK;
+}
+int csr_pixel_unshuffle2(const void* src, void* dst, int32_t n, int32_t h, int32_t w, int32_t c, void* stream) {
+  if (!src || !dst || n < 1 || h < 1 || w < 1 || c < 8 || c % 8) return fail(CSR_ERR_BAD_ARG, "csr_pixel_unshuffle2: bad arguments");
+  CSR_CUDA(launch_pixel_unshuffle2(src, dst, n, h, w, c, reinterpret_cast<cudaStream_t>(stream)));
   ++g_launches;
   return CSR_OK;
 }

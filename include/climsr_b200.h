@@ -270,16 +270,29 @@ int     csr_linear_forward(const float* x, const float* w, const float* b, float
 int     csr_linear_backward(const float* x, const float* w, const float* gy, float* dx, float* dw, float* db, int32_t n,
                             int32_t k, int32_t j, void* stream);
 
-/* ---- RCAN generator (SURVEY section 8f row 4; inference) ---------------------------------------------------------------
- * climsr.models.rcan.RCAN.forward (climsr/models/rcan.py:175-186): every 3x3 conv (+ ReLU, + the ResidualGroup / body skips as
- * epilogue residuals) runs on csr_conv2d_nhwc; these two entry points are the rest of an RCAB and of the Upsampler.
+/* ---- RCAN generator (SURVEY section 8f row 4) --------------------------------------------------------------------------
+ * climsr.models.rcan.RCAN.forward (climsr/models/rcan.py:175-186) and its autograd backward: every 3x3 conv (+ ReLU, + the
+ * ResidualGroup / body skips as epilogue residuals) runs on csr_conv2d_nhwc, its input gradient on the same entry point with
+ * transposed weights (ReLU' as a gate with gate_neg = 0) and its weight gradient on csr_conv2d_wgrad; these entry points are the
+ * rest of an RCAB and of the Upsampler.
  *   csr_channel_attention  out = res * sigmoid(W2 relu(W1 avgpool(res) + b1) + b2) + x        (CALayer + RCAB skip, rcan.py:50-101)
  *                          res, x, out: bf16 NHWC (n,h,w,c); w1 (c_reduced, c), w2 (c, c_reduced) fp32; pooled_scratch: n*c floats
- *   csr_pixel_shuffle2     dst (n,2h,2w,c) = nn.PixelShuffle(2)(src (n,h,w,4c))                 (Upsampler, rcan.py:30-36)          */
+ *                          (on return: the per-image channel sums of res, which the backward takes as `pooled`)
+ *   csr_channel_attention_backward   its adjoint w.r.t. res given dout = dL/dout: dres = dout * gate + d(avgpool)/dres, gate
+ *                          recomputed from `pooled`; dw1, db1, dw2, db2 (fp32, shapes of w1, b1, w2, b2) are ACCUMULATED (+=).
+ *                          The skip gradient dL/dx = dout is not written.  scratch: csr_channel_attention_backward_scratch_bytes
+ *   csr_pixel_shuffle2     dst (n,2h,2w,c) = nn.PixelShuffle(2)(src (n,h,w,4c))                 (Upsampler, rcan.py:30-36)
+ *   csr_pixel_unshuffle2   dst (n,h,w,4c) = nn.PixelUnshuffle(2)(src (n,2h,2w,c)), the adjoint of csr_pixel_shuffle2          */
 int     csr_channel_attention(const void* res, const void* x, const float* w1, const float* b1, const float* w2, const float* b2,
                               void* out, float* pooled_scratch, int32_t n, int32_t h, int32_t w, int32_t c, int32_t c_reduced,
                               void* stream);
+size_t  csr_channel_attention_backward_scratch_bytes(int32_t n, int32_t c);
+int     csr_channel_attention_backward(const void* dout, const void* res, const float* pooled, const float* w1, const float* b1,
+                                       const float* w2, const float* b2, void* dres, float* dw1, float* db1, float* dw2,
+                                       float* db2, void* scratch, size_t scratch_bytes, int32_t n, int32_t h, int32_t w,
+                                       int32_t c, int32_t c_reduced, void* stream);
 int     csr_pixel_shuffle2(const void* src, void* dst, int32_t n, int32_t h, int32_t w, int32_t c, void* stream);
+int     csr_pixel_unshuffle2(const void* src, void* dst, int32_t n, int32_t h, int32_t w, int32_t c, void* stream);
 
 /* ---- gradient exchange of data-parallel training (SURVEY section 8e: "bf16 gradients are reduced with NCCL over NVLink,
  * bucketed and overlapped with backward"; replaces the gradient all-reduce of Lightning's DDP plugin, conf/trainer/
