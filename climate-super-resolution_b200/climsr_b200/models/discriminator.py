@@ -220,8 +220,19 @@ class Discriminator(nn.Module):
         return self._forward_saving(x, save=False)[0]
 
     # ------------------------------------------------------------------ CUDA-graph slots
+    def _check_bn_momentum(self) -> None:
+        """A training-mode forward updates the running statistics with a fixed ``momentum``, which graph replays bake into their
+        launches.  PyTorch's ``momentum=None`` (cumulative average, factor 1 / num_batches_tracked, a new value every call) is
+        rejected instead of silently replaced."""
+        if not self.training:
+            return
+        for i, (_, bn, _) in enumerate(self._layers()[0]):
+            if bn.track_running_stats and bn.momentum is None:
+                raise CsrError(f"BatchNorm of discriminator stage {i + 1} has momentum=None (cumulative moving average): not supported "
+                               "by climsr_b200 Discriminator in training mode - set a float momentum (PyTorch's default is 0.1)")
+
     def _graph_key(self, x: Tensor, save: bool):
-        bn_mode = tuple(self.training or not st[1].track_running_stats for st in self._layers()[0])
+        bn_mode = tuple((self.training or not st[1].track_running_stats, st[1].momentum, st[1].eps) for st in self._layers()[0])
         ptrs = tuple(t.data_ptr() for t in self.parameters()) + tuple(t.data_ptr() for t in self.buffers())
         return (x.device, x.shape[0], save, bn_mode, ptrs)
 
@@ -230,6 +241,7 @@ class Discriminator(nn.Module):
 
     def _forward_saving(self, x: Tensor, save: bool = True):
         """(scores, saved, lease).  Eager for the first calls of a kind, then a graph replay on a leased slot."""
+        self._check_bn_momentum()
         with torch.cuda.device(x.device):
             self._refresh_packs(False)
             if not self._graphs_usable(x):
@@ -335,10 +347,12 @@ class Discriminator(nn.Module):
                 nbytes = lib.csr_disc_bn_scratch_bytes(c)
                 scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev)
                 training = self.training or not bn.track_running_stats
+                if training and bn.track_running_stats and bn.momentum is None:
+                    self._check_bn_momentum()
                 if training and bn.track_running_stats and bn.num_batches_tracked is not None:
                     bn.num_batches_tracked += 1
                 check(lib.csr_disc_bn_forward(sa.data_ptr(), C.byref(va), n, f32(bn.weight).data_ptr(), f32(bn.bias).data_ptr(), float(bn.eps),
-                                              float(bn.momentum if bn.momentum is not None else 0.1),
+                                              float(bn.momentum if bn.momentum is not None else 0.0),     # unused without running statistics
                                               _ptr(bn.running_mean if bn.track_running_stats else None),
                                               _ptr(bn.running_var if bn.track_running_stats else None), 1 if training else 0,
                                               scale.data_ptr(), shift.data_ptr(), mean.data_ptr(), invstd.data_ptr(), scratch.data_ptr(), nbytes,

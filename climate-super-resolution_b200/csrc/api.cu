@@ -2167,7 +2167,7 @@ int csr_disc_bn_forward(const void* src, const CsrView* view, int32_t n, const f
   if (!mean || !invstd || !scratch || scratch_bytes < csr_disc_bn_scratch_bytes(v.C)) return fail(CSR_ERR_WORKSPACE, "BatchNorm scratch / statistics buffers");
   if ((running_mean == nullptr) != (running_var == nullptr)) return fail(CSR_ERR_BAD_ARG, "running_mean and running_var go together");
   CSR_CUDA(launch_disc_bn_stats(src, v, n, reinterpret_cast<double*>(scratch), s));
-  CSR_CUDA(launch_disc_bn_finalize(reinterpret_cast<double*>(scratch), v.C, (double)n * v.Hl * v.Wl, gamma, beta, eps, momentum, running_mean,
+  CSR_CUDA(launch_disc_bn_finalize(reinterpret_cast<double*>(scratch), src, v, (double)n * v.Hl * v.Wl, gamma, beta, eps, momentum, running_mean,
                                    running_var, scale, shift, mean, invstd, s));
   g_launches += 2;
   return CSR_OK;
@@ -2214,7 +2214,7 @@ int csr_linear_backward(const float* x, const float* w, const float* gy, float* 
                         void* stream) {
   if (!x || !w || !gy || n < 1 || k < 1 || j < 1) return fail(CSR_ERR_BAD_ARG, "csr_linear_backward: bad arguments");
   CSR_CUDA(launch_linear_backward(x, w, gy, dx, dw, db, n, k, j, reinterpret_cast<cudaStream_t>(stream)));
-  g_launches += (dx ? 1 : 0) + (dw ? 1 : 0);
+  g_launches += (dx ? 1 : 0) + ((dw || db) ? 1 : 0);
   return CSR_OK;
 }
 

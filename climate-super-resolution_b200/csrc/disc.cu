@@ -130,13 +130,19 @@ __device__ __forceinline__ void block_reduce_to_sums(const float (&s)[8], const 
 }
 
 // ---- BatchNorm2d, training mode (batch statistics over the logical pixels) ---------------------------------------------
-// sums[c] += x, sums[C + c] += x^2 (double atomics; a few hundred blocks)
+// The sums are taken of x - pivot[c], pivot = the channel's first logical pixel (image 0, pixel (0, 0)): with raw x, the fp32
+// per-thread partials of x^2 carry mean^2 and the variance E[x^2] - mean^2 cancels their rounding error into the result
+// (invstd 1.8e-4 off at mean = 100 std, 16 x 128 x 128 pixels); around a pivot a few std from the mean nothing cancels.
+__device__ __forceinline__ long bn_pivot_index(const DiscView& v) { return (static_cast<long>(v.off) * v.Ws + v.off) * v.C; }
+
+// sums[c] += x - pivot[c], sums[C + c] += (x - pivot[c])^2 (double atomics; a few hundred blocks)
 __global__ void disc_bn_stats_kernel(const __nv_bfloat16* __restrict__ src, DiscView v, int N, double* __restrict__ sums) {
   const int c8n = v.C >> 3;
   const int c8 = threadIdx.x % c8n;                       // blockDim.x is a multiple of C/8: a thread keeps its channel group
   const int lanes = blockDim.x / c8n;
   const long npix = static_cast<long>(N) * v.Hl * v.Wl;
-  float s[8], q[8];
+  float s[8], q[8], piv[8];
+  unpack8(*reinterpret_cast<const uint4*>(src + bn_pivot_index(v) + c8 * 8), piv);
 #pragma unroll
   for (int k = 0; k < 8; ++k) s[k] = q[k] = 0.f;
   for (long p = blockIdx.x * static_cast<long>(lanes) + threadIdx.x / c8n; p < npix; p += static_cast<long>(gridDim.x) * lanes) {
@@ -147,21 +153,27 @@ __global__ void disc_bn_stats_kernel(const __nv_bfloat16* __restrict__ src, Disc
     float f[8];
     unpack8(*reinterpret_cast<const uint4*>(src + ((static_cast<long>(n) * v.Hs + v.off + v.step * i) * v.Ws + v.off + v.step * j) * v.C + c8 * 8), f);
 #pragma unroll
-    for (int k = 0; k < 8; ++k) { s[k] += f[k]; q[k] += f[k] * f[k]; }
+    for (int k = 0; k < 8; ++k) {
+      const float d = f[k] - piv[k];                      // exact: two bf16 values
+      s[k] += d;
+      q[k] += d * d;
+    }
   }
   block_reduce_to_sums(s, q, v.C, c8, c8n, sums);
 }
 
-// mean / biased variance -> scale = gamma * invstd, shift = beta - mean * scale; saves (mean, invstd) for the backward and
+// mean = pivot + sum(x - pivot) / M, biased variance from the pivot-shifted sums -> scale = gamma * invstd, shift = beta - mean * scale; saves (mean, invstd) for the backward and
 // updates the running statistics like nn.BatchNorm2d (momentum, unbiased variance).
-__global__ void disc_bn_finalize_kernel(const double* __restrict__ sums, int C, double count, const float* __restrict__ gamma,
-                                        const float* __restrict__ beta, float eps, float momentum, float* __restrict__ running_mean,
+__global__ void disc_bn_finalize_kernel(const double* __restrict__ sums, const __nv_bfloat16* __restrict__ src, DiscView v, double count,
+                                        const float* __restrict__ gamma, const float* __restrict__ beta, float eps, float momentum, float* __restrict__ running_mean,
                                         float* __restrict__ running_var, float* __restrict__ scale, float* __restrict__ shift,
                                         float* __restrict__ mean_out, float* __restrict__ invstd_out) {
+  const int C = v.C;
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= C) return;
-  const double mean = sums[c] / count;
-  const double var = fmax(sums[C + c] / count - mean * mean, 0.0);
+  const double d = sums[c] / count;                       // mean of x - pivot
+  const double mean = static_cast<double>(__bfloat162float(src[bn_pivot_index(v) + c])) + d;
+  const double var = fmax(sums[C + c] / count - d * d, 0.0);
   const float invstd = static_cast<float>(1.0 / sqrt(var + static_cast<double>(eps)));
   const float sc = gamma[c] * invstd;
   scale[c] = sc;
@@ -334,6 +346,14 @@ __global__ void linear_bwd_w_kernel(const float* __restrict__ gy, const float* _
     }
   }
 }
+// db[j] += sum_n gy[n][j] alone (dW not wanted); same summation order as linear_bwd_w_kernel
+__global__ void linear_bwd_b_kernel(const float* __restrict__ gy, float* __restrict__ db, int N, int J) {
+  for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < J; j += gridDim.x * blockDim.x) {
+    float sb = 0.f;
+    for (int n = 0; n < N; ++n) sb += gy[static_cast<long>(n) * J + j];
+    db[j] += sb;
+  }
+}
 
 inline int grid_for(long total, int block, int cap = 148 * 8) {
   long g = (total + block - 1) / block;
@@ -367,11 +387,11 @@ cudaError_t launch_disc_bn_stats(const void* src, const DiscView& v, int N, doub
       reinterpret_cast<const __nv_bfloat16*>(src), v, N, sums);
   return cudaGetLastError();
 }
-cudaError_t launch_disc_bn_finalize(const double* sums, int C, double count, const float* gamma, const float* beta, float eps, float momentum,
-                                    float* running_mean, float* running_var, float* scale, float* shift, float* mean, float* invstd,
-                                    cudaStream_t s) {
-  disc_bn_finalize_kernel<<<(C + 127) / 128, 128, 0, s>>>(sums, C, count, gamma, beta, eps, momentum, running_mean, running_var, scale, shift, mean,
-                                                          invstd);
+cudaError_t launch_disc_bn_finalize(const double* sums, const void* src, const DiscView& v, double count, const float* gamma, const float* beta,
+                                    float eps, float momentum, float* running_mean, float* running_var, float* scale, float* shift, float* mean,
+                                    float* invstd, cudaStream_t s) {
+  disc_bn_finalize_kernel<<<(v.C + 127) / 128, 128, 0, s>>>(sums, reinterpret_cast<const __nv_bfloat16*>(src), v, count, gamma, beta, eps,
+                                                            momentum, running_mean, running_var, scale, shift, mean, invstd);
   return cudaGetLastError();
 }
 cudaError_t launch_disc_bn_eval(int C, const float* gamma, const float* beta, float eps, const float* running_mean, const float* running_var,
@@ -411,6 +431,7 @@ cudaError_t launch_linear_backward(const float* x, const float* W, const float* 
                                    cudaStream_t s) {
   if (dx) linear_bwd_x_kernel<<<grid_for(static_cast<long>(N) * K, 256), 256, 0, s>>>(gy, W, dx, N, K, J);
   if (dW) linear_bwd_w_kernel<<<grid_for(static_cast<long>(J) * K, 256), 256, 0, s>>>(gy, x, dW, db, N, K, J);
+  else if (db) linear_bwd_b_kernel<<<grid_for(J, 256), 256, 0, s>>>(gy, db, N, J);
   return cudaGetLastError();
 }
 

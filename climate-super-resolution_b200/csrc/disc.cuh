@@ -15,7 +15,7 @@ struct DiscView {
 cudaError_t launch_disc_gather(const void* src, const DiscView& v, int N, void* dst, int pad, const float* scale, const float* shift, cudaStream_t s);
 cudaError_t launch_disc_collect(const void* dP, const DiscView& v, int N, int pad, const void* act, float gate_neg, void* g, cudaStream_t s);
 cudaError_t launch_disc_bn_stats(const void* src, const DiscView& v, int N, double* sums, cudaStream_t s);
-cudaError_t launch_disc_bn_finalize(const double* sums, int C, double count, const float* gamma, const float* beta, float eps, float momentum,
+cudaError_t launch_disc_bn_finalize(const double* sums, const void* src, const DiscView& v, double count, const float* gamma, const float* beta, float eps, float momentum,
                                     float* running_mean, float* running_var, float* scale, float* shift, float* mean, float* invstd, cudaStream_t s);
 cudaError_t launch_disc_bn_eval(int C, const float* gamma, const float* beta, float eps, const float* running_mean, const float* running_var,
                                 float* scale, float* shift, cudaStream_t s);

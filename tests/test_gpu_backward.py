@@ -28,6 +28,17 @@ WGRAD_CASES = [
     (1, 24, 24, 192, 64, 3, 0),         # gc=32 conv5: two 128-channel chunks
     (1, 1, 1, 64, 64, 3, 0),            # single pixel
     (1, 113, 113, 64, 64, 3, 0),        # Europe-extent LR raster
+    # the discriminator's ten convs at the GAN step's batch 16 (same-convs over the padded maps; job mode from 128 channels on)
+    (16, 130, 130, 1, 64, 3, 0),        # stage 1 conv_a: one input channel in a 64-channel buffer
+    (16, 130, 130, 64, 64, 3, 0),       # stage 1 conv_b
+    (16, 66, 66, 64, 128, 3, 0),        # stage 2 conv_a
+    (16, 66, 66, 128, 128, 3, 0),       # stage 2 conv_b
+    (16, 34, 34, 128, 256, 3, 0),       # stage 3 conv_a
+    (16, 34, 34, 256, 256, 3, 0),       # stage 3 conv_b
+    (16, 18, 18, 256, 512, 3, 0),       # stage 4 conv_a
+    (16, 18, 18, 512, 512, 3, 0),       # stage 4 conv_b
+    (16, 8, 8, 512, 512, 3, 0),         # conv4
+    (16, 6, 6, 512, 512, 3, 0),         # conv5
 ]
 
 
@@ -40,11 +51,15 @@ def test_wgrad_matches_autograd(n, h, w, cin, cout, k, up2):
     gy = (torch.rand((n, cout, s * h, s * w), generator=g) * 2 - 1).to(torch.bfloat16).float()
     wt = torch.zeros((cout, cin, k, k), dtype=torch.float64, requires_grad=True)
     xin = F.interpolate(x, scale_factor=2, mode="nearest") if up2 else x
-    (dw_ref,) = torch.autograd.grad(F.conv2d(xin.double(), wt, None, padding=k // 2), wt, gy.double())
+    # fp64 on the GPU for the large layers (the same fp64 arithmetic, seconds instead of minutes on the host)
+    dev = "cuda" if n * h * w * cin * cout > 1 << 26 else "cpu"
+    wt = wt.detach().to(dev).requires_grad_(True)
+    (dw_ref,) = torch.autograd.grad(F.conv2d(xin.to(dev).double(), wt, None, padding=k // 2), wt, gy.to(dev).double())
+    dw_ref = dw_ref.cpu()
     db_ref = gy.double().sum(dim=(0, 2, 3))
     xb = torch.zeros((n, h, w, (cin + 63) // 64 * 64), dtype=torch.bfloat16)
     xb[..., :cin] = x.permute(0, 2, 3, 1).to(torch.bfloat16)
-    gb = torch.full((n, s * h, s * w, 64), 3.0, dtype=torch.bfloat16)      # channels >= cout must never be used
+    gb = torch.full((n, s * h, s * w, (cout + 63) // 64 * 64), 3.0, dtype=torch.bfloat16)      # channels >= cout must never be used
     gb[..., :cout] = gy.permute(0, 2, 3, 1).to(torch.bfloat16)
     dw = torch.ones((cout, cin, k, k), device="cuda")                        # accumulate semantics: dw += scale * grad
     db = torch.ones((cout,), device="cuda")

@@ -19,10 +19,12 @@ def _bf(t):
     return t.to(torch.bfloat16).float()
 
 
-def _ref_conv(x, w, b, act):
+def _ref_conv(x, w, b, act, slope=0.0):
     y = F.conv2d(_bf(x).double(), _bf(w).double(), b.double(), padding=(w.shape[2] // 2, w.shape[3] // 2))
     if act == "lrelu":
         y = F.leaky_relu(y, 0.2)
+    elif act == "lrelu_slope":
+        y = F.leaky_relu(y, slope)
     elif act == "relu":
         y = F.relu(y)
     return y.float()
@@ -52,12 +54,26 @@ CONV_CASES = [
     (1, 113, 113, 64, 64, 3, "lrelu", 64),     # Europe-extent LR raster
     (2, 9, 11, 64, 24, 3, "relu", 64),         # cout multiple of 8 but not 16
     (1, 7, 33, 64, 20, 3, "none", 64),         # ragged cout: per-element store path
+    # the discriminator's ten convs at the GAN step's batch 16, as the same-convs over their padded maps it runs
+    # ("lrelu_slope=s": LeakyReLU(s) epilogue; stride 2 reads every second pixel of the same-conv's output)
+    (16, 130, 130, 1, 64, 3, "lrelu_slope=0.01", 64),      # stage 1 conv_a: one input channel in a 64-channel buffer
+    (16, 130, 130, 64, 64, 3, "lrelu_slope=0.01", 64),     # stage 1 conv_b (stride 2)
+    (16, 66, 66, 64, 128, 3, "lrelu_slope=0.01", 64),      # stage 2 conv_a
+    (16, 66, 66, 128, 128, 3, "lrelu_slope=0.01", 128),    # stage 2 conv_b
+    (16, 34, 34, 128, 256, 3, "lrelu_slope=0.01", 128),    # stage 3 conv_a
+    (16, 34, 34, 256, 256, 3, "lrelu_slope=0.01", 256),    # stage 3 conv_b: k-block weight streaming, output-channel parts
+    (16, 18, 18, 256, 512, 3, "lrelu_slope=0.01", 256),    # stage 4 conv_a
+    (16, 18, 18, 512, 512, 3, "lrelu_slope=0.01", 512),    # stage 4 conv_b
+    (16, 8, 8, 512, 512, 3, "lrelu_slope=0.2", 512),       # conv4 (valid)
+    (16, 6, 6, 512, 512, 3, "none", 512),                  # conv5 (valid)
 ]
 
 
 @pytest.mark.parametrize("n,h,w,cin,cout,k,act,in_c", CONV_CASES)
 def test_conv_matches_fp32_reference(n, h, w, cin, cout, k, act, in_c):
     from climsr_b200 import ops
+    act, _, slope = act.partition("=")
+    slope = float(slope or 0.0)
     g = torch.Generator().manual_seed(n * 1000 + h * 10 + cin + k)
     x = torch.rand((n, cin, h, w), generator=g) * 2 - 1
     wt = (torch.rand((cout, cin, k, k), generator=g) * 2 - 1) / (cin * k * k) ** 0.5
@@ -65,9 +81,11 @@ def test_conv_matches_fp32_reference(n, h, w, cin, cout, k, act, in_c):
     xin = _nhwc(x, in_c)
     if cin % 16 == 0 and in_c > cin:
         xin[..., cin:] = 9.0          # channels beyond cin must never be multiplied
-    out = ops.conv2d_nhwc(xin, wt.cuda(), b.cuda(), act=act)
+    out = ops.conv2d_nhwc(xin, wt.cuda(), b.cuda(), act=act, act_slope=slope)
     got = out[..., :cout].float().cpu().permute(0, 3, 1, 2)
-    want = _ref_conv(x, wt, b, act)
+    # fp64 on the GPU for the large layers (the same fp64 arithmetic, seconds instead of minutes on the host)
+    dev = "cuda" if n * h * w * cin * cout > 1 << 26 else "cpu"
+    want = _ref_conv(x.to(dev), wt.to(dev), b.to(dev), act, slope).cpu()
     assert torch.isfinite(got).all()
     # bf16 output rounding: half an ulp relative (2^-9) plus fp32 accumulation noise
     assert float((got - want).abs().max()) <= 2.0 ** -8 * max(1.0, float(want.abs().max()))
