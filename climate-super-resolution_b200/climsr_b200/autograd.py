@@ -35,8 +35,7 @@ class GeneratorFunction(torch.autograd.Function):
         module._fwd_serial += 1
         module._train_plan = plan
         # an optimizer step normally follows: whatever the version counters say, the next inference forward repacks
-        module._packed_key = None
-        module._packed_bwd_key = None
+        module._invalidate_packs()
         ctx.module, ctx.plan, ctx.serial, ctx.dev = module, plan, module._fwd_serial, dev
         ctx.shapes = [tuple(p.shape) for p in params]
         ctx.set_materialize_grads(False)

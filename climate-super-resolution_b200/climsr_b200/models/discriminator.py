@@ -32,6 +32,7 @@ from torch import Tensor
 
 from .. import ops
 from .._lib import CsrError, View, check, current_stream_ptr, lib
+from ._common import DerivedState, f32, flat_grad_views
 
 SLOPE = 0.01            # nn.LeakyReLU() default, discriminator.py:15,23
 SLOPE_TAIL = 0.2        # discriminator.py:33
@@ -130,7 +131,8 @@ class _Lease:
         self.release()
 
 
-class Discriminator(nn.Module):
+class Discriminator(DerivedState, nn.Module):
+    _DERIVED = ("_slots", "_calls")
     use_cuda_graphs = True          # replay forward / backward as CUDA graphs from the third call of a kind on
     _EAGER_CALLS = 2                # calls of a kind that run eagerly first (module load, attribute set-up, both calls of a first GAN batch)
 
@@ -156,26 +158,12 @@ class Discriminator(nn.Module):
     def _packed(self, conv: nn.Conv2d, transposed: bool):
         """(scratch, True): the layer's packed bf16 weight tiles, re-packed (csr_conv2d_pack, outside any graph) only when the
         weights changed - the four forwards and two backwards of a GAN batch (pl_gan.py:28-61) see at most two weight versions.
-        Keyed like the generator's pack cache: storage pointer, version counter and the process-wide optimizer-step epoch (fused
-        optimizers do not bump version counters).  The scratch tensor of a layer is never reallocated, so captured graphs that
-        read it stay valid across weight updates."""
-        from .esrgan import _WEIGHT_EPOCH
-        cache = self.__dict__.setdefault("_pack_cache", {})
-        w, b = conv.weight, conv.bias
-        key = (w.data_ptr(), w._version, b.data_ptr(), b._version, _WEIGHT_EPOCH[0], w.device)
-        ent = cache.get((id(conv), transposed))
-        if ent is not None and ent[1] == key:
-            return ent[0], True
-        if ent is not None and ent[0].device == w.device:
-            scratch = ent[0]
-        else:
-            nbytes = ops.conv2d_scratch_bytes(conv.out_channels, conv.in_channels, 3, 3, False) if not transposed else \
-                ops.conv2d_scratch_bytes(conv.in_channels, conv.out_channels, 3, 3, True)
-            scratch = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=w.device)
+        Keyed like the generator's pack cache (``weights_key``).  The scratch tensor of a layer is reallocated only when its
+        device changes, so captured graphs that read it stay valid across weight updates."""
+        scratch, pre, new = self._layer_pack(conv, transposed, pack=True)
+        if new:
             self.__dict__["_slots"] = {}                      # new scratch storage: graphs captured over the old one are stale
-        ops.conv2d_pack(w, None if transposed else b, scratch, transposed)
-        cache[(id(conv), transposed)] = (scratch, key)
-        return scratch, True
+        return scratch, pre
 
     def _refresh_packs(self, transposed: bool) -> None:
         stages, conv4, conv5, _, _ = self._layers()
@@ -184,21 +172,6 @@ class Discriminator(nn.Module):
             self._packed(conv_b, transposed)
         self._packed(conv4, transposed)
         self._packed(conv5, transposed)
-
-    def __getstate__(self):
-        state = dict(self.__dict__)
-        for k in ("_pack_cache", "_slots", "_calls"):
-            state.pop(k, None)
-        return state
-
-    def __deepcopy__(self, memo):
-        import copy
-        new = self.__class__.__new__(self.__class__)
-        memo[id(self)] = new
-        for k, v in self.__dict__.items():
-            if k not in ("_pack_cache", "_slots", "_calls"):
-                new.__dict__[k] = copy.deepcopy(v, memo)
-        return new
 
     # ------------------------------------------------------------------ layer table
     def _layers(self):
@@ -313,14 +286,7 @@ class Discriminator(nn.Module):
             graph.replay()
             # the static buffers are overwritten by the next replay: hand out copies (one for all parameter gradients)
             dx_out = dx.clone() if dx is not None else None
-            if flat is not None:
-                fc = flat.clone()
-                out, off = [], 0
-                for g in grads:
-                    out.append(fc[off:off + g.numel()].view(g.shape))
-                    off += g.numel()
-            else:
-                out = grads
+            out = flat_grad_views(grads, gy.device, flat.clone())[1] if flat is not None else grads
             lease.release()
             return dx_out, out
 
@@ -329,7 +295,6 @@ class Discriminator(nn.Module):
         dev = x.device
         n = x.shape[0]
         stages, conv4, conv5, lin0, lin1 = self._layers()
-        f32 = lambda t: t.detach().contiguous().float()  # noqa: E731
         with torch.cuda.device(dev):
             a0 = ops.nchw_to_nhwc_bf16(x.detach(), 64)                            # (N,128,128,64), channel 0 = the image, the rest zero
             buf, view = a0, View(128, 128, 64, 0, 1, 128, 128)
@@ -388,7 +353,6 @@ class Discriminator(nn.Module):
         dev = gy.device
         n = sv["n"]
         stages, conv4, conv5, lin0, lin1 = self._layers()
-        f32 = lambda t: t.detach().contiguous().float()  # noqa: E731
         grads = {}
         # every parameter gradient is a view of ONE zeroed buffer (parameters() order): one memset instead of 24, and one copy when a
         # graph replay hands the gradients out
@@ -396,15 +360,8 @@ class Discriminator(nn.Module):
         flat = None
         gviews = {}
         if need_params:
-            total = sum(m.weight.numel() + m.bias.numel() for m in mods)
-            flat = torch.zeros(total, dtype=torch.float32, device=dev)
-            off = 0
-            for m in mods:
-                wv = flat[off:off + m.weight.numel()].view(m.weight.shape)
-                off += m.weight.numel()
-                bv = flat[off:off + m.bias.numel()].view(m.bias.shape)
-                off += m.bias.numel()
-                gviews[m] = (wv, bv)
+            flat, views = flat_grad_views([t for m in mods for t in (m.weight, m.bias)], dev)
+            gviews = {m: (views[2 * i], views[2 * i + 1]) for i, m in enumerate(mods)}
         else:                                                     # frozen parameters: BatchNorm backward still writes its two sums
             for m in mods:
                 if isinstance(m, nn.BatchNorm2d):

@@ -13,30 +13,13 @@ csr_plan_forward on torch's current CUDA stream.  There is no eager / CPU fallba
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Optional, Tuple
 
 import torch
 import torch.nn as nn
 from torch import Tensor
 
 from .._lib import CsrError, NetDesc, check, current_stream_ptr, lib
-
-# Parameter version counters do not see every update: torch.optim.*(fused=True).step() and ``p.data.mul_()`` leave
-# ``p._version`` unchanged.  A process-wide optimizer post-step hook therefore bumps this epoch, which is part of the
-# pack-cache key: the first forward after ANY optimizer step repacks.  (Direct ``.data`` surgery - EMA, SWA - must call
-# ``ESRGANGenerator.mark_weights_dirty()``.)
-_WEIGHT_EPOCH = [0]
-
-
-def _bump_weight_epoch(*_args, **_kwargs) -> None:
-    _WEIGHT_EPOCH[0] += 1
-
-
-try:   # torch >= 2.0
-    from torch.optim.optimizer import register_optimizer_step_post_hook as _reg_post_hook
-    _reg_post_hook(_bump_weight_epoch)
-except Exception:   # pragma: no cover - without the hook every forward of a module in train() mode repacks (see below)
-    _reg_post_hook = None
+from ._common import DerivedState, _reg_post_hook, _SRCNNParams, check_generator_inputs, f32, weights_key
 
 
 class _RDBParams(nn.Module):
@@ -61,17 +44,10 @@ class _RRDBParams(nn.Module):
         self.RDB3 = _RDBParams(nf, gc)
 
 
-class _SRCNNParams(nn.Module):
-    """Names of SRCNN (srcnn.py:6-11)."""
+class ESRGANGenerator(DerivedState, nn.Module):
+    _DERIVED = ("_packed", "_packed_key", "_plans", "_packed_bwd", "_packed_bwd_key", "_ordered_cache", "_seg_cache", "_goff_cache",
+                "_train_plan", "_grad_sync")
 
-    def __init__(self, in_channels: int = 3, out_channels: int = 1):
-        super().__init__()
-        self.conv1 = nn.Conv2d(in_channels, 64, kernel_size=9, padding=4)
-        self.conv2 = nn.Conv2d(64, 32, kernel_size=1, padding=0)
-        self.conv3 = nn.Conv2d(32, out_channels, kernel_size=5, padding=2)
-
-
-class ESRGANGenerator(nn.Module):
     def __init__(self, in_channels: int = 3, out_channels: int = 3, nf: int = 64, nb: int = 23, gc: int = 32,
                  scaling_factor: int = 4, **kwargs):
         super().__init__()
@@ -92,61 +68,29 @@ class ESRGANGenerator(nn.Module):
         self.conv_last = nn.Conv2d(nf, out_channels, 3, 1, 1, bias=True)
         self.srcnn = _SRCNNParams(in_channels=3, out_channels=out_channels)
         self._desc = NetDesc(in_channels, out_channels, nf, nb, gc, scaling_factor)
-        self._packed: Optional[Tensor] = None
-        self._packed_key: Optional[Tuple] = None
-        self._plans: Dict[Tuple, Tuple[int, Tensor]] = {}
-        self._packed_bwd: Optional[Tensor] = None
-        self._packed_bwd_key: Optional[Tuple] = None
-        self._fwd_serial = 0
-        self._grad_sync = None
-        self._dirty = False
-        self._train_plan = None       # plan of the latest training forward: its saved activations belong to a live autograd node
-        self._ordered_cache = None
-        self._seg_cache = None
-        self._goff_cache = None
-
-    # derived device state (plans, packed blobs, pointer caches) is never copied or pickled: copy.deepcopy (EMA / SWA
-    # shadows) and torch.save(module) would otherwise duplicate raw CsrPlan* handles -> shared workspaces, double free
-    _DERIVED = ("_packed", "_packed_key", "_plans", "_packed_bwd", "_packed_bwd_key", "_ordered_cache", "_seg_cache", "_goff_cache",
-                "_train_plan", "_grad_sync")
+        self._reset_derived()
 
     def _reset_derived(self) -> None:
         self._packed = self._packed_key = self._packed_bwd = self._packed_bwd_key = None
         self._plans = {}
-        self._ordered_cache = self._seg_cache = self._goff_cache = self._train_plan = self._grad_sync = None
+        self._ordered_cache = self._seg_cache = self._goff_cache = self._grad_sync = None
+        self._train_plan = None       # plan of the latest training forward: its saved activations belong to a live autograd node
         self._fwd_serial = 0
         self._dirty = False
-
-    def __getstate__(self):
-        state = dict(self.__dict__)
-        for k in self._DERIVED:
-            state.pop(k, None)
-        return state
-
-    def __setstate__(self, state):
-        super().__setstate__(state)
-        self._reset_derived()
-
-    def __deepcopy__(self, memo):
-        import copy
-        cls = self.__class__
-        new = cls.__new__(cls)
-        memo[id(self)] = new
-        for k, v in self.__dict__.items():
-            if k not in self._DERIVED:
-                new.__dict__[k] = copy.deepcopy(v, memo)
-        new._reset_derived()
-        return new
 
     def mark_weights_dirty(self) -> None:
         """Call after changing parameters behind autograd's back (``p.data`` updates): the next forward repacks."""
         self._dirty = True
 
+    def _invalidate_packs(self) -> None:
+        """The next forward and backward pack, whatever the cache keys say."""
+        self._packed_key = self._packed_bwd_key = None
+
     def _apply(self, fn, *args, **kwargs):
         # .cuda() / .to() / .float(): parameter storage moves, cached pointers and plans of the old device are stale
         out = super()._apply(fn, *args, **kwargs)
         self._ordered_cache = None
-        self._packed_key = self._packed_bwd_key = None
+        self._invalidate_packs()
         return out
 
     # ------------------------------------------------------------------ weights
@@ -175,7 +119,7 @@ class ESRGANGenerator(nn.Module):
         """bf16 UMMA weight tiles + fp32 biases; rebuilt when any parameter changed (optimizer step, load_state_dict)."""
         pairs = self._ordered_params()
         dev = pairs[0][0].device
-        key = (dev, _WEIGHT_EPOCH[0]) + tuple((p.data_ptr(), p._version) for wb in pairs for p in wb)
+        key = weights_key((p for wb in pairs for p in wb), dev)
         # a module in train() mode without the optimizer hook cannot trust version counters at all
         force = force or self._dirty or (_reg_post_hook is None and self.training)
         if self._packed is not None and key == self._packed_key and not force:
@@ -189,8 +133,7 @@ class ESRGANGenerator(nn.Module):
         n = len(pairs)
         wp, bp = (C.c_void_p * n)(), (C.c_void_p * n)()
         for i, (w, b) in enumerate(pairs):
-            wc = w.detach().contiguous().float()
-            bc = b.detach().contiguous().float()
+            wc, bc = f32(w), f32(b)
             keep += [wc, bc]
             wp[i], bp[i] = wc.data_ptr(), bc.data_ptr()
         with torch.cuda.device(dev):
@@ -204,7 +147,7 @@ class ESRGANGenerator(nn.Module):
         """Transposed / flipped bf16 tiles for the input-gradient convs; rebuilt when any weight changed."""
         pairs = self._ordered_params()
         dev = pairs[0][0].device
-        key = (dev,) + tuple((w.data_ptr(), w._version) for w, _ in pairs)
+        key = weights_key((p for wb in pairs for p in wb), dev)
         if self._packed_bwd is not None and key == self._packed_bwd_key and not force:
             return self._packed_bwd
         nbytes = lib.csr_packed_weight_bytes_bwd(C.byref(self._desc))
@@ -214,7 +157,7 @@ class ESRGANGenerator(nn.Module):
         keep = []
         wp = (C.c_void_p * n)()
         for i, (w, _) in enumerate(pairs):
-            wc = w.detach().contiguous().float()
+            wc = f32(w)
             keep.append(wc)
             wp[i] = wc.data_ptr()
         with torch.cuda.device(dev):
@@ -296,16 +239,7 @@ class ESRGANGenerator(nn.Module):
 
     # ------------------------------------------------------------------ forward
     def forward(self, x: Tensor, elev: Tensor, mask: Tensor) -> Tensor:
-        if x.dim() != 4 or elev.dim() != 4 or mask.dim() != 4:
-            raise ValueError("expected x (N,C,h,w), elev (N,1,4h,4w), mask (N,1,4h,4w)")
-        n, c, h, w = x.shape
-        if c != self.in_channels:
-            raise ValueError(f"x has {c} channels, generator was built with in_channels={self.in_channels}")
-        hr_shape = (n, 1, 4 * h, 4 * w)
-        if tuple(elev.shape) != hr_shape or tuple(mask.shape) != hr_shape:
-            raise ValueError(f"elev/mask must have shape {hr_shape}, got {tuple(elev.shape)} / {tuple(mask.shape)}")
-        if not x.is_cuda:
-            raise CsrError("climsr_b200 ESRGANGenerator runs on CUDA (sm_100a) only; there is no CPU fallback")
+        check_generator_inputs(x, elev, mask, self.in_channels, "generator", "ESRGANGenerator")
         if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters())):
             from ..autograd import generator_apply
             return generator_apply(self, x, elev, mask)

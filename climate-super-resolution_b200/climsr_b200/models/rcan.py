@@ -32,6 +32,7 @@ from torch import Tensor
 
 from .. import ops
 from .._lib import CsrError, check, current_stream_ptr, lib
+from ._common import DerivedState, _SRCNNParams, check_generator_inputs, f32, flat_grad_views
 
 
 def default_conv(in_channels: int, out_channels: int, kernel_size: int, bias: bool = True) -> nn.Module:
@@ -62,15 +63,7 @@ class _ResidualGroupParams(nn.Module):
         self.body = nn.Sequential(*body)
 
 
-class _SRCNNParams(nn.Module):
-    def __init__(self, in_channels: int = 3, out_channels: int = 1):
-        super().__init__()
-        self.conv1 = nn.Conv2d(in_channels, 64, kernel_size=9, padding=4)
-        self.conv2 = nn.Conv2d(64, 32, kernel_size=1, padding=0)
-        self.conv3 = nn.Conv2d(32, out_channels, kernel_size=5, padding=2)
-
-
-class RCAN(nn.Module):
+class RCAN(DerivedState, nn.Module):
     def __init__(self, n_resgroups: int = 10, n_resblocks: int = 20, n_feats: int = 64, reduction: int = 16, scaling_factor: int = 4,
                  in_channels: int = 3, out_channels: int = 1, conv=default_conv, **kwargs):
         super().__init__()
@@ -118,63 +111,20 @@ class RCAN(nn.Module):
             if len(missing) > 0:
                 raise KeyError(f'missing keys in state_dict: "{missing}"')
 
-    # ------------------------------------------------------------------ packed-weight cache (see Discriminator._packed)
-    def _packed(self, conv: nn.Conv2d, transposed: bool = False, force: bool = False):
-        """(scratch, prepacked): the layer's pack scratch and whether it already holds the current weights.  force: the caller packs
-        in its conv call (training: optimizers such as fused AdamW update weights without bumping the version counters), and the
-        entry is left without a key so that the next inference forward repacks too."""
-        from .esrgan import _WEIGHT_EPOCH
-        cache = self.__dict__.setdefault("_pack_cache", {})
-        w, b = conv.weight, conv.bias
-        key = (w.data_ptr(), w._version, b.data_ptr(), b._version, _WEIGHT_EPOCH[0], w.device)
-        ent = cache.get((id(conv), transposed))
-        if not force and ent is not None and ent[1] == key:
-            return ent[0], True
-        kh, kw = conv.kernel_size
-        nbytes = ops.conv2d_scratch_bytes(conv.in_channels, conv.out_channels, kh, kw, True) if transposed else \
-            ops.conv2d_scratch_bytes(conv.out_channels, conv.in_channels, kh, kw)
-        scratch = ent[0] if ent is not None and ent[0].numel() >= nbytes and ent[0].device == w.device else \
-            torch.empty(max(nbytes, 16), dtype=torch.uint8, device=w.device)
-        cache[(id(conv), transposed)] = (scratch, None if force else key)
-        return scratch, False
-
-    def __getstate__(self):
-        state = dict(self.__dict__)
-        state.pop("_pack_cache", None)
-        return state
-
-    def __deepcopy__(self, memo):
-        import copy
-        new = self.__class__.__new__(self.__class__)
-        memo[id(self)] = new
-        for k, v in self.__dict__.items():
-            if k != "_pack_cache":
-                new.__dict__[k] = copy.deepcopy(v, memo)
-        return new
-
     def _conv(self, inp: Tensor, conv: nn.Conv2d, act: str = "none", res1=None, out_mode: str = "nhwc", train: bool = False) -> Tensor:
-        scratch, pre = self._packed(conv, force=train)
-        return ops.conv2d_nhwc(inp, conv.weight.detach().contiguous().float(), conv.bias.detach().contiguous().float(), act=act, res1=res1,
-                               out_mode=out_mode, scratch=scratch, prepacked=pre)
+        # training packs in every conv call: fused optimizers update the weights without bumping their version counters
+        scratch, pre, _ = self._layer_pack(conv, force=train)
+        return ops.conv2d_nhwc(inp, f32(conv.weight), f32(conv.bias), act=act, res1=res1, out_mode=out_mode, scratch=scratch, prepacked=pre)
 
     def _conv_t(self, g: Tensor, conv: nn.Conv2d, res1=None, res2=None, gate=None) -> Tensor:
         """Input gradient of ``conv`` (+ res1 + res2, then * ReLU'(gate)), packed transposed on every call."""
-        scratch, _ = self._packed(conv, transposed=True, force=True)
-        return ops.conv2d_nhwc(g, conv.weight.detach().contiguous().float(), None, transposed=True, res1=res1, res2=res2, gate=gate,
+        scratch, _, _ = self._layer_pack(conv, transposed=True, force=True)
+        return ops.conv2d_nhwc(g, f32(conv.weight), None, transposed=True, res1=res1, res2=res2, gate=gate,
                                gate_neg=0.0, scratch=scratch)
 
     # ------------------------------------------------------------------ forward (rcan.py:175-186)
     def forward(self, x: Tensor, elev: Tensor, mask: Tensor) -> Tensor:
-        if x.dim() != 4 or elev.dim() != 4 or mask.dim() != 4:
-            raise ValueError("expected x (N,C,h,w), elev (N,1,4h,4w), mask (N,1,4h,4w)")
-        n, c, h, w = x.shape
-        if c != self.in_channels:
-            raise ValueError(f"x has {c} channels, RCAN was built with in_channels={self.in_channels}")
-        hr_shape = (n, 1, 4 * h, 4 * w)
-        if tuple(elev.shape) != hr_shape or tuple(mask.shape) != hr_shape:
-            raise ValueError(f"elev/mask must have shape {hr_shape}, got {tuple(elev.shape)} / {tuple(mask.shape)}")
-        if not x.is_cuda:
-            raise CsrError("climsr_b200 RCAN runs on CUDA (sm_100a) only; there is no CPU fallback")
+        check_generator_inputs(x, elev, mask, self.in_channels, "RCAN", "RCAN")
         if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters())):
             if not self.training:
                 raise CsrError("climsr_b200 RCAN trains in train() mode only (eval() mode runs the inference path): call .train() "
@@ -188,7 +138,6 @@ class RCAN(nn.Module):
         n, _, h, w = x.shape
         dev = x.device
         train = saved is not None
-        f32 = lambda t: t.detach().contiguous().float()  # noqa: E731
         with torch.cuda.device(dev):
             a = ops.nchw_to_nhwc_bf16(x.detach(), 64)
             head = self._conv(a, self.head[0], train=train)                      # x = self.head(x)
@@ -239,12 +188,8 @@ class RCAN(nn.Module):
         dev = grad_out.device
         n, h, w = sv["n"], sv["h"], sv["w"]
         params = list(self.parameters())
-        flat = torch.zeros(sum(p.numel() for p in params), dtype=torch.float32, device=dev)
-        views, off = {}, 0
-        for p in params:
-            views[p] = flat[off:off + p.numel()].view(p.shape)
-            off += p.numel()
-        f32 = lambda t: t.detach().contiguous().float()  # noqa: E731
+        _, grads = flat_grad_views(params, dev)
+        views = dict(zip(params, grads))
 
         def wgrad(x, g, conv):
             ops.conv2d_wgrad(x, g, tuple(conv.weight.shape), dw=views[conv.weight], db=views[conv.bias])
@@ -302,7 +247,7 @@ class RCAN(nn.Module):
             # dL/dhead = g + d_res (body skip): the weight gradient is linear in it - two accumulating calls instead of an add pass
             wgrad(sv["a"], g, self.head[0])
             wgrad(sv["a"], d_res, self.head[0])
-        return [views[p] for p in params]
+        return grads
 
 
 class _RCANFunction(torch.autograd.Function):

@@ -117,11 +117,11 @@ def test_derived_device_state_is_never_copied_or_pickled():
     net._plans.clear()
 
 
-def test_optimizer_steps_invalidate_the_pack_cache_key():
+def test_optimizer_steps_bump_the_shared_weight_epoch():
     """Fused optimizers do not bump parameter version counters; a process-wide optimizer post-step hook bumps the epoch that is
-    part of the pack-cache key (climsr_b200/models/esrgan.py)."""
+    part of the pack-cache key (climsr_b200/models/_common.py)."""
     from climsr_b200.models import ESRGANGenerator
-    from climsr_b200.models import esrgan as E
+    from climsr_b200.models import _common as E
     net = ESRGANGenerator(4, 1, 64, 1, 16)
     for p in net.parameters():
         p.grad = torch.zeros_like(p)
@@ -132,3 +132,62 @@ def test_optimizer_steps_invalidate_the_pack_cache_key():
     assert net._dirty is False
     net.mark_weights_dirty()
     assert net._dirty is True
+
+
+@pytest.mark.parametrize("kind", ["rcan", "discriminator"])
+def test_rcan_and_discriminator_derived_state_is_never_copied_or_pickled(kind):
+    """copy.deepcopy / torch.save of RCAN and Discriminator leave their weight packs and captured graphs behind."""
+    import copy
+    import io
+    from climsr_b200.models.discriminator import Discriminator
+    from climsr_b200.models.rcan import RCAN
+    net = RCAN(n_resgroups=1, n_resblocks=1) if kind == "rcan" else Discriminator()
+    conv = next(m for m in net.modules() if isinstance(m, torch.nn.Conv2d))
+    net._layer_pack(conv, force=True)          # a CPU scratch: sized and allocated, nothing packed
+    assert net._pack_cache._entries
+    if kind == "discriminator":
+        net._slots = {("key",): [object()]}
+        net._calls = {("key",): 3}
+    buf = io.BytesIO()
+    torch.save(net, buf)
+    buf.seek(0)
+    for twin in (copy.deepcopy(net), torch.load(buf, weights_only=False)):
+        assert not any(k in twin.__dict__ for k in ("_pack_cache", "_slots", "_calls"))
+        assert list(twin.state_dict()) == list(net.state_dict())
+        assert all(torch.equal(a, b) for a, b in zip(net.state_dict().values(), twin.state_dict().values()))
+        assert all(a.data_ptr() != b.data_ptr() for a, b in zip(net.parameters(), twin.parameters()))
+
+
+def test_weights_key_follows_optimizer_steps_and_in_place_updates():
+    from climsr_b200.models._common import weights_key
+    conv = torch.nn.Conv2d(4, 8, 3)
+    params = list(conv.parameters())
+    key = weights_key(params, conv.weight.device)
+    assert weights_key(params, conv.weight.device) == key
+    for p in params:
+        p.grad = torch.ones_like(p)
+    torch.optim.AdamW(params, lr=1e-3, fused=False).step()
+    stepped = weights_key(params, conv.weight.device)
+    assert stepped != key
+    with torch.no_grad():
+        conv.bias.add_(1.0)
+    assert weights_key(params, conv.weight.device) != stepped
+
+
+def test_layer_pack_cache_keys_and_forced_packs():
+    """A hit reuses the scratch as prepacked; a forced call (the conv packs) leaves no key, so the next call packs again; an
+    optimizer step invalidates every entry; the scratch is allocated once per layer and device."""
+    from climsr_b200.models._common import LayerPackCache
+    conv = torch.nn.Conv2d(64, 64, 3, padding=1)
+    cache = LayerPackCache()
+    scratch, pre, new = cache.get(conv)
+    assert (pre, new) == (False, True) and scratch.dtype == torch.uint8 and scratch.numel() > 0
+    assert cache.get(conv) == (scratch, True, False)
+    assert cache.get(conv, force=True) == (scratch, False, False)
+    assert cache.get(conv) == (scratch, False, False)
+    assert cache.get(conv) == (scratch, True, False)
+    conv.weight.grad = torch.zeros_like(conv.weight)
+    torch.optim.SGD([conv.weight], lr=0.0).step()
+    assert cache.get(conv) == (scratch, False, False)
+    transposed, pre, new = cache.get(conv, transposed=True)
+    assert transposed is not scratch and (pre, new) == (False, True)
