@@ -29,12 +29,7 @@ static int g_opt_pdl = 1;
 static long long* g_trace = nullptr;
 static unsigned long long* g_timeline = nullptr;   // csr_debug_set_timeline
 static int g_timeline_cap = 0;
-static int g_opt_force_sw = 0;
-static int g_opt_max_slots = 8;
 static int g_opt_no_tma_store = 0;
-static int g_opt_two_acc = 0;
-static int g_opt_force_generic = 0;
-static int g_opt_one_mma = 0;
 static int g_opt_graphs = 1;
 static int g_opt_graph_max_px = 1 << 21;   // forward: replay a CUDA graph up to this many HR pixels per call (larger batches are GPU-bound)
 static int g_opt_wgrad_atomic = 1;      // weight-gradient partial sums through red.global.add.v4.f32 instead of per-CTA slices + reduce kernel
@@ -53,7 +48,6 @@ static int g_opt_fuse_tail = 3;         // inference, second MMA over the staged
                                         // nine tap planes inside HRconv's epilogue (+ tap_sum_kernel)
 static int g_opt_dense = 1;             // conv1..conv4 of every gc = 16 dense block as ONE persistent launch with tile-level dependencies (rdb_tc.cu)
 static int g_opt_early = 1;             // early-release epilogue (conv_tc.cu, EARLY_T) for the wide residual-free layers
-static int g_dbg_wgrad[5] = {0, 0, 0, 0, 0};   // a_lbo, a_sbo, b_lbo, b_sbo, flags overrides of the MN-major descriptors
 
 static int fail(int code, const char* fmt, ...) {
   va_list ap;
@@ -263,11 +257,11 @@ struct Tiling {
   int SW, TH, TW, win_rows, win_bytes, slot_bytes, n_slots, stage_bytes;
   double eff;   // useful fraction of the MMA rows (with the small penalties applied by choose_tiling)
 };
+constexpr int kMaxSlots = 8;   // deepest window ring of a conv or dense-block launch
 static int choose_tiling(int H, int W, int KH, int KW, int w_bytes, int n_kblocks, int stage_row_bytes, int n_stage, Tiling* out,
                          int row_bytes = 128, int tall = 1, int extra_slot_bytes = 0) {
   double best = -1;
   for (int SW = 16; SW <= 128; SW *= 2) {
-    if (g_opt_force_sw && SW != g_opt_force_sw) continue;
     // The epilogue sums the folded horizontal taps with warp shuffles: a window row must not straddle two warps.
     if (KW > 1 && SW > 32) continue;
     const int TW = SW - (KW - 1);
@@ -278,7 +272,7 @@ static int choose_tiling(int H, int W, int KH, int KW, int w_bytes, int n_kblock
     const int slot_bytes = (int)align_up(win_bytes, 1024) + (int)align_up(extra_slot_bytes, 1024);   // + a streamed weight k-block
     const int stage_bytes = stage_row_bytes ? (int)align_up((size_t)TH * TW * stage_row_bytes, 1024) : 0;
     const int fixed = 1024 + (int)align_up(w_bytes, 128) + 256 + 512 + n_stage * stage_bytes;
-    const int slots = std::min(g_opt_max_slots, (kSmemLimit - fixed) / slot_bytes);
+    const int slots = std::min(kMaxSlots, (kSmemLimit - fixed) / slot_bytes);
     if (slots < 1) continue;
     const double tiles = (double)ceil_div(H, TH * tall) * ceil_div(W, TW) * tall;
     double eff = (double)H * W / (tiles * kTileM);
@@ -337,7 +331,7 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
   p.store_mode = tma_out ? kStoreStaged : io.out_kind == kOutBf16 ? kStoreDirect : io.out_kind == kOutF32Planar ? kStoreF32Planar : kStoreF32Nhwc;
   p.stage_row_bytes = tma_out ? pp.n_store * 2 : 0;
   // four tiles in flight in the epilogue when four accumulators fit in TMEM and a warp then owns <= 4 chunks of 8 channels
-  p.n_acc = (4 * p.KW * p.npad <= 512 && p.npad <= 32 && !g_opt_two_acc) ? 4 : 2;
+  p.n_acc = (4 * p.KW * p.npad <= 512 && p.npad <= 32) ? 4 : 2;
   p.n_groups = p.n_acc;
   Tiling tl;
   int rc = CSR_OK;
@@ -389,7 +383,7 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
   // buffers; KW <= 2 layers also get four accumulator buffers (4 x KW x 64 <= 512 TMEM columns).
   const bool early_plain = !has_res && p.n_groups == 1 &&
       ((p.KW == 3 && p.PW == 1 && (p.act == 0 || p.act == 1)) || (p.KW == 2 && p.PW <= 1 && p.act == 1) || (p.KW == 1 && p.PW == 0 && p.act == 2));
-  if (g_opt_early && early_plain && !p.tall_shift && tma_out && p.npad == 64 && pp.n_store == 64 && !g_opt_force_generic) {
+  if (g_opt_early && early_plain && !p.tall_shift && tma_out && p.npad == 64 && pp.n_store == 64) {
     Tiling te2, te1;
     const bool ok2 = choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, 2, &te2, p.box_c * 2) == CSR_OK;
     const bool ok1 = choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, 1, &te1, p.box_c * 2) == CSR_OK;
@@ -404,7 +398,7 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
       p.early = 1;
       p.n_groups = 1;
       p.n_stage = stages;
-      if (4 * p.KW * p.npad <= 512 && !g_opt_two_acc) p.n_acc = 4;
+      if (4 * p.KW * p.npad <= 512) p.n_acc = 4;
     }
   }
   // Hybrid tap fold (conv_tc.cu HYB_T) for the early-release 64-channel 3x3 / 2x2 layers, which are epilogue-bound: the last horizontal
@@ -412,7 +406,7 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
   // accumulator columns to read and one shuffle-sum fewer, at 22 % more MMA time.
   if (g_opt_hyb && p.early && ((p.KW == 3 && p.PW == 1) || (p.KW == 2 && p.PW <= 1)) && p.box_c == 64 && !p.stream_w) {
     p.hyb = 1;
-    if (4 * (p.KW - 1) * p.npad <= 512 && !g_opt_two_acc) p.n_acc = 4;
+    if (4 * (p.KW - 1) * p.npad <= 512) p.n_acc = 4;
   }
   p.SW = tl.SW; p.TH = tl.TH; p.TW = tl.TW;
   p.sw_shift = 0;
@@ -428,7 +422,6 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
   p.win_rows = tl.win_rows; p.win_bytes = tl.win_bytes; p.slot_bytes = tl.slot_bytes; p.n_slots = tl.n_slots;
   p.win_slot_bytes = (int)align_up(tl.win_bytes, 1024);
   p.stage_bytes = tl.stage_bytes;
-  p.n_mma = g_opt_one_mma ? 1 : 2;
   int cols = 32;
   while (cols < p.n_acc * (p.hyb ? p.KW - 1 : p.KW) * p.npad) cols *= 2;
   if (cols > 512 || p.KW * p.npad > 256) return fail(CSR_ERR_UNSUPPORTED, "KW*npad = %d exceeds the UMMA N / TMEM budget", p.KW * p.npad);
@@ -436,7 +429,6 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
   p.trace = g_trace;
   p.trace_cta = g_opt_trace_cta;
   p.use_pdl = g_opt_pdl;
-  p.force_generic = g_opt_force_generic;
   p.s1 = io.s1; p.s2 = io.s2;
   p.r1 = io.r1; p.r1_C = io.r1_C; p.r1_coff = io.r1_coff + pp.co_lo;
   p.r2 = io.r2; p.r2_C = io.r2_C; p.r2_coff = io.r2_coff + pp.co_lo;
@@ -498,8 +490,6 @@ static int build_wgrad(int sms, int N, int H, int W, int KW, int PW, int dy_off,
   p.gc0[0] = gA_c0; p.gc0[1] = gB_c0;
   p.dacc = dacc; p.ld_n = ld_n; p.part_stride = part_stride;
   p.n_parts = std::min(p.num_tiles, sms);
-  p.dbg_a_lbo = g_dbg_wgrad[0]; p.dbg_a_sbo = g_dbg_wgrad[1]; p.dbg_b_lbo = g_dbg_wgrad[2]; p.dbg_b_sbo = g_dbg_wgrad[3];
-  p.dbg_flags = g_dbg_wgrad[4];
   int rc = encode_act_map(&wl->tx0, x, N, H, W, x_C, p.SW, p.TH + n_dy);
   if (rc) return rc;
   wl->tx1 = wl->tx0;
@@ -933,13 +923,13 @@ static int build_dense(const std::vector<PackLayer>& packs, int li, int N, int H
   if ((long long)p.tiles_per_img * N >= (1 << 24) || p.tiles_per_img >= (1 << 16)) return fail(CSR_ERR_UNSUPPORTED, "dense-block kernel: too many windows");
   p.magic_img = ((1ull << 40) / (unsigned)p.tiles_per_img) + 1;
   p.magic_row = ((1ull << 40) / (unsigned)p.tiles_x) + 1;
-  p.win_bytes = tl.win_bytes; p.slot_bytes = tl.slot_bytes; p.n_slots = std::min(tl.n_slots, 8);
+  p.win_bytes = tl.win_bytes; p.slot_bytes = tl.slot_bytes; p.n_slots = tl.n_slots;
   p.stage_bytes = (int)align_up((size_t)p.TH * p.TW * 32, 1024);
   if (dense_smem_bytes(p) > (size_t)kSmemLimit) return fail(CSR_ERR_UNSUPPORTED, "dense-block kernel needs %zu bytes of shared memory", dense_smem_bytes(p));
   return encode_act_map(&dl->tmap, buf, N, H, W, C, p.SW, 2 * p.TH + 2, 64);
 }
 
-static bool dense_enabled(const CsrNetDesc& d) { return g_opt_dense && d.gc == 16 && !g_opt_force_generic; }
+static bool dense_enabled(const CsrNetDesc& d) { return g_opt_dense && d.gc == 16; }
 
 // The four convs of dense block j (concat buffer `buf`, pack layers li..li+3) as ONE persistent launch with tile-level
 // dependencies between the layers: conv1..conv4 of the forward, or with `gate` the backward's four gated input-gradient convs.
@@ -1409,23 +1399,18 @@ int csr_device_check(void) {
 }
 
 int csr_set_option(int32_t key, int32_t value) {
-  // the table with defaults and meanings is in INTEGRATION.md section 6.  Keys 8, 9, 13, 14, 16, 28, 29 and 32 are retired (they
-  // selected removed kernel variants): do not reuse them, callers of older versions may still set them
+  // the table with defaults and meanings is in INTEGRATION.md section 6.  Keys 2, 3, 5, 6, 7, 8, 9, 13, 14, 16, 20-24, 28, 29 and 32
+  // are retired (they selected removed kernel variants or measured-and-rejected settings of the default kernels): do not reuse them,
+  // callers of older versions may still set them
   switch (key) {
     case 1: g_opt_pdl = value ? 1 : 0; return CSR_OK;              // programmatic dependent launch on/off
-    case 2: g_opt_force_sw = value; return CSR_OK;                 // debug: force the window pitch
-    case 3: g_opt_max_slots = value < 1 ? 1 : value; return CSR_OK;
     case 4: g_opt_no_tma_store = value ? 1 : 0; return CSR_OK;     // debug: per-element stores instead of the staged copy-out
-    case 5: g_opt_two_acc = value ? 1 : 0; return CSR_OK;          // debug: never more than two accumulator buffers
-    case 6: g_opt_force_generic = value ? 1 : 0; return CSR_OK;    // debug: runtime-switched kernels only
-    case 7: g_opt_one_mma = value ? 1 : 0; return CSR_OK;          // debug: a single MMA issuer warp
     case 11: g_opt_graphs = value ? 1 : 0; return CSR_OK;          // CUDA-graph replay of plan forward / backward_flat
     case 12: g_opt_graph_max_px = value; return CSR_OK;
     case 15: g_opt_trace_cta = value; return CSR_OK;
     case 17: g_opt_narrow_box = value ? 1 : 0; return CSR_OK;
     case 18: g_opt_tall = value ? 1 : 0; return CSR_OK;
     case 19: g_opt_eight_acc = value ? 1 : 0; return CSR_OK;
-    case 20: case 21: case 22: case 23: case 24: g_dbg_wgrad[key - 20] = value; return CSR_OK;
     case 25: g_opt_wgrad_atomic = value ? 1 : 0; return CSR_OK;    // plans created afterwards
     case 27: g_opt_dense = value ? 1 : 0; return CSR_OK;           // plans created afterwards
     case 36: g_opt_tap_pack = value ? 1 : 0; return CSR_OK;

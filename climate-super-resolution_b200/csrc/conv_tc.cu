@@ -274,7 +274,6 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
       }
     }
   } else if (warp <= kMmaWarps) {
-    if (warp > p.n_mma) goto done;                       // single-issuer launches: warp 2 idles
     // ===================== MMA issuers (warps 1 and 2 take alternate tiles) =====================
     // tcgen05.mma issue proceeds at execution pace (the issuing thread stalls while the tensor pipe is busy), so with a
     // single issuer the ~600 clk of mbarrier round trips between tiles leave the pipe idle.  With two issuers one warp's
@@ -307,7 +306,7 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
     };
     if (mw) ring_advance(p.n_kblocks);
     int entry = mw * p.n_kblocks;                                            // ring entry index of (tile, kb)
-    for (int it = mw; ; it += p.n_mma) {
+    for (int it = mw; ; it += kMmaWarps) {
       const int t = blockIdx.x + it * static_cast<int>(gridDim.x);
       if (t >= p.num_tiles) break;
       if (lane == 0) CSR_TRACE(1, it, 0);
@@ -317,15 +316,13 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
       if (lane == 0) CSR_TRACE(1, it, 1);
       const uint32_t d_tmem = tmem_base + buf * nacc;
       for (int kb = 0; kb < p.n_kblocks; ++kb, ++entry) {
-        if (p.n_mma > 1) {
-          const int need = entry - S;
-          if (need >= 0 && ((need / p.n_kblocks) & 1) != mw) {
-            while (progress[1 - mw] <= static_cast<uint32_t>(need)) {
-            }
+        const int need = entry - S;
+        if (need >= 0 && ((need / p.n_kblocks) & 1) != mw) {
+          while (progress[1 - mw] <= static_cast<uint32_t>(need)) {
           }
         }
         mbar_wait_spin(bar_a_full(slot), phase);
-        if (p.n_mma > 1) progress[mw] = static_cast<uint32_t>(entry) + 1u;
+        progress[mw] = static_cast<uint32_t>(entry) + 1u;
         tc_fence_after();
         if (kb == 0 && lane == 0) CSR_TRACE(1, it, 2);
         const int ks_here = min(4, ksteps_total - kb * 4);
@@ -380,11 +377,9 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
         if (kb == p.n_kblocks - 1 && lane == 0) CSR_TRACE(1, it, 3);
         ring_advance(1);
       }
-      if (p.n_mma > 1) {                                                   // skip the other issuer's tile
-        ring_advance(p.n_kblocks);
-        entry += p.n_kblocks;
-      }
-      buf += p.n_mma * tall;
+      ring_advance(p.n_kblocks);                                           // skip the other issuer's tile
+      entry += p.n_kblocks;
+      buf += kMmaWarps * tall;
       if (buf >= NA) { buf -= NA; acc_phase ^= 1; }
       if (lane == 0) CSR_TRACE(1, it, 6);
     }
@@ -735,7 +730,6 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
     }
   }
 
-done:
   tc_fence_before();
   __syncthreads();
   timeline_end(p.timeline, p.launch_id);
@@ -788,19 +782,19 @@ int launch_conv_tc(const ConvParams& p, const CUtensorMap& tmap, int num_sms, cu
   if (p.tall_shift) {
     // two-M-tile windows: the thin layers only (four accumulator buffers)
     if ((p.n_acc != 4 && p.n_acc != 8) || p.n_groups != 4) return static_cast<int>(cudaErrorInvalidValue);
-    if (p.store_mode == kStoreStaged && !p.force_generic && p.KW == 3 && p.PW == 1 && p.act == 1 && res == 0)
+    if (p.store_mode == kStoreStaged && p.KW == 3 && p.PW == 1 && p.act == 1 && res == 0)
       return launch_t<3, 1, 1, 0, 1, 1>(p, tmap, num_sms, stream);         // RDB conv1-4
-    if (p.store_mode == kStoreStaged && !p.force_generic && p.KW == 1 && p.PW == 0 && p.act == 2 && res == 0)
+    if (p.store_mode == kStoreStaged && p.KW == 1 && p.PW == 0 && p.act == 2 && res == 0)
       return launch_t<1, 0, 2, 0, 1, 1>(p, tmap, num_sms, stream);         // srcnn.conv2
-    if (p.store_mode == kStoreStaged && !p.force_generic && p.KW == 3 && p.PW == 1 && p.act == 0 && res == 4)
+    if (p.store_mode == kStoreStaged && p.KW == 3 && p.PW == 1 && p.act == 0 && res == 4)
       return launch_t<3, 1, 0, 4, 1, 1>(p, tmap, num_sms, stream);         // dense-block input gradients of x1..x4 (gated)
-    if (p.store_mode == kStoreStaged && !p.force_generic && p.KW == 3 && p.PW == 1 && p.act == 0 && res == 5)
+    if (p.store_mode == kStoreStaged && p.KW == 3 && p.PW == 1 && p.act == 0 && res == 5)
       return launch_t<3, 1, 0, 5, 1, 1>(p, tmap, num_sms, stream);
-    if (p.store_mode == kStoreStaged && !p.force_generic && p.KW == 1 && p.PW == 0 && p.act == 0 && res == 4)
+    if (p.store_mode == kStoreStaged && p.KW == 1 && p.PW == 0 && p.act == 0 && res == 4)
       return launch_t<1, 0, 0, 4, 1, 1>(p, tmap, num_sms, stream);         // srcnn.conv3 input gradient over the gradient im2col
-    if (p.store_mode == kStoreF32Planar && !p.force_generic && p.KW == 3 && p.PW == 1 && p.act == 0 && res == 0)
+    if (p.store_mode == kStoreF32Planar && p.KW == 3 && p.PW == 1 && p.act == 0 && res == 0)
       return launch_t<3, 1, 0, 0, 3, 1>(p, tmap, num_sms, stream);         // conv_last
-    if (p.store_mode == kStoreF32Planar && !p.force_generic && p.KW == 5 && p.PW == 2 && p.act == 0 && res == 0)
+    if (p.store_mode == kStoreF32Planar && p.KW == 5 && p.PW == 2 && p.act == 0 && res == 0)
       return launch_t<5, 2, 0, 0, 3, 1>(p, tmap, num_sms, stream);         // srcnn.conv3
     switch (p.KW) {
       case 1: return launch_t<1, 0, -1, -1, -1, 1>(p, tmap, num_sms, stream);
@@ -810,7 +804,7 @@ int launch_conv_tc(const ConvParams& p, const CUtensorMap& tmap, int num_sms, cu
   }
   if (p.early) {
     // wide residual-free layers with the early-release epilogue (one 16-warp group, two staging buffers)
-    if (p.store_mode != kStoreStaged || p.n_groups != 1 || p.n_stage < 1 || p.n_stage > 2 || p.npad != 64 || res != 0 || p.force_generic)
+    if (p.store_mode != kStoreStaged || p.n_groups != 1 || p.n_stage < 1 || p.n_stage > 2 || p.npad != 64 || res != 0)
       return static_cast<int>(cudaErrorInvalidValue);
     if (p.fuse2 == 2) {
       // HRconv (3x3, LeakyReLU) + the nine tap planes of conv_last (3x3, 64 -> 1) in one launch
@@ -841,7 +835,7 @@ int launch_conv_tc(const ConvParams& p, const CUtensorMap& tmap, int num_sms, cu
     return static_cast<int>(cudaErrorInvalidValue);
   }
 #define CSR_CASE(KW_, PW_, ACT_, RES_, ST_)                                                                  \
-  if (p.store_mode == (ST_ == 1 ? kStoreStaged : kStoreF32Planar) && !p.force_generic && p.KW == KW_ &&   \
+  if (p.store_mode == (ST_ == 1 ? kStoreStaged : kStoreF32Planar) && p.KW == KW_ &&                         \
       p.PW == PW_ && p.act == ACT_ && res == RES_)                                                           \
     return launch_t<KW_, PW_, ACT_, RES_, ST_>(p, tmap, num_sms, stream);
   // the layer shapes of the generator forward (esrgan.py / srcnn.py) ...

@@ -40,14 +40,12 @@ struct ConvParams {
   int n_kblocks;   // ceil(cin / 64)
   int n_slots;     // activation-window ring depth
   int w_bytes;     // packed weights: KH * (cin/16) * KW * npad * 32
-  int n_mma;       // MMA issuer warps in use (2; 1 = debug)
   int n_acc;       // accumulator buffers in TMEM (2, 4 or 8); n_acc * KW * npad <= 512
   int n_groups;    // epilogue warp groups (1, 2 or 4; n_groups divides n_acc): one staging buffer each
   int n_stage;     // staging buffers in shared memory: n_groups, or 2 for the early-release epilogue
   int hyb;         // 1 = hybrid tap fold (conv_tc.cu HYB_T): 3x3 early-release layers, accumulators of 2*npad columns
   int early;       // 1 = early-release epilogue (conv_tc.cu, EARLY_T): wide residual-free layers, one 16-warp group
   int tmem_cols;   // power of two >= max(32, n_acc*KW*npad)
-  int force_generic;  // debug: skip the compile-time specialised kernels
   int trace_cta;   // debug: the CTA whose role timestamps go to `trace`
   int box_c;       // channels per window pixel in shared memory: 64 (128-byte rows), or 32 / 16 for single-k-block layers with cin <= 32 / 16
   int tall_shift;  // 1: a window holds TWO vertically adjacent M tiles (2*TH + KH - 1 rows, one TMA load, one MMA-issuer iteration,

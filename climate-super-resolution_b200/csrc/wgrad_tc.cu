@@ -123,13 +123,9 @@ wgrad_tc_kernel(const WgradParams p, const __grid_constant__ CUtensorMap tx0, co
     const uint32_t idesc = make_idesc_bf16_mn(128, p.n_cols);
     // MN-major, 128B swizzle: 64 channels (128 B) contiguous per pixel; LBO = byte distance to the next 64-channel box,
     // SBO = byte distance between groups of 8 pixels (8 x 128 B when pixels are consecutive lines).
-    const uint32_t a_lbo = p.dbg_a_lbo ? p.dbg_a_lbo : x_pitch;
-    const uint32_t a_sbo = p.dbg_a_sbo ? p.dbg_a_sbo : 1024u;
-    const uint32_t b_lbo = p.dbg_b_lbo ? p.dbg_b_lbo : static_cast<uint32_t>(p.g_box_bytes);
-    const uint32_t b_sbo = p.dbg_b_sbo ? p.dbg_b_sbo : 1024u;
-    const uint32_t a_hi = (a_sbo >> 4) | (1u << 14) | (2u << 29);
-    const uint32_t b_hi = (b_sbo >> 4) | (1u << 14) | (2u << 29);
-    const uint32_t a_lo_fixed = ((a_lbo >> 4) & 0x3FFFu) << 16, b_lo_fixed = ((b_lbo >> 4) & 0x3FFFu) << 16;
+    const uint32_t hi = (1024u >> 4) | (1u << 14) | (2u << 29);   // both operands: SBO 1024 B, version 1, SWIZZLE_128B
+    const uint32_t a_lo_fixed = ((x_pitch >> 4) & 0x3FFFu) << 16;
+    const uint32_t b_lo_fixed = ((static_cast<uint32_t>(p.g_box_bytes) >> 4) & 0x3FFFu) << 16;
     int stage = 0;
     uint32_t phase = 0;
     bool first = true;
@@ -146,7 +142,7 @@ wgrad_tc_kernel(const WgradParams p, const __grid_constant__ CUtensorMap tx0, co
             for (int j = 0; j < 8; ++j) {
               const uint32_t a_lo = (((a0 + j * 2048u) >> 4) & 0x3FFFu) | a_lo_fixed;
               const uint32_t b_lo = (((sb + g_off + j * 2048u) >> 4) & 0x3FFFu) | b_lo_fixed;
-              umma_bf16_split(d_tmem, a_lo, a_hi, b_lo, b_hi, idesc, (first && j == 0) ? 0u : 1u);
+              umma_bf16_split(d_tmem, a_lo, hi, b_lo, hi, idesc, (first && j == 0) ? 0u : 1u);
             }
           }
         }

@@ -40,8 +40,6 @@ struct WgradParams {
   int KH, PH, per_dy;
   int x_coff, g_coff;        // first channel of the layer's input / output gradient inside their buffers
   long job_stride;
-  // debug overrides of the MN-major descriptor fields (0 = default)
-  int dbg_a_lbo, dbg_a_sbo, dbg_b_lbo, dbg_b_sbo, dbg_flags;
 };
 
 int launch_wgrad_tc(const WgradParams& p, const CUtensorMap& tx0, const CUtensorMap& tx1, const CUtensorMap& tg0, const CUtensorMap& tg1,

@@ -1,7 +1,7 @@
 """Bring-up diagnostics for the tcgen05 conv kernel on a real B200 (run through gpurun, not pytest).
 
     python tests/gpu_selftest.py            # runs every case in a subprocess (a trapped kernel kills only its case)
-    python tests/gpu_selftest.py --case conv_basic --base-off 0
+    python tests/gpu_selftest.py --case conv_basic --pdl 0
 
 Each case compares the CUDA path with torch CPU fp32 on bf16-rounded operands (oracle side only).
 """
@@ -238,12 +238,12 @@ CASES = {
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--case", default=None)
-    ap.add_argument("--base-off", type=int, default=0)
+    ap.add_argument("--pdl", type=int, default=0, help="programmatic dependent launch (option 1) off / on")
     ap.add_argument("--cases", default=",".join(CASES))
     a = ap.parse_args()
     if a.case:
         from climsr_b200._lib import lib
-        lib.csr_set_option(1, a.base_off)
+        lib.csr_set_option(1, a.pdl)
         ok = CASES[a.case]()
         sys.exit(0 if ok else 1)
     summary = []
@@ -251,9 +251,9 @@ def main():
         for name in a.cases.split(","):
             if mode == 1 and name in ("layout", "metrics"):
                 continue
-            print(f"== case {name} (A base_offset mode {mode})", flush=True)
+            print(f"== case {name} (PDL {'on' if mode else 'off'})", flush=True)
             try:
-                r = subprocess.run([sys.executable, __file__, "--case", name, "--base-off", str(mode)], timeout=300,
+                r = subprocess.run([sys.executable, __file__, "--case", name, "--pdl", str(mode)], timeout=300,
                                    capture_output=True, text=True)
                 out = (r.stdout + r.stderr).strip().splitlines()
                 print("\n".join(out[-60:]))
@@ -262,10 +262,10 @@ def main():
                 print("  TIMEOUT")
                 summary.append((name, mode, "timeout"))
         if all(rc == 0 for (_, m, rc) in summary if m == mode):
-            break   # this descriptor mode passes everything: no need to try the other
+            break   # everything passes with this PDL setting: no need to try the other
     print("== summary")
     for name, mode, rc in summary:
-        print(f"  {name:20s} mode {mode}: {'PASS' if rc == 0 else 'FAIL(' + str(rc) + ')'}")
+        print(f"  {name:20s} PDL {mode}: {'PASS' if rc == 0 else 'FAIL(' + str(rc) + ')'}")
 
 
 if __name__ == "__main__":

@@ -59,9 +59,9 @@ def test_argument_validation_without_gpu():
 
 
 def test_retired_option_keys_are_rejected():
-    """Keys of the removed kernel variants are unknown keys; 26 and 35 take only 0 / 1."""
+    """Keys of the removed kernel variants and debug settings are unknown keys; 26 and 35 take only 0 / 1."""
     from climsr_b200._lib import lib
-    for key in (8, 9, 13, 14, 16, 28, 29, 32):
+    for key in (2, 3, 5, 6, 7, 8, 9, 13, 14, 16, 20, 21, 22, 23, 24, 28, 29, 32):
         assert lib.csr_set_option(key, 0) == -1 and lib.csr_set_option(key, 1) == -1, key
     for key in (26, 35):
         assert lib.csr_set_option(key, 2) == -1 and lib.csr_set_option(key, -1) == -1, key

@@ -21,6 +21,7 @@ WGRAD_CASES = [
     # n, h, w, cin, cout, k, up2
     (1, 8, 14, 64, 16, 1, 0),
     (1, 8, 14, 128, 64, 1, 0),
+    (1, 8, 14, 64, 16, 3, 0),           # RDB conv1
     (2, 16, 16, 80, 16, 3, 0),          # RDB conv2
     (2, 33, 45, 128, 64, 3, 0),         # RDB conv5, ragged tiles
     (1, 20, 40, 32, 1, 5, 0),           # srcnn.conv3

@@ -11,10 +11,6 @@ from climsr_b200.models import ESRGANGenerator  # noqa: E402
 
 VARIANTS = {
     "default": {},
-    "one_mma": {7: 1},
-    "two_acc": {5: 1},
-    "slots4": {3: 4},
-    "slots3": {3: 3},
     "no_pdl": {1: 0},
     "no_eight_acc": {19: 0},
     "no_narrow_box": {17: 0},
@@ -23,8 +19,8 @@ VARIANTS = {
 
 
 def run(name, opts, n=64, h=64, w=64, steps=20):
-    for k in (1, 3, 5, 7, 17, 18, 19):
-        lib.csr_set_option(k, {1: 1, 3: 8, 17: 1, 18: 1, 19: 1}.get(k, 0))
+    for k in (1, 17, 18, 19):
+        lib.csr_set_option(k, 1)
     for k, v in opts.items():
         lib.csr_set_option(k, v)
     torch.manual_seed(0)

@@ -54,8 +54,6 @@ def run(name, n, h, w, cin, cout, k, in_c, act="lrelu", out_coff=0, res=False, i
 
 
 if __name__ == "__main__":
-    if os.environ.get("CSR_SLOTS"):
-        lib.csr_set_option(3, int(os.environ["CSR_SLOTS"]))
     if os.environ.get("CSR_CONV5"):
         run("rdb.conv5+res", 64, 64, 64, 128, 64, 3, 128, act="none", res=True)
         sys.exit(0)
