@@ -90,6 +90,8 @@ def _load():
         "csr_conv2d_wgrad": (C.c_int, [wd, vp, vp, vp, vp, vp, sz, vp]),
         "csr_nchw_f32_to_nhwc_bf16": (C.c_int, [vp, vp, i32, i32, i32, i32, i32, i32, vp]),
         "csr_nhwc_bf16_to_nchw_f32": (C.c_int, [vp, vp, i32, i32, i32, i32, i32, i32, vp]),
+        "csr_nchw_f32_to_nhwc_split": (C.c_int, [vp, vp, i32, i32, i32, i32, i32, vp]),
+        "csr_maxpool2x2_split": (C.c_int, [vp, vp, i32, i32, i32, i32, vp]),
         "csr_pixel_loss_scratch_bytes": (sz, [C.c_int64]),
         "csr_l1_loss": (C.c_int, [vp, vp, vp, C.c_int64, vp, vp, sz, vp]),
         "csr_mse_loss": (C.c_int, [vp, vp, vp, C.c_int64, vp, vp, sz, vp]),
@@ -128,7 +130,8 @@ EXPORTS = ("csr_abi_version", "csr_last_error", "csr_device_check", "csr_set_opt
            "csr_plan_forward", "csr_plan_num_launches", "csr_plan_destroy", "csr_train_workspace_bytes", "csr_train_plan_create",
            "csr_packed_weight_bytes_bwd", "csr_pack_weights_bwd", "csr_plan_backward", "csr_plan_num_backward_ops", "csr_plan_buffer", "csr_plan_grad_floats", "csr_plan_graph_status", "csr_plan_grad_offset",
            "csr_plan_backward_flat", "csr_plan_backward_segments", "csr_plan_backward_flat_seg", "csr_generator_forward", "csr_conv2d_scratch_bytes",
-           "csr_conv2d_nhwc", "csr_conv2d_pack", "csr_conv2d_wgrad_scratch_bytes", "csr_conv2d_wgrad", "csr_nchw_f32_to_nhwc_bf16", "csr_nhwc_bf16_to_nchw_f32", "csr_pixel_loss_scratch_bytes", "csr_l1_loss", "csr_mse_loss",
+           "csr_conv2d_nhwc", "csr_conv2d_pack", "csr_conv2d_wgrad_scratch_bytes", "csr_conv2d_wgrad", "csr_nchw_f32_to_nhwc_bf16", "csr_nhwc_bf16_to_nchw_f32",
+           "csr_nchw_f32_to_nhwc_split", "csr_maxpool2x2_split", "csr_pixel_loss_scratch_bytes", "csr_l1_loss", "csr_mse_loss",
            "csr_metrics_scratch_bytes", "csr_masked_metrics", "csr_minmax_normalize", "csr_minmax_denormalize_mask", "csr_disc_gather", "csr_disc_collect", "csr_disc_bn_scratch_bytes", "csr_disc_bn_forward",
            "csr_disc_bn_backward", "csr_disc_flatten", "csr_disc_unflatten", "csr_linear_forward", "csr_linear_backward",
            "csr_channel_attention", "csr_channel_attention_backward_scratch_bytes", "csr_channel_attention_backward", "csr_pixel_shuffle2",

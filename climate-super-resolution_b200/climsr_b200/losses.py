@@ -1,7 +1,9 @@
 """Pixel losses of the training step (mirror of ``self.loss = L1Loss() / MSELoss()``, climsr/core/task.py:141, used un-masked
 over all pixels in climsr/task/pl_generator_pre_training.py:29-30 and climsr/task/pl_gan.py:41).
 
-One CUDA pass produces the loss value and d loss / d sr; backward is a scalar multiply.  No CPU fallback."""
+One CUDA pass produces the loss value and d loss / d sr; backward is a scalar multiply.  No CPU fallback.
+
+The GAN step's VGG19 perceptual term is ``PerceptualLoss`` (climsr_b200/perceptual.py, re-exported here)."""
 from __future__ import annotations
 
 import torch
@@ -58,3 +60,6 @@ class L1Loss(torch.nn.Module):
 class MSELoss(torch.nn.Module):
     def forward(self, sr: Tensor, hr: Tensor) -> Tensor:
         return mse_loss(sr, hr)
+
+
+from .perceptual import PerceptualLoss  # noqa: E402,F401  (imports this package's models; kept last)

@@ -1,4 +1,4 @@
-"""Host-side plumbing shared by the three native models (ESRGANGenerator, RCAN, Discriminator): when a weight pack is stale,
+"""Host-side plumbing shared by the native models (ESRGANGenerator, RCAN, Discriminator, the VGG19 of PerceptualLoss): when a weight pack is stale,
 the per-layer conv pack cache, derived device state that is never copied or pickled, flat gradient buffers, and the SRCNN tail
 the two generators share with their input checks."""
 from __future__ import annotations
@@ -48,29 +48,37 @@ class LayerPackCache:
     def __init__(self):
         self._entries = {}
 
-    def get(self, conv: nn.Conv2d, transposed: bool = False, force: bool = False, pack: bool = False):
+    def get(self, conv: nn.Conv2d, transposed: bool = False, force: bool = False, pack: bool = False, weight_fn=None,
+            variant=None):
         """(scratch, prepacked, new): the layer's pack scratch, whether it already holds the current weights, and whether the
         scratch was just allocated (graphs captured over an older one are stale).
 
         force: the caller packs in its conv call (training: fused optimizers update weights without bumping the version
         counters); the entry is left without a key so that the next call that does not force repacks too.
-        pack: pack here (csr_conv2d_pack, outside any graph) when the weights changed, so that prepacked is always True."""
+        pack: pack here (csr_conv2d_pack, outside any graph) when the weights changed, so that prepacked is always True.
+        weight_fn: the layer executes ``weight_fn(conv.weight)`` (same output channels, any input channels) instead of its own
+        weight - the [W | W] weights of a conv over hi/lo activation pairs; ``variant`` names that form in the cache slot.
+        The key is still that of conv.weight / conv.bias."""
         w, b = conv.weight, conv.bias
-        slot = (conv, transposed)
+        if weight_fn is not None and transposed:
+            raise ValueError("weight_fn applies to forward packs only")
+        slot = (conv, transposed) if variant is None else (conv, transposed, variant)
         ent = self._entries.get(slot)
         key = None if force else weights_key((w, b), w.device)
         if key is not None and ent is not None and ent[1] == key:
             return ent[0], True, False
         new = ent is None or ent[0].device != w.device
+        ew = weight_fn(w.detach()) if weight_fn is not None and (new or pack) else None
         if new:
             kh, kw = conv.kernel_size
+            cin = conv.in_channels if ew is None else ew.shape[1]
             nbytes = ops.conv2d_scratch_bytes(conv.in_channels, conv.out_channels, kh, kw, True) if transposed else \
-                ops.conv2d_scratch_bytes(conv.out_channels, conv.in_channels, kh, kw)
+                ops.conv2d_scratch_bytes(conv.out_channels, cin, kh, kw)
             scratch = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=w.device)
         else:
             scratch = ent[0]
         if pack:
-            ops.conv2d_pack(w, None if transposed else b, scratch, transposed)
+            ops.conv2d_pack(w if ew is None else ew, None if transposed else b, scratch, transposed)
         self._entries[slot] = (scratch, key)
         return scratch, pack, new
 
@@ -86,12 +94,13 @@ class DerivedState:
     def _reset_derived(self) -> None:
         pass
 
-    def _layer_pack(self, conv: nn.Conv2d, transposed: bool = False, force: bool = False, pack: bool = False):
+    def _layer_pack(self, conv: nn.Conv2d, transposed: bool = False, force: bool = False, pack: bool = False, weight_fn=None,
+                    variant=None):
         """``LayerPackCache.get`` on this module's cache, created on first use."""
         cache = self.__dict__.get("_pack_cache")
         if cache is None:
             cache = self.__dict__["_pack_cache"] = LayerPackCache()
-        return cache.get(conv, transposed, force, pack)
+        return cache.get(conv, transposed, force, pack, weight_fn, variant)
 
     def __getstate__(self):
         return {k: v for k, v in self.__dict__.items() if k not in self._DERIVED and k != "_pack_cache"}

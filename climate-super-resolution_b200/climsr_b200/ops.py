@@ -10,7 +10,7 @@ from torch import Tensor
 from ._lib import ConvDesc, WgradDesc, check, current_stream_ptr, lib
 
 ACT = {"none": 0, "lrelu": 1, "relu": 2, "lrelu_slope": 4}
-OUT_MODE = {"nhwc": 0, "f32_planar": 2, "f32_nhwc": 3}
+OUT_MODE = {"nhwc": 0, "f32_planar": 2, "f32_nhwc": 3, "split": 4}
 
 
 def nchw_to_nhwc_bf16(x: Tensor, dst_c: int = 64) -> Tensor:
@@ -31,6 +31,26 @@ def nhwc_bf16_to_nchw(x: Tensor, c: int, coff: int = 0) -> Tensor:
     return out
 
 
+def nchw_to_nhwc_split(x: Tensor, dst_c: int = 16, out: Optional[Tensor] = None) -> Tensor:
+    """fp32 NCHW (c <= 3) -> bf16 NHWC hi/lo pairs [hi_0..hi_{c-1}, lo_0..lo_{c-1}, 0...] with dst_c channels per pixel
+    (csr_nchw_f32_to_nhwc_split).  ``out``: an (n, h, w, dst_c) bf16 view to write instead of a new buffer."""
+    n, c, h, w = x.shape
+    if out is None:
+        out = torch.empty((n, h, w, dst_c), dtype=torch.bfloat16, device=x.device)
+    xs = x.contiguous().float()
+    check(lib.csr_nchw_f32_to_nhwc_split(xs.data_ptr(), out.data_ptr(), n, c, h, w, dst_c, current_stream_ptr()),
+          "csr_nchw_f32_to_nhwc_split")
+    return out
+
+
+def maxpool2x2_split(x: Tensor) -> Tensor:
+    """nn.MaxPool2d(2) of the values hi + lo held by a bf16 NHWC (n, h, w, 2c) hi/lo buffer, re-split (csr_maxpool2x2_split)."""
+    n, h, w, c2 = x.shape
+    out = torch.empty((n, h // 2, w // 2, c2), dtype=torch.bfloat16, device=x.device)
+    check(lib.csr_maxpool2x2_split(x.data_ptr(), out.data_ptr(), n, h, w, c2 // 2, current_stream_ptr()), "csr_maxpool2x2_split")
+    return out
+
+
 def conv2d_nhwc(inp: Tensor, weight: Tensor, bias: Optional[Tensor], *, act: str = "none", out: Optional[Tensor] = None,
                 out_coff: int = 0, out_mode: str = "nhwc", in_coff: int = 0, in_up2: bool = False, transposed: bool = False,
                 res1: Optional[Tensor] = None, res1_coff: int = 0, scale1: float = 1.0,
@@ -40,7 +60,8 @@ def conv2d_nhwc(inp: Tensor, weight: Tensor, bias: Optional[Tensor], *, act: str
     """One KxK stride-1 'same' conv on a bf16 NHWC buffer via csr_conv2d_nhwc.
 
     Reads input channels [in_coff, in_coff+cin); writes act(conv+bias) (then *scale1+res1, *scale2+res2, lrelu-gate) into
-    channels [out_coff, out_coff+cout) of `out` (allocated as a 64-channel-padded buffer when None).  in_up2: the input
+    channels [out_coff, out_coff+cout) of `out` (allocated as a 64-channel-padded buffer when None; out_mode "split": hi in
+    [out_coff, out_coff+cout), lo in [out_coff+cout, out_coff+2*cout), a 2*cout-channel buffer when None).  in_up2: the input
     is nearest-x2 upsampled first (output is 2h x 2w).  transposed: `weight` is the forward layer's OIHW tensor and the
     op computed is that layer's input gradient (cin/cout swap roles).
     """
@@ -54,6 +75,8 @@ def conv2d_nhwc(inp: Tensor, weight: Tensor, bias: Optional[Tensor], *, act: str
     if out is None:
         if mode == 2:
             out = torch.empty((n, 1, s * h, s * w), dtype=torch.float32, device=inp.device)
+        elif mode == 4:
+            out = torch.empty((n, h, w, out_coff + 2 * cout), dtype=torch.bfloat16, device=inp.device)
         else:
             oc = (out_coff + cout + 63) // 64 * 64
             # every channel of every pixel is written when the layer fills the buffer exactly: no zero fill needed then

@@ -50,7 +50,7 @@ class SuperResolutionTask(nn.Module):
         self.loss = losses.MSELoss() if generator_type == "srcnn" else losses.L1Loss()
         self.pixel_level_criterion = losses.L1Loss()                    # pl_gan.py:20
         self.adversarial_criterion = nn.BCEWithLogitsLoss()             # pl_gan.py:21 (a scalar epilogue on N logits)
-        self.perceptual_criterion = perceptual_criterion               # pl_gan.py:19 (VGG19 features: out of scope, optional plug-in)
+        self.perceptual_criterion = perceptual_criterion               # pl_gan.py:19 (losses.PerceptualLoss: VGG19 features; None = term off)
         self.pixel_level_loss_factor = pixel_level_loss_factor          # conf/task/gan_training.yaml:6-8
         self.perceptual_loss_factor = perceptual_loss_factor
         self.adversarial_loss_factor = adversarial_loss_factor

@@ -302,10 +302,11 @@ struct DenseLaunch {
   size_t w_off[kDenseMaxLayers], b_off[kDenseMaxLayers];   // offsets into the packed blob (resolved at forward time)
 };
 
-enum OutKind { kOutBf16 = 0, kOutF32Planar = 1, kOutF32Nhwc = 2 };
+enum OutKind { kOutBf16 = 0, kOutF32Planar = 1, kOutF32Nhwc = 2, kOutBf16Split = 3 };
 struct ConvIO {
   const void* in = nullptr; int in_C = 0, cin_off = 0;
   void* out = nullptr; int out_C = 0, out_coff = 0; int out_kind = kOutBf16;
+  int split_off = 0;       // kOutBf16Split: channel distance from a hi value to its lo
   int act = CSR_ACT_NONE;
   const void* r1 = nullptr; int r1_C = 0, r1_coff = 0; float s1 = 1.f;
   const void* r2 = nullptr; int r2_C = 0, r2_coff = 0; float s2 = 1.f;
@@ -315,7 +316,9 @@ struct ConvIO {
 // H, W: spatial size of the launch's input (for an up2 layer: the low-resolution input; its output is 2H x 2W).
 static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int W, const ConvIO& io, ConvLaunch* cl) {
   if (io.in_C % 8 != 0 || io.cin_off % 8 != 0) return fail(CSR_ERR_BAD_ARG, "input buffer channels (%d) / offset (%d) must be multiples of 8", io.in_C, io.cin_off);
-  if (io.out_kind == kOutBf16 && ((io.out_C % 8) || (io.out_coff % 8))) return fail(CSR_ERR_BAD_ARG, "output channel stride/offset must be multiples of 8");
+  const bool split = io.out_kind == kOutBf16Split;
+  if ((io.out_kind == kOutBf16 || split) && ((io.out_C % 8) || (io.out_coff % 8))) return fail(CSR_ERR_BAD_ARG, "output channel stride/offset must be multiples of 8");
+  if (split && (pp.n_store % 8 || io.split_off % 8)) return fail(CSR_ERR_UNSUPPORTED, "hi/lo output needs output channels in multiples of 8");
   ConvParams& p = cl->p;
   memset(&p, 0, sizeof(p));
   p.N = N; p.H = H; p.W = W;
@@ -327,8 +330,10 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
   p.n_kblocks = ceil_div(p.cin, 64);
   p.w_bytes = pp.w_bytes;
   const int up = pp.phase >= 0 ? 2 : 1;
-  const bool tma_out = io.out_kind == kOutBf16 && pp.n_store % 8 == 0 && !g_opt_no_tma_store;
-  p.store_mode = tma_out ? kStoreStaged : io.out_kind == kOutBf16 ? kStoreDirect : io.out_kind == kOutF32Planar ? kStoreF32Planar : kStoreF32Nhwc;
+  // hi/lo pairs are only ever staged: a staging buffer holds the hi tile and then the lo tile (stage_mult = 2)
+  const bool tma_out = split || (io.out_kind == kOutBf16 && pp.n_store % 8 == 0 && !g_opt_no_tma_store);
+  const int stage_mult = split ? 2 : 1;
+  p.store_mode = split ? kStoreBf16Split : tma_out ? kStoreStaged : io.out_kind == kOutBf16 ? kStoreDirect : io.out_kind == kOutF32Planar ? kStoreF32Planar : kStoreF32Nhwc;
   p.stage_row_bytes = tma_out ? pp.n_store * 2 : 0;
   // four tiles in flight in the epilogue when four accumulators fit in TMEM and a warp then owns <= 4 chunks of 8 channels
   p.n_acc = (4 * p.KW * p.npad <= 512 && p.npad <= 32) ? 4 : 2;
@@ -351,10 +356,10 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
     p.stream_w = 1;
     p.n_groups = 1;                                        // one staging buffer: two (window + weight k-block) slots of ~96 KB must fit
     p.wkb_bytes = pp.kh * 4 * pp.kw * pp.npad * 32;
-    rc = choose_tiling(H, W, pp.kh, pp.kw, 0, p.n_kblocks, p.stage_row_bytes, p.n_groups, &tl, 128, 1, p.wkb_bytes);
+    rc = choose_tiling(H, W, pp.kh, pp.kw, 0, p.n_kblocks, p.stage_row_bytes, p.n_groups * stage_mult, &tl, 128, 1, p.wkb_bytes);
     if (!rc && tl.n_slots < 2) rc = fail(CSR_ERR_UNSUPPORTED, "streamed-weight conv: window ring too shallow");
-  } else rc = choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, p.n_groups, &tl, p.box_c * 2);
-  if (!rc && g_opt_tall && p.n_acc == 4 && p.n_groups == 4) {
+  } else rc = choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, p.n_groups * stage_mult, &tl, p.box_c * 2);
+  if (!rc && g_opt_tall && p.n_acc == 4 && p.n_groups == 4 && !split) {
     Tiling t2;   // taken unless the second M tile would mostly hang below the image
     if (choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, p.n_groups, &t2, p.box_c * 2, 2) == CSR_OK &&
         t2.eff >= 0.85 * tl.eff && t2.n_slots >= 2) {
@@ -372,7 +377,7 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
     // one tile shorten its latency chain (-2 % per inference step).  RDB conv5 and the gated input-gradient convs of the backward
     // lose with it: there the single group paces the tile.
     Tiling t1;
-    if (choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, 1, &t1, p.box_c * 2) == CSR_OK) {
+    if (choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, stage_mult, &t1, p.box_c * 2) == CSR_OK) {
       tl = t1;
       p.n_groups = 1;
     }
@@ -383,7 +388,7 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
   // buffers; KW <= 2 layers also get four accumulator buffers (4 x KW x 64 <= 512 TMEM columns).
   const bool early_plain = !has_res && p.n_groups == 1 &&
       ((p.KW == 3 && p.PW == 1 && (p.act == 0 || p.act == 1)) || (p.KW == 2 && p.PW <= 1 && p.act == 1) || (p.KW == 1 && p.PW == 0 && p.act == 2));
-  if (g_opt_early && early_plain && !p.tall_shift && tma_out && p.npad == 64 && pp.n_store == 64) {
+  if (g_opt_early && early_plain && !split && !p.tall_shift && tma_out && p.npad == 64 && pp.n_store == 64) {
     Tiling te2, te1;
     const bool ok2 = choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, 2, &te2, p.box_c * 2) == CSR_OK;
     const bool ok1 = choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, 1, &te1, p.box_c * 2) == CSR_OK;
@@ -422,6 +427,11 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
   p.win_rows = tl.win_rows; p.win_bytes = tl.win_bytes; p.slot_bytes = tl.slot_bytes; p.n_slots = tl.n_slots;
   p.win_slot_bytes = (int)align_up(tl.win_bytes, 1024);
   p.stage_bytes = tl.stage_bytes;
+  if (split) {
+    p.stage_lo_bytes = tl.stage_bytes;
+    p.stage_bytes = 2 * tl.stage_bytes;
+    p.split_off = io.split_off;
+  }
   int cols = 32;
   while (cols < p.n_acc * (p.hyb ? p.KW - 1 : p.KW) * p.npad) cols *= 2;
   if (cols > 512 || p.KW * p.npad > 256) return fail(CSR_ERR_UNSUPPORTED, "KW*npad = %d exceeds the UMMA N / TMEM budget", p.KW * p.npad);
@@ -1883,8 +1893,15 @@ static int conv_desc_to_layer(const CsrConvDesc* d, LayerSpec* L) {
   if (d->n < 1 || d->h < 1 || d->w < 1 || d->cin < 1 || d->cout < 1) return fail(CSR_ERR_BAD_ARG, "non-positive conv shape");
   if (!(d->kh & 1) || !(d->kw & 1) || d->kh > 9 || d->kw > 9) return fail(CSR_ERR_UNSUPPORTED, "kernel %dx%d (odd, <= 9 supported)", d->kh, d->kw);
   if (d->cout > 1024) return fail(CSR_ERR_UNSUPPORTED, "cout %d > 1024", d->cout);
-  if (d->out_mode != CSR_OUT_BF16_NHWC && d->out_mode != CSR_OUT_F32_PLANAR && d->out_mode != CSR_OUT_F32_NHWC)
+  if (d->out_mode != CSR_OUT_BF16_NHWC && d->out_mode != CSR_OUT_F32_PLANAR && d->out_mode != CSR_OUT_F32_NHWC && d->out_mode != CSR_OUT_BF16_SPLIT)
     return fail(CSR_ERR_BAD_ARG, "unknown out_mode %d", d->out_mode);
+  if (d->out_mode == CSR_OUT_BF16_SPLIT) {
+    if (d->kh != 3 || d->kw != 3 || d->act != CSR_ACT_RELU || d->in_up2 || d->transposed)
+      return fail(CSR_ERR_UNSUPPORTED, "hi/lo bf16 output is implemented for plain 3x3 convs with ReLU only");
+    if (d->cout % 8 || d->out_c < d->out_coff + 2 * d->cout)
+      return fail(CSR_ERR_UNSUPPORTED, "hi/lo bf16 output needs cout %% 8 == 0 and out_c >= out_coff + 2 cout (cout %d, out_c %d, out_coff %d)",
+                  d->cout, d->out_c, d->out_coff);
+  }
   if (d->out_mode == CSR_OUT_F32_PLANAR && d->cout != 1) return fail(CSR_ERR_UNSUPPORTED, "fp32 planar output needs cout == 1");
   if (d->in_up2 && (d->kh != 3 || d->kw != 3)) return fail(CSR_ERR_UNSUPPORTED, "nearest-x2 input needs a 3x3 kernel");
   if (d->in_up2 && d->transposed) return fail(CSR_ERR_UNSUPPORTED, "in_up2 and transposed cannot be combined");
@@ -1938,7 +1955,10 @@ int csr_conv2d_nhwc(const CsrConvDesc* d, const void* in, const float* weight, c
   ConvIO io;
   io.in = in; io.in_C = d->in_c; io.cin_off = d->in_coff;
   io.out = out; io.out_C = d->out_c; io.out_coff = d->out_coff;
-  io.out_kind = d->out_mode == CSR_OUT_BF16_NHWC ? kOutBf16 : d->out_mode == CSR_OUT_F32_PLANAR ? kOutF32Planar : kOutF32Nhwc;
+  io.out_kind = d->out_mode == CSR_OUT_BF16_NHWC ? kOutBf16 : d->out_mode == CSR_OUT_F32_PLANAR ? kOutF32Planar :
+                d->out_mode == CSR_OUT_BF16_SPLIT ? kOutBf16Split : kOutF32Nhwc;
+  io.split_off = d->cout;
+  if (d->out_mode == CSR_OUT_BF16_SPLIT && (res1 || res2 || gate)) return fail(CSR_ERR_UNSUPPORTED, "hi/lo bf16 output takes no residual / gate operand");
   io.act = d->act;
   io.r1 = res1; io.r1_C = d->res1_c; io.r1_coff = d->res1_coff; io.s1 = d->scale1;
   io.r2 = res2; io.r2_C = d->res2_c; io.r2_coff = d->res2_coff; io.s2 = d->scale2;
@@ -1953,7 +1973,7 @@ int csr_conv2d_nhwc(const CsrConvDesc* d, const void* in, const float* weight, c
   // Equal output-channel parts of a residual-free layer go out as ONE launch (gridDim.y = parts): a 512-channel layer over an
   // 8 x 8 map is 8 parts of ~16 tiles each - one after the other they would leave nine SMs in ten idle.
   const std::vector<PackPart>& parts = packs[0].parts;
-  bool merge = parts.size() > 1 && !res1 && !res2 && !gate && d->out_mode == CSR_OUT_BF16_NHWC;
+  bool merge = parts.size() > 1 && !res1 && !res2 && !gate && (d->out_mode == CSR_OUT_BF16_NHWC || d->out_mode == CSR_OUT_BF16_SPLIT);
   for (size_t i = 1; merge && i < parts.size(); ++i)
     merge = parts[i].phase < 0 && parts[i].npad == parts[0].npad && parts[i].n_store == parts[0].npad && parts[0].n_store == parts[0].npad &&
             parts[i].w_bytes == parts[0].w_bytes && parts[i].w_off - parts[i - 1].w_off == parts[1].w_off - parts[0].w_off &&
@@ -2039,6 +2059,28 @@ int csr_nhwc_bf16_to_nchw_f32(const void* src, float* dst, int32_t n, int32_t c,
                               void* stream) {
   if (!src || !dst) return fail(CSR_ERR_BAD_ARG, "null pointer");
   CSR_CUDA(launch_nhwc_to_nchw(src, dst, n, c, h, w, src_c, src_coff, reinterpret_cast<cudaStream_t>(stream)));
+  ++g_launches;
+  return CSR_OK;
+}
+
+// ---- hi/lo bf16 activations (perceptual loss) -----------------------------------------------------------
+int csr_nchw_f32_to_nhwc_split(const float* src, void* dst, int32_t n, int32_t c, int32_t h, int32_t w, int32_t dst_c, void* stream) {
+  if (!src || !dst) return fail(CSR_ERR_BAD_ARG, "null pointer");
+  if (n < 1 || h < 1 || w < 1) return fail(CSR_ERR_BAD_ARG, "non-positive shape %dx%dx%d", n, h, w);
+  if (c < 1 || c > 3 || dst_c % 8 || dst_c < 2 * c || dst_c > 64)
+    return fail(CSR_ERR_UNSUPPORTED, "split conversion: c=%d (1..3), dst_c=%d (multiple of 8, 2c..64)", c, dst_c);
+  if (reinterpret_cast<uintptr_t>(dst) % 16) return fail(CSR_ERR_BAD_ARG, "dst must be 16-byte aligned");
+  CSR_CUDA(launch_nchw_to_nhwc_split(src, dst, n, c, h, w, dst_c, reinterpret_cast<cudaStream_t>(stream)));
+  ++g_launches;
+  return CSR_OK;
+}
+
+int csr_maxpool2x2_split(const void* src, void* dst, int32_t n, int32_t h, int32_t w, int32_t c, void* stream) {
+  if (!src || !dst) return fail(CSR_ERR_BAD_ARG, "null pointer");
+  if (n < 1) return fail(CSR_ERR_BAD_ARG, "non-positive batch %d", n);
+  if (h < 2 || w < 2 || c < 8 || c % 8) return fail(CSR_ERR_UNSUPPORTED, "split max pool: h=%d, w=%d (>= 2), c=%d (multiple of 8)", h, w, c);
+  if ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) % 16) return fail(CSR_ERR_BAD_ARG, "src / dst must be 16-byte aligned");
+  CSR_CUDA(launch_maxpool2x2_split(src, dst, n, h, w, c, reinterpret_cast<cudaStream_t>(stream)));
   ++g_launches;
   return CSR_OK;
 }

@@ -134,7 +134,8 @@ __device__ __forceinline__ uint4 ldg16(const void* base, size_t pix, int C, int 
 //   KW_T  horizontal taps (0 = runtime p.KW, taps gathered one at a time);  PW_T left padding when KW_T > 0
 //   ACT_T activation (-1 = runtime p.act);  RES_T bit0 r1, bit1 r2, bit2 gate (-1 = runtime pointers)
 //   ST_T  1 = staged bf16 stores only, 3 = fp32 planar single-channel output only (conv_last, srcnn.conv3: just channel 0
-//         is computed), -1 = runtime p.store_mode
+//         is computed), 4 = staged hi/lo bf16 pairs (kStoreBf16Split: the VGG19 convs of the perceptual loss), -1 = runtime
+//         p.store_mode
 //   TALL_T 1 = two M tiles per window (ConvParams::tall_shift), compile-time so that the common kernels carry none of it
 //   HYB_T 1 = (3x3, early-release epilogue) only TWO of the three horizontal taps are folded into N: per (dy, k-step) one N = 2*npad MMA
 //            (taps dx = 0, 1) plus one N = npad MMA for tap dx = 2 whose A operand starts one pixel later and which accumulates into the
@@ -409,7 +410,7 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
     const bool has_r1 = RES_T >= 0 ? (RES_T & 1) != 0 : p.r1 != nullptr;
     const bool has_r2 = RES_T >= 0 ? (RES_T & 2) != 0 : p.r2 != nullptr;
     const bool has_gate = RES_T >= 0 ? (RES_T & 4) != 0 : p.gate != nullptr;
-    const bool tma_store = ST_T >= 0 ? ST_T == 1 : (p.store_mode == kStoreStaged);
+    const bool tma_store = ST_T >= 0 ? (ST_T == 1 || ST_T == 4) : (p.store_mode == kStoreStaged);
     const bool need_pix = !tma_store || has_r1 || has_r2 || has_gate;    // warp-uniform
     const uint32_t swz = (p.stage_row_bytes == 128) ? static_cast<uint32_t>(srow & 7) : 0u;   // SWIZZLE_128B staging rows
     const uint32_t srow_addr = stage_addr + static_cast<uint32_t>(g) * p.stage_bytes + static_cast<uint32_t>(srow * p.stage_row_bytes);
@@ -678,7 +679,17 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
             if (has_gate) gate8(v, q2[j], p.gate_neg);
             else if (has_r2) fma_residual8(v, q2[j], p.s2);
           }
-          if (tma_store) {
+          if constexpr (ST_T == 4) {
+            // hi tile and lo tile side by side in the staging buffer, same swizzle
+            if (col_ok && ch0 < p.n_store) {
+              uint32_t hi[4], lo[4];
+#pragma unroll
+              for (int i = 0; i < 4; ++i) split_bf16x2(v[2 * i], v[2 * i + 1], &hi[i], &lo[i]);
+              const uint32_t a = srow_addr + ((static_cast<uint32_t>(c) ^ swz) << 4);
+              st_shared_v4(a, hi[0], hi[1], hi[2], hi[3]);
+              st_shared_v4(a + static_cast<uint32_t>(p.stage_lo_bytes), lo[0], lo[1], lo[2], lo[3]);
+            }
+          } else if (tma_store) {
             if (col_ok && ch0 < p.n_store)
               st_shared_v4(srow_addr + ((static_cast<uint32_t>(c) ^ swz) << 4), pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]),
                            pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
@@ -721,6 +732,10 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
           if (ok) {
             const uint4 val = ld_shared_v4(pc_s[k]);
             *reinterpret_cast<uint4*>(tile_out + pc_d[k]) = val;
+            if constexpr (ST_T == 4) {
+              const uint4 lo = ld_shared_v4(pc_s[k] + static_cast<uint32_t>(p.stage_lo_bytes));
+              *reinterpret_cast<uint4*>(tile_out + pc_d[k] + p.split_off) = lo;
+            }
           }
         }
       }
@@ -779,6 +794,12 @@ static int launch_t(const ConvParams& p, const CUtensorMap& tmap, int num_sms, c
 int launch_conv_tc(const ConvParams& p, const CUtensorMap& tmap, int num_sms, cudaStream_t stream) {
   const int res = (p.r1 ? 1 : 0) | (p.r2 ? 2 : 0) | (p.gate ? 4 : 0);
   if ((res & 6) == 6) return static_cast<int>(cudaErrorInvalidValue);   // r2 and gate share an operand slot
+  // hi/lo bf16 pairs (the VGG19 convs of the perceptual loss): one specialisation, no runtime-switch fallback
+  if (p.store_mode == kStoreBf16Split) {
+    if (p.KW == 3 && p.PW == 1 && p.act == 2 && res == 0 && !p.tall_shift && !p.early && !p.fuse2 && !p.hyb)
+      return launch_t<3, 1, 2, 0, 4>(p, tmap, num_sms, stream);
+    return static_cast<int>(cudaErrorInvalidValue);
+  }
   if (p.tall_shift) {
     // two-M-tile windows: the thin layers only (four accumulator buffers)
     if ((p.n_acc != 4 && p.n_acc != 8) || p.n_groups != 4) return static_cast<int>(cudaErrorInvalidValue);

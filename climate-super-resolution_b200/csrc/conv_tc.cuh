@@ -18,7 +18,9 @@ enum StoreMode {
   kStoreStaged = 0,     // bf16 NHWC through a swizzled shared-memory staging tile, copied out as whole pixel rows
   kStoreDirect = 1,     // bf16 NHWC, per-element global stores (ragged channel counts)
   kStoreF32Planar = 2,  // fp32 (N,1,H,W), channel 0 only
-  kStoreF32Nhwc = 3     // fp32 NHWC (n_store channels per pixel, pitch out_C): gradient / debug outputs
+  kStoreF32Nhwc = 3,    // fp32 NHWC (n_store channels per pixel, pitch out_C): gradient / debug outputs
+  kStoreBf16Split = 4   // staged like kStoreStaged, as a hi/lo bf16 pair: hi = bf16(v) at channel c, lo = bf16(v - hi) at channel
+                        // split_off + c (VGG features of the perceptual loss: the pair carries v to fp32 precision)
 };
 
 struct ConvParams {
@@ -85,7 +87,9 @@ struct ConvParams {
   int out_sy, out_sx, out_oy, out_ox;   // conv-output pixel (y,x) lives at buffer pixel (y*out_sy+out_oy, x*out_sx+out_ox)
   int out_H, out_W;                     // spatial size of the output buffer
   int stage_row_bytes; // kStoreStaged: bytes per staged pixel (n_store * 2: 16..128)
-  int stage_bytes;     // one staging buffer (TH*TW*stage_row_bytes rounded up to 1024)
+  int stage_bytes;     // one staging buffer (TH*TW*stage_row_bytes rounded up to 1024; twice that for kStoreBf16Split)
+  int stage_lo_bytes;  // kStoreBf16Split: offset of the lo tile inside a staging buffer (the hi tile is at 0)
+  int split_off;       // kStoreBf16Split: channel distance between a hi value and its lo (the layer's total output channels)
   long long* trace;    // debug: per-role clock64 timestamps of CTA 0 (nullptr = off), [3 roles][64 tiles][4 events]
   unsigned long long* timeline;   // debug (csr_debug_set_timeline): [2*launch_id] = earliest CTA start after griddepcontrol.wait,
   int launch_id;                  // [2*launch_id + 1] = latest CTA end, in globaltimer ns - the in-situ timeline of a forward

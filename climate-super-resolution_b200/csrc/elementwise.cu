@@ -141,6 +141,71 @@ __global__ void nchw_to_nhwc_kernel(const float* __restrict__ src, __nv_bfloat16
   }
 }
 
+// ---- hi/lo bf16 activations (perceptual loss, CSR_OUT_BF16_SPLIT) ------------------------------------------------
+// fp32 NCHW (n,c,h,w), c <= 3 -> bf16 NHWC (n,h,w,dst_c): channels [hi_0..hi_{c-1}, lo_0..lo_{c-1}, 0...], hi = bf16(x),
+// lo = bf16(x - hi).  The input needs the pair too: one bf16 ulp near 1 (0.0039) is larger than the differences between
+// hr and sr the loss has to resolve.
+__global__ void nchw_to_nhwc_split_kernel(const float* __restrict__ src, __nv_bfloat16* __restrict__ dst, long npix_per_img,
+                                          long total_pix, int c, int dst_c) {
+  for (long p = blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x; p < total_pix; p += static_cast<long>(gridDim.x) * blockDim.x) {
+    const long n = p / npix_per_img;
+    const long r = p - n * npix_per_img;
+    float f[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+      if (i < c) {
+        const float x = src[(n * c + i) * npix_per_img + r];
+        const float hi = __bfloat162float(__float2bfloat16_rn(x));
+        f[i] = hi;                                        // exact bf16 values: pack_bf16x2 below does not round them again
+        f[c + i] = __bfloat162float(__float2bfloat16_rn(x - hi));
+      }
+    }
+    uint4* o = reinterpret_cast<uint4*>(dst + p * dst_c);
+    o[0] = make_uint4(pack_bf16x2(f[0], f[1]), pack_bf16x2(f[2], f[3]), pack_bf16x2(f[4], f[5]), pack_bf16x2(f[6], f[7]));
+    for (int k = 1; k < (dst_c >> 3); ++k) o[k] = make_uint4(0u, 0u, 0u, 0u);
+  }
+}
+
+// nn.MaxPool2d(2) (ceil_mode=False) over hi/lo pairs: src (n,h,w,2c) -> dst (n,h/2,w/2,2c).  One thread per (output pixel,
+// 8 channels): 16-byte loads of the hi and lo vectors of the four window pixels; hi + lo is exact in fp32, so the max of
+// the sums re-splits into the winning pixel's own pair.  Window order and the NaN rule are those of F.max_pool2d
+// ((v > m) || isnan(v), starting from -inf): the first maximum wins, a NaN anywhere in the window is the result.
+__global__ void maxpool2x2_split_kernel(const __nv_bfloat16* __restrict__ src, __nv_bfloat16* __restrict__ dst, int h, int w, int c,
+                                        long total) {
+  const int ho = h >> 1, wo = w >> 1, g8 = c >> 3;
+  for (long i = blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x; i < total; i += static_cast<long>(gridDim.x) * blockDim.x) {
+    const int g = static_cast<int>(i % g8);
+    long q = i / g8;
+    const int x = static_cast<int>(q % wo);
+    q /= wo;
+    const int y = static_cast<int>(q % ho);
+    const long n = q / ho;
+    float m[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) m[j] = -INFINITY;
+#pragma unroll
+    for (int t = 0; t < 4; ++t) {
+      const long pix = (n * h + 2 * y + (t >> 1)) * w + 2 * x + (t & 1);
+      const __nv_bfloat16* base = src + pix * 2 * c + g * 8;
+      const uint4 hv = __ldg(reinterpret_cast<const uint4*>(base));
+      const uint4 lv = __ldg(reinterpret_cast<const uint4*>(base + c));
+      const uint32_t hw[4] = {hv.x, hv.y, hv.z, hv.w}, lw[4] = {lv.x, lv.y, lv.z, lv.w};
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        const float v0 = bf16lo(hw[k]) + bf16lo(lw[k]), v1 = bf16hi(hw[k]) + bf16hi(lw[k]);
+        if (v0 > m[2 * k] || isnan(v0)) m[2 * k] = v0;
+        if (v1 > m[2 * k + 1] || isnan(v1)) m[2 * k + 1] = v1;
+      }
+    }
+    uint32_t hi[4], lo[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) split_bf16x2(m[2 * k], m[2 * k + 1], &hi[k], &lo[k]);
+    __nv_bfloat16* o = dst + ((n * ho + y) * wo + x) * 2 * c + g * 8;
+    *reinterpret_cast<uint4*>(o) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+    *reinterpret_cast<uint4*>(o + c) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+  }
+}
+
 // SRCNN input as an x-im2col buffer: torch.cat([out, elev, mask], 1) (esrgan.py:100) followed by the horizontal half of
 // srcnn.conv1's 9x9 window.  For pixel (n,y,x) channel dx*3 + c (dx = 0..8, c = 0: conv_last output, 1: elev, 2: mask)
 // holds source c at (y, x+dx-4), zero outside the image (the conv's zero padding); channels 27..31 are zero.  The 9x9
@@ -403,6 +468,17 @@ cudaError_t launch_pack_bias(const float* b, float* dst, int cout, int co_lo, in
 cudaError_t launch_nchw_to_nhwc(const float* src, void* dst, int n, int c, int h, int w, int dst_c, int zero_to, cudaStream_t s) {
   const long per = static_cast<long>(h) * w, total = per * n;
   nchw_to_nhwc_kernel<<<grid_for(total, 256), 256, 0, s>>>(src, reinterpret_cast<__nv_bfloat16*>(dst), per, total, c, dst_c, zero_to);
+  return cudaGetLastError();
+}
+cudaError_t launch_nchw_to_nhwc_split(const float* src, void* dst, int n, int c, int h, int w, int dst_c, cudaStream_t s) {
+  const long per = static_cast<long>(h) * w, total = per * n;
+  nchw_to_nhwc_split_kernel<<<grid_for(total, 256), 256, 0, s>>>(src, reinterpret_cast<__nv_bfloat16*>(dst), per, total, c, dst_c);
+  return cudaGetLastError();
+}
+cudaError_t launch_maxpool2x2_split(const void* src, void* dst, int n, int h, int w, int c, cudaStream_t s) {
+  const long total = static_cast<long>(n) * (h >> 1) * (w >> 1) * (c >> 3);
+  maxpool2x2_split_kernel<<<grid_for(total, 256), 256, 0, s>>>(reinterpret_cast<const __nv_bfloat16*>(src), reinterpret_cast<__nv_bfloat16*>(dst),
+                                                               h, w, c, total);
   return cudaGetLastError();
 }
 cudaError_t launch_pack_srcnn_in(const float* t, const float* elev, const float* mask, void* dst, int W, long total_pix, int dst_c,

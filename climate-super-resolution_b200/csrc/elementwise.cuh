@@ -17,6 +17,9 @@ cudaError_t launch_pack_weight(const float* w, void* dst, int cout, int cin, int
                                float wscale, int co_lo, int npad, int cin_pad, cudaStream_t s);
 cudaError_t launch_pack_bias(const float* b, float* dst, int cout, int co_lo, int npad, cudaStream_t s);
 cudaError_t launch_nchw_to_nhwc(const float* src, void* dst, int n, int c, int h, int w, int dst_c, int zero_to, cudaStream_t s);
+// hi/lo bf16 activations of the perceptual loss (CSR_OUT_BF16_SPLIT): input conversion and 2x2 max pool
+cudaError_t launch_nchw_to_nhwc_split(const float* src, void* dst, int n, int c, int h, int w, int dst_c, cudaStream_t s);
+cudaError_t launch_maxpool2x2_split(const void* src, void* dst, int n, int h, int w, int c, cudaStream_t s);
 cudaError_t launch_pack_srcnn_in(const float* t, const float* elev, const float* mask, void* dst, int W, long total_pix, int dst_c,
                                  cudaStream_t s);
 cudaError_t launch_nhwc_to_nchw(const void* src, float* dst, int n, int c, int h, int w, int src_c, int src_coff, cudaStream_t s);

@@ -209,5 +209,10 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
 }
 __device__ __forceinline__ float bf16lo(uint32_t v) { return __uint_as_float(v << 16); }
 __device__ __forceinline__ float bf16hi(uint32_t v) { return __uint_as_float(v & 0xFFFF0000u); }
+// hi/lo bf16 pair of two fp32 values: hi = bf16(v), lo = bf16(v - hi) (v - hi is exact in fp32; hi + lo is v to ~2^-16 relative)
+__device__ __forceinline__ void split_bf16x2(float a, float b, uint32_t* hi, uint32_t* lo) {
+  *hi = pack_bf16x2(a, b);
+  *lo = pack_bf16x2(a - bf16lo(*hi), b - bf16hi(*hi));
+}
 
 }  // namespace csr

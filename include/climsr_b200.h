@@ -65,7 +65,11 @@ typedef enum CsrAct { CSR_ACT_NONE = 0, CSR_ACT_LRELU02 = 1, CSR_ACT_RELU = 2,
 typedef enum CsrOutMode {
   CSR_OUT_BF16_NHWC = 0,     /* bf16, channel slice [out_coff, out_coff+cout) of an NHWC buffer          */
   CSR_OUT_F32_PLANAR = 2,    /* fp32 (N,1,H,W); cout must be 1                                            */
-  CSR_OUT_F32_NHWC = 3       /* fp32 NHWC, channel slice [out_coff, out_coff+cout) (gradients, debugging) */
+  CSR_OUT_F32_NHWC = 3,      /* fp32 NHWC, channel slice [out_coff, out_coff+cout) (gradients, debugging) */
+  CSR_OUT_BF16_SPLIT = 4     /* hi/lo bf16 pair of every output value v: hi = bf16(v) at channel out_coff + c, lo = bf16(v - hi)
+                                at channel out_coff + cout + c (hi + lo carries v to ~2^-16 relative).  A following conv over the
+                                2*cout channels with weights [W | W] computes W (hi + lo) in fp32.  3x3 convs with CSR_ACT_RELU and
+                                no residual / gate only; cout % 8 == 0, out_c >= out_coff + 2*cout.  (The VGG19 perceptual loss.) */
 } CsrOutMode;
 
 typedef struct CsrConvDesc {
@@ -211,6 +215,17 @@ int     csr_nchw_f32_to_nhwc_bf16(const float* src, void* dst, int32_t n, int32_
 /* bf16 NHWC channel slice -> fp32 NCHW (n,c,h,w)                                                 */
 int     csr_nhwc_bf16_to_nchw_f32(const void* src, float* dst, int32_t n, int32_t c, int32_t h, int32_t w,
                                   int32_t src_c, int32_t src_coff, void* stream);
+
+/* ---- hi/lo bf16 activations (VGG19 perceptual loss; see CSR_OUT_BF16_SPLIT) ---------------------------------------
+ * A value v is held as the pair hi = bf16(v), lo = bf16(v - hi): C channels are stored as 2C channels [hi_0..hi_{C-1} |
+ * lo_0..lo_{C-1}].
+ *   csr_nchw_f32_to_nhwc_split  fp32 NCHW (n,c,h,w), c <= 3 -> bf16 NHWC (n,h,w,dst_c) = [hi_0..hi_{c-1}, lo_0..lo_{c-1}, 0...];
+ *                               dst_c a multiple of 8, 2c <= dst_c <= 64
+ *   csr_maxpool2x2_split        nn.MaxPool2d(2) (floor, NaN-propagating) of hi + lo (exact in fp32), re-split:
+ *                               src (n,h,w,2c) -> dst (n,h/2,w/2,2c); h, w >= 2, c % 8 == 0                                */
+int     csr_nchw_f32_to_nhwc_split(const float* src, void* dst, int32_t n, int32_t c, int32_t h, int32_t w, int32_t dst_c,
+                                   void* stream);
+int     csr_maxpool2x2_split(const void* src, void* dst, int32_t n, int32_t h, int32_t w, int32_t c, void* stream);
 
 /* ---- pixel loss of the training step: mean over all numel elements, value AND gradient in one HBM pass --------
  * out[0] = mean |sr - hr| (L1, esrgan) or mean (sr - hr)^2 (MSE, srcnn);  grad (nullable, numel floats) = d out / d sr.

@@ -10,7 +10,11 @@ climsr/models/discriminator.py:5-46 (eight reflection-padded 3x3 convs, stride 1
 stride-1 ones, two valid 3x3 convs, Linear 8192 -> 100 -> 1) run under bf16 autocast + channels_last; per-rank BatchNorm
 statistics (sync_batchnorm: False).  Multi-GPU: torchrun, bf16 bucketed all-reduce of both parameter sets.
 
-    python tools/bench_gan_step.py [--batch 16] [--steps 20]
+--perceptual cuda adds the 1.0 * perceptual term on this repo's path (climsr_b200.losses.PerceptualLoss, seeded VGG19 weights: hi/lo
+bf16 activations on the tcgen05 convs), --perceptual torch the same term as stock PyTorch fp32 with TF32 off (the accuracy-equivalent
+cuDNN arm of tools/bench_perceptual.py); the default, off, leaves it out as before.
+
+    python tools/bench_gan_step.py [--batch 16] [--steps 20] [--perceptual off|cuda|torch]
 """
 import argparse
 import json
@@ -50,6 +54,7 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--disc", default="cuda", choices=["cuda", "torch"])
+    ap.add_argument("--perceptual", default="off", choices=["off", "cuda", "torch"])
     args = ap.parse_args()
     world, rank, local = (int(os.environ.get(k, d)) for k, d in (("WORLD_SIZE", "1"), ("RANK", "0"), ("LOCAL_RANK", "0")))
     torch.cuda.set_device(local)
@@ -72,6 +77,14 @@ def main():
     hr = torch.rand(n, 1, 4 * h, 4 * h, device=dev) * 2 - 1
     real, fake = torch.ones((n, 1), device=dev), torch.zeros((n, 1), device=dev)
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(6)]
+    perc = None
+    if args.perceptual != "off":
+        sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+        from bench_perceptual import TorchPerceptual
+        perc = losses.PerceptualLoss(seed=0).to(dev)
+        if args.perceptual == "torch":
+            torch.backends.cudnn.allow_tf32 = False
+            perc = TorchPerceptual(perc).to(dev)
 
     def d_scores(a, b):
         if args.disc == "cuda":
@@ -92,6 +105,8 @@ def main():
         s_real, s_fake = d_scores(hr, sr)
         adv = (relativistic(s_fake, s_real, real) + relativistic(s_real, s_fake, fake)) / 2
         loss_g = 0.01 * losses.l1_loss(sr, hr) + 0.005 * adv
+        if perc is not None:
+            loss_g = loss_g + 1.0 * perc(hr, sr)
         loss_g.backward()
         for p_ in D.parameters():
             p_.requires_grad_(True)
@@ -130,9 +145,15 @@ def main():
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     if rank == 0:
+        extra = {}
+        if perc is not None:
+            from bench_perceptual import gpu_identity
+            extra = gpu_identity(local)
         print(json.dumps({"workload": f"cfg3 GAN step, batch {n}/GPU of 128x128 HR, Hydra generator (CUDA path) + " +
                                       ("discriminator on the CUDA path" if args.disc == "cuda" else "stock PyTorch discriminator (bf16 autocast, channels_last)") +
-                                      ", perceptual term disabled", "n_gpus": world,
+                                      (", perceptual term disabled" if perc is None else
+                                       f", perceptual term on the {'CUDA path (hi/lo bf16)' if args.perceptual == 'cuda' else 'cuDNN fp32 (TF32 off)'}"),
+                          **extra, "n_gpus": world,
                           "ms_per_step_max_over_ranks": float(t), "hr_mpx_s": world * n * 128 * 128 / float(t) / 1e3,
                           "split_ms_rank0": {"G_forward_train": ms[0], "D(hr),D(sr)_fwd + loss_G backward (through D and G) + allreduce + G step": ms[1],
                                              "G_forward_again (common_step of optimizer 1)": ms[2], "D fwd x2 + D backward + allreduce + D step": ms[3]}}))
