@@ -8,6 +8,7 @@
 #include <map>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/climsr_b200.h"
@@ -43,7 +44,7 @@ static int g_opt_dense_min = 2;         // ... only when a block has at least th
                                         // across layers and the counters only cost (cfg1 / one Europe raster / cfg3: 7-10 % slower, r02 A/B)
 static int g_opt_tap_pack = 1;          // conv_last's tap sum fused with the SRCNN input im2col (tap_pack_kernel)
 static int g_opt_hyb = 1;               // hybrid tap fold (conv_tc.cu HYB_T) on the early-release layers (HRconv 338 -> 294 us)
-static int g_opt_merge_phases = 1;      // sub-pixel phase pairs of nearest-x2 + conv as one launch (gridDim.y)
+static int g_opt_merge_phases = 1;      // sub-pixel phase pairs of nearest-x2 + conv as one launch (gridDim.y, emit_conv)
 static int g_opt_fuse_tail = 3;         // inference, second MMA over the staged tile: bit 0 srcnn.conv2 inside srcnn.conv1's epilogue, bit 1 conv_last's
                                         // nine tap planes inside HRconv's epilogue (+ tap_sum_kernel)
 static int g_opt_dense = 1;             // conv1..conv4 of every gc = 16 dense block as ONE persistent launch with tile-level dependencies (rdb_tc.cu)
@@ -307,13 +308,14 @@ struct ConvIO {
   const void* in = nullptr; int in_C = 0, cin_off = 0;
   void* out = nullptr; int out_C = 0, out_coff = 0; int out_kind = kOutBf16;
   int split_off = 0;       // kOutBf16Split: channel distance from a hi value to its lo
-  int act = CSR_ACT_NONE;
+  int act = CSR_ACT_NONE; float act_slope = 0.f;   // act_slope: CSR_ACT_LRELU's negative slope
   const void* r1 = nullptr; int r1_C = 0, r1_coff = 0; float s1 = 1.f;
   const void* r2 = nullptr; int r2_C = 0, r2_coff = 0; float s2 = 1.f;
   const void* gate = nullptr; int gate_C = 0, gate_coff = 0, gate_from = 0; float gate_neg = 0.2f;
 };
 
-// H, W: spatial size of the launch's input (for an up2 layer: the low-resolution input; its output is 2H x 2W).
+// H, W: spatial size of the launch's input (for an up2 layer: the low-resolution input; its output is 2H x 2W).  cl->tmap is left to
+// the caller: emit_conv encodes the input map of the launches it keeps, bwd_build a sub-pixel phase view.
 static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int W, const ConvIO& io, ConvLaunch* cl) {
   if (io.in_C % 8 != 0 || io.cin_off % 8 != 0) return fail(CSR_ERR_BAD_ARG, "input buffer channels (%d) / offset (%d) must be multiples of 8", io.in_C, io.cin_off);
   const bool split = io.out_kind == kOutBf16Split;
@@ -383,6 +385,7 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
     }
   }
   p.act = io.act;
+  p.act_slope = io.act_slope;
   p.n_stage = p.n_groups;
   // Early-release epilogue (conv_tc.cu, EARLY_T): wide residual-free layers that run with one 16-warp group.  Two staging
   // buffers; KW <= 2 layers also get four accumulator buffers (4 x KW x 64 <= 512 TMEM columns).
@@ -451,7 +454,7 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
   p.out_H = up * H; p.out_W = up * W;
   cl->w_off = pp.w_off; cl->b_off = pp.b_off;
   if (conv_smem_bytes(p) > (size_t)kSmemLimit) return fail(CSR_ERR_UNSUPPORTED, "conv needs %zu bytes of shared memory", conv_smem_bytes(p));
-  return encode_act_map(&cl->tmap, io.in, N, H, W, io.in_C, p.SW, p.win_rows, p.box_c);
+  return CSR_OK;
 }
 
 // ------------------------------------------------------------------------------------------- weight gradient
@@ -552,56 +555,20 @@ static size_t wgrad_jobs_scratch_floats(const LayerSpec& L) {
   const long jobs = (long)ceil_div(L.cin, 128) * ceil_div(L.cout, n_cols) * ceil_div(L.kh, per);
   return (size_t)jobs * per * L.kw * 128 * n_cols;
 }
-static int run_wgrad_layer_jobs(const LayerSpec& L, int N, int H, int W, const void* x, int x_C, int x_coff, const void* g, int g_C, int g_coff,
-                                float scale, float* dw, float* db, float* scratch, int sms, cudaStream_t s) {
-  const int n_cols = L.cout >= 128 ? 128 : (L.cout + 15) / 16 * 16;
-  if (L.cout > 128 && L.cout % 128) return fail(CSR_ERR_UNSUPPORTED, "wgrad: cout %d > 128 must be a multiple of 128", L.cout);
-  const int per = wgrad_taps_per_launch(L.kw, n_cols);
-  WgradLaunch wl;
-  int rc = build_wgrad(sms, N, H, W, L.kw, L.kw / 2, -(L.kh / 2), std::min(per, L.kh), x, x_C, x_coff, g, g_C, g_coff, n_cols > 64 ? g : nullptr,
-                       n_cols > 64 ? g_C : 0, n_cols > 64 ? g_coff + 64 : 0, n_cols, scratch, 0, n_cols, &wl);
-  if (rc) return rc;
-  WgradParams& p = wl.p;
-  p.jobs_ci = ceil_div(L.cin, 128); p.jobs_co = ceil_div(L.cout, n_cols); p.jobs_dy = ceil_div(L.kh, per);
-  p.KH = L.kh; p.PH = L.kh / 2; p.per_dy = per; p.x_coff = x_coff; p.g_coff = g_coff;
-  p.job_stride = (long)per * L.kw * 128 * n_cols;
-  p.ld_n = n_cols;
-  p.atomic = 1;
-  const int jobs = p.jobs_ci * p.jobs_co * p.jobs_dy;
-  p.splits = std::max(1, std::min(p.num_tiles, sms / jobs));
-  CSR_CUDA(cudaMemsetAsync(scratch, 0, (size_t)jobs * p.job_stride * sizeof(float), s));
-  int e = launch_wgrad_tc(p, wl.tx0, wl.tx1, wl.tg0, wl.tg1, sms, s);
-  if (e) return fail(CSR_ERR_CUDA, "wgrad (job mode) launch failed: %s", cudaGetErrorString((cudaError_t)e));
-  CSR_CUDA(launch_wgrad_scatter_jobs(scratch, dw, L.cout, L.cin, L.kh, L.kw, n_cols, p.jobs_co, p.jobs_dy, per, p.job_stride, scale, s));
-  g_launches += 3;
-  if (db) {
-    const long npix = (long)N * H * W;
-    if (L.cout > 128 && L.cout % 128 == 0) {
-      CSR_CUDA(launch_bias_grad_wide(g, npix, g_C, g_coff, L.cout / 128, scale, db, s));
-      ++g_launches;
-    } else {
-      for (int co = 0; co < L.cout; co += 128) {
-        float* dbs[1] = {db + co};
-        CSR_CUDA(launch_bias_grad(g, npix, g_C, g_coff + co, std::min(128, L.cout - co), scale, dbs, 1, s));
-        ++g_launches;
-      }
-    }
-  }
-  return CSR_OK;
-}
-
 // ------------------------------------------------------------------------------------------- launch lists
 // One launch of a launch list: a plan's forward or backward (CsrPlan::fwd / bwd) or one layer's weight gradient.  Operands that
 // change from call to call are null here and supplied by run_ops from its Bindings; every other pointer is fixed when the op is built.
 struct Op {
-  enum Kind { kNchw, kConv, kDense, kTapSum, kTapPack, kPackSrcnn, kGcol, kScale, kWgrad, kReduce, kScatter, kBias, kBiasPlanar, kMemset } kind;
+  enum Kind { kNchw, kConv, kDense, kTapSum, kTapPack, kPackSrcnn, kGcol, kScale, kWgrad, kReduce, kScatter, kScatterJobs, kBias, kBiasWide,
+              kBiasPlanar, kMemset } kind;
   ConvLaunch conv;               // kConv; p.out == nullptr: the caller's `out`
   DenseLaunch dense;             // kDense: conv1..conv4 of a dense block, or (backward) its four gated input-gradient convs (rdb_tc.cu)
   WgradLaunch wg;                // kWgrad
   // kScatter / kBias*: which layer's gradient (index into Bindings::dw / db), and how
   int layer = -1, fold = 0, phase = -1, ci0 = 0, ci_n = 0, col0 = 0, ld_n = 0, n_parts = 0, nseg = 1;
   int taps_t = 0;                         // kScatter: columns are taps of a single-output-channel layer (dw[ci][tap])
-  int cout = 0, cin = 0, kh = 0, kw = 0;  // kScatter: the forward layer's shape; kGcol: taps
+  int cout = 0, cin = 0, kh = 0, kw = 0;  // kScatter / kScatterJobs: the forward layer's shape; kGcol: taps
+  int jobs_co = 0, jobs_dy = 0, per_dy = 0;   // kScatterJobs: the job grid of the kWgrad op before it (WgradParams), job stride in `count`
   int seg_layers[4] = {-1, -1, -1, -1};   // kBias with nseg > 1: one layer per channel segment
   int N = 0, H = 0, W = 0;                // kNchw: the input grid (C channels); kTapSum / kTapPack / kPackSrcnn / kGcol: the HR grid
   float scale = 1.f;
@@ -681,6 +648,11 @@ static int run_ops(const std::vector<Op>& ops, size_t lo, size_t hi, const Bindi
         CSR_CUDA(launch_wgrad_scatter(reinterpret_cast<const float*>(op.src), op.ld_n, b.dw[op.layer], op.cout, op.cin, op.kh, op.kw, op.fold, op.phase,
                                       op.ci0, op.ci_n, op.col0, op.scale, op.taps_t, s));
         break;
+      case Op::kScatterJobs:
+        if (!b.dw[op.layer]) return fail(CSR_ERR_BAD_ARG, "null weight-gradient pointer for layer %d", op.layer);
+        CSR_CUDA(launch_wgrad_scatter_jobs(reinterpret_cast<const float*>(op.src), b.dw[op.layer], op.cout, op.cin, op.kh, op.kw, op.ld_n, op.jobs_co,
+                                           op.jobs_dy, op.per_dy, op.count, op.scale, s));
+        break;
       case Op::kBias: {
         float* dbs[4] = {nullptr, nullptr, nullptr, nullptr};
         for (int q = 0; q < op.nseg; ++q) {
@@ -690,6 +662,10 @@ static int run_ops(const std::vector<Op>& ops, size_t lo, size_t hi, const Bindi
         CSR_CUDA(launch_bias_grad(op.src, op.count, op.C, op.coff, op.cout, op.scale, dbs, op.nseg, s));
         break;
       }
+      case Op::kBiasWide:
+        if (!b.db[op.layer]) return fail(CSR_ERR_BAD_ARG, "null bias-gradient pointer for layer %d", op.layer);
+        CSR_CUDA(launch_bias_grad_wide(op.src, op.count, op.C, op.coff, op.cout / 128, op.scale, b.db[op.layer], s));
+        break;
       case Op::kBiasPlanar:
         CSR_CUDA(launch_bias_grad_planar(op.src ? reinterpret_cast<const float*>(op.src) : b.grad_out, op.count, op.scale, b.db[op.layer], s));
         break;
@@ -706,6 +682,71 @@ static Op memset_op(void* dst, size_t bytes) {
   Op op;
   op.kind = Op::kMemset; op.dst = dst; op.count = (long)bytes;
   return op;
+}
+
+// A pack part without the inputs that only set its per-part launch fields: w_off / b_off (weights, bias), co_lo (out_coff), ph (PH) and
+// the row bit a of a sub-pixel phase 2a + b (out_oy).  build_conv is a function of the part, so two parts of the same shape build the
+// same launch up to those fields.
+static PackPart part_shape(PackPart pp) {
+  pp.w_off = pp.b_off = 0;
+  pp.co_lo = pp.ph = 0;
+  if (pp.phase >= 0) pp.phase &= 1;
+  return pp;
+}
+static_assert(std::has_unique_object_representations_v<PackPart>, "part shapes are compared with memcmp: PackPart must have no padding");
+
+// The conv launches of one layer (all its pack parts), appended to `ops`.  Parts of the same shape go out as ONE launch with the parts
+// on gridDim.y (ConvParams::parts) when their per-part fields step by constant strides: the output-channel parts of a wide layer (a
+// 512-channel layer over an 8 x 8 map is 8 parts of ~16 tiles: one after the other they would leave nine SMs in ten idle) and, with
+// option 34, the two sub-pixel phases of nearest-x2 + conv that share a kernel specialisation (PW = 1 - b; phases a = 0, 1 on
+// gridDim.y).  Residual / gate operands are not offset per part, and fp32 outputs keep one launch per part: only residual-free bf16
+// layers are merged.  Only the launches that go out are built (csr_conv2d_nhwc is called ~100 times per discriminator step).
+static int emit_conv(std::vector<Op>& ops, const PackLayer& pl, int N, int H, int W, const ConvIO& io) {
+  const std::vector<PackPart>& parts = pl.parts;
+  const bool mergeable = parts.size() > 1 && !io.r1 && !io.r2 && !io.gate && (io.out_kind == kOutBf16 || io.out_kind == kOutBf16Split);
+  thread_local std::vector<char> merged;                   // thread_local: no allocation per call
+  thread_local std::vector<PackPart> shape;
+  merged.assign(mergeable ? parts.size() : 0, 0);
+  shape.clear();
+  if (mergeable)
+    for (const PackPart& q : parts) shape.push_back(part_shape(q));
+  auto row = [](const PackPart& q) { return q.phase >= 0 ? q.phase >> 1 : 0; };
+  auto steps = [&](const PackPart& a, const PackPart& b, long long d[5]) {
+    d[0] = (long long)b.w_off - (long long)a.w_off; d[1] = (long long)b.b_off - (long long)a.b_off;
+    d[2] = b.co_lo - a.co_lo; d[3] = b.ph - a.ph; d[4] = row(b) - row(a);
+  };
+  for (size_t i = 0; i < parts.size(); ++i) {
+    if (mergeable && merged[i]) continue;
+    Op op;
+    op.kind = Op::kConv;
+    int rc = build_conv(pl, parts[i], N, H, W, io, &op.conv);
+    if (rc) return rc;
+    if (mergeable) {
+      auto same = [&](size_t j) { return !merged[j] && !memcmp(&shape[i], &shape[j], sizeof(PackPart)); };
+      long long d0[5], d[5];
+      size_t prev = i, count = 1;
+      bool steady = true;
+      for (size_t j = i + 1; j < parts.size(); ++j) {
+        if (!same(j)) continue;
+        steps(parts[prev], parts[j], count == 1 ? d0 : d);
+        if (count > 1) steady = steady && !memcmp(d, d0, sizeof(d));
+        prev = j;
+        ++count;
+      }
+      if (count > 1 && steady && (g_opt_merge_phases || (!d0[3] && !d0[4]))) {
+        for (size_t j = i + 1; j < parts.size(); ++j)
+          if (same(j)) merged[j] = 1;
+        ConvParams& p = op.conv.p;
+        p.parts = (int)count;
+        p.part_w_bytes = (int)d0[0]; p.part_b_floats = (int)(d0[1] / (long long)sizeof(float));
+        p.part_c = (int)d0[2]; p.part_ph = (int)d0[3]; p.part_oy = (int)d0[4];
+      }
+    }
+    rc = encode_act_map(&op.conv.tmap, io.in, N, H, W, io.in_C, op.conv.p.SW, op.conv.p.win_rows, op.conv.p.box_c);
+    if (rc) return rc;
+    ops.push_back(op);
+  }
+  return CSR_OK;
 }
 
 // One weight-gradient accumulation group: the GEMM launches `wg` sum into dacc[0, floats).  Option 25 on: dacc is zeroed and the
@@ -760,6 +801,38 @@ static int emit_wgrad(std::vector<Op>& ops, const LayerSpec& L, int layer, int N
   }
   if (bias) {
     Op bo; bo.kind = Op::kBias; bo.layer = layer; bo.src = g; bo.count = (long)N * H * W * (L.up2 ? 4 : 1); bo.C = g_C; bo.coff = g_coff;
+    bo.cout = L.cout; bo.scale = scale;
+    ops.push_back(bo);
+  }
+  return CSR_OK;
+}
+
+// Job mode (wgrad_jobs_applicable): one GEMM launch for the whole layer, its per-job sums scattered into Bindings::dw [layer].
+static int emit_wgrad_jobs(std::vector<Op>& ops, const LayerSpec& L, int layer, int N, int H, int W, const void* x, int x_C, int x_coff, const void* g,
+                           int g_C, int g_coff, float scale, bool bias, float* scratch, int sms) {
+  const int n_cols = L.cout >= 128 ? 128 : (L.cout + 15) / 16 * 16;
+  if (L.cout > 128 && L.cout % 128) return fail(CSR_ERR_UNSUPPORTED, "wgrad: cout %d > 128 must be a multiple of 128", L.cout);
+  const int per = wgrad_taps_per_launch(L.kw, n_cols);
+  Op op; op.kind = Op::kWgrad;
+  int rc = build_wgrad(sms, N, H, W, L.kw, L.kw / 2, -(L.kh / 2), std::min(per, L.kh), x, x_C, x_coff, g, g_C, g_coff, n_cols > 64 ? g : nullptr,
+                       n_cols > 64 ? g_C : 0, n_cols > 64 ? g_coff + 64 : 0, n_cols, scratch, 0, n_cols, &op.wg);
+  if (rc) return rc;
+  WgradParams& p = op.wg.p;
+  p.jobs_ci = ceil_div(L.cin, 128); p.jobs_co = ceil_div(L.cout, n_cols); p.jobs_dy = ceil_div(L.kh, per);
+  p.KH = L.kh; p.PH = L.kh / 2; p.per_dy = per; p.x_coff = x_coff; p.g_coff = g_coff;
+  p.job_stride = (long)per * L.kw * 128 * n_cols;
+  p.ld_n = n_cols;
+  p.atomic = 1;
+  const int jobs = p.jobs_ci * p.jobs_co * p.jobs_dy;
+  p.splits = std::max(1, std::min(p.num_tiles, sms / jobs));
+  ops.push_back(memset_op(scratch, (size_t)jobs * p.job_stride * sizeof(float)));
+  ops.push_back(op);
+  Op sc; sc.kind = Op::kScatterJobs; sc.src = scratch; sc.layer = layer; sc.cout = L.cout; sc.cin = L.cin; sc.kh = L.kh; sc.kw = L.kw; sc.ld_n = n_cols;
+  sc.jobs_co = p.jobs_co; sc.jobs_dy = p.jobs_dy; sc.per_dy = per; sc.count = p.job_stride; sc.scale = scale;
+  ops.push_back(sc);
+  if (bias) {
+    // > 128 output channels (a multiple of 128 here): every 128-channel chunk in one launch
+    Op bo; bo.kind = L.cout > 128 ? Op::kBiasWide : Op::kBias; bo.layer = layer; bo.src = g; bo.count = (long)N * H * W; bo.C = g_C; bo.coff = g_coff;
     bo.cout = L.cout; bo.scale = scale;
     ops.push_back(bo);
   }
@@ -969,41 +1042,9 @@ static int plan_build(CsrPlan* P, const WsPtrs& ws, const std::vector<LayerSpec>
   }
   int li = 0;
   auto add = [&](int H, int W, const ConvIO& io, bool advance = true) -> int {
-    const PackLayer& pl = packs[li];
-    const size_t first = ops.size();
-    for (const PackPart& pp : pl.parts) {
-      Op op; op.kind = Op::kConv;
-      int rc = build_conv(pl, pp, N, H, W, io, &op.conv);
-      if (rc) return rc;
-      ops.push_back(op);
-    }
-    // nearest-x2 + conv = four sub-pixel phases (a, b) in phase order 2a + b: the two phases with the same b share the kernel
-    // specialisation (PW = 1 - b) and go out as ONE launch with a on gridDim.y (weights / bias at a constant stride, PH = 1 - a,
-    // output rows 2y + a): two launches instead of four, each over twice the tiles
-    if (g_opt_merge_phases && pl.parts.size() == 4 && pl.parts[0].phase == 0 && pl.parts[3].phase == 3 && !io.r1 && !io.r2 && !io.gate) {
-      ConvLaunch& a0 = ops[first].conv; ConvLaunch& a1 = ops[first + 1].conv;
-      const ConvLaunch& c2 = ops[first + 2].conv; const ConvLaunch& c3 = ops[first + 3].conv;
-      auto pair_ok = [](const ConvLaunch& u, const ConvLaunch& v) {
-        return u.p.PW == v.p.PW && u.p.KW == v.p.KW && u.p.KH == v.p.KH && u.p.num_tiles == v.p.num_tiles && u.p.SW == v.p.SW && u.p.TH == v.p.TH &&
-               u.p.n_slots == v.p.n_slots && u.p.w_bytes == v.p.w_bytes && u.p.early == v.p.early && u.p.n_acc == v.p.n_acc &&
-               u.p.out_ox == v.p.out_ox && u.p.store_mode == v.p.store_mode && v.w_off > u.w_off && v.b_off > u.b_off;
-      };
-      if (pair_ok(a0, c2) && pair_ok(a1, c3)) {
-        auto merge2 = [](ConvLaunch& u, const ConvLaunch& v) {
-          u.p.parts = 2;
-          u.p.part_w_bytes = (int)(v.w_off - u.w_off);
-          u.p.part_b_floats = (int)((v.b_off - u.b_off) / sizeof(float));
-          u.p.part_c = 0;
-          u.p.part_ph = v.p.PH - u.p.PH;
-          u.p.part_oy = v.p.out_oy - u.p.out_oy;
-        };
-        merge2(a0, c2);
-        merge2(a1, c3);
-        ops.resize(first + 2);
-      }
-    }
+    const int rc = emit_conv(ops, packs[li], N, H, W, io);
     if (advance) ++li;
-    return CSR_OK;
+    return rc;
   };
   int rc;
   // conv_first (esrgan.py:90) has two consumers: the first RRDB (reads x from its concat buffer) and the trunk skip-add
@@ -1012,7 +1053,7 @@ static int plan_build(CsrPlan* P, const WsPtrs& ws, const std::vector<LayerSpec>
   rc = add(h, w, io_of(ws.xin, 64, cat(0), C, 0, CSR_ACT_NONE), false);
   if (rc) return rc;
   ConvParams& f = ops[c0].conv.p;
-  if (g_opt_merge_phases && ops.size() == c0 + 1 && f.early && f.store_mode == kStoreStaged && f.KW == 3 && f.act == 0 && !f.r1) {
+  if (ops.size() == c0 + 1 && f.early && f.store_mode == kStoreStaged && f.KW == 3 && f.act == 0 && !f.r1) {
     // ... with the early-release epilogue the staged tile is simply stored twice (conv_tc.cu, out_dup)
     f.out_dup = ws.fea0; f.dup_C = 64; f.dup_coff = 0;
     ++li;
@@ -1208,28 +1249,23 @@ static int bwd_build(CsrPlan* P, const WsPtrs& ws, const std::vector<LayerSpec>&
   // the parts of backward layer bi
   auto dgrad = [&](int Hh, int Ww, const ConvIO& io, const void* phase_src = nullptr) -> int {
     const PackLayer& pl = packs[bi];
-    const bool up2 = B[bi].up2 != 0;
+    if (!B[bi++].up2) return emit_conv(ops, pl, N, Hh, Ww, io);
     for (const PackPart& pp : pl.parts) {
       Op op;
       op.kind = Op::kConv;
+      // phases accumulate into the same low-resolution gradient: first writes, later ones add, the last one gates
       ConvIO io2 = io;
-      if (up2) {
-        // phases accumulate into the same low-resolution gradient: first writes, later ones add, the last one gates
-        if (pp.phase > 0) { io2.r1 = io.out; io2.r1_C = io.out_C; io2.r1_coff = io.out_coff; io2.s1 = 1.f; }
-        if (pp.phase < 3) io2.gate = nullptr;
-      }
+      if (pp.phase > 0) { io2.r1 = io.out; io2.r1_C = io.out_C; io2.r1_coff = io.out_coff; io2.s1 = 1.f; }
+      if (pp.phase < 3) io2.gate = nullptr;
       // build as a plain (non-up2) conv on the low-resolution grid: output view is dense, INPUT view is the strided phase
       PackPart q = pp;
-      if (up2) q.phase = -1;
+      q.phase = -1;
       int rc = build_conv(pl, q, N, Hh, Ww, io2, &op.conv);
       if (rc) return rc;
-      if (up2) {
-        rc = encode_phase_map(&op.conv.tmap, phase_src, N, Hh, Ww, io.in_C, pp.phase, op.conv.p.SW, op.conv.p.win_rows);
-        if (rc) return rc;
-      }
+      rc = encode_phase_map(&op.conv.tmap, phase_src, N, Hh, Ww, io.in_C, pp.phase, op.conv.p.SW, op.conv.p.win_rows);
+      if (rc) return rc;
       ops.push_back(op);
     }
-    ++bi;
     return CSR_OK;
   };
   auto wgrad_plain = [&](int layer, int Hh, int Ww, const void* x, int x_C, int x_coff, const void* g, int g_C, int g_coff, float scale) -> int {
@@ -1427,7 +1463,7 @@ int csr_set_option(int32_t key, int32_t value) {
     case 35:                                                       // plans created afterwards
       if (value != 0 && value != 1) return fail(CSR_ERR_BAD_ARG, "option 35: 0 or 1");
       g_opt_hyb = value; return CSR_OK;
-    case 34: g_opt_merge_phases = value ? 1 : 0; return CSR_OK;    // plans created afterwards
+    case 34: g_opt_merge_phases = value ? 1 : 0; return CSR_OK;    // plans created afterwards, single convs called afterwards
     case 33: g_opt_fuse_tail = value & 3; return CSR_OK;       // plans created afterwards
     case 31: if (value < 0 || value > 64) return fail(CSR_ERR_BAD_ARG, "option 31: windows per SM in [0, 64]"); g_opt_dense_min = value; return CSR_OK;
     case 30: g_opt_reserve_sms = value < 0 ? 0 : value; return CSR_OK;
@@ -1951,7 +1987,6 @@ int csr_conv2d_nhwc(const CsrConvDesc* d, const void* in, const float* weight, c
   const auto packs = pack_layout({L}, &total, true);
   if (scratch_bytes < total) return fail(CSR_ERR_WORKSPACE, "scratch %zu < %zu bytes", scratch_bytes, total);
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  uint8_t* base = reinterpret_cast<uint8_t*>(scratch);
   ConvIO io;
   io.in = in; io.in_C = d->in_c; io.cin_off = d->in_coff;
   io.out = out; io.out_C = d->out_c; io.out_coff = d->out_coff;
@@ -1959,7 +1994,7 @@ int csr_conv2d_nhwc(const CsrConvDesc* d, const void* in, const float* weight, c
                 d->out_mode == CSR_OUT_BF16_SPLIT ? kOutBf16Split : kOutF32Nhwc;
   io.split_off = d->cout;
   if (d->out_mode == CSR_OUT_BF16_SPLIT && (res1 || res2 || gate)) return fail(CSR_ERR_UNSUPPORTED, "hi/lo bf16 output takes no residual / gate operand");
-  io.act = d->act;
+  io.act = d->act; io.act_slope = d->act_slope;
   io.r1 = res1; io.r1_C = d->res1_c; io.r1_coff = d->res1_coff; io.s1 = d->scale1;
   io.r2 = res2; io.r2_C = d->res2_c; io.r2_coff = d->res2_coff; io.s2 = d->scale2;
   io.gate = gate; io.gate_C = d->gate_c; io.gate_coff = d->gate_coff; io.gate_from = d->gate_from; io.gate_neg = d->gate_neg;
@@ -1970,34 +2005,14 @@ int csr_conv2d_nhwc(const CsrConvDesc* d, const void* in, const float* weight, c
     rc = conv2d_pack_parts(L, packs[0], weight, bias, scratch, s);
     if (rc) return rc;
   }
-  // Equal output-channel parts of a residual-free layer go out as ONE launch (gridDim.y = parts): a 512-channel layer over an
-  // 8 x 8 map is 8 parts of ~16 tiles each - one after the other they would leave nine SMs in ten idle.
-  const std::vector<PackPart>& parts = packs[0].parts;
-  bool merge = parts.size() > 1 && !res1 && !res2 && !gate && (d->out_mode == CSR_OUT_BF16_NHWC || d->out_mode == CSR_OUT_BF16_SPLIT);
-  for (size_t i = 1; merge && i < parts.size(); ++i)
-    merge = parts[i].phase < 0 && parts[i].npad == parts[0].npad && parts[i].n_store == parts[0].npad && parts[0].n_store == parts[0].npad &&
-            parts[i].w_bytes == parts[0].w_bytes && parts[i].w_off - parts[i - 1].w_off == parts[1].w_off - parts[0].w_off &&
-            parts[i].b_off - parts[i - 1].b_off == parts[1].b_off - parts[0].b_off && parts[i].co_lo - parts[i - 1].co_lo == parts[0].npad;
-  for (size_t i = 0; i < parts.size(); ++i) {
-    const PackPart& pp = parts[i];
-    ConvLaunch cl;
-    rc = build_conv(packs[0], pp, d->n, d->h, d->w, io, &cl);
-    if (rc) return rc;
-    cl.p.act_slope = d->act_slope;
-    cl.p.wpk = base + pp.w_off;
-    cl.p.bias = reinterpret_cast<const float*>(base + pp.b_off);
-    if (merge) {
-      cl.p.parts = (int)parts.size();
-      cl.p.part_w_bytes = (int)(parts[1].w_off - parts[0].w_off);
-      cl.p.part_b_floats = (int)((parts[1].b_off - parts[0].b_off) / sizeof(float));
-      cl.p.part_c = parts[0].npad;
-    }
-    int e = launch_conv_tc(cl.p, cl.tmap, di.sms, s);
-    if (e) return fail(CSR_ERR_CUDA, "conv launch failed: %s", cudaGetErrorString((cudaError_t)e));
-    ++g_launches;
-    if (merge) break;
-  }
-  return CSR_OK;
+  // RCAN training is bound by host time per call (~4 us): reuse the list's storage instead of allocating it every call
+  thread_local std::vector<Op> ops;
+  ops.clear();
+  rc = emit_conv(ops, packs[0], d->n, d->h, d->w, io);
+  if (rc) return rc;
+  Bindings b;
+  b.packed = scratch;
+  return run_ops(ops, 0, ops.size(), b, di.sms, s);
 }
 
 // ---- single-layer weight gradient (building block; used by the parity tests) ---------------------------
@@ -2022,26 +2037,30 @@ int csr_conv2d_wgrad(const CsrWgradDesc* d, const void* x, const void* g, float*
   if (rc) return rc;
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   float* dacc = reinterpret_cast<float*>(scratch);
-  if (wgrad_jobs_applicable(L, d->n, d->h, d->w, di.sms))
-    return run_wgrad_layer_jobs(L, d->n, d->h, d->w, x, d->x_c, d->x_coff, g, d->g_c, d->g_coff, d->scale, dw, db, dacc, di.sms, s);
-  // Output channels in chunks whose KW x chunk accumulator columns fit the 512 TMEM columns (one chunk for every layer up to 5x5 / 64
-  // channels; the 9x9 srcnn.conv1 with 64 output channels takes two).
-  const int ekw = L.up2 ? 2 : L.kw;
-  const int chunk = std::max(16, std::min((L.cout + 15) / 16 * 16, 512 / ekw / 16 * 16));
-  for (int co0 = 0; co0 < L.cout; co0 += chunk) {
-    LayerSpec Lc = L;
-    Lc.cout = std::min(chunk, L.cout - co0);
-    std::vector<Op> ops;
-    rc = emit_wgrad(ops, Lc, 0, d->n, d->h, d->w, x, d->x_c, d->x_coff, g, d->g_c, d->g_coff + co0, d->scale, db != nullptr, dacc, di.sms);
+  std::vector<Op> ops;
+  std::vector<float*> dws, dbs;                            // op layer k: output-channel chunk k
+  if (wgrad_jobs_applicable(L, d->n, d->h, d->w, di.sms)) {
+    rc = emit_wgrad_jobs(ops, L, 0, d->n, d->h, d->w, x, d->x_c, d->x_coff, g, d->g_c, d->g_coff, d->scale, db != nullptr, dacc, di.sms);
     if (rc) return rc;
-    float* dwc = dw + (size_t)co0 * L.cin * L.kh * L.kw;
-    float* dbc = db ? db + co0 : nullptr;
-    Bindings b;
-    b.dw = &dwc; b.db = &dbc;
-    rc = run_ops(ops, 0, ops.size(), b, di.sms, s);
-    if (rc) return rc;
+    dws.push_back(dw); dbs.push_back(db);
+  } else {
+    // Output channels in chunks whose KW x chunk accumulator columns fit the 512 TMEM columns (one chunk for every layer up to 5x5 / 64
+    // channels; the 9x9 srcnn.conv1 with 64 output channels takes two).
+    const int ekw = L.up2 ? 2 : L.kw;
+    const int chunk = std::max(16, std::min((L.cout + 15) / 16 * 16, 512 / ekw / 16 * 16));
+    for (int co0 = 0; co0 < L.cout; co0 += chunk) {
+      LayerSpec Lc = L;
+      Lc.cout = std::min(chunk, L.cout - co0);
+      rc = emit_wgrad(ops, Lc, (int)dws.size(), d->n, d->h, d->w, x, d->x_c, d->x_coff, g, d->g_c, d->g_coff + co0, d->scale, db != nullptr, dacc,
+                      di.sms);
+      if (rc) return rc;
+      dws.push_back(dw + (size_t)co0 * L.cin * L.kh * L.kw);
+      dbs.push_back(db ? db + co0 : nullptr);
+    }
   }
-  return CSR_OK;
+  Bindings b;
+  b.dw = dws.data(); b.db = dbs.data();
+  return run_ops(ops, 0, ops.size(), b, di.sms, s);
 }
 
 // ---- layout helpers -----------------------------------------------------------------------------------

@@ -92,12 +92,6 @@ __device__ __forceinline__ void pack_weight_body(const float* __restrict__ w, __
   }
 }
 
-__global__ void pack_weight_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ dst, int cout, int cin, int kh,
-                                   int kw, int fold, int phase, int transposed, float wscale, int co_lo, int npad, int cin_pad) {
-  pack_weight_body(w, dst, cout, cin, kh, kw, fold, phase, transposed, wscale, co_lo, npad, cin_pad, 0, 0, 0, 0,
-                   blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x, static_cast<long>(gridDim.x) * blockDim.x);
-}
-
 // All layers of the generator in ONE launch (training repacks every optimizer step: ~360 layer parts): blockIdx.y = job.
 __global__ void pack_jobs_kernel(const PackJob* __restrict__ jobs) {
   const PackJob j = jobs[blockIdx.y];
@@ -112,11 +106,6 @@ __global__ void pack_jobs_kernel(const PackJob* __restrict__ jobs) {
       j.bdst[threadIdx.x] = (j.b && co < j.cout) ? j.b[co] : 0.f;
     }
   }
-}
-
-__global__ void pack_bias_kernel(const float* __restrict__ b, float* __restrict__ dst, int cout, int co_lo, int npad) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < npad) dst[i] = (co_lo + i < cout) ? b[co_lo + i] : 0.f;
 }
 
 // ---- activations -----------------------------------------------------------------------------------------
@@ -453,18 +442,6 @@ static inline int grid_for(long total, int block, int cap = 148 * 16) {
   return static_cast<int>(g);
 }
 
-cudaError_t launch_pack_weight(const float* w, void* dst, int cout, int cin, int kh, int kw, int fold, int phase, int transposed,
-                               float wscale, int co_lo, int npad, int cin_pad, cudaStream_t s) {
-  const int ekh = phase >= 0 ? 2 : kh, ekw = phase >= 0 ? 2 : (fold ? 1 : kw);
-  const long total = static_cast<long>(ekh) * ekw * (cin_pad >> 4) * npad * 16;
-  pack_weight_kernel<<<grid_for(total, 256), 256, 0, s>>>(w, reinterpret_cast<__nv_bfloat16*>(dst), cout, cin, kh, kw, fold, phase,
-                                                          transposed, wscale, co_lo, npad, cin_pad);
-  return cudaGetLastError();
-}
-cudaError_t launch_pack_bias(const float* b, float* dst, int cout, int co_lo, int npad, cudaStream_t s) {
-  pack_bias_kernel<<<(npad + 127) / 128, 128, 0, s>>>(b, dst, cout, co_lo, npad);
-  return cudaGetLastError();
-}
 cudaError_t launch_nchw_to_nhwc(const float* src, void* dst, int n, int c, int h, int w, int dst_c, int zero_to, cudaStream_t s) {
   const long per = static_cast<long>(h) * w, total = per * n;
   nchw_to_nhwc_kernel<<<grid_for(total, 256), 256, 0, s>>>(src, reinterpret_cast<__nv_bfloat16*>(dst), per, total, c, dst_c, zero_to);

@@ -2,7 +2,7 @@
 #include <cuda_runtime.h>
 
 namespace csr {
-// one layer part of a batched weight pack (see pack_weight_kernel for the field meanings)
+// one layer part of a batched weight pack (see pack_weight_body for the field meanings)
 struct PackJob {
   const float* w; const float* b; void* dst; float* bdst;
   int cout, cin, kh, kw, fold, phase, transposed; float wscale; int co_lo, npad, cin_pad;
@@ -13,9 +13,6 @@ struct PackJob {
   int ci_lo, ci_n, src_ci_off, src_cin;
 };
 cudaError_t launch_pack_jobs(const PackJob* jobs_dev, int njobs, cudaStream_t s);
-cudaError_t launch_pack_weight(const float* w, void* dst, int cout, int cin, int kh, int kw, int fold, int phase, int transposed,
-                               float wscale, int co_lo, int npad, int cin_pad, cudaStream_t s);
-cudaError_t launch_pack_bias(const float* b, float* dst, int cout, int co_lo, int npad, cudaStream_t s);
 cudaError_t launch_nchw_to_nhwc(const float* src, void* dst, int n, int c, int h, int w, int dst_c, int zero_to, cudaStream_t s);
 // hi/lo bf16 activations of the perceptual loss (CSR_OUT_BF16_SPLIT): input conversion and 2x2 max pool
 cudaError_t launch_nchw_to_nhwc_split(const float* src, void* dst, int n, int c, int h, int w, int dst_c, cudaStream_t s);
