@@ -49,6 +49,7 @@ static int g_opt_fuse_tail = 3;         // inference, second MMA over the staged
                                         // nine tap planes inside HRconv's epilogue (+ tap_sum_kernel)
 static int g_opt_dense = 1;             // conv1..conv4 of every gc = 16 dense block as ONE persistent launch with tile-level dependencies (rdb_tc.cu)
 static int g_opt_early = 1;             // early-release epilogue (conv_tc.cu, EARLY_T) for the wide residual-free layers
+static int g_opt_whole_row = 1;         // whole-row tiles (SW = W) for the trunk's 3x3 convs over 32- / 64-pixel-wide maps (choose_tiling)
 
 static int fail(int code, const char* fmt, ...) {
   va_list ap;
@@ -257,32 +258,46 @@ static std::vector<PackLayer> pack_layout(const std::vector<LayerSpec>& layers, 
 struct Tiling {
   int SW, TH, TW, win_rows, win_bytes, slot_bytes, n_slots, stage_bytes;
   double eff;   // useful fraction of the MMA rows (with the small penalties applied by choose_tiling)
+  int whole_row;   // SW == TW == W: no halo columns (ConvParams / DenseParams::whole_row)
+  int n_stage;     // staging buffers the shape was sized with (whole rows may take fewer than asked for, see choose_tiling)
 };
 constexpr int kMaxSlots = 8;   // deepest window ring of a conv or dense-block launch
+// whole_row (option 37): 1 = also consider whole-row tiles of a 3x3 conv over a 32- or 64-pixel-wide map (SW = TW = W, TH = 128 / W,
+// no halo columns: 20 % fewer M tiles than SW = 16 at W = 64, 33 % fewer than SW = 16 at W = 32); 2 = the same, and if n_stage = 2
+// staging buffers leave room for one window slot only, size it with ONE staging buffer the two epilogue groups share in tile order
+// (RDB conv5: 144 KB of weights + 2 x 32 KB slots + 2 x 16 KB staging buffers do not fit 227 KB).
 static int choose_tiling(int H, int W, int KH, int KW, int w_bytes, int n_kblocks, int stage_row_bytes, int n_stage, Tiling* out,
-                         int row_bytes = 128, int tall = 1, int extra_slot_bytes = 0) {
+                         int row_bytes = 128, int tall = 1, int extra_slot_bytes = 0, int whole_row = 0) {
   double best = -1;
-  for (int SW = 16; SW <= 128; SW *= 2) {
-    // The epilogue sums the folded horizontal taps with warp shuffles: a window row must not straddle two warps.
-    if (KW > 1 && SW > 32) continue;
-    const int TW = SW - (KW - 1);
-    if (TW < 1) continue;
+  auto consider = [&](int SW, bool wr, int nst) {
+    const int TW = wr ? SW : SW - (KW - 1);
+    if (TW < 1) return 0;
     const int TH = kTileM / SW;
     const int win_rows = tall * TH + KH - 1;
     const int win_bytes = win_rows * SW * row_bytes;
     const int slot_bytes = (int)align_up(win_bytes, 1024) + (int)align_up(extra_slot_bytes, 1024);   // + a streamed weight k-block
     const int stage_bytes = stage_row_bytes ? (int)align_up((size_t)TH * TW * stage_row_bytes, 1024) : 0;
-    const int fixed = 1024 + (int)align_up(w_bytes, 128) + 256 + 512 + n_stage * stage_bytes;
+    const int fixed = 1024 + (int)align_up(w_bytes, 128) + 256 + 512 + nst * stage_bytes + (wr ? kXchgBytes : 0);
     const int slots = std::min(kMaxSlots, (kSmemLimit - fixed) / slot_bytes);
-    if (slots < 1) continue;
+    if (slots < 1) return 0;
     const double tiles = (double)ceil_div(H, TH * tall) * ceil_div(W, TW) * tall;
     double eff = (double)H * W / (tiles * kTileM);
     if (slots < std::min(2, n_kblocks + 1)) eff *= 0.7;  // no load/MMA overlap
     eff -= 1e-4 * win_bytes / (double)(kTileM * 128);    // tie-break: less halo traffic
     if (eff > best) {
       best = eff;
-      *out = {SW, TH, TW, win_rows, win_bytes, slot_bytes, slots, stage_bytes, eff};
+      *out = {SW, TH, TW, win_rows, win_bytes, slot_bytes, slots, stage_bytes, eff, wr ? 1 : 0, nst};
     }
+    return slots;
+  };
+  for (int SW = 16; SW <= 128; SW *= 2) {
+    // The epilogue sums the folded horizontal taps with warp shuffles: a window row must not straddle two warps (except for
+    // whole-row tiles, which hand the taps at the warp boundary over through shared memory).
+    if (KW > 1 && SW > 32) continue;
+    consider(SW, false, n_stage);
+  }
+  if (whole_row && g_opt_whole_row && KH == 3 && KW == 3 && (W == 32 || W == 64)) {
+    if (consider(W, true, n_stage) < std::min(2, n_kblocks + 1) && whole_row == 2 && n_stage == 2) consider(W, true, 1);
   }
   if (best < 0) return fail(CSR_ERR_UNSUPPORTED, "no tile shape fits shared memory (weights %d bytes, %dx%d kernel)", w_bytes, KH, KW);
   return CSR_OK;
@@ -360,7 +375,14 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
     p.wkb_bytes = pp.kh * 4 * pp.kw * pp.npad * 32;
     rc = choose_tiling(H, W, pp.kh, pp.kw, 0, p.n_kblocks, p.stage_row_bytes, p.n_groups * stage_mult, &tl, 128, 1, p.wkb_bytes);
     if (!rc && tl.n_slots < 2) rc = fail(CSR_ERR_UNSUPPORTED, "streamed-weight conv: window ring too shallow");
-  } else rc = choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, p.n_groups * stage_mult, &tl, p.box_c * 2);
+  } else {
+    // whole-row tiles for the trunk's one-residual convs (RDB conv5, trunk_conv: conv_tc.cu WR_T), which share a staging buffer if need
+    // be.  Not for the RDB3 conv5 with its second residual: with one shared staging buffer its longer epilogue paces the tiles
+    // (50.7 -> 66 us per launch at cfg2 on a B200, while the plain conv5 goes 37 -> 35.5 us)
+    const bool wr = !split && tma_out && pp.phase < 0 && pp.kh == 3 && pp.kw == 3 && pp.ph == 1 && pp.pw == 1 && io.act == CSR_ACT_NONE &&
+                    io.r1 && !io.r2 && !io.gate && p.n_acc == 2 && p.box_c == 64;
+    rc = choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, p.n_groups * stage_mult, &tl, p.box_c * 2, 1, 0, wr ? 2 : 0);
+  }
   if (!rc && g_opt_tall && p.n_acc == 4 && p.n_groups == 4 && !split) {
     Tiling t2;   // taken unless the second M tile would mostly hang below the image
     if (choose_tiling(H, W, pp.kh, pp.kw, p.w_bytes, p.n_kblocks, p.stage_row_bytes, p.n_groups, &t2, p.box_c * 2, 2) == CSR_OK &&
@@ -386,7 +408,7 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
   }
   p.act = io.act;
   p.act_slope = io.act_slope;
-  p.n_stage = p.n_groups;
+  p.n_stage = tl.whole_row ? tl.n_stage : p.n_groups;
   // Early-release epilogue (conv_tc.cu, EARLY_T): wide residual-free layers that run with one 16-warp group.  Two staging
   // buffers; KW <= 2 layers also get four accumulator buffers (4 x KW x 64 <= 512 TMEM columns).
   const bool early_plain = !has_res && p.n_groups == 1 &&
@@ -417,6 +439,7 @@ static int build_conv(const PackLayer& pl, const PackPart& pp, int N, int H, int
     if (4 * (p.KW - 1) * p.npad <= 512) p.n_acc = 4;
   }
   p.SW = tl.SW; p.TH = tl.TH; p.TW = tl.TW;
+  p.whole_row = tl.whole_row;
   p.sw_shift = 0;
   while ((1 << p.sw_shift) < p.SW) ++p.sw_shift;
   p.tiles_x = ceil_div(W, p.TW);
@@ -995,10 +1018,10 @@ static int build_dense(const std::vector<PackLayer>& packs, int li, int N, int H
   }
   p.wbuf_bytes = (int)align_up(wmax, 1024);
   Tiling tl;
-  int rc = choose_tiling(H, W, 3, 3, 2 * p.wbuf_bytes, 2, 32, 4, &tl, 128, 2);
+  int rc = choose_tiling(H, W, 3, 3, 2 * p.wbuf_bytes, 2, 32, 4, &tl, 128, 2, 0, 1);
   if (rc) return rc;
   if (tl.n_slots < 3) return fail(CSR_ERR_UNSUPPORTED, "dense-block kernel: window ring too shallow");
-  p.SW = tl.SW; p.TH = tl.TH; p.TW = tl.TW;
+  p.SW = tl.SW; p.TH = tl.TH; p.TW = tl.TW; p.whole_row = tl.whole_row;
   while ((1 << p.sw_shift) < p.SW) ++p.sw_shift;
   p.tiles_x = ceil_div(W, p.TW); p.tiles_y = ceil_div(H, 2 * p.TH);
   p.tiles_per_img = p.tiles_x * p.tiles_y;
@@ -1467,6 +1490,7 @@ int csr_set_option(int32_t key, int32_t value) {
     case 33: g_opt_fuse_tail = value & 3; return CSR_OK;       // plans created afterwards
     case 31: if (value < 0 || value > 64) return fail(CSR_ERR_BAD_ARG, "option 31: windows per SM in [0, 64]"); g_opt_dense_min = value; return CSR_OK;
     case 30: g_opt_reserve_sms = value < 0 ? 0 : value; return CSR_OK;
+    case 37: g_opt_whole_row = value ? 1 : 0; return CSR_OK;       // plans created afterwards, single convs called afterwards
     case 26:                                                       // early-release epilogue of the wide residual-free layers
       if (value != 0 && value != 1) return fail(CSR_ERR_BAD_ARG, "option 26: 0 or 1");
       g_opt_early = value; return CSR_OK;

@@ -152,17 +152,23 @@ __device__ __forceinline__ uint4 ldg16(const void* base, size_t pix, int C, int 
 //          ~2450 clk per 128 x 64 tile against ~1400 clk of MMAs, because an accumulator stayed busy for the whole
 //          ~1000-clk arithmetic phase and only two of them fit TMEM; tools/tmem_probe.cu shows the TMEM read port itself
 //          delivers a 128 x 192 fp32 tile to 16 warps in ~260 clk.)
-template <int KW_T, int PW_T, int ACT_T, int RES_T, int ST_T, int TALL_T = 0, int EARLY_T = 0, int FUSE_T = 0, int HYB_T = 0>
+//   WR_T 1 = whole-row tiles (ConvParams::whole_row: 3x3 over a 32- or 64-pixel-wide map, RDB conv5 and trunk_conv): the window
+//          starts at x = 0 and every GEMM row is an output pixel (m -> row m >> sw_shift, x = m & (W-1)); the edge taps come from
+//          row_edge_put / row_edge_get (ptx.cuh) instead of halo columns, and with n_stage < n_groups the two epilogue groups share
+//          one staging buffer in tile order (the 144 KB of conv5 weights leave room for two 32 KB window slots only then)
+template <int KW_T, int PW_T, int ACT_T, int RES_T, int ST_T, int TALL_T = 0, int EARLY_T = 0, int FUSE_T = 0, int HYB_T = 0, int WR_T = 0>
 __global__ void __launch_bounds__(kConvThreads, 1)
 conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
   static_assert(!HYB_T || EARLY_T, "hybrid tap fold: early-release epilogue only");
+  static_assert(!WR_T || (KW_T == 3 && PW_T == 1 && ST_T == 1 && !TALL_T && !EARLY_T), "whole-row tiles: staged 3x3 layers");
   extern __shared__ uint8_t smem_raw[];
   // 1024-byte alignment: the 128B-swizzle pattern repeats every 8 rows x 128 B.
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t slots_addr = smem_base;
   const uint32_t stage_addr = slots_addr + static_cast<uint32_t>(p.n_slots) * p.slot_bytes;   // one staging buffer per epilogue group
   const uint32_t w_addr = stage_addr + static_cast<uint32_t>(p.n_stage) * p.stage_bytes;
-  const int w_local = p.stream_w ? 0 : p.w_bytes;       // resident weight bytes
+  const int stream_w = WR_T ? 0 : p.stream_w;          // (whole-row layers keep their weights resident)
+  const int w_local = stream_w ? 0 : p.w_bytes;         // resident weight bytes
   // fused 1x1 successor (FUSE_T): its packed weights and bias sit right behind the layer's own weights
   const uint32_t w2_addr = w_addr + ((w_local + 127) & ~127);
   const uint32_t b2_addr = w2_addr + (FUSE_T ? static_cast<uint32_t>(p.w2_bytes) : 0u);
@@ -180,6 +186,7 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
   auto bar_acc_empty = [&](int b) { return bar_addr + 8u * (9 + 2 * S + b); };
   const uint32_t bar_d2 = bar_addr + 8u * (17 + 2 * S);              // FUSE_T: the second MMA of a tile has completed
   const uint32_t tmem_slot_addr = bar_addr + 8u * (18 + 2 * S);      // [0] TMEM base, [1..2] issuer progress words
+  const uint32_t xchg_addr = (tmem_slot_addr + 12u + 15u) & ~15u;    // WR_T: 96 zero bytes, then the row_edge_put / row_edge_get slots
   uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
   float* bias_s = reinterpret_cast<float*>(smem_gen + (bias_addr - smem_base));
   volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(smem_gen + (tmem_slot_addr - smem_base));
@@ -213,7 +220,7 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
     fence_mbar_init();
     fence_proxy_async_smem();
   }
-  if (threadIdx.x == 0 && !p.stream_w) {
+  if (threadIdx.x == 0 && !stream_w) {
     // layer weights (constant data, not produced by the previous kernel): resident for the whole CTA
     const uint8_t* wsrc = reinterpret_cast<const uint8_t*>(p.wpk) + static_cast<size_t>(blockIdx.y) * p.part_w_bytes;
     mbar_arrive_expect_tx(bar_w, p.w_bytes + (FUSE_T ? p.w2_bytes : 0));
@@ -228,6 +235,7 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
     tmem_relinquish();
   }
   for (int i = threadIdx.x; i < p.npad; i += blockDim.x) bias_s[i] = p.bias[blockIdx.y * p.part_b_floats + i];
+  if (WR_T && threadIdx.x < 6) st_shared_v4(xchg_addr + 16u * threadIdx.x, 0u, 0u, 0u, 0u);
   if constexpr (FUSE_T) {
     float* bias2_s = reinterpret_cast<float*>(smem_gen + (b2_addr - smem_base));
     for (int i = threadIdx.x; i < 32; i += blockDim.x) bias2_s[i] = (p.b2 && i < p.n2) ? p.b2[i] : 0.f;
@@ -256,7 +264,7 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
         mbar_wait_spin(bar_a_empty(slot), phase ^ 1);
         if (kb == 0 && lane == 0) CSR_TRACE(0, pit, 1);
         if (elect_one()) {
-          if (p.stream_w) {
+          if (stream_w) {
             // streamed weights: this k-block's packed weights travel with the window (same barrier)
             const int ks_here = min(4, (p.cin >> 4) - kb * 4);
             const int wbytes = p.KH * ks_here * (KW * p.npad) * 32;
@@ -268,7 +276,8 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
           } else {
             mbar_arrive_expect_tx(bar_a_full(slot), p.win_bytes);
           }
-          tma_load_4d(slots_addr + slot * p.slot_bytes, &tmap, bar_a_full(slot), p.cin_off + kb * 64, tl.x0 - p.PW, tl.y0 - ph_eff, tl.n);
+          tma_load_4d(slots_addr + slot * p.slot_bytes, &tmap, bar_a_full(slot), p.cin_off + kb * 64, tl.x0 - (WR_T ? 0 : p.PW), tl.y0 - ph_eff,
+                      tl.n);
         }
         __syncwarp();
         if (++slot == S) { slot = 0; phase ^= 1; }
@@ -294,7 +303,7 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
     const uint32_t a_hi = ((8u * row_bytes) >> 4) | (1u << 14) | (a_layout << 29);   // SBO = 8 rows, version 1
     const uint32_t b_hi = (256u >> 4) | (1u << 14);                           // SBO 256 B, version 1, no swizzle
     const uint32_t a_lbo = (16u >> 4) << 16, b_lbo = (128u >> 4) << 16;
-    if (!p.stream_w) mbar_wait_spin(bar_w, 0);
+    if (!stream_w) mbar_wait_spin(bar_w, 0);
     tc_fence_after();
     // window-slot ring position of k-block 0 of this warp's first tile (the ring is shared by both issuers: tile `it`
     // owns ring entries it*n_kblocks .. it*n_kblocks + n_kblocks-1)
@@ -328,7 +337,7 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
         if (kb == 0 && lane == 0) CSR_TRACE(1, it, 2);
         const int ks_here = min(4, ksteps_total - kb * 4);
         uint32_t a16 = ((slots_addr + slot * p.slot_bytes) >> 4) | a_lbo;
-        uint32_t b16 = (p.stream_w ? ((slots_addr + slot * p.slot_bytes + p.win_slot_bytes) >> 4)
+        uint32_t b16 = (stream_w ? ((slots_addr + slot * p.slot_bytes + p.win_slot_bytes) >> 4)
                                    : ((w_addr >> 4) + static_cast<uint32_t>(kb) * kb_w16)) | b_lbo;
         if (elect_one()) {
           const bool last_kb = kb == p.n_kblocks - 1;
@@ -404,8 +413,20 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
     const int tx = m & (p.SW - 1);                       // window column
     const int n_chunks = ST_T == 3 ? 1 : p.npad >> 3;     // fp32 planar output: one channel, so one chunk (and of it only v[0] is live)
     const int PW = KW_T ? PW_T : p.PW;
-    const bool col_ok = (tx >= PW) && (tx < PW + p.TW);
-    const int srow = ty * p.TW + (tx - PW);              // staging row of this thread's pixel
+    const int x_off = WR_T ? 0 : PW;                     // window column of the tile's first output
+    const bool col_ok = WR_T || ((tx >= PW) && (tx < PW + p.TW));
+    const int srow = ty * p.TW + (tx - x_off);           // staging row of this thread's pixel
+    // WR_T: one staging buffer for both groups (ConvParams::whole_row), turns passed in tile order through barriers 13 / 14
+    const bool shared_stage = WR_T && p.n_stage < NG;
+    const int sg = shared_stage ? 0 : g;
+    // WR_T, 64-pixel rows: warps of TMEM lane quadrants 2k and 2k+1 (same group and chunks) hold the two halves of a row.  Their
+    // exchanges alternate between two slots by chunk parity (n_chunks is even, so also across tiles): the pair's next barrier
+    // orders the reads of one exchange before the slot's reuse
+    const bool row_pair = WR_T && p.SW == 64;
+    const bool row_left = (lane_grp & 1) == 0;
+    const int pair_bar = 5 + ((g * cstep + sub) << 1) + (lane_grp >> 1);   // 5..12
+    uint32_t xdst, xsrc;
+    edge_addrs(xchg_addr + 96u + static_cast<uint32_t>(pair_bar - 5) * 128u, xchg_addr, row_pair, row_left, lane, &xdst, &xsrc);
     const int act = ACT_T >= 0 ? ACT_T : p.act;
     const bool has_r1 = RES_T >= 0 ? (RES_T & 1) != 0 : p.r1 != nullptr;
     const bool has_r2 = RES_T >= 0 ? (RES_T & 2) != 0 : p.r2 != nullptr;
@@ -413,8 +434,8 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
     const bool tma_store = ST_T >= 0 ? (ST_T == 1 || ST_T == 4) : (p.store_mode == kStoreStaged);
     const bool need_pix = !tma_store || has_r1 || has_r2 || has_gate;    // warp-uniform
     const uint32_t swz = (p.stage_row_bytes == 128) ? static_cast<uint32_t>(srow & 7) : 0u;   // SWIZZLE_128B staging rows
-    const uint32_t srow_addr = stage_addr + static_cast<uint32_t>(g) * p.stage_bytes + static_cast<uint32_t>(srow * p.stage_row_bytes);
-    const uint32_t sbuf = stage_addr + static_cast<uint32_t>(g) * p.stage_bytes;
+    const uint32_t srow_addr = stage_addr + static_cast<uint32_t>(sg) * p.stage_bytes + static_cast<uint32_t>(srow * p.stage_row_bytes);
+    const uint32_t sbuf = stage_addr + static_cast<uint32_t>(sg) * p.stage_bytes;
     const uint32_t t_lane = tmem_base + (static_cast<uint32_t>(lane_grp * 32) << 16);
     const int d0 = -PW, d1 = 1 - PW, d2 = 2 - PW;
     // Staged stores: the group's output tile sits in shared memory as TH*TW rows of stage_row_bytes; it is copied out in
@@ -610,7 +631,7 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
       uint4 q1[4], q2[4];
       if (need_pix) {
         y = tl.y0 + ty;
-        x = tl.x0 - PW + tx;
+        x = tl.x0 - x_off + tx;
         valid = col_ok && (y < p.H) && (x < p.W);
         pix = (static_cast<size_t>(tl.n) * p.H + y) * p.W + x;
 #pragma unroll
@@ -625,7 +646,11 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
             q2[j] = (on && has_r2) ? ldg16(p.r2, pix, p.r2_C, p.r2_coff + ch0) : make_uint4(0, 0, 0, 0);
         }
       }
-      if (tma_store) named_bar_sync(1 + g, gthreads);   // every thread of the group has copied out the previous tile
+      if (shared_stage) {
+        if (it > 0) named_bar_sync(13 + g, 2 * gthreads);   // the other group has copied out tile it-1 (and so, before it, this one it-2)
+      } else if (tma_store) {
+        named_bar_sync(1 + g, gthreads);                  // every thread of the group has copied out the previous tile
+      }
       if (tracer) CSR_TRACE(2, it, 0);
       const uint32_t t_addr = t_lane + buf * nacc;
       mbar_wait(bar_acc_full(buf), acc_phase);             // the one bounded wait (see mbar_wait_spin)
@@ -662,6 +687,14 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
             tmem_ld8(t_addr + p.npad + ch0, r1);
             tmem_ld8(t_addr + 2 * p.npad + ch0, r2);
             tmem_ld_wait();
+            if constexpr (WR_T) {
+              const uint32_t xo = (j & 1) * 64u;
+              if (row_pair) {
+                row_edge_put(r0, r2, xdst + xo, lane, row_left);
+                named_bar_sync(pair_bar, 64);
+              }
+              row_edge_get(r0, r2, xsrc + xo, lane);
+            }
             gather_add8(v, r0, d0, lane);
             gather_add8(v, r1, d1, lane);
             gather_add8(v, r2, d2, lane);
@@ -738,6 +771,8 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
             }
           }
         }
+        if (shared_stage && blockIdx.x + (it + 1) * static_cast<int>(gridDim.x) < p.num_tiles)
+          named_bar_arrive(13 + (g ^ 1), 2 * gthreads);    // the staging buffer passes to the other group's tile it+1
       }
       if (tracer) CSR_TRACE(2, it, 2);
       buf += NG;
@@ -758,16 +793,16 @@ conv_tc_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmap) {
 size_t conv_smem_bytes(const ConvParams& p) {
   return 1024 /*alignment slack*/ + static_cast<size_t>(p.n_slots) * p.slot_bytes + static_cast<size_t>(p.n_stage) * p.stage_bytes +
          (((p.stream_w ? 0 : p.w_bytes) + 127) & ~127) + (p.fuse2 ? p.w2_bytes + 128 : 0) + 256 /*bias*/ +
-         8 * (18 + 2 * p.n_slots) + 32;
+         8 * (18 + 2 * p.n_slots) + 32 + (p.whole_row ? kXchgBytes : 0);
 }
 
-template <int KW_T, int PW_T, int ACT_T, int RES_T, int ST_T, int TALL_T = 0, int EARLY_T = 0, int FUSE_T = 0, int HYB_T = 0>
+template <int KW_T, int PW_T, int ACT_T, int RES_T, int ST_T, int TALL_T = 0, int EARLY_T = 0, int FUSE_T = 0, int HYB_T = 0, int WR_T = 0>
 static int launch_t(const ConvParams& p, const CUtensorMap& tmap, int num_sms, cudaStream_t stream) {
   const size_t smem = conv_smem_bytes(p);
   if (smem > static_cast<size_t>(kSmemLimit)) return static_cast<int>(cudaErrorInvalidValue);
   // the attribute is per device (and per template instantiation): one process may drive several GPUs
   static bool configured[64] = {};
-  auto kern = conv_tc_kernel<KW_T, PW_T, ACT_T, RES_T, ST_T, TALL_T, EARLY_T, FUSE_T, HYB_T>;
+  auto kern = conv_tc_kernel<KW_T, PW_T, ACT_T, RES_T, ST_T, TALL_T, EARLY_T, FUSE_T, HYB_T, WR_T>;
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return static_cast<int>(cudaErrorInvalidDevice);
   if (!configured[dev]) {
@@ -794,6 +829,13 @@ static int launch_t(const ConvParams& p, const CUtensorMap& tmap, int num_sms, c
 int launch_conv_tc(const ConvParams& p, const CUtensorMap& tmap, int num_sms, cudaStream_t stream) {
   const int res = (p.r1 ? 1 : 0) | (p.r2 ? 2 : 0) | (p.gate ? 4 : 0);
   if ((res & 6) == 6) return static_cast<int>(cudaErrorInvalidValue);   // r2 and gate share an operand slot
+  if (p.whole_row) {
+    // whole-row tiles: the trunk's one-residual convs only (RDB conv5, trunk_conv)
+    if (p.store_mode != kStoreStaged || p.KW != 3 || p.PW != 1 || p.act != 0 || res != 1 || p.tall_shift || p.early || p.fuse2 || p.hyb ||
+        p.n_groups != 2 || p.n_stage < 1 || p.SW != p.W || p.TW != p.W || (p.W != 32 && p.W != 64))
+      return static_cast<int>(cudaErrorInvalidValue);
+    return launch_t<3, 1, 0, 1, 1, 0, 0, 0, 0, 1>(p, tmap, num_sms, stream);
+  }
   // hi/lo bf16 pairs (the VGG19 convs of the perceptual loss): one specialisation, no runtime-switch fallback
   if (p.store_mode == kStoreBf16Split) {
     if (p.KW == 3 && p.PW == 1 && p.act == 2 && res == 0 && !p.tall_shift && !p.early && !p.fuse2 && !p.hyb)

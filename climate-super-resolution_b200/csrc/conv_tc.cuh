@@ -13,6 +13,10 @@ constexpr int kConvThreads = 32 * (1 + kMmaWarps) + kEpilogueThreads;   // warp0
 constexpr int kTileM = 128;           // window positions (UMMA M) per tile = TH * SW
 constexpr int kSmemLimit = 232448;    // 227 KB opt-in dynamic shared memory per CTA on sm_100
 constexpr int kMaxNpad = 64;          // output channels per launch part (epilogue: <= 2 chunks of 8 per warp)
+// Whole-row tiles: 96 zero bytes (the taps beyond an image edge, read at +0 and +64 like the two slots) and, for 64-pixel-wide maps,
+// where a row spans two epilogue warps, two 64-byte slots per warp pair (eight pairs, named barriers 5..12) to swap their boundary
+// taps; + alignment
+constexpr int kXchgBytes = 96 + 8 * 128 + 16;
 
 enum StoreMode {
   kStoreStaged = 0,     // bf16 NHWC through a swizzled shared-memory staging tile, copied out as whole pixel rows
@@ -34,6 +38,8 @@ struct ConvParams {
   int n_store;     // real output channels
   // tiling: a tile is TH rows x SW window columns of which TW = SW-(KW-1) are real outputs (columns [PW, PW+TW))
   int SW, sw_shift, TH, TW;
+  int whole_row;   // 1: SW == TW == W (3x3, W = 32 or 64): a window holds whole image rows from x = 0, no halo columns
+                   //    (conv_tc.cu WR_T); with n_stage < n_groups the two epilogue groups take one staging buffer in tile order
   int tiles_x, tiles_y, num_tiles, tiles_per_img;
   unsigned long long magic_img, magic_row;   // floor(2^40/d)+1 for d = tiles_per_img, tiles_x (num_tiles < 2^24)
   int win_rows;    // TH + KH - 1

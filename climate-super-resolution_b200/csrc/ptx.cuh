@@ -107,6 +107,9 @@ __device__ __forceinline__ void bulk_wait_group() { asm volatile("cp.async.bulk.
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
+__device__ __forceinline__ void named_bar_arrive(int id, int nthreads) {
+  asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+}
 // fire-and-forget vector fp32 add into global memory (sm_90+): one L2 atomic per 16 bytes
 __device__ __forceinline__ void red_add_v4_f32(float* ptr, float a, float b, float c, float d) {
   asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(ptr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
@@ -213,6 +216,42 @@ __device__ __forceinline__ float bf16hi(uint32_t v) { return __uint_as_float(v &
 __device__ __forceinline__ void split_bf16x2(float a, float b, uint32_t* hi, uint32_t* lo) {
   *hi = pack_bf16x2(a, b);
   *lo = pack_bf16x2(a - bf16lo(*hi), b - bf16hi(*hi));
+}
+
+// ---------------------------------------------------------------- whole-row tiles (conv_tc.cu / rdb_tc.cu, WR_T)
+// The epilogue sums the folded 3x3 taps as out[m] = D[m-1][tap 0] + D[m][tap 1] + D[m+1][tap 2] with warp shuffles that wrap
+// around the warp: lane 0 receives lane 31's tap-0 value, lane 31 lane 0's tap-2 value.  These two helpers put into those two
+// source registers what the edge pixels need instead - +0 at an image edge (exactly what a zero-filled halo column contributed),
+// or, where a 64-pixel row spans two warps (`left`: the TMEM lane quadrant with pixels 0..31 of the row), the other warp's
+// boundary value - so the summation order, and with it every output bit, is that of a tiling with halo columns.
+// 64 bytes per chunk and warp pair: the left warp's lane-31 tap 0, then the right warp's lane-0 tap 2.  row_edge_put: `dst` = this
+// thread's half of the slot.  row_edge_get (after the pair's named barrier): lane 31 reloads tap 0, lane 0 tap 2 from `src` = the
+// other warp's half of the slot, or 32 zero bytes (edge_addrs).
+__device__ __forceinline__ void edge_addrs(uint32_t slot, uint32_t zeros, bool pair, bool left, int lane, uint32_t* dst, uint32_t* src) {
+  *dst = left ? slot : slot + 32u;
+  *src = !pair ? zeros : lane == 31 ? (left ? zeros : slot) : (left ? slot + 32u : zeros);
+}
+// predicated forms (one SETP, no branch): the exchange sits in the epilogue's unrolled chunk loop, inside the instruction-cache budget
+__device__ __forceinline__ void st_shared_v8_if(bool pred, uint32_t addr, const uint32_t (&t)[8]) {
+  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %0, 0;\n\t"
+               "@p st.shared.v4.b32 [%1], {%2, %3, %4, %5};\n\t@p st.shared.v4.b32 [%1+16], {%6, %7, %8, %9};\n\t}"
+               ::"r"(static_cast<uint32_t>(pred)), "r"(addr), "r"(t[0]), "r"(t[1]), "r"(t[2]), "r"(t[3]), "r"(t[4]), "r"(t[5]), "r"(t[6]), "r"(t[7])
+               : "memory");
+}
+__device__ __forceinline__ void ld_shared_v8_if(bool pred, uint32_t addr, uint32_t (&t)[8]) {
+  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %8, 0;\n\t"
+               "@p ld.shared.v4.b32 {%0, %1, %2, %3}, [%9];\n\t@p ld.shared.v4.b32 {%4, %5, %6, %7}, [%9+16];\n\t}"
+               : "+r"(t[0]), "+r"(t[1]), "+r"(t[2]), "+r"(t[3]), "+r"(t[4]), "+r"(t[5]), "+r"(t[6]), "+r"(t[7])
+               : "r"(static_cast<uint32_t>(pred)), "r"(addr)
+               : "memory");
+}
+__device__ __forceinline__ void row_edge_put(const uint32_t (&t0)[8], const uint32_t (&t2)[8], uint32_t dst, int lane, bool left) {
+  st_shared_v8_if(left && lane == 31, dst, t0);
+  st_shared_v8_if(!left && lane == 0, dst, t2);
+}
+__device__ __forceinline__ void row_edge_get(uint32_t (&t0)[8], uint32_t (&t2)[8], uint32_t src, int lane) {
+  ld_shared_v8_if(lane == 31, src, t0);
+  ld_shared_v8_if(lane == 0, src, t2);
 }
 
 }  // namespace csr

@@ -15,6 +15,10 @@
 // conv_tc_kernel<3,1,1,0,1,0,1> (two M tiles per window, horizontal taps folded into N = 48, eight accumulators, four
 // epilogue groups), so the results are bit-identical to four per-layer launches.
 //
+// Whole-row windows (WR_T, DenseParams::whole_row): on a 32- or 64-pixel-wide map a window is 2*TH whole image rows starting at
+// x = 0 - no halo columns, every GEMM row an output - and depends on at most three windows of the previous layer (above, itself,
+// below).  The edge taps come from row_edge_put / row_edge_get (ptx.cuh), so the outputs stay bit-identical.
+//
 // Deadlock freedom: the grid never exceeds the SM count and every CTA takes a whole SM (shared memory), so all CTAs are
 // co-resident once the previous grid has drained; within a CTA layer k never waits for layer k+1.  Every wait on another
 // CTA is bounded and traps instead of hanging.
@@ -86,6 +90,7 @@ __device__ __forceinline__ void gather_add8(float (&acc)[8], const uint32_t (&ra
 
 }  // namespace
 
+template <int WR_T>
 __global__ void __launch_bounds__(kConvThreads, 1)
 dense_block_kernel(const DenseParams p, const __grid_constant__ CUtensorMap tmap) {
   extern __shared__ uint8_t smem_raw[];
@@ -104,6 +109,7 @@ dense_block_kernel(const DenseParams p, const __grid_constant__ CUtensorMap tmap
   auto bar_acc_full = [&](int b) { return bar_addr + 8u * (4 + 2 * S + b); };
   auto bar_acc_empty = [&](int b) { return bar_addr + 8u * (4 + 2 * S + kAcc + b); };
   const uint32_t tmem_slot_addr = bar_addr + 8u * (4 + 2 * S + 2 * kAcc);
+  const uint32_t xchg_addr = (tmem_slot_addr + 12u + 15u) & ~15u;            // WR_T: 96 zero bytes, then the row_edge_put / get slots
   uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
   float* bias_s = reinterpret_cast<float*>(smem_gen + (bias_addr - smem_base));
   volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(smem_gen + (tmem_slot_addr - smem_base));
@@ -146,6 +152,7 @@ dense_block_kernel(const DenseParams p, const __grid_constant__ CUtensorMap tmap
     tmem_relinquish();
   }
   for (int i = threadIdx.x; i < nl * kNpad; i += blockDim.x) bias_s[i] = p.L[i / kNpad].bias[i % kNpad];
+  if (WR_T && threadIdx.x < 6) st_shared_v4(xchg_addr + 16u * threadIdx.x, 0u, 0u, 0u, 0u);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -166,9 +173,10 @@ dense_block_kernel(const DenseParams p, const __grid_constant__ CUtensorMap tmap
       for (int t = blockIdx.x; t < p.num_tiles; t += G) {
         const Win w = decode_win(p, t);
         if (l > 0) {
-          // the windows of layer l-1 this window reads (1-pixel halo): itself and its <= 8 neighbours inside the image
-          if (lane < 9) {
-            const int dy = lane / 3 - 1, dx = lane - (lane / 3) * 3 - 1;
+          // the windows of layer l-1 this window reads (1-pixel halo): itself and its <= 8 neighbours inside the image (whole rows:
+          // the window above and below)
+          if (lane < (WR_T ? 3 : 9)) {
+            const int dy = WR_T ? lane - 1 : lane / 3 - 1, dx = WR_T ? 0 : lane - (lane / 3) * 3 - 1;
             const int yy = w.ty + dy, xx = w.tx + dx;
             if (yy >= 0 && yy < p.tiles_y && xx >= 0 && xx < p.tiles_x) {
               const int idx = w.n * p.tiles_per_img + yy * p.tiles_x + xx;
@@ -189,7 +197,7 @@ dense_block_kernel(const DenseParams p, const __grid_constant__ CUtensorMap tmap
           mbar_wait_spin(bar_a_empty(slot), phase ^ 1);
           if (elect_one()) {
             mbar_arrive_expect_tx(bar_a_full(slot), p.win_bytes);
-            tma_load_4d(slots_addr + slot * p.slot_bytes, &tmap, bar_a_full(slot), kb * 64, w.x0 - 1, w.y0 - 1, w.n);
+            tma_load_4d(slots_addr + slot * p.slot_bytes, &tmap, bar_a_full(slot), kb * 64, w.x0 - (WR_T ? 0 : 1), w.y0 - 1, w.n);
           }
           __syncwarp();
           if (++slot == S) { slot = 0; phase ^= 1; }
@@ -294,8 +302,15 @@ dense_block_kernel(const DenseParams p, const __grid_constant__ CUtensorMap tmap
     const int m_row = lane_grp * 32 + lane;
     const int ty = m_row >> p.sw_shift;
     const int tx = m_row & (p.SW - 1);
-    const bool col_ok = (tx >= 1) && (tx < 1 + p.TW);
-    const int srow = ty * p.TW + (tx - 1);
+    const int x_off = WR_T ? 0 : 1;                       // window column of the window's first output
+    const bool col_ok = WR_T || ((tx >= 1) && (tx < 1 + p.TW));
+    const int srow = ty * p.TW + (tx - x_off);
+    // WR_T, 64-pixel rows: the warps of TMEM lane quadrants 2k and 2k+1 of a group hold the two halves of a row
+    const bool row_pair = WR_T && p.SW == 64;
+    const bool row_left = (lane_grp & 1) == 0;
+    const int pair = (g << 1) + (lane_grp >> 1);          // 0..7
+    uint32_t xdst, xsrc;                                  // 64 bytes per chunk
+    edge_addrs(xchg_addr + 96u + static_cast<uint32_t>(pair) * 128u, xchg_addr, row_pair, row_left, lane, &xdst, &xsrc);
     const uint32_t sbuf = stage_addr + static_cast<uint32_t>(g) * p.stage_bytes;
     const uint32_t srow_addr = sbuf + static_cast<uint32_t>(srow * 32);
     const uint32_t t_lane = tmem_base + (static_cast<uint32_t>(lane_grp * 32) << 16);
@@ -327,7 +342,7 @@ dense_block_kernel(const DenseParams p, const __grid_constant__ CUtensorMap tmap
       // accumulator - fetch it before waiting for the MMAs
       uint4 gq[2] = {make_uint4(0x3f803f80u, 0x3f803f80u, 0x3f803f80u, 0x3f803f80u), make_uint4(0x3f803f80u, 0x3f803f80u, 0x3f803f80u, 0x3f803f80u)};
       if (p.gate) {
-        const int y = y0 + ty, x = w.x0 - 1 + tx;
+        const int y = y0 + ty, x = w.x0 - x_off + tx;
         if (col_ok && y < p.H && x < p.W) {
           const uint4* gsrc = reinterpret_cast<const uint4*>(reinterpret_cast<const __nv_bfloat16*>(p.gate) +
                                                              ((static_cast<size_t>(w.n) * p.H + y) * p.W + x) * p.gate_C + p.L[l].gate_coff);
@@ -346,6 +361,16 @@ dense_block_kernel(const DenseParams p, const __grid_constant__ CUtensorMap tmap
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(bar_acc_empty(buf));       // the accumulator lives in registers now
+      if constexpr (WR_T) {
+        // one exchange per M tile (both chunks); the group's barriers below order the partner's reads before the next tile's writes
+        if (row_pair) {
+          row_edge_put(raw[0][0], raw[0][2], xdst, lane, row_left);
+          row_edge_put(raw[1][0], raw[1][2], xdst + 64u, lane, row_left);
+          named_bar_sync(5 + pair, 64);
+        }
+        row_edge_get(raw[0][0], raw[0][2], xsrc, lane);
+        row_edge_get(raw[1][0], raw[1][2], xsrc + 64u, lane);
+      }
 #pragma unroll
       for (int jj = 0; jj < 2; ++jj) {
         float v[8];
@@ -411,20 +436,22 @@ dense_block_kernel(const DenseParams p, const __grid_constant__ CUtensorMap tmap
 
 size_t dense_smem_bytes(const DenseParams& p) {
   return 1024 + static_cast<size_t>(p.n_slots) * p.slot_bytes + static_cast<size_t>(kGroups) * p.stage_bytes + 2u * p.wbuf_bytes +
-         kDenseMaxLayers * kNpad * 4 + 8 * (4 + 2 * p.n_slots + 2 * kAcc) + 32;
+         kDenseMaxLayers * kNpad * 4 + 8 * (4 + 2 * p.n_slots + 2 * kAcc) + 32 + (p.whole_row ? kXchgBytes : 0);
 }
 
 int launch_dense_block(const DenseParams& p, const CUtensorMap& tmap, int num_sms, cudaStream_t stream) {
   const size_t smem = dense_smem_bytes(p);
   if (smem > static_cast<size_t>(kSmemLimit) || p.n_layers < 1 || p.n_layers > kDenseMaxLayers || p.n_slots < 2)
     return static_cast<int>(cudaErrorInvalidValue);
-  static bool configured[64] = {};
+  if (p.whole_row && (p.SW != p.W || p.TW != p.W || (p.W != 32 && p.W != 64) || p.tiles_x != 1)) return static_cast<int>(cudaErrorInvalidValue);
+  static bool configured[2][64] = {};
+  auto kern = p.whole_row ? dense_block_kernel<1> : dense_block_kernel<0>;
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return static_cast<int>(cudaErrorInvalidDevice);
-  if (!configured[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(dense_block_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit);
+  if (!configured[p.whole_row][dev]) {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit);
     if (e != cudaSuccess) return static_cast<int>(e);
-    configured[dev] = true;
+    configured[p.whole_row][dev] = true;
   }
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(p.num_tiles < num_sms ? p.num_tiles : num_sms);
@@ -436,7 +463,7 @@ int launch_dense_block(const DenseParams& p, const CUtensorMap& tmap, int num_sm
   attr[0].val.programmaticStreamSerializationAllowed = p.use_pdl ? 1 : 0;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  return static_cast<int>(cudaLaunchKernelEx(&cfg, dense_block_kernel, p, tmap));
+  return static_cast<int>(cudaLaunchKernelEx(&cfg, kern, p, tmap));
 }
 
 }  // namespace csr

@@ -22,6 +22,7 @@ struct DenseLayerParams {
 struct DenseParams {
   int N, H, W;
   int SW, sw_shift, TH, TW;                       // window pitch, rows per M tile, output columns per tile (SW - 2)
+  int whole_row;                                  // 1: SW == TW == W (32 or 64), windows of whole image rows (rdb_tc.cu WR_T)
   int tiles_x, tiles_y, num_tiles, tiles_per_img; // in WINDOWS of two vertically adjacent M tiles (2*TH output rows)
   unsigned long long magic_img, magic_row;        // floor(2^40/d)+1 for d = tiles_per_img, tiles_x
   int win_bytes;     // (2*TH + 2) * SW * 128
