@@ -872,7 +872,7 @@ struct CsrPlan {
   int train = 0;
   std::vector<csr::Op> fwd, bwd;        // forward (op 0: the input conversion) and, in training plans, backward launch lists
   std::vector<size_t> dbg_cat;          // csr_plan_buffer: byte offsets of the concat buffers / HR-tail activations inside the workspace
-  size_t dbg_tail[5] = {0, 0, 0, 0, 0};  // m1, hrA, hrB, hrD, hrE
+  size_t dbg_tail[9] = {};              // csr_plan_buffer kinds 1..9: m1, hrA, hrB, hrD, hrE, fea0, t0, hrC, tlast
   int ccat = 0;
   unsigned int* flags = nullptr;        // completion counters of the dense-block launches
   size_t flags_bytes = 0;
@@ -1625,6 +1625,7 @@ static int plan_create_impl(const CsrNetDesc* net, int32_t n, int32_t h, int32_t
   P->flags = reinterpret_cast<unsigned int*>(base + L.flags); P->flags_bytes = L.flags_bytes;
   P->dbg_cat = L.cat; P->ccat = L.ccat;
   P->dbg_tail[0] = L.m1; P->dbg_tail[1] = L.hrA; P->dbg_tail[2] = L.hrB; P->dbg_tail[3] = L.hrD; P->dbg_tail[4] = L.hrE;
+  P->dbg_tail[5] = L.fea0; P->dbg_tail[6] = L.t0; P->dbg_tail[7] = L.hrC; P->dbg_tail[8] = L.tlast;
   const WsPtrs ws = ws_carve(L, workspace);
   rc = plan_build(P, ws, layers);
   if (!rc && train) {
@@ -1880,9 +1881,13 @@ int csr_plan_backward_flat(CsrPlan* P, const void* packed_bwd, const float* grad
 }
 
 int csr_plan_buffer(const CsrPlan* P, int32_t kind, int32_t index, size_t* offset_bytes, int32_t* dims4) {
-  // test hook: where an activation buffer of the plan lives inside the caller's workspace (bf16 NHWC; dims4 = n, h, w, channel pitch).
-  // kind 0: concat buffer `index` (training plans keep one per dense block: [x | x1 | x2 | x3 | x4]), 1: upconv1 output, 2: upconv2 output,
-  // 3: HRconv output, 4: srcnn.conv1 output, 5: srcnn.conv2 output
+  // test hook: where an activation buffer of the plan lives inside the caller's workspace (dims4 = n, h, w, channel pitch; bf16 NHWC
+  // except kind 9).  kind 0: concat buffer `index` ([x | x1 | x2 | x3 | x4]), 1: upconv1 output, 2: upconv2 output, 3: HRconv output,
+  // 4: srcnn.conv1 output, 5: srcnn.conv2 output, 6: fea0 (conv_first output), 7: t0 (trunk_conv + fea0), 8: hrC (SRCNN input
+  // im2col, channel dx*3 + c), 9: tlast (conv_last output, fp32 planar).  Training plans keep all of them, one concat buffer per
+  // dense block.  Inference plans rotate three concat buffers (RDB3 writes the RRDB output over buffer 0's x), share kinds 2 / 4 and
+  // 3 / 5 (fused tail, option 33 = 3: kind 2 keeps upconv2's output; kind 3 holds conv_last's tap planes, then srcnn.conv2's output)
+  // and leave kind 9 unwritten while option 36 is on.  The header spells this out.
   if (!P || !offset_bytes || !dims4) return fail(CSR_ERR_BAD_ARG, "null pointer");
   const int h = P->h, w = P->w;
   if (kind == 0) {
@@ -1891,10 +1896,11 @@ int csr_plan_buffer(const CsrPlan* P, int32_t kind, int32_t index, size_t* offse
     dims4[0] = P->N; dims4[1] = h; dims4[2] = w; dims4[3] = P->ccat;
     return CSR_OK;
   }
-  if (kind < 1 || kind > 5) return fail(CSR_ERR_BAD_ARG, "unknown buffer kind %d", kind);
+  if (kind < 1 || kind > 9) return fail(CSR_ERR_BAD_ARG, "unknown buffer kind %d", kind);
   *offset_bytes = P->dbg_tail[kind - 1];
-  const int s = kind == 1 ? 2 : 4;
-  dims4[0] = P->N; dims4[1] = s * h; dims4[2] = s * w; dims4[3] = (kind == 5) ? P->srcnn_pitch : 64;
+  const int s = (kind == 6 || kind == 7) ? 1 : kind == 1 ? 2 : 4;
+  dims4[0] = P->N; dims4[1] = s * h; dims4[2] = s * w;
+  dims4[3] = (kind == 5 || kind == 8) ? P->srcnn_pitch : kind == 9 ? 1 : 64;
   return CSR_OK;
 }
 

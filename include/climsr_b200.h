@@ -155,10 +155,27 @@ size_t  csr_packed_weight_bytes_bwd(const CsrNetDesc* net);
 int     csr_pack_weights_bwd(const CsrNetDesc* net, const float* const* w, void* packed, size_t packed_bytes, void* stream);
 int     csr_plan_backward(CsrPlan* plan, const void* packed_bwd, const float* grad_out,
                           float* const* dw, float* const* db, void* stream);
-/* test hook: byte offset (inside the workspace given to csr_*plan_create) and dims {n, h, w, channel pitch} of a bf16 NHWC activation
- * buffer of the plan.  kind 0: concat buffer `index` ([x | x1..x4]; one per dense block in training plans), 1: upconv1 output,
- * 2: upconv2 output, 3: HRconv output, 4: srcnn.conv1 output, 5: srcnn.conv2 output.  The parity tests read the activation SIGNS of a
- * training forward from these to run the fp32 oracle with the same LeakyReLU / ReLU masks. */
+/* test hook: byte offset (inside the workspace given to csr_*plan_create) and dims {n, h, w, channel pitch} of an activation buffer of
+ * the plan; bf16 NHWC except kind 9.  The parity tests read a forward's operands and results from these.  After a forward:
+ *   kind 0  concat buffer `index`, [x | x1 | x2 | x3 | x4] of a dense block                        (n, h, w, concat pitch)
+ *   kind 1  upconv1 output                                                                         (n, 2h, 2w, 64)
+ *   kind 2  upconv2 output                                                                         (n, 4h, 4w, 64)
+ *   kind 3  HRconv output                                                                          (n, 4h, 4w, 64)
+ *   kind 4  srcnn.conv1 output                                                                     (n, 4h, 4w, 64)
+ *   kind 5  srcnn.conv2 output, 32 channels                                                        (n, 4h, 4w, SRCNN pitch)
+ *   kind 6  conv_first output, the trunk skip (fea0)                                               (n, h, w, 64)
+ *   kind 7  trunk_conv output + fea0                                                               (n, h, w, 64)
+ *   kind 8  SRCNN input im2col: channel dx*3 + c = bf16 of (conv_last output, elev, mask)[c] at x + dx - 4, zero outside the
+ *           image; channels 27..31 zero, 32.. not written                                          (n, 4h, 4w, SRCNN pitch)
+ *   kind 9  conv_last output, fp32 planar                                                          (n, 4h, 4w, 1)
+ * The SRCNN pitch is 64 in training plans, 32 in inference plans.  Training plans keep all of these, one concat buffer per dense
+ * block (3 nb + 1; buffer 3 nb is the trunk output).  Inference plans reuse memory:
+ *   - three concat buffers rotate (index = dense block mod 3), and RRDB i's RDB3 writes the RRDB output over buffer 0's x, so
+ *     buffer 0's x is the last RRDB's output and kind 6 is the only surviving copy of conv_first's output;
+ *   - kinds 2 and 4 share memory, and so do kinds 3 and 5.  With the default fused tail (option 33 = 3) HRconv's output is never
+ *     written: its epilogue writes conv_last's nine fp32 tap planes into kind 3's memory, srcnn.conv1's output is never written
+ *     (srcnn.conv2 runs in its epilogue), so kind 2 / 4 still holds upconv2's output and kind 3 / 5 ends as srcnn.conv2's output;
+ *   - kind 9 is not written while option 36 is on: the tap sum and the im2col then run as one kernel straight into kind 8. */
 int     csr_plan_buffer(const CsrPlan* plan, int32_t kind, int32_t index, size_t* offset_bytes, int32_t dims4[4]);
 int     csr_plan_num_backward_ops(const CsrPlan* plan);
 /* Same backward, all gradients in ONE flat fp32 buffer (OVERWRITTEN, not accumulated): layer i's dW at float offset

@@ -109,6 +109,27 @@ def test_conv_epilogue_variants():
     buf = _nhwc(r2, 64)
     ops.conv2d_nhwc(_nhwc(x, 64), wt.cuda(), b.cuda(), out=buf, res1=_nhwc(r1, 64), scale1=0.2, res2=buf, scale2=0.2)
     assert float((buf.float().cpu().permute(0, 3, 1, 2) - want).abs().max()) <= 2.0 ** -7
+    # one-residual 3x3 conv over 128 channels on 32- and 64-pixel-wide maps (RDB conv5 shape): whole-row tiles (option 37), also
+    # in place (out aliases res1); bit-identical to the tiling with halo columns
+    from climsr_b200._lib import lib
+    for wd in (32, 64):
+        x5 = torch.rand((n, 128, 13, wd), generator=g) * 2 - 1
+        w5 = (torch.rand((64, 128, 3, 3), generator=g) * 2 - 1) / 34
+        r5 = torch.rand((n, 64, 13, wd), generator=g) * 2 - 1
+        want = _ref_conv(x5, w5, b, "none") * 0.2 + _bf(r5)
+        outs = []
+        try:
+            for whole_row in (1, 0):
+                lib.csr_set_option(37, whole_row)
+                outs.append(ops.conv2d_nhwc(_nhwc(x5, 128), w5.cuda(), b.cuda(), res1=_nhwc(r5, 64), scale1=0.2))
+                buf = _nhwc(r5, 64)
+                ops.conv2d_nhwc(_nhwc(x5, 128), w5.cuda(), b.cuda(), out=buf, res1=buf, scale1=0.2)
+                outs.append(buf)
+        finally:
+            lib.csr_set_option(37, 1)
+        assert float((outs[0].float().cpu().permute(0, 3, 1, 2) - want).abs().max()) <= 2.0 ** -7, wd
+        for o in outs[1:]:
+            assert torch.equal(o, outs[0]), wd
     # nearest x2 then conv + lrelu (esrgan.py:94,97): executed as four 2x2 sub-pixel convs with summed weights
     out = ops.conv2d_nhwc(_nhwc(x, 64), wt.cuda(), b.cuda(), act="lrelu", in_up2=True)
     up = F.interpolate(_bf(x), scale_factor=2, mode="nearest")
