@@ -8,6 +8,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libclimsr_b200.so")
 
 CSR_OK = 0
+CSR_ERR_BAD_ARG = -1            # CsrStatus in include/climsr_b200.h
 NUM_METRICS = 18
 METRIC_KEYS = ("acc@0.1", "acc@0.25", "acc@0.5", "acc@0.75", "acc@1", "acc@01.25", "acc@1.5", "acc@2", "psnr", "ssim", "mae",
                "mse", "rmse", "mape", "smape", "r2", "l1_loss", "mse_loss")   # key names of core/task.py:318-334 (typo kept)

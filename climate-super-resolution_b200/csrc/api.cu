@@ -873,6 +873,7 @@ struct CsrPlan {
   std::vector<csr::Op> fwd, bwd;        // forward (op 0: the input conversion) and, in training plans, backward launch lists
   std::vector<size_t> dbg_cat;          // csr_plan_buffer: byte offsets of the concat buffers / HR-tail activations inside the workspace
   size_t dbg_tail[9] = {};              // csr_plan_buffer kinds 1..9: m1, hrA, hrB, hrD, hrE, fea0, t0, hrC, tlast
+  struct { size_t gO, gcolB, gT, gP, gQ, gm1, gt0, gcat[3]; } dbg_grad = {};   // kinds 10..17 (training plans)
   int ccat = 0;
   unsigned int* flags = nullptr;        // completion counters of the dense-block launches
   size_t flags_bytes = 0;
@@ -1626,6 +1627,7 @@ static int plan_create_impl(const CsrNetDesc* net, int32_t n, int32_t h, int32_t
   P->dbg_cat = L.cat; P->ccat = L.ccat;
   P->dbg_tail[0] = L.m1; P->dbg_tail[1] = L.hrA; P->dbg_tail[2] = L.hrB; P->dbg_tail[3] = L.hrD; P->dbg_tail[4] = L.hrE;
   P->dbg_tail[5] = L.fea0; P->dbg_tail[6] = L.t0; P->dbg_tail[7] = L.hrC; P->dbg_tail[8] = L.tlast;
+  P->dbg_grad = {L.gO, L.gcolB, L.gT, L.gP, L.gQ, L.gm1, L.gt0, {L.gcat[0], L.gcat[1], L.gcat[2]}};
   const WsPtrs ws = ws_carve(L, workspace);
   rc = plan_build(P, ws, layers);
   if (!rc && train) {
@@ -1831,7 +1833,9 @@ int csr_plan_backward_segments(CsrPlan* P, int32_t nseg) {
     if (k == nseg) oi = P->bwd.size();
     else
       while (oi < P->bwd.size() && done_at[oi] > target) ++oi;
-    if (oi <= prev_op && k < nseg) continue;
+    // no op left for this slice: skip it (with nseg near grad_floats the suffix is complete before k == nseg, and a last
+    // segment would run nothing)
+    if (oi <= prev_op) continue;
     P->seg_op.push_back(prev_op);
     P->seg_lo.push_back(done_at[oi]);
     P->seg_hi.push_back(prev_lo);
@@ -1887,13 +1891,27 @@ int csr_plan_buffer(const CsrPlan* P, int32_t kind, int32_t index, size_t* offse
   // im2col, channel dx*3 + c), 9: tlast (conv_last output, fp32 planar).  Training plans keep all of them, one concat buffer per
   // dense block.  Inference plans rotate three concat buffers (RDB3 writes the RRDB output over buffer 0's x), share kinds 2 / 4 and
   // 3 / 5 (fused tail, option 33 = 3: kind 2 keeps upconv2's output; kind 3 holds conv_last's tap planes, then srcnn.conv2's output)
-  // and leave kind 9 unwritten while option 36 is on.  The header spells this out.
+  // and leave kind 9 unwritten while option 36 is on.  Kinds 10..17 (training plans only) are the backward's gradient buffers:
+  // 10: gO (25-tap im2col of dL/dout), 11: gcolB (9-tap im2col of dL/d(conv_last output)), 12: gT (dL/d[conv_last output, elev,
+  // mask]), 13 / 14: gP / gQ (HR-tail ping-pong), 15: gm1, 16: gt0, 17: gradient concat buffer `index` (0..2).  The header spells
+  // this out.
   if (!P || !offset_bytes || !dims4) return fail(CSR_ERR_BAD_ARG, "null pointer");
   const int h = P->h, w = P->w;
   if (kind == 0) {
     if (index < 0 || (size_t)index >= P->dbg_cat.size()) return fail(CSR_ERR_BAD_ARG, "concat buffer index %d out of range", index);
     *offset_bytes = P->dbg_cat[index];
     dims4[0] = P->N; dims4[1] = h; dims4[2] = w; dims4[3] = P->ccat;
+    return CSR_OK;
+  }
+  if (kind >= 10 && kind <= 17) {
+    if (!P->train) return fail(CSR_ERR_BAD_ARG, "buffer kind %d exists in training plans only", kind);
+    if (kind == 17 && (index < 0 || index > 2)) return fail(CSR_ERR_BAD_ARG, "gradient concat buffer index %d out of range", index);
+    const size_t off[8] = {P->dbg_grad.gO, P->dbg_grad.gcolB, P->dbg_grad.gT, P->dbg_grad.gP, P->dbg_grad.gQ, P->dbg_grad.gm1,
+                           P->dbg_grad.gt0, kind == 17 ? P->dbg_grad.gcat[index] : 0};
+    const int pitch[8] = {32, 16, 16, 64, 64, 64, 64, P->ccat};
+    const int s = kind <= 14 ? 4 : kind == 15 ? 2 : 1;
+    *offset_bytes = off[kind - 10];
+    dims4[0] = P->N; dims4[1] = s * h; dims4[2] = s * w; dims4[3] = pitch[kind - 10];
     return CSR_OK;
   }
   if (kind < 1 || kind > 9) return fail(CSR_ERR_BAD_ARG, "unknown buffer kind %d", kind);

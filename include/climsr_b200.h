@@ -175,7 +175,16 @@ int     csr_plan_backward(CsrPlan* plan, const void* packed_bwd, const float* gr
  *   - kinds 2 and 4 share memory, and so do kinds 3 and 5.  With the default fused tail (option 33 = 3) HRconv's output is never
  *     written: its epilogue writes conv_last's nine fp32 tap planes into kind 3's memory, srcnn.conv1's output is never written
  *     (srcnn.conv2 runs in its epilogue), so kind 2 / 4 still holds upconv2's output and kind 3 / 5 ends as srcnn.conv2's output;
- *   - kind 9 is not written while option 36 is on: the tap sum and the im2col then run as one kernel straight into kind 8. */
+ *   - kind 9 is not written while option 36 is on: the tap sum and the im2col then run as one kernel straight into kind 8.
+ * Training plans also expose the backward's gradient buffers (CSR_ERR_BAD_ARG on an inference plan).  Each is complete once the
+ * backward has run past the layer that writes it, and later layers overwrite the ping-pong ones:
+ *   kind 10  gO: im2col of bf16(dL/dout), channel dy*5 + dx = dL/dout at (y - dy + 2, x - dx + 2)  (n, 4h, 4w, 32)
+ *   kind 11  gcolB: the same 3x3 im2col of kind 12's channel 0                                     (n, 4h, 4w, 16)
+ *   kind 12  gT: dL/d[conv_last output, elev, mask] (channels 0..2)                                 (n, 4h, 4w, 16)
+ *   kind 13  gP, kind 14 gQ: HR-tail gradient ping-pong                                             (n, 4h, 4w, 64)
+ *   kind 15  gm1: dL/d(upconv1 output)                                                              (n, 2h, 2w, 64)
+ *   kind 16  gt0: dL/d(trunk_conv output + fea0)                                                    (n, h, w, 64)
+ *   kind 17  gradient concat buffer `index` (0..2), [g_y | g4 | g3 | g2 | g1] of a dense block      (n, h, w, concat pitch) */
 int     csr_plan_buffer(const CsrPlan* plan, int32_t kind, int32_t index, size_t* offset_bytes, int32_t dims4[4]);
 int     csr_plan_num_backward_ops(const CsrPlan* plan);
 /* Same backward, all gradients in ONE flat fp32 buffer (OVERWRITTEN, not accumulated): layer i's dW at float offset

@@ -34,7 +34,7 @@ pytestmark = pytest.mark.gpu
 
 REL = 2.0 ** -12
 K_INNER = 1.0 / 4
-OPTION_DEFAULTS = {27: 1, 31: 2, 33: 3, 36: 1, 37: 1}
+OPTION_DEFAULTS = {25: 1, 27: 1, 31: 2, 33: 3, 36: 1, 37: 1}
 
 
 @contextmanager
